@@ -2,13 +2,14 @@
 """bench.py — the BASELINE.json workloads on B200 through the C-ABI (SURVEY.md 8d).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  Default = the headline, config 2.
 
   c2  uniform-random batched incr building ~1.5 B nnz over 13 M rows per GPU, then 500 M point gets
       at 50 % hits.  A step = one batch of 2^26 incr ops per GPU; the timed steps are the LAST K
       batches of the 2 B-op stream (K = 30: the whole build from empty; smaller K: the first batches
-      are applied untimed, so the timed region still ends at ~1.5 B nnz).
+      are applied untimed, so the timed region still ends at ~1.5 B nnz; larger K: the stream goes on).
   c3  co-occurrence build (examples/cf_recommender.c:35-47): Zipf(1.1) baskets of 8 over 4 M items,
       all-pairs incr + column-0 totals, 2^24 baskets = 1.07 B ops in 16 steps of 2^26; then gets.
   c4  read path: 13 M rows with Zipf(1.7) row lengths 1 .. 10^6 (~1.4 B nnz) are built, then every
@@ -62,7 +63,10 @@ WORKLOADS = {
 def parse():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=None, help="timed steps (default: the whole workload)")
+    p.add_argument("--steps", type=int, default=None,
+                   help="timed steps (default: the whole workload); past the workload's own length the stream goes on and "
+                        "the arena grows with it, and all K batches (8 B per op) are resident at once, so device memory "
+                        "bounds K (c2 at full scale: 0.5 GiB of batches + 1.7 GiB of arena per step)")
     p.add_argument("--warmup", type=int, default=3)
     p.add_argument("--impl", default="ours", choices=["ours", "reference"])
     p.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
@@ -79,7 +83,13 @@ def parse():
     p.add_argument("--cpu-secs", type=float, default=12.0, help="target seconds of CPU work for cpu_baseline")
     p.add_argument("--ref-step", type=int, default=None, help="ops (c4: rows) per step of the reference arm")
     p.add_argument("--parity-ops", type=int, default=3_000_000, help="ops of the parity prefix (whole job)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the timed path computed in its last step as DIR/<name>.npy "
+                        "(float64, fixed seeded samples, at most 64 MB) so that two builds can be compared output for output")
+    a = p.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs records the GPU path: use it with --impl ours")
+    return a
 
 
 # ------------------------------------------------------------------------------ clocks
@@ -148,6 +158,29 @@ def thread_candidates():
 
 def scaled(a, v):
     return max(1, int(v * a.scale))
+
+
+DUMP_SAMPLE = 1 << 21        # entries per dumped array over the whole job (N ranks: 1/N each): 16 MB in float64
+
+
+def dump_index(n: int, k: int = DUMP_SAMPLE) -> np.ndarray:
+    """Sorted positions of a fixed, seeded sample of k out of n outputs (all n when n <= k)."""
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    return np.unique(np.random.default_rng(20240611).integers(0, n, k))
+
+
+def write_dump(job, arrays: dict):
+    """--dump-outputs: every array as DIR/<name>.npy in float64 (u32 values and i64 offsets are exact there);
+    at N > 1 every rank writes its own share as <name>.rank<r>.npy."""
+    os.makedirs(job.a.dump_outputs, exist_ok=True)
+    sfx = f".rank{job.rank}" if job.world > 1 else ""
+    for name, arr in arrays.items():
+        if not isinstance(arr, np.ndarray):
+            arr = arr.cpu().numpy()
+        if arr.dtype == np.int32:
+            arr = arr.view(np.uint32)
+        np.save(os.path.join(job.a.dump_outputs, f"{name}{sfx}.npy"), arr.astype(np.float64))
 
 
 # ====================================================================================================
@@ -391,7 +424,11 @@ class WriteWorkload:
         if a.arena_gib is not None:
             self.arena = a.arena_gib
         self.n_batches = max(1, -(-total // (self.B * W)))       # batches per rank
-        self.K = min(a.steps or self.n_batches, self.n_batches)
+        if a.steps and a.steps > self.n_batches:                 # more steps than the workload has: the stream goes on
+            if a.arena_gib is None:                              # and the arena grows with the ops it has to hold
+                self.arena = -(-self.arena * a.steps // self.n_batches)
+            self.n_batches = a.steps
+        self.K = a.steps or self.n_batches
         self.prefill = self.n_batches - self.K
         self.gets = scaled(a, cfg["gets"])
         self.n_build = self.n_batches * self.B * W
@@ -520,6 +557,10 @@ def run_write_workload(job: Job, name: str):
     m.set_kernel_timing(False)
     clocks = job.sampler.window(wall0, wall1)
     value = K * B * world / (ms_build * 1e-3) / 1e6
+    dump = {}
+    if a.dump_outputs:      # incr_batch hands nothing back: its result is the cells it wrote, read back before close
+        pick = torch.from_numpy(dump_index(B, DUMP_SAMPLE // world)).to(job.dev)
+        dump_keys = xs[K - 1][pick].contiguous(), ys[K - 1][pick].contiguous()
     del xs, ys
     nnz_local, rows_local = m.stat("nnz"), m.stat("rows")
     vsum_local = m.stat("value_sum")     # every op added 1: the table-wide sum must equal the op count
@@ -584,6 +625,8 @@ def run_write_workload(job: Job, name: str):
             get_sweep[f"{bs}:{mode}"] = round(tot * world / (ms_v * 1e-3) / 1e6, 1)
         get_same = get_same and bool((out[:tot] == ref_out[:tot]).all().item())
     m.set_get_slices(int(os.environ.get("SMATRIX_GET_SLICES", "1"), 0))
+    if a.dump_outputs:
+        dump["get_values"] = ref_out[torch.from_numpy(dump_index(G, DUMP_SAMPLE // world)).to(job.dev)]
     del ref_out
     hits = int((out != 0).sum().item())
     first_q = rank * G
@@ -613,6 +656,10 @@ def run_write_workload(job: Job, name: str):
                  "getrow_value_sum": int(pairs[1::2].to(torch.int64).sum().item())}
         del pairs, offs, ids, sample
 
+    if a.dump_outputs:
+        dump["incr_values"] = m.get_batch(*dump_keys, job.ibuf(dump_keys[0].numel()))
+        write_dump(job, dump)
+        del dump, dump_keys
     m.close()
     torch.cuda.empty_cache()      # the timed batches are back with the driver before the next tables reserve their arenas
 
@@ -955,6 +1002,8 @@ def run_c4(job: Job):
     launches = m.stat("launches") - launches0
     m.set_kernel_timing(False)
     clocks = job.sampler.window(wall0, wall1)
+    if a.dump_outputs:
+        dump_c4_last_step(job, rl_out[cut[K - 1]:cut[K]], offsets[:cut[K] - cut[K - 1] + 1], pairs)
     rowlen_ok = bool((rl_out.to(torch.int64) == my_lens).all().item())   # no column 0 here: rowlen = distinct columns
     last_val_sum = int(pairs[1:2 * step_pairs[-1]:2].to(torch.int64).sum().item())
     pairs_total, rows_asked = job.sum_over_ranks(got_pairs, n_mine)
@@ -1042,6 +1091,22 @@ def run_c4(job: Job):
         "table": stats, "clocks": clocks, "gpu_launches": launches, "step_ms": step_ms,
         "roofline": roofline, "e2e": e2e, "cpu_baseline": cpu,
     }
+
+
+def dump_c4_last_step(job: Job, rowlen, offsets, pairs):
+    """The last step's answers: rowlens, and the getrow pairs of a seeded sample of its rows (at most
+    DUMP_SAMPLE pairs over the job), each row sorted by column because a row's pairs come back in table order."""
+    torch, k = job.torch, DUMP_SAMPLE // job.world
+    offs = offsets.cpu().numpy()
+    rows = dump_index(len(offs) - 1, (1 << 16) // job.world)
+    lens = offs[rows + 1] - offs[rows]
+    keep = np.cumsum(lens) <= k
+    rows, lens = rows[keep], lens[keep]
+    at = np.repeat(offs[rows] - np.cumsum(lens) + lens, lens) + np.arange(int(lens.sum()))
+    got = pairs.view(-1, 2)[torch.from_numpy(at).to(job.dev)].cpu().numpy().view(np.uint32)
+    row_of = np.repeat(np.arange(len(rows)), lens)
+    write_dump(job, {"rowlen": rowlen[torch.from_numpy(dump_index(rowlen.numel(), k)).to(job.dev)],
+                     "getrow_lengths": lens, "getrow_pairs": got[np.lexsort((got[:, 0], row_of))]})
 
 
 def run_parity_c4(job: Job, m, cfg, lens, offs, R):

@@ -103,6 +103,87 @@ def test_round2_bench_lines(name, metric, n):
         assert d["get_mops"] > 1.5 * g["input_order"]["get_mops"]
 
 
+def _bench_dump(tmp_path, *args):
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--warmup", "1", "--no-e2e", "--no-cpu",
+                        "--no-probes", "--no-parity", "--dump-outputs", str(out), *args],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout.strip().splitlines()[-1])
+    assert sum(f.stat().st_size for f in out.iterdir()) <= 64 << 20
+    import numpy as np
+    got = {f.name[:-4]: np.load(f) for f in out.iterdir()}
+    assert all(a.dtype == np.float64 for a in got.values())
+    return d, got
+
+
+def _counts(keys, q):
+    """How often every query key occurs in the build stream = its cell value (every op adds 1)."""
+    import numpy as np
+    uk, cnt = np.unique(keys, return_counts=True)
+    pos = np.minimum(np.searchsorted(uk, q), len(uk) - 1)
+    return np.where(uk[pos] == q, cnt[pos], 0)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("wl", ["c2", "c3"])
+def test_dump_outputs_of_the_write_workloads_are_the_streams_answers(tmp_path, wl):
+    """--dump-outputs on a small write workload with --steps past the workload's own length (c2: 20 batches,
+    c3: 11): the step count is honoured, and the dumped cells of the last batch and the sampled get answers equal
+    the counts of their keys in the whole build stream, generated again on the host by the CPU checker."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from libsmatrix_b200.workloads import zipf_thresholds
+    from oracle import cpu
+    B, K = 1 << 20, {"c2": 24, "c3": 12}[wl]
+    d, got = _bench_dump(tmp_path, "--workload", wl, "--steps", str(K), "--scale", "0.01", "--batch", str(B))
+    assert set(got) == {"incr_values", "get_values"}
+    assert d["steps"] == K and d["checks"]["ops_applied"] == K * B and d["checks"]["value_sum_ok"]
+    cfg, rows, G = bench.WORKLOADS[wl], d["config"]["rows"], d["config"]["gets"]
+    if wl == "c2":
+        xs, ys = cpu.gen_c2_ops(cfg["seed"], 0, K * B, rows, cfg["ycols"])
+        qx, qy = cpu.gen_c2_queries(cfg["seed_get"], cfg["seed"], 0, G, K * B, rows, cfg["ycols"])
+    else:
+        thr = zipf_thresholds(rows, cfg["zipf_s"])
+        xs, ys = cpu.gen_c3_ops(cfg["seed"], 0, K * B, thr)
+        qx, qy = cpu.gen_c3_queries(cfg["seed_get"], cfg["seed"], 0, G, K * B, thr)
+    keys = xs.astype(np.uint64) << np.uint64(32) | ys
+    last = keys[(K - 1) * B:][bench.dump_index(B)]
+    assert (got["incr_values"] == _counts(keys, last)).all() and (got["incr_values"] >= 1).all()
+    idx = bench.dump_index(G)
+    q = (qx.astype(np.uint64) << np.uint64(32) | qy)[idx]
+    assert (got["get_values"] == _counts(keys, q)).all()
+    assert (got["get_values"][idx % 2 == 1] == 0).all() and (got["get_values"][idx % 2 == 0] >= 1).all()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_read_workload_are_the_last_steps_rows(tmp_path):
+    """--dump-outputs on a small c4 run: the last step's rowlens are the generated row lengths, and the sampled
+    rows' getrow pairs, column-sorted, are the (column, value) ops the host generator wrote into them."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from libsmatrix_b200.workloads import zipf_thresholds
+    from oracle import cpu
+    K = 4
+    d, got = _bench_dump(tmp_path, "--workload", "c4", "--steps", str(K), "--scale", "0.02")
+    assert set(got) == {"rowlen", "getrow_lengths", "getrow_pairs"} and d["steps"] == K
+    cfg, R = bench.WORKLOADS["c4"], d["config"]["rows"]
+    thr = zipf_thresholds(d["config"]["kmax"], cfg["zipf_s"])
+    lens = cpu.gen_c4_lens(cfg["seed"], 0, R, thr).astype(np.uint64)
+    offs = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
+    lo, hi = (K - 1) * R // K, R
+    assert (got["rowlen"] == lens[lo:hi][bench.dump_index(hi - lo)]).all()
+    rows = lo + bench.dump_index(hi - lo, 1 << 16)[:len(got["getrow_lengths"])]
+    assert len(rows) > 0 and (got["getrow_lengths"] == lens[rows]).all()
+    _, ys, vs = cpu.gen_c4_ops(cfg["seed"], int(offs[lo]), int(offs[hi] - offs[lo]), offs)
+    at = np.concatenate([np.arange(offs[r], offs[r + 1]) for r in rows]).astype(np.int64) - int(offs[lo])
+    row_of = np.repeat(np.arange(len(rows)), lens[rows].astype(np.int64))
+    order = np.lexsort((ys[at], row_of))
+    assert (got["getrow_pairs"] == np.stack([ys[at][order], vs[at][order]], 1)).all()
+
+
 def test_full_scale_parity_record():
     d = json.load(open(os.path.join(ROOT, "profiles", "r2_fullscale_parity.json")))
     assert d["ok"] and d["row_digest_mismatches"] == 0 and d["get_mismatches"] == 0

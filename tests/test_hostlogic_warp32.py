@@ -77,8 +77,14 @@ def test_chunks_without_column0(make, monkeypatch):
 
 def test_snapshot_export_kernels(sim32, tmp_path, monkeypatch):
     """K9: the row blocks of the .smx file are laid out by k_snap_* (one warp per row, linear probing in the reference's
-    y % size layout) — both directions against the reference's own file mode, and a round trip with big rows."""
+    y % size layout) — both directions against the reference's own file mode."""
     import snapshot_suite as ss
     monkeypatch.setenv("SMATRIX_DIR_LOG2", "6")
     ss.scenario_snapshot_interchange(lambda f: SparseMatrix(f, _lib_path=sim32), tmp_path)
+
+
+def test_snapshot_export_kernels_roundtrip(sim32, tmp_path, monkeypatch):
+    """K9: the same kernels, ours -> ours with big rows (no reference build needed)."""
+    import snapshot_suite as ss
+    monkeypatch.setenv("SMATRIX_DIR_LOG2", "6")
     ss.scenario_snapshot_roundtrip_big(lambda f: SparseMatrix(f, _lib_path=sim32), tmp_path, n_rows=1500)
