@@ -61,6 +61,7 @@ struct smatrix_s {
   int dir_in_arena; /* the directory was carved from the slab arena: never cudaFree'd on its own */
   uint64_t dir_cap;
   uint32_t dir_log_min;
+  uint64_t shrink_refused; /* largest directory size a shrink was refused at (a row would sit too far from home) */
   smx_ctl_t* d_ctl;
   smx_ctl_t* h_ctl; /* pinned */
 
@@ -457,7 +458,7 @@ static double ln_unit(double r) {
   return 2.0 * sum - (double)k * 0.69314718055994530942;
 }
 #define SMX_SKETCH_BITS_LOG 25u
-static void resize_dir(smatrix_t* s, uint64_t new_cap);
+static int resize_dir(smatrix_t* s, uint64_t new_cap, int shrink);
 static uint64_t pow2_at_least(uint64_t v);
 static void presize_dir(smatrix_t* s, const smx_ops_t* ops) {
   const uint64_t n = ops->n, used = s->h_ctl->dir_used;
@@ -479,7 +480,7 @@ static void presize_dir(smatrix_t* s, const smx_ops_t* ops) {
   if (est > (double)n) est = (double)n;
   const uint64_t cap = pow2_at_least((uint64_t)(4.0 * ((double)used + 1.1 * est)) + 64);
   if (s->debug) fprintf(stderr, "[smatrix] presize: %llu ops, %.0f zero bits, ~%.0f distinct rows\n", (unsigned long long)n, zeros, est);
-  if (cap > s->dir_cap) resize_dir(s, cap);
+  if (cap > s->dir_cap) resize_dir(s, cap, 0);
 }
 
 static uint64_t pow2_at_least(uint64_t v) {
@@ -488,7 +489,11 @@ static uint64_t pow2_at_least(uint64_t v) {
   return p;
 }
 
-static void resize_dir(smatrix_t* s, uint64_t new_cap) {
+/* Re-place every row into a directory of new_cap entries.  A shrink is abandoned (the current directory stays,
+ * returns 0) when it would put a row SMX_DIR_CREATE_STEPS or more probe steps from its home: dir_find refuses to
+ * create a row that far out, so the next new row on such a chain (rows whose mix_row share their low bits) would
+ * grow the directory all the way back, and the shrink after the chunk would undo that again, batch after batch. */
+static int resize_dir(smatrix_t* s, uint64_t new_cap, int shrink) {
   double t0 = now_ns();
   if (s->debug)
     fprintf(stderr, "[smatrix] directory %llu -> %llu entries (rows %llu, refused ops %u of which directory-full %u)\n",
@@ -502,10 +507,26 @@ static void resize_dir(smatrix_t* s, uint64_t new_cap) {
                            : (smx_row_t*)dmalloc(s, (size_t)new_cap * sizeof(smx_row_t));
   CK(cudaMemsetAsync(nd, 0, (size_t)new_cap * sizeof(smx_row_t), s->stream));
   CK(cudaMemsetAsync(s->d_ctl->slice_used, 0, sizeof(uint32_t) * SMX_DIR_SLICES, s->stream));
+  CK(cudaMemsetAsync(&s->d_ctl->dir_probe_max, 0, 4, s->stream));
   smx_view_t to = view_for(s, nd, new_cap);
   smx_launch_dir_rehash(s->stream, from, to);
   s->n_launches++;
+  if (shrink) copy_d2h(s, &s->h_small[39], &s->d_ctl->dir_probe_max, 4, s->stream); /* read in the same wait */
   CK(cudaStreamSynchronize(s->stream));
+  if (shrink && s->h_small[39] >= SMX_DIR_CREATE_STEPS) {
+    if (s->debug)
+      fprintf(stderr, "[smatrix] shrink to %llu entries refused: a row would sit %u probe steps from its home\n",
+              (unsigned long long)new_cap, s->h_small[39]);
+    if (in_arena) slab_give_back(s, (char*)nd, (size_t)new_cap * sizeof(smx_row_t));
+    else CK(cudaFree(nd));
+    /* the rehash counted the rows per slice of the new directory: put back the counts of the current one
+     * (as of the last read_ctl, which followed the chunk's last update launch) */
+    copy_h2d(s, s->d_ctl->slice_used, s->h_ctl->slice_used, sizeof(uint32_t) * SMX_DIR_SLICES, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    s->shrink_refused = new_cap;
+    s->phase_ns[PH_DIR] += now_ns() - t0;
+    return 0;
+  }
   if (!s->dir_in_arena) CK(cudaFree(s->dir));
   else slab_give_back(s, (char*)s->dir, (size_t)s->dir_cap * sizeof(smx_row_t)); /* the old directory's arena space */
   s->dir = nd;
@@ -513,6 +534,7 @@ static void resize_dir(smatrix_t* s, uint64_t new_cap) {
   s->dir_cap = new_cap;
   s->n_dir_grows++;
   s->phase_ns[PH_DIR] += now_ns() - t0;
+  return 1;
 }
 
 /* ------------------------------------------------------------------------------ write path */
@@ -557,7 +579,7 @@ static void run_pass(smatrix_t* s, smx_ops_t ops, int op, int pass, const uint32
       uint64_t cap = pow2_at_least(need);
       if (cap < s->dir_cap * 2) cap = s->dir_cap * 2;
       if (cap > s->dir_cap * 64) cap = s->dir_cap * 64;
-      resize_dir(s, cap);
+      resize_dir(s, cap, 0);
     } else if (!c.n_grow && c.n_defer >= prev_defer) {
       smx_die("update pass made no progress (%u ops deferred)", c.n_defer);
     }
@@ -575,7 +597,8 @@ static void maybe_shrink_dir(smatrix_t* s) {
   uint64_t fit = pow2_at_least(4 * (used ? used : 1));
   const uint64_t floor_cap = 1ull << s->dir_log_min;
   if (fit < floor_cap) fit = floor_cap;
-  if (fit * 4 <= s->dir_cap) resize_dir(s, fit);
+  /* rows are never removed, so a size at which a shrink was refused stays out of reach: not tried again */
+  if (fit * 4 <= s->dir_cap && fit > s->shrink_refused) resize_dir(s, fit, 1);
 }
 
 /* directory slices of a batch: 2^parts_log of them, slice(x) = (mix_row(x) & (dir_cap - 1)) >> shift */

@@ -60,6 +60,7 @@ typedef struct {
 
 /* ---- device control block (counters the host reads back after every round) -------------- */
 #define SMX_DIR_SLICES 256u      /* occupancy is tracked (and limited) per directory slice     */
+#define SMX_DIR_CREATE_STEPS 256u /* dir_find creates a row at most this many probe steps - 1 from its home */
 typedef struct {
   /* persistent */
   unsigned long long dir_used;   /* rows in the directory (sum of slice_used, set by the host's readers) */
@@ -74,7 +75,7 @@ typedef struct {
   uint32_t n_mid;                /*           rows whose OLD bucket is 2^SMX_MID_LOG .. 2^(SMX_BIG_LOG-1) */
   uint32_t n_recycled;           /* planned buckets taken from the free lists                */
   uint32_t n_spill;              /* cells k_migrate_tiles could not place inside their tile (spill list length) */
-  uint32_t pad_round;
+  uint32_t dir_probe_max;        /* largest probe step at which k_dir_rehash placed a row (zeroed before it runs) */
   unsigned long long plan_bytes; /* bytes of FRESH slab planned by grow_plan                 */
   unsigned long long need_zero;  /* planned buckets that are filled in place (global CAS) and so
                                     need a zeroed region; shared-memory-built buckets do not  */

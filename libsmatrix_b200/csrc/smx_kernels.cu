@@ -215,7 +215,7 @@ __device__ __forceinline__ int dir_find(const smx_view_t& V, uint32_t x, bool cr
     if (!create) return DIR_MISS;
     const uint32_t sl = (uint32_t)(pos >> V.slice_shift);
     uint32_t* slice = &V.ctl->slice_used[sl];
-    if (step >= 256 || __ldcg(slice) >= V.slice_limit) return DIR_FULL;
+    if (step >= SMX_DIR_CREATE_STEPS || __ldcg(slice) >= V.slice_limit) return DIR_FULL;
     const ull fresh = (ull)x | ((ull)(SMX_META_USED | SMX_INLINE_LOG) << 32);
     ull old = atomicCAS((ull*)e, 0ull, fresh);
     if (old == 0ull) {
@@ -785,7 +785,8 @@ k_zero_old_big(smx_view_t V, smx_lists_t S, uint32_t big_first) {
  * ---------------------------------------------------------------------------------------- */
 __global__ void __launch_bounds__(SMX_BLOCK) k_dir_rehash(smx_view_t from, smx_view_t to) {
   const ull mask = to.dir_cap - 1;
-  ull moved = 0;
+  uint32_t far = 0; /* largest probe step of this thread's rows: the host refuses a shrink that puts a row beyond
+                       dir_find's create limit */
   for (ull pos = blockIdx.x * blockDim.x + threadIdx.x; pos < from.dir_cap;
        pos += (ull)gridDim.x * blockDim.x) {
     const smx_row_t* o = from.dir + pos;
@@ -801,12 +802,12 @@ __global__ void __launch_bounds__(SMX_BLOCK) k_dir_rehash(smx_view_t from, smx_v
         dst[1] = a[1]; dst[2] = a[2]; dst[3] = a[3];
         dst[4] = b[0]; dst[5] = b[1]; dst[6] = b[2]; dst[7] = b[3];
         atomicAdd(&to.ctl->slice_used[q >> to.slice_shift], 1u);
+        if (step > far) far = step < 0xFFFFFFFFull ? (uint32_t)step : 0xFFFFFFFFu;
         break;
       }
     }
-    ++moved;
   }
-  (void)moved;
+  if (far) atomicMax(&to.ctl->dir_probe_max, far);
 }
 
 /* between the EARLY and LATE passes: column 0 of these rows turns non-zero HERE in input order, so
