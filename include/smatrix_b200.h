@@ -19,7 +19,9 @@ extern "C" {
  * SMATRIX_RECYCLE (free lists of vacated buckets on/off), SMATRIX_PRESIZE (distinct-row estimate
  * that sizes the directory before a chunk of new rows, on/off), SMATRIX_GET_SLICES / SMATRIX_GET_SLICE_MIN
  * (see smatrix_b200_set_get_slices), SMATRIX_WIDE_SLICES (default 1: a write chunk without ops on column 0
- * is ordered over 256 directory slices instead of 128 + their column-0 twins). */
+ * is ordered over 256 directory slices instead of 128 + their column-0 twins), SMATRIX_TOPK_PAIRS (default
+ * 2^28: smatrix_cf_topk_batch scores and ranks the items of a call in pieces whose rows hold at most that
+ * many pairs, 32 bytes of device scratch per pair; a row longer than that is a piece of its own). */
 smatrix_t* smatrix_b200_open(const char* fname, int device);
 /* the same with the slab arena given explicitly (bytes; 0 = segments on demand) instead of through
  * $SMATRIX_ARENA_GIB — for hosts that open several handles with different needs from several threads */
@@ -66,7 +68,9 @@ enum {
   SMX_STAT_SLICED_GETS = 24,/* point reads answered in directory-slice order so far (see set_get_slices)  */
   SMX_STAT_WIDE_CHUNKS = 25,/* write chunks without ops on column 0 that were ordered over 256 slices ($SMATRIX_WIDE_SLICES) */
   SMX_STAT_NS_ALLOC = 26,   /* host time inside cudaMalloc on behalf of this handle so far, ns */
-  SMX_STAT_ALLOCS = 27      /* number of those cudaMalloc calls */
+  SMX_STAT_ALLOCS = 27,     /* number of those cudaMalloc calls */
+  SMX_STAT_TOPK_BIG = 28,   /* top-k segments (items) longer than 4096 pairs: ranked by the multi-block radix select */
+  SMX_STAT_TOPK_PASSES = 29 /* digit passes that select ran so far */
 };
 uint64_t smatrix_b200_stat(smatrix_t* self, int which);
 
@@ -182,6 +186,13 @@ void smatrix_b200_pair_cols(smatrix_t* self, const uint32_t* d_pairs, uint64_t t
 void smatrix_b200_cf_scores_totals(smatrix_t* self, size_t n, const uint64_t* d_offsets, const uint32_t* d_pairs,
                                    const uint32_t* d_a_tot, const uint32_t* d_b_tot, uint32_t* d_ids,
                                    double* d_scores);
+/* The selection of smatrix_cf_topk_batch over any CSR of (id, double) pairs on the device: segment i is
+ * d_ids / d_scores[d_offsets[i] .. d_offsets[i+1]); its first min(k, len) pairs by score descending, then id
+ * ascending, go to d_counts[i] and row i of d_out_ids / d_out_scores[n*k] (slots past the count: id
+ * 0xFFFFFFFF, score -1.0).  Ids must be unique inside a segment.  1 <= k <= 1024.  All arrays DEVICE. */
+void smatrix_b200_topk_segments(smatrix_t* self, size_t n, const uint64_t* d_offsets, const uint32_t* d_ids,
+                                const double* d_scores, uint32_t k, uint32_t* d_counts, uint32_t* d_out_ids,
+                                double* d_out_scores);
 int  smatrix_b200_is_device_ptr(smatrix_t* self, const void* p);   /* device (or managed) memory? */
 /* peers in the SAME process (one thread per GPU) need no IPC: enable direct access to `peer_device` */
 int  smatrix_b200_enable_peer(smatrix_t* self, int peer_device);

@@ -70,6 +70,17 @@ uint64_t smatrix_getrow_batch(smatrix_t* self, const uint32_t* xs, size_t n, uin
 uint64_t smatrix_cf_neighbors_batch(smatrix_t* self, const uint32_t* items, size_t n,
                                     uint64_t* offsets, uint32_t* ids, double* scores, uint64_t cap);
 
+/* The recommendation itself: for every item, the first min(k, len) entries of exactly the list
+ * smatrix_cf_neighbors_batch returns for it (column-0 pair included), ordered by score descending, then
+ * id ascending, so the answer is unique and bit-exact.  The ranking runs on the device; the neighbour
+ * lists never leave it.  Fixed-width, row-major outputs: counts[n] = min(k, len); ids[n*k] and
+ * scores[n*k], where the slots past counts[i] hold id 0xFFFFFFFF and score -1.0.  An absent item or an
+ * empty row has count 0.  1 <= k <= 1024.  `items` may be host or device; the three outputs are all host
+ * or all device (host outputs: n * (12k + 4) bytes come down).  Items are processed in pieces whose rows
+ * hold at most $SMATRIX_TOPK_PAIRS pairs (see smatrix_b200.h). */
+void smatrix_cf_topk_batch(smatrix_t* self, const uint32_t* items, size_t n, uint32_t k,
+                           uint32_t* counts, uint32_t* ids, double* scores);
+
 #ifdef __cplusplus
 }
 #endif

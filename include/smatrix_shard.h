@@ -92,6 +92,13 @@ uint64_t smatrix_b200_shard_getrow_batch(smatrix_shard_t* self, const uint32_t* 
 uint64_t smatrix_b200_shard_cf_neighbors_batch(smatrix_shard_t* self, const uint32_t* items, size_t n,
                                                uint64_t* offsets, uint32_t* ids, double* scores, uint64_t cap);
 
+/* The top k neighbours of this rank's items across ranks: same contract as smatrix_cf_topk_batch (counts[n],
+ * ids / scores[n*k], 1 <= k <= 1024).  The scores come as in smatrix_b200_shard_cf_neighbors_batch and are
+ * ranked by smatrix_b200_topk_segments on this rank's GPU.  One piece per call: this rank's row buffer and
+ * scratch hold all the pairs of its items at once, as cf_neighbors_batch needs for a full fill. */
+void smatrix_b200_shard_cf_topk_batch(smatrix_shard_t* self, const uint32_t* items, size_t n, uint32_t k,
+                                      uint32_t* counts, uint32_t* ids, double* scores);
+
 /* Host wall-clock accounting of this rank since the last reset (not collective): time spent routing
  * (count, count exchange, scatter over NVLink, arrival barrier), time spent applying the inbox,
  * number of routes, bytes this rank stored into OTHER ranks' inboxes. */

@@ -40,6 +40,8 @@ PROTOTYPES = {
                                           C.c_uint64]),
     "smatrix_cf_neighbors_batch": (C.c_uint64, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                                C.c_void_p, C.c_uint64]),
+    "smatrix_cf_topk_batch": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p, C.c_void_p,
+                                     C.c_void_p]),
     # include/smatrix_b200.h
     "smatrix_b200_open": (C.c_void_p, [C.c_char_p, C.c_int]),
     "smatrix_b200_open_arena": (C.c_void_p, [C.c_char_p, C.c_int, C.c_size_t]),
@@ -89,6 +91,8 @@ PROTOTYPES = {
     "smatrix_b200_pair_cols": (None, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "smatrix_b200_cf_scores_totals": (None, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p]),
+    "smatrix_b200_topk_segments": (None, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
+                                          C.c_void_p, C.c_void_p, C.c_void_p]),
     "smatrix_b200_enable_peer": (C.c_int, [C.c_void_p, C.c_int]),
     "smatrix_b200_is_device_ptr": (C.c_int, [C.c_void_p, C.c_void_p]),
     "smatrix_b200_memcpy_async": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int]),
@@ -122,6 +126,8 @@ PROTOTYPES.update({
     "smatrix_b200_shard_rowlen_batch": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "smatrix_b200_shard_cf_neighbors_batch": (C.c_uint64, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                                           C.c_void_p, C.c_uint64]),
+    "smatrix_b200_shard_cf_topk_batch": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p,
+                                                C.c_void_p, C.c_void_p]),
     "smatrix_b200_shard_getrow_batch": (C.c_uint64, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                                     C.c_uint64]),
     "smatrix_b200_shard_stat": (C.c_uint64, [C.c_void_p, C.c_int]),
@@ -135,7 +141,8 @@ STAT = {"rows": 0, "nnz": 1, "dir_cap": 2, "slab_bytes": 3, "device_bytes": 4, "
         "rounds": 6, "row_grows": 7, "dir_grows": 8, "kernel_ns": 9, "ns_partition": 10, "ns_upsert": 11,
         "ns_grow_plan": 12, "ns_slab": 13, "ns_migrate": 14, "ns_dir": 15, "value_sum": 16,
         "live_bucket_bytes": 17, "free_bytes": 18, "recycled": 19, "h2d_bytes": 20, "d2h_bytes": 21, "bucket_bytes": 22, "spilled": 23,
-        "sliced_gets": 24, "wide_chunks": 25, "ns_alloc": 26, "allocs": 27}
+        "sliced_gets": 24, "wide_chunks": 25, "ns_alloc": 26, "allocs": 27,
+        "topk_big": 28, "topk_passes": 29}
 
 _cache: dict[str, C.CDLL] = {}
 

@@ -114,6 +114,19 @@ struct smatrix_s {
   uint32_t* d_cursors;
   size_t d_big_bytes;
   uint32_t n_big_rows;
+  /* top-k (smatrix_cf_topk_batch, smatrix_b200_topk_segments): scratch that grows with slack, so that calls of
+   * similar size make no cudaMalloc */
+  uint32_t topk_pairs;  /* SMATRIX_TOPK_PAIRS: pairs per piece of a cf_topk_batch call */
+  uint32_t* tk_ctl;     /* 16 control words + the list of big segments */
+  uint64_t* tk_off;     /* row offsets of the whole call (piece cuts) */
+  void* tk_big;         /* select state + histograms of the big segments */
+  uint32_t* tk_cids;    /* compaction regions of the big segments */
+  double* tk_cscores;
+  uint32_t* tk_ids;     /* scores of a piece */
+  double* tk_scores;
+  void* tk_out;         /* a piece's answers on their way to host outputs */
+  size_t tk_bytes[8];
+  uint64_t n_topk_big, n_topk_passes;
 
   unsigned long long* free_ptr[SMX_CLASSES]; /* device stacks of vacated buckets, per size class */
   uint32_t free_cap[SMX_CLASSES];
@@ -1244,6 +1257,134 @@ uint64_t smatrix_cf_neighbors_batch(smatrix_t* s, const uint32_t* items, size_t 
   return total;
 }
 
+/* ------------------------------------------------------------------------------ top-k */
+/* top-k scratch buffer `b` (an index into tk_bytes) of at least `need` bytes; grows with slack */
+static void* tk_buf(smatrix_t* s, void** p, int b, size_t need) {
+  if (need > s->tk_bytes[b]) {
+    if (*p) { CK(cudaStreamSynchronize(s->stream)); cudaFree(*p); }
+    s->tk_bytes[b] = need + need / 4 + 4096;
+    *p = dmalloc(s, s->tk_bytes[b]);
+  }
+  return *p;
+}
+
+/* the selection of smatrix_b200_topk_segments on device arrays, enqueued on s->stream (synchronises to read
+ * the number of big segments and, per digit pass, how many are still selecting) */
+static void topk_run(smatrix_t* s, uint32_t n, const uint64_t* d_off, const uint32_t* d_ids, const double* d_scores,
+                     uint32_t k, uint32_t* d_counts, uint32_t* d_oids, double* d_oscores) {
+  if (!n) return;
+  uint32_t* ctl = (uint32_t*)tk_buf(s, (void**)&s->tk_ctl, 0, (size_t)n * 4 + 64);
+  uint32_t* big_list = ctl + 16;
+  CK(cudaMemsetAsync(ctl, 0, 64, s->stream));
+  smx_launch_topk_classify(s->stream, n, d_off, big_list, ctl);
+  copy_d2h(s, &s->h_small[40], ctl, 16, s->stream);
+  smx_launch_topk_small(s->stream, n, d_off, d_ids, d_scores, k, d_counts, d_oids, d_oscores);
+  s->n_launches += 3;
+  CK(cudaStreamSynchronize(s->stream));
+  const uint32_t n_big = s->h_small[40];
+  if (!n_big) return;
+  uint64_t big_pairs;
+  memcpy(&big_pairs, &s->h_small[42], 8);
+  void* big = tk_buf(s, &s->tk_big, 2, smx_topk_big_bytes(n_big));
+  tk_buf(s, (void**)&s->tk_cids, 3, (size_t)big_pairs * 4);
+  tk_buf(s, (void**)&s->tk_cscores, 4, (size_t)big_pairs * 8);
+  CK(cudaMemsetAsync(big, 0, smx_topk_big_bytes(n_big), s->stream));
+  smx_launch_topk_init(s->stream, big_list, n_big, d_off, big, ctl);
+  s->n_launches++;
+  for (uint32_t pass = 1;; pass++) { /* every pass fixes one more digit of the k-th key */
+    if (pass > smx_topk_max_passes()) smx_die("topk: the select did not end after %u digit passes", pass - 1);
+    CK(cudaMemsetAsync(ctl + 1, 0, 4, s->stream));
+    smx_launch_topk_pass(s->stream, big, n_big, k, d_ids, d_scores, s->tk_cids, s->tk_cscores, ctl);
+    copy_d2h(s, &s->h_small[44], ctl + 1, 4, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    s->n_launches += 3;
+    s->n_topk_passes++;
+    if (!s->h_small[44]) break;
+  }
+  smx_launch_topk_finish(s->stream, big, n_big, s->tk_cids, s->tk_cscores, k, d_counts, d_oids, d_oscores);
+  s->n_launches++;
+  s->n_topk_big += n_big;
+}
+
+void smatrix_b200_topk_segments(smatrix_t* s, size_t n, const uint64_t* d_offsets, const uint32_t* d_ids,
+                                const double* d_scores, uint32_t k, uint32_t* d_counts, uint32_t* d_out_ids,
+                                double* d_out_scores) {
+  if (k < 1 || k > SMX_TOPK_MAX_K) smx_die("topk_segments: k = %u is outside 1..%u", k, SMX_TOPK_MAX_K);
+  if (n >= 0xFFFFFFFFull) smx_die("topk_segments: too many segments in one call");
+  if (!n) return;
+  enter(s);
+  topk_run(s, (uint32_t)n, d_offsets, d_ids, d_scores, k, d_counts, d_out_ids, d_out_scores);
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+}
+
+/* the top k neighbours of every item, ranked on the device: scores as smatrix_cf_neighbors_batch computes them,
+ * for pieces of items whose pairs fit SMATRIX_TOPK_PAIRS, each piece selected by topk_run */
+void smatrix_cf_topk_batch(smatrix_t* s, const uint32_t* items, size_t n, uint32_t k, uint32_t* counts, uint32_t* ids,
+                           double* scores) {
+  if (k < 1 || k > SMX_TOPK_MAX_K) smx_die("cf_topk_batch: k = %u is outside 1..%u", k, SMX_TOPK_MAX_K);
+  if (n >= 0xFFFFFFFFull) smx_die("cf_topk_batch: too many items in one call");
+  if (!n) return;
+  enter(s);
+  const int out_dev = is_device_ptr(counts);
+  if (is_device_ptr(ids) != out_dev || is_device_ptr(scores) != out_dev)
+    smx_die("batch arrays must be all host or all device pointers");
+  const uint32_t nn = (uint32_t)n;
+  const uint32_t tiles = smx_scan_scratch_items(nn);
+  ensure_tmp(s, (size_t)nn * 8, ((size_t)nn + 1 + tiles) * 8);
+  const uint32_t* d_items = items;
+  if (!is_device_ptr(items)) {
+    copy_h2d(s, s->d_tmp, items, (size_t)nn * 4, s->stream);
+    d_items = s->d_tmp;
+  }
+  uint32_t* d_cnt = s->d_tmp + nn;
+  /* the row lengths of the whole call decide where the pieces end */
+  uint64_t* d_all = (uint64_t*)tk_buf(s, (void**)&s->tk_off, 1, ((size_t)nn + 1) * 8);
+  smx_launch_row_counts(s->stream, view_of(s), d_items, nn, d_cnt, NULL, NULL, NULL);
+  smx_launch_scan(s->stream, d_cnt, nn, 0, d_all, s->d_tmp64 + (size_t)nn + 1);
+  s->n_launches += 4;
+  for (uint32_t lo = 0, hi; lo < nn; lo = hi) {
+    smx_launch_topk_cut(s->stream, d_all, nn, lo, s->topk_pairs, s->d_small);
+    copy_d2h(s, &s->h_small[45], s->d_small, 4, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    hi = s->h_small[45];
+    const uint32_t np = hi - lo;
+    const uint64_t total = plan_rows(s, d_items + lo, np, d_cnt); /* the piece's offsets: d_tmp64[0..np] */
+    tk_buf(s, (void**)&s->tk_ids, 5, (size_t)total * 4);
+    tk_buf(s, (void**)&s->tk_scores, 6, (size_t)total * 8);
+    if (total) {
+      if (total * 8 > s->d_rowbuf_bytes) {
+        if (s->d_rowbuf) cudaFree(s->d_rowbuf);
+        s->d_rowbuf_bytes = (size_t)total * 8 + (size_t)total * 2 + 4096;
+        s->d_rowbuf = (uint32_t*)dmalloc(s, s->d_rowbuf_bytes);
+      }
+      smx_launch_getrow_fill(s->stream, view_of(s), s->d_info, np, s->d_tmp64, 0, s->d_rowbuf, s->d_big, s->n_big_rows,
+                             s->d_cursors);
+      smx_launch_cf_scores(s->stream, view_of(s), d_items + lo, np, s->d_tmp64, s->d_rowbuf, s->tk_ids, s->tk_scores);
+      s->n_launches += 2;
+    }
+    uint32_t* oc = counts + lo;
+    uint32_t* oi = ids + (size_t)lo * k;
+    double* os = scores + (size_t)lo * k;
+    if (!out_dev) {
+      char* o = (char*)tk_buf(s, &s->tk_out, 7, (size_t)np * (12ull * k + 4));
+      os = (double*)o;
+      oi = (uint32_t*)(o + (size_t)np * k * 8);
+      oc = oi + (size_t)np * k;
+    }
+    topk_run(s, np, s->d_tmp64, s->tk_ids, s->tk_scores, k, oc, oi, os);
+    if (!out_dev) {
+      copy_d2h(s, counts + lo, oc, (size_t)np * 4, s->stream);
+      copy_d2h(s, ids + (size_t)lo * k, oi, (size_t)np * k * 4, s->stream);
+      copy_d2h(s, scores + (size_t)lo * k, os, (size_t)np * k * 8, s->stream);
+    }
+  }
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+}
+
 /* ------------------------------------------------------------------------------ single ops */
 static uint32_t single_write(smatrix_t* s, int api_op, uint32_t x, uint32_t y, uint32_t v) {
   enter(s);
@@ -1608,6 +1749,8 @@ smatrix_t* smatrix_b200_open_arena(const char* fname, int device, size_t arena_b
   if (s->stage_max < 1024) s->stage_max = 1024;
   s->get_slices = (int)env_u32("SMATRIX_GET_SLICES", 1);
   s->get_slice_min = env_u32("SMATRIX_GET_SLICE_MIN", 1u << 22);
+  s->topk_pairs = env_u32("SMATRIX_TOPK_PAIRS", 1u << 28);
+  if (s->topk_pairs < 1) s->topk_pairs = 1;
   s->get_flags = s->get_slices & SMX_GET_FLAGS;
   s->get_slices = (s->get_slices & 3) > 2 ? 2 : (s->get_slices & 3);
   s->part_min = env_u32("SMATRIX_PARTITION_MIN", 1u << 20);
@@ -1690,6 +1833,9 @@ void smatrix_close(smatrix_t* s) {
   if (s->d_rowbuf) cudaFree(s->d_rowbuf);
   if (s->d_info) cudaFree(s->d_info);
   if (s->d_spill) cudaFree(s->d_spill);
+  void* tk[] = {s->tk_ctl, s->tk_off, s->tk_big, s->tk_cids, s->tk_cscores, s->tk_ids, s->tk_scores, s->tk_out};
+  for (size_t b = 0; b < sizeof tk / sizeof tk[0]; b++)
+    if (tk[b]) cudaFree(tk[b]);
   if (s->bo_cap) {
     cudaFree(s->bo_addr[0]); cudaFree(s->bo_addr[1]); cudaFree(s->bo_idx[0]); cudaFree(s->bo_idx[1]);
     cudaFree(s->bo_seg); cudaFree(s->bo_tiles); cudaFree(s->bo_out); cudaFree(s->bo_sort);
@@ -1802,6 +1948,8 @@ uint64_t smatrix_b200_stat(smatrix_t* s, int which) {
     case SMX_STAT_WIDE_CHUNKS: r = s->n_wide_chunks; break;
     case SMX_STAT_NS_ALLOC: r = (uint64_t)s->alloc_ns; break;
     case SMX_STAT_ALLOCS: r = s->n_allocs; break;
+    case SMX_STAT_TOPK_BIG: r = s->n_topk_big; break;
+    case SMX_STAT_TOPK_PASSES: r = s->n_topk_passes; break;
     case SMX_STAT_H2D_BYTES: r = s->h2d_bytes; break;
     case SMX_STAT_D2H_BYTES: r = s->d2h_bytes; break;
     case SMX_STAT_DIR_CAP: r = s->dir_cap; break;
@@ -1810,6 +1958,7 @@ uint64_t smatrix_b200_stat(smatrix_t* s, int which) {
       r = s->seg_bytes + s->dir_cap * sizeof(smx_row_t) + (uint64_t)s->list_cap * (6 * 4 + sizeof(smx_plan_t)) +
           (uint64_t)s->stage_cap * 24 + s->d_tmp_bytes + s->d_tmp64_bytes + s->d_rowbuf_bytes +
           (uint64_t)s->addrs_cap * 8 + (uint64_t)s->part_cap * 16;
+      for (int b = 0; b < 8; b++) r += s->tk_bytes[b];
       break;
     case SMX_STAT_LAUNCHES: r = s->n_launches; break;
     case SMX_STAT_ROUNDS: r = s->n_rounds; break;

@@ -185,6 +185,25 @@ void smx_launch_cf_scores(smx_stream_t stream, smx_view_t v, const uint32_t* ite
 void smx_launch_pair_cols(smx_stream_t stream, const uint32_t* pairs, uint64_t total, uint32_t* cols);
 void smx_launch_cf_scores_totals(smx_stream_t stream, uint32_t n, const uint64_t* offsets, const uint32_t* pairs,
                                  const uint32_t* a_tot, const uint32_t* b_tot, uint32_t* ids, double* scores);
+/* top-k per segment (kernel comment in smx_kernels.cu).  offsets[0..n] index ids / scores; outputs are k slots
+ * per segment.  Big segments: classify -> (host reads ctl) -> init -> passes until ctl[1] (segments still
+ * selecting) is 0 -> finish.  ctl: 16 zeroed words (big count, active count, big pairs as u64, region cursor as
+ * u64).  big_scratch: smx_topk_big_bytes(n_big) bytes, zeroed before init; c_ids / c_scores: big pairs slots. */
+#define SMX_TOPK_MAX_K 1024u
+size_t smx_topk_big_bytes(uint32_t n_big);
+uint32_t smx_topk_max_passes(void); /* digits of the 96-bit key */
+void smx_launch_topk_small(smx_stream_t stream, uint32_t n, const uint64_t* offsets, const uint32_t* ids,
+                           const double* scores, uint32_t k, uint32_t* counts, uint32_t* out_ids, double* out_scores);
+void smx_launch_topk_classify(smx_stream_t stream, uint32_t n, const uint64_t* offsets, uint32_t* big_list,
+                              uint32_t* ctl);
+void smx_launch_topk_init(smx_stream_t stream, const uint32_t* big_list, uint32_t n_big, const uint64_t* offsets,
+                          void* big_scratch, uint32_t* ctl);
+void smx_launch_topk_pass(smx_stream_t stream, void* big_scratch, uint32_t n_big, uint32_t k, const uint32_t* ids,
+                          const double* scores, uint32_t* c_ids, double* c_scores, uint32_t* ctl);
+void smx_launch_topk_finish(smx_stream_t stream, const void* big_scratch, uint32_t n_big, const uint32_t* c_ids,
+                            const double* c_scores, uint32_t k, uint32_t* counts, uint32_t* out_ids, double* out_scores);
+void smx_launch_topk_cut(smx_stream_t stream, const uint64_t* offsets, uint32_t n, uint32_t lo, uint64_t budget,
+                         uint32_t* out);
 void smx_launch_list_rows(smx_stream_t stream, smx_view_t v, uint32_t* keys, uint32_t* counter /* zeroed */);
 void smx_launch_row_slog(smx_stream_t stream, smx_view_t v, const uint32_t* xs, uint32_t n, uint32_t* out);
 void smx_launch_snap_units(smx_stream_t stream, const uint32_t* counts, const uint32_t* slogs, uint32_t n,

@@ -1303,6 +1303,303 @@ k_cf_scores_totals(uint32_t n, const ull* offsets, const uint32_t* pairs, const 
   }
 }
 
+/* ---- top-k per segment of (id, score) pairs (smatrix_cf_topk_batch, smatrix_b200_topk_segments) ------------
+ * Order: score descending, then id ascending.  The key of a pair is 96 bits: the score mapped to an order-
+ * preserving uint64 (flip every bit of a negative, set the sign bit of a positive), then ~id, so a larger key
+ * is always better and keys inside a segment are unique.  Three size classes, like getrow's:
+ *   k_topk_warp    segments of <= TOPK_WARP_MAX pairs: one warp per segment, bitonic sort in shared memory
+ *   k_topk_block   <= TOPK_BLOCK_MAX pairs: one block per segment, the same sort over 48 KB of shared memory
+ *   big segments   MSB radix select over the key, TOPK_DIGIT_BITS per pass, for all big segments of a call at
+ *                  once: k_topk_hist (TOPK_BIG_BLOCKS blocks per segment build shared-memory histograms of the
+ *                  candidates and merge them with one global atomic per bin), k_topk_pick (one thread per
+ *                  segment: the digit of the k-th key), k_topk_compact (the pairs at or above the boundary go to
+ *                  a private region once they are at most half the segment, and again once they fit).  When the
+ *                  pairs above the boundary plus the candidates fit TOPK_BLOCK_MAX, k_topk_finish sorts them.
+ * Launches are bounded by the number of digits, not by the number of segments.  The CPU tests lower the class
+ * thresholds and the digit width with -D so that rows of a few thousand pairs take every path. */
+#ifndef TOPK_WARP_MAX
+#define TOPK_WARP_MAX 256u
+#endif
+#ifndef TOPK_BLOCK_MAX
+#define TOPK_BLOCK_MAX 4096u /* 4096 x 12 B = the 48 KB of static shared memory a block may have */
+#endif
+#ifndef TOPK_DIGIT_BITS
+#define TOPK_DIGIT_BITS 8u
+#endif
+#define TOPK_RADIX (1u << TOPK_DIGIT_BITS)
+#define TOPK_BIG_BLOCKS (SMX_WARP > 1 ? 32u : 2u) /* grid.x per big segment (grid.y = segments) */
+static_assert(32u % TOPK_DIGIT_BITS == 0u, "a digit must not straddle the score / id boundary of the key");
+static_assert((TOPK_WARP_MAX & (TOPK_WARP_MAX - 1u)) == 0u && (TOPK_BLOCK_MAX & (TOPK_BLOCK_MAX - 1u)) == 0u,
+              "the bitonic sorts need power-of-two buffers");
+static_assert(TOPK_BLOCK_MAX >= SMX_TOPK_MAX_K && TOPK_WARP_MAX < TOPK_BLOCK_MAX, "size classes");
+
+__device__ __forceinline__ ull topk_map(double d) {
+#ifdef SMX_HOSTSIM
+  ull b;
+  memcpy(&b, &d, 8);
+#else
+  const ull b = (ull)__double_as_longlong(d);
+#endif
+  return (b >> 63) ? ~b : (b | (1ull << 63));
+}
+__device__ __forceinline__ double topk_unmap(ull m) {
+  const ull b = (m >> 63) ? (m & ~(1ull << 63)) : ~m;
+#ifdef SMX_HOSTSIM
+  double d;
+  memcpy(&d, &b, 8);
+  return d;
+#else
+  return __longlong_as_double((long long)b);
+#endif
+}
+/* a ranks before b */
+__device__ __forceinline__ bool topk_better(ull a_hi, uint32_t a_id, ull b_hi, uint32_t b_id) {
+  return a_hi > b_hi || (a_hi == b_hi && a_id < b_id);
+}
+/* the top `bits` bits of key (hi, lo) compared with those of the prefix: -1, 0, 1 */
+__device__ __forceinline__ int topk_cmp_top(ull hi, uint32_t lo, ull p_hi, uint32_t p_lo, uint32_t bits) {
+  if (bits == 0u) return 0;
+  if (bits <= 64u) {
+    const ull a = hi >> (64u - bits), b = p_hi >> (64u - bits);
+    return a < b ? -1 : (a > b ? 1 : 0);
+  }
+  if (hi != p_hi) return hi < p_hi ? -1 : 1;
+  const uint32_t a = (uint32_t)((ull)lo >> (96u - bits)), b = (uint32_t)((ull)p_lo >> (96u - bits));
+  return a < b ? -1 : (a > b ? 1 : 0);
+}
+/* the digit below the top `bits` bits */
+__device__ __forceinline__ uint32_t topk_digit(ull hi, uint32_t lo, uint32_t bits) {
+  if (bits < 64u) return (uint32_t)(hi >> (64u - bits - TOPK_DIGIT_BITS)) & (TOPK_RADIX - 1u);
+  return (lo >> (96u - bits - TOPK_DIGIT_BITS)) & (TOPK_RADIX - 1u);
+}
+
+template <bool BLOCK>
+__device__ __forceinline__ void topk_sync() {
+  if (BLOCK) __syncthreads(); else __syncwarp();
+}
+/* bitonic sort of N (power of two) keys, best first, by the T threads of a warp or a block (t = own index) */
+template <bool BLOCK>
+__device__ void topk_sort(ull* hi, uint32_t* id, uint32_t N, uint32_t t, uint32_t T) {
+  for (uint32_t run = 2; run <= N; run <<= 1)
+    for (uint32_t j = run >> 1; j > 0; j >>= 1) {
+      for (uint32_t i = t; i < N; i += T) {
+        const uint32_t l = i ^ j;
+        if (l <= i) continue;
+        const ull hi_i = hi[i], hi_l = hi[l];
+        const uint32_t id_i = id[i], id_l = id[l];
+        const bool swap = (i & run) == 0 ? topk_better(hi_l, id_l, hi_i, id_i) : topk_better(hi_i, id_i, hi_l, id_l);
+        if (swap) {
+          hi[i] = hi_l; hi[l] = hi_i;
+          id[i] = id_l; id[l] = id_i;
+        }
+      }
+      topk_sync<BLOCK>();
+    }
+}
+/* one segment of len <= buffer size pairs: stage, sort, write k slots (count[0] = min(k, len); the slots past
+ * it get id 0xFFFFFFFF and score -1.0) */
+template <bool BLOCK>
+__device__ void topk_segment(const uint32_t* ids, const double* scores, uint32_t len, uint32_t k, ull* hi,
+                             uint32_t* id, uint32_t t, uint32_t T, uint32_t* count, uint32_t* out_ids,
+                             double* out_scores) {
+  uint32_t N = 1u;
+  while (N < len) N <<= 1;
+  for (uint32_t i = t; i < N; i += T) {
+    const bool real = i < len;
+    hi[i] = real ? topk_map(scores[i]) : 0ull; /* padding ranks after every real key */
+    id[i] = real ? ids[i] : 0xFFFFFFFFu;
+  }
+  topk_sync<BLOCK>();
+  topk_sort<BLOCK>(hi, id, N, t, T);
+  const uint32_t c = len < k ? len : k;
+  for (uint32_t r = t; r < k; r += T) {
+    out_ids[r] = r < c ? id[r] : 0xFFFFFFFFu;
+    out_scores[r] = r < c ? topk_unmap(hi[r]) : -1.0;
+  }
+  if (t == 0u) *count = c;
+  topk_sync<BLOCK>(); /* before the buffers take the next segment */
+}
+
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_warp(uint32_t n, const ull* offsets, const uint32_t* ids, const double* scores, uint32_t k, uint32_t* counts,
+            uint32_t* out_ids, double* out_scores) {
+  __shared__ ull s_hi[SMX_BLOCK / SMX_WARP][TOPK_WARP_MAX];
+  __shared__ uint32_t s_id[SMX_BLOCK / SMX_WARP][TOPK_WARP_MAX];
+  const uint32_t lane = lane_id(), wib = threadIdx.x / SMX_WARP;
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) / SMX_WARP;
+  const uint32_t nwarps = gridDim.x * blockDim.x / SMX_WARP;
+  for (uint32_t i = warp; i < n; i += nwarps) {
+    const ull lo = offsets[i], len = offsets[i + 1] - lo;
+    if (len > TOPK_WARP_MAX) continue;
+    topk_segment<false>(ids + lo, scores + lo, (uint32_t)len, k, s_hi[wib], s_id[wib], lane, SMX_WARP, counts + i,
+                        out_ids + (ull)i * k, out_scores + (ull)i * k);
+  }
+}
+
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_block(uint32_t n, const ull* offsets, const uint32_t* ids, const double* scores, uint32_t k, uint32_t* counts,
+             uint32_t* out_ids, double* out_scores) {
+  __shared__ ull s_hi[TOPK_BLOCK_MAX];
+  __shared__ uint32_t s_id[TOPK_BLOCK_MAX];
+  for (uint32_t i = blockIdx.x; i < n; i += gridDim.x) {
+    const ull lo = offsets[i], len = offsets[i + 1] - lo;
+    if (len <= TOPK_WARP_MAX || len > TOPK_BLOCK_MAX) continue;
+    topk_segment<true>(ids + lo, scores + lo, (uint32_t)len, k, s_hi, s_id, threadIdx.x, blockDim.x, counts + i,
+                       out_ids + (ull)i * k, out_scores + (ull)i * k);
+  }
+}
+
+/* the select state of one big segment.  Its pairs live in the input arrays (src_kind 0) or, once compacted, in
+ * its region of the compaction buffers (src_kind 1; the region has `len` slots: the first compaction writes at
+ * its start, a second one into its upper half, which the first one's output never reaches). */
+typedef struct {
+  ull pre_hi;         /* the key bits fixed so far, left-aligned; the rest zero        */
+  ull len, reg;       /* segment length, start of its compaction region              */
+  ull src_off, src_len, from_off, from_len;
+  uint32_t pre_lo, bits; /* key bits fixed so far (a multiple of TOPK_DIGIT_BITS)     */
+  uint32_t item;      /* segment index                                               */
+  uint32_t above;     /* pairs above the prefix range: all of them are in the top k  */
+  uint32_t cand;      /* pairs inside the prefix range                               */
+  uint32_t done, compact, cursor, src_kind, from_kind;
+} topk_state_t;
+
+/* big segments -> list; ctl[0] = their number, ctl[2..3] = their pairs (u64) */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_classify(uint32_t n, const ull* offsets, uint32_t* big_list, uint32_t* ctl) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const ull len = offsets[i + 1] - offsets[i];
+    if (len <= TOPK_BLOCK_MAX) continue;
+    big_list[agg_inc(&ctl[0])] = i;
+    atomicAdd((ull*)(ctl + 2), len);
+  }
+}
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_init(const uint32_t* big_list, uint32_t n_big, const ull* offsets, topk_state_t* st_all, ull* reg_cursor) {
+  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n_big; j += gridDim.x * blockDim.x) {
+    const uint32_t i = big_list[j];
+    topk_state_t st;
+    memset(&st, 0, sizeof st);
+    st.item = i;
+    st.src_off = offsets[i];
+    st.len = st.src_len = offsets[i + 1] - st.src_off;
+    st.cand = (uint32_t)st.len;
+    st.reg = atomicAdd(reg_cursor, st.len);
+    st_all[j] = st;
+  }
+}
+
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_hist(const topk_state_t* st_all, uint32_t first, const uint32_t* ids, const double* scores,
+            const uint32_t* c_ids, const double* c_scores, uint32_t* hist) {
+  __shared__ uint32_t s_h[TOPK_RADIX];
+  const uint32_t j = first + blockIdx.y;
+  const topk_state_t st = st_all[j];
+  if (st.done) return;
+  for (uint32_t b = threadIdx.x; b < TOPK_RADIX; b += blockDim.x) s_h[b] = 0u;
+  __syncthreads();
+  const uint32_t* sid = (st.src_kind ? c_ids : ids) + st.src_off;
+  const double* ssc = (st.src_kind ? c_scores : scores) + st.src_off;
+  for (ull p = (ull)blockIdx.x * blockDim.x + threadIdx.x; p < st.src_len; p += (ull)gridDim.x * blockDim.x) {
+    const ull hk = topk_map(ssc[p]);
+    const uint32_t lk = ~sid[p];
+    if (topk_cmp_top(hk, lk, st.pre_hi, st.pre_lo, st.bits) == 0) atomicAdd(&s_h[topk_digit(hk, lk, st.bits)], 1u);
+  }
+  __syncthreads();
+  for (uint32_t b = threadIdx.x; b < TOPK_RADIX; b += blockDim.x)
+    if (s_h[b]) atomicAdd(&hist[(ull)j * TOPK_RADIX + b], s_h[b]);
+}
+
+/* one thread per big segment: the boundary digit = the bin that holds the k-th key among the candidates */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_pick(topk_state_t* st_all, uint32_t n_big, uint32_t k, uint32_t* hist, uint32_t* active) {
+  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n_big; j += gridDim.x * blockDim.x) {
+    topk_state_t st = st_all[j];
+    if (st.done) {
+      st_all[j].compact = 0u; /* its last compaction ran in the pass that finished it */
+      continue;
+    }
+    uint32_t* h = hist + (ull)j * TOPK_RADIX;
+    const uint32_t need = k - st.above; /* >= 1: above < k always */
+    uint32_t cum = 0u, b = TOPK_RADIX - 1u;
+    for (;; --b) {
+      if (cum + h[b] >= need || b == 0u) break;
+      cum += h[b];
+    }
+    st.above += cum;
+    st.cand = h[b];
+    if (st.bits < 64u) st.pre_hi |= (ull)b << (64u - st.bits - TOPK_DIGIT_BITS);
+    else st.pre_lo |= b << (96u - st.bits - TOPK_DIGIT_BITS);
+    st.bits += TOPK_DIGIT_BITS;
+    for (uint32_t d = 0; d < TOPK_RADIX; ++d) h[d] = 0u;
+    const ull keep = (ull)st.above + st.cand;
+    st.done = keep <= TOPK_BLOCK_MAX;
+    st.compact = st.src_kind == 0u ? (st.done || 2ull * keep <= st.len) : (st.done && st.src_len != keep);
+    if (st.compact) {
+      st.from_kind = st.src_kind; st.from_off = st.src_off; st.from_len = st.src_len;
+      st.src_kind = 1u;
+      st.src_off = st.reg + (st.from_kind ? st.len / 2u : 0ull);
+      st.src_len = keep;
+      st.cursor = 0u;
+    }
+    if (!st.done) atomicAdd(active, 1u);
+    st_all[j] = st;
+  }
+}
+
+/* the pairs whose top `bits` key bits are >= the prefix: into the segment's region (one atomic per block tile) */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_compact(topk_state_t* st_all, uint32_t first, const uint32_t* ids, const double* scores, uint32_t* c_ids,
+               double* c_scores) {
+  __shared__ uint32_t s_base;
+  const uint32_t j = first + blockIdx.y;
+  const topk_state_t st = st_all[j];
+  if (!st.compact) return;
+  const uint32_t* sid = (st.from_kind ? c_ids : ids) + st.from_off;
+  const double* ssc = (st.from_kind ? c_scores : scores) + st.from_off;
+  for (ull p0 = (ull)blockIdx.x * blockDim.x; p0 < st.from_len; p0 += (ull)gridDim.x * blockDim.x) {
+    const ull p = p0 + threadIdx.x;
+    uint32_t id = 0u;
+    double sc = 0.0;
+    bool keep = false;
+    if (p < st.from_len) {
+      id = sid[p];
+      sc = ssc[p];
+      keep = topk_cmp_top(topk_map(sc), ~id, st.pre_hi, st.pre_lo, st.bits) >= 0;
+    }
+    ull total;
+    const uint32_t w = (uint32_t)block_exclusive_scan(keep ? 1ull : 0ull, &total);
+    if (threadIdx.x == 0) s_base = total ? atomicAdd(&st_all[j].cursor, (uint32_t)total) : 0u;
+    __syncthreads();
+    if (keep) {
+      c_ids[st.src_off + s_base + w] = id;
+      c_scores[st.src_off + s_base + w] = sc;
+    }
+    __syncthreads(); /* s_base is rewritten by the next tile */
+  }
+}
+
+/* one block per big segment: sort what the select kept (<= TOPK_BLOCK_MAX pairs) and write the first k */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_topk_finish(const topk_state_t* st_all, uint32_t first, const uint32_t* c_ids, const double* c_scores, uint32_t k,
+              uint32_t* counts, uint32_t* out_ids, double* out_scores) {
+  __shared__ ull s_hi[TOPK_BLOCK_MAX];
+  __shared__ uint32_t s_id[TOPK_BLOCK_MAX];
+  const topk_state_t st = st_all[first + blockIdx.x];
+  topk_segment<true>(c_ids + st.src_off, c_scores + st.src_off, (uint32_t)st.src_len, k, s_hi, s_id, threadIdx.x,
+                     blockDim.x, counts + st.item, out_ids + (ull)st.item * k, out_scores + (ull)st.item * k);
+}
+
+/* one thread: the end of the piece that starts at item lo = the last item whose pairs still fit the budget
+ * (at least one item: a row over the budget is a piece of its own) -> out[0] */
+__global__ void k_topk_cut(const ull* offsets, uint32_t n, uint32_t lo, ull budget, uint32_t* out) {
+  uint32_t a = lo + 1u, b = n; /* answer in [a, b] */
+  while (a < b) {
+    const uint32_t m = a + (b - a + 1u) / 2u;
+    if (offsets[m] - offsets[lo] <= budget) a = m; else b = m - 1u;
+  }
+  out[0] = a;
+}
+
 /* ---- snapshot support (file mode, reference src/smatrix.c:30-72) --------------------------- */
 /* all row ids of the directory, in no particular order */
 __global__ void __launch_bounds__(SMX_BLOCK) k_list_rows(smx_view_t V, uint32_t* keys, uint32_t* counter) {
@@ -2202,6 +2499,61 @@ extern "C" void smx_launch_cf_scores_totals(smx_stream_t st, uint32_t n, const u
   if (!n) return;
   SMX_LAUNCH(k_cf_scores_totals, grid_for((ull)n * SMX_WARP), SMX_BLOCK, st, n, (const ull*)offsets, pairs, a_tot,
              b_tot, ids, scores);
+}
+extern "C" uint32_t smx_topk_max_passes(void) { return 96u / TOPK_DIGIT_BITS; }
+extern "C" size_t smx_topk_big_bytes(uint32_t n_big) {
+  return (size_t)n_big * (sizeof(topk_state_t) + TOPK_RADIX * 4u);
+}
+extern "C" void smx_launch_topk_small(smx_stream_t st, uint32_t n, const uint64_t* offsets, const uint32_t* ids,
+                                      const double* scores, uint32_t k, uint32_t* counts, uint32_t* out_ids,
+                                      double* out_scores) {
+  if (!n) return;
+  SMX_LAUNCH(k_topk_warp, grid_for((ull)n * SMX_WARP), SMX_BLOCK, st, n, (const ull*)offsets, ids, scores, k, counts,
+             out_ids, out_scores);
+  const uint32_t cap = (uint32_t)smx_grid_blocks();
+  SMX_LAUNCH(k_topk_block, n < cap ? n : cap, SMX_BLOCK, st, n, (const ull*)offsets, ids, scores, k, counts, out_ids,
+             out_scores);
+}
+extern "C" void smx_launch_topk_classify(smx_stream_t st, uint32_t n, const uint64_t* offsets, uint32_t* big_list,
+                                         uint32_t* ctl) {
+  if (!n) return;
+  SMX_LAUNCH(k_topk_classify, grid_for(n), SMX_BLOCK, st, n, (const ull*)offsets, big_list, ctl);
+}
+extern "C" void smx_launch_topk_init(smx_stream_t st, const uint32_t* big_list, uint32_t n_big, const uint64_t* offsets,
+                                     void* big_scratch, uint32_t* ctl) {
+  if (!n_big) return;
+  SMX_LAUNCH(k_topk_init, grid_for(n_big), SMX_BLOCK, st, big_list, n_big, (const ull*)offsets,
+             (topk_state_t*)big_scratch, (ull*)(ctl + 4));
+}
+extern "C" void smx_launch_topk_pass(smx_stream_t st, void* big_scratch, uint32_t n_big, uint32_t k,
+                                     const uint32_t* ids, const double* scores, uint32_t* c_ids, double* c_scores,
+                                     uint32_t* ctl) {
+  topk_state_t* state = (topk_state_t*)big_scratch;
+  uint32_t* hist = (uint32_t*)(state + n_big);
+  for (uint32_t first = 0; first < n_big; first += 32768u) {
+    const uint32_t cnt = (n_big - first < 32768u) ? n_big - first : 32768u;
+    SMX_LAUNCH(k_topk_hist, dim3(TOPK_BIG_BLOCKS, cnt, 1u), SMX_BLOCK, st, state, first, ids, scores, c_ids, c_scores,
+               hist);
+  }
+  SMX_LAUNCH(k_topk_pick, grid_for(n_big), SMX_BLOCK, st, state, n_big, k, hist, ctl + 1);
+  for (uint32_t first = 0; first < n_big; first += 32768u) {
+    const uint32_t cnt = (n_big - first < 32768u) ? n_big - first : 32768u;
+    SMX_LAUNCH(k_topk_compact, dim3(TOPK_BIG_BLOCKS, cnt, 1u), SMX_BLOCK, st, state, first, ids, scores, c_ids,
+               c_scores);
+  }
+}
+extern "C" void smx_launch_topk_finish(smx_stream_t st, const void* big_scratch, uint32_t n_big, const uint32_t* c_ids,
+                                       const double* c_scores, uint32_t k, uint32_t* counts, uint32_t* out_ids,
+                                       double* out_scores) {
+  for (uint32_t first = 0; first < n_big; first += 32768u) {
+    const uint32_t cnt = (n_big - first < 32768u) ? n_big - first : 32768u;
+    SMX_LAUNCH(k_topk_finish, cnt, SMX_BLOCK, st, (const topk_state_t*)big_scratch, first, c_ids, c_scores, k, counts,
+               out_ids, out_scores);
+  }
+}
+extern "C" void smx_launch_topk_cut(smx_stream_t st, const uint64_t* offsets, uint32_t n, uint32_t lo, uint64_t budget,
+                                    uint32_t* out) {
+  SMX_LAUNCH(k_topk_cut, 1, 1, st, (const ull*)offsets, n, lo, (ull)budget, out);
 }
 extern "C" void smx_launch_sum_values(smx_stream_t st, smx_view_t v, uint32_t* big_list, uint32_t* big_counter) {
   SMX_LAUNCH(k_sum_values, grid_for(v.dir_cap * SMX_WARP), SMX_BLOCK, st, v, big_list, big_counter);

@@ -804,16 +804,23 @@ uint64_t smatrix_b200_shard_getrow_batch(smatrix_shard_t* sh, const uint32_t* xs
   return total;
 }
 
-/* The read side of the co-occurrence recommender across ranks (examples/cf_recommender.c:50-86, same
- * contract as smatrix_cf_neighbors_batch): the rows come through the getrow route; the totals
- * (value at (item, 0) and at (neighbour, 0)) are two sharded gets; the scores are computed where the
- * pairs landed. */
-uint64_t smatrix_b200_shard_cf_neighbors_batch(smatrix_shard_t* sh, const uint32_t* items, size_t n,
-                                               uint64_t* offsets, uint32_t* ids, double* scores, uint64_t cap) {
-  if (n >= 0xFFFFFFFEull) rt_die(sh, "cf_neighbors_batch: too many items in one call");
+/* The collective core of both CF calls: rows through the getrow route, totals through two sharded gets, scores
+ * on this rank's GPU.  Returns the total; when any rank fills, c->scratch holds (with `extra` more bytes at
+ * c->extra) and, if this rank filled, c->off / c->ids / c->scores are its CSR of scores on the device.  The
+ * caller frees c->scratch. */
+typedef struct {
+  char* scratch;
+  void* extra;
+  uint64_t* off;
+  uint32_t* ids;
+  double* scores;
+  int filled;
+} rt_cf_t;
+static uint64_t rt_cf_scores(smatrix_shard_t* sh, const uint32_t* items, size_t n, int want, uint64_t cap,
+                             uint64_t* offsets, size_t extra, rt_cf_t* c) {
   const uint32_t* d_items = rt_ids_on_device(sh, items, n);
   int filled = 0, any = 0;
-  const uint64_t total = rt_getrow_core(sh, d_items, n, ids != NULL && scores != NULL, cap, &filled, &any);
+  const uint64_t total = rt_getrow_core(sh, d_items, n, want, cap, &filled, &any);
   if (offsets) {
     if (n) {
       smatrix_b200_memcpy(sh->local, offsets, sh->inbox + OFF_OFS(sh->cap), (n + 1) * 8);
@@ -822,12 +829,15 @@ uint64_t smatrix_b200_shard_cf_neighbors_batch(smatrix_shard_t* sh, const uint32
       smatrix_b200_memcpy(sh->local, offsets, &zero, 8);
     }
   }
+  memset(c, 0, sizeof *c);
+  c->filled = filled;
   if (!any) return total;
   /* scratch on my GPU: neighbour ids, their totals, my items' totals, zeros (column 0), scores, and a
    * copy of the CSR offsets + items (the gets below reuse the inbox's local arrays) */
   const size_t np = filled ? (size_t)total : 0, nn = filled ? n : 0;
   const size_t big = np > nn ? np : nn;
-  char* scratch = (char*)smatrix_b200_dev_alloc(sh->local, big * 4 * 2 + np * 4 + nn * 4 * 2 + np * 8 + (nn + 1) * 8 + 256);
+  char* scratch = (char*)smatrix_b200_dev_alloc(sh->local, big * 4 * 2 + np * 4 + nn * 4 * 2 + np * 8 + (nn + 1) * 8 +
+                                                extra + 256);
   uint32_t* d_zero = (uint32_t*)scratch;
   uint32_t* d_cols = d_zero + big;
   uint32_t* d_btot = d_cols + big;
@@ -843,12 +853,63 @@ uint64_t smatrix_b200_shard_cf_neighbors_batch(smatrix_shard_t* sh, const uint32
   }
   rt_read_piece(sh, RT_GET, d_cols, d_zero, np, d_btot);                  /* collective: n = 0 on ranks that do not fill */
   rt_read_piece(sh, RT_GET, d_keep, d_zero, nn, d_atot);
-  if (filled) {
-    /* the ids go out through d_cols' slot again (same values), the scores through d_scores */
-    smatrix_b200_cf_scores_totals(sh->local, n, d_off, (const uint32_t*)sh->rowbuf, d_atot, d_btot, d_cols, d_scores);
-    smatrix_b200_memcpy(sh->local, ids, d_cols, (size_t)total * 4);
-    smatrix_b200_memcpy(sh->local, scores, d_scores, (size_t)total * 8);
-  }
-  smatrix_b200_dev_free(sh->local, scratch);
+  /* the ids go out through d_cols' slot again (same values), the scores through d_scores */
+  if (filled) smatrix_b200_cf_scores_totals(sh->local, n, d_off, (const uint32_t*)sh->rowbuf, d_atot, d_btot, d_cols, d_scores);
+  c->scratch = scratch;
+  c->extra = d_scores + np;
+  c->off = d_off;
+  c->ids = d_cols;
+  c->scores = d_scores;
   return total;
+}
+
+/* The read side of the co-occurrence recommender across ranks (examples/cf_recommender.c:50-86, same
+ * contract as smatrix_cf_neighbors_batch): the rows come through the getrow route; the totals
+ * (value at (item, 0) and at (neighbour, 0)) are two sharded gets; the scores are computed where the
+ * pairs landed. */
+uint64_t smatrix_b200_shard_cf_neighbors_batch(smatrix_shard_t* sh, const uint32_t* items, size_t n,
+                                               uint64_t* offsets, uint32_t* ids, double* scores, uint64_t cap) {
+  if (n >= 0xFFFFFFFEull) rt_die(sh, "cf_neighbors_batch: too many items in one call");
+  rt_cf_t c;
+  const uint64_t total = rt_cf_scores(sh, items, n, ids != NULL && scores != NULL, cap, offsets, 0, &c);
+  if (c.filled) {
+    smatrix_b200_memcpy(sh->local, ids, c.ids, (size_t)total * 4);
+    smatrix_b200_memcpy(sh->local, scores, c.scores, (size_t)total * 8);
+  }
+  if (c.scratch) smatrix_b200_dev_free(sh->local, c.scratch);
+  return total;
+}
+
+void smatrix_b200_shard_cf_topk_batch(smatrix_shard_t* sh, const uint32_t* items, size_t n, uint32_t k,
+                                      uint32_t* counts, uint32_t* ids, double* scores) {
+  if (k < 1 || k > 1024u) rt_die(sh, "cf_topk_batch: k = %u is outside 1..1024", k);
+  if (n >= 0xFFFFFFFEull) rt_die(sh, "cf_topk_batch: too many items in one call");
+  const int out_dev = rt_is_dev(sh, counts);
+  if (n && (rt_is_dev(sh, ids) != out_dev || rt_is_dev(sh, scores) != out_dev))
+    rt_die(sh, "batch arrays must be all host or all device pointers");
+  /* room for the answers on the device when they go to host arrays, and for all-zero offsets when this rank's
+   * rows are empty (then it fills nothing but still ranks: every count is 0) */
+  const size_t out_bytes = out_dev ? 0 : n * (12ull * k + 4);
+  rt_cf_t c;
+  rt_cf_scores(sh, items, n, 1, ~0ull, NULL, out_bytes + (n + 1) * 8 + 64, &c);
+  if (n) {
+    char* extra = c.scratch ? (char*)(((uintptr_t)c.extra + 7) & ~(uintptr_t)7)
+                            : (char*)smatrix_b200_dev_alloc(sh->local, out_bytes + (n + 1) * 8 + 64);
+    const uint64_t* d_off = c.off;
+    if (!c.filled) {
+      smatrix_b200_memset0(sh->local, extra, (n + 1) * 8);
+      d_off = (const uint64_t*)extra;
+    }
+    double* os = out_dev ? scores : (double*)(extra + (n + 1) * 8);
+    uint32_t* oi = out_dev ? ids : (uint32_t*)(os + n * k);
+    uint32_t* oc = out_dev ? counts : oi + n * k;
+    smatrix_b200_topk_segments(sh->local, n, d_off, c.ids, c.scores, k, oc, oi, os);
+    if (!out_dev) {
+      smatrix_b200_memcpy(sh->local, counts, oc, n * 4);
+      smatrix_b200_memcpy(sh->local, ids, oi, n * k * 4);
+      smatrix_b200_memcpy(sh->local, scores, os, n * k * 8);
+    }
+    if (!c.scratch) smatrix_b200_dev_free(sh->local, extra);
+  }
+  if (c.scratch) smatrix_b200_dev_free(sh->local, c.scratch);
 }

@@ -22,6 +22,37 @@ def _is_torch(a) -> bool:
     return type(a).__module__.startswith("torch")
 
 
+TOPK_MAX_K = 1024
+
+
+def _topk_call(fn, items, k):
+    """fn(items_ptr, n, k, counts_ptr, ids_ptr, scores_ptr) on outputs allocated where `items` lives."""
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= int(k) <= TOPK_MAX_K:
+        raise ValueError(f"k must be an integer in 1..{TOPK_MAX_K}, got {k!r}")
+    k = int(k)
+    if _is_torch(items) and items.is_cuda:
+        import torch
+        if items.dtype not in (torch.int32, torch.uint32):
+            raise TypeError("torch batch arrays must be int32/uint32")
+        items = items.contiguous()
+        n = items.numel()
+        counts = torch.empty(n, dtype=torch.int32, device=items.device)
+        ids = torch.empty((n, k), dtype=torch.int32, device=items.device)
+        scores = torch.empty((n, k), dtype=torch.float64, device=items.device)
+        torch.cuda.current_stream(items.device).synchronize()      # the items may still be in flight on torch's stream
+        fn(items.data_ptr(), n, k, counts.data_ptr(), ids.data_ptr(), scores.data_ptr())
+        return counts, ids, scores
+    if _is_torch(items):
+        items = items.numpy()
+    items = np.ascontiguousarray(items, dtype=np.uint32)
+    n = len(items)
+    counts = np.empty(n, dtype=np.uint32)
+    ids = np.empty((n, k), dtype=np.uint32)
+    scores = np.empty((n, k), dtype=np.float64)
+    fn(items.ctypes.data, n, k, counts.ctypes.data, ids.ctypes.data, scores.ctypes.data)
+    return counts, ids, scores
+
+
 class DevPtr:
     """A raw device array of `n` uint32 (library- or peer-allocated memory that is not a tensor)."""
     __slots__ = ("ptr", "n")
@@ -279,6 +310,13 @@ class SparseMatrix:
             self._lib.smatrix_cf_neighbors_batch(self._handle(), items.ctypes.data, n, offsets.ctypes.data,
                                                  ids.ctypes.data, scores.ctypes.data, total)
         return offsets, ids, scores
+
+    def cf_topk_batch(self, items, k: int):
+        """The k best neighbours of every item, ranked on the device (score descending, then id ascending) ->
+        (counts[n], ids[n, k], scores[n, k]); slots past counts[i] hold id 0xFFFFFFFF and score -1.0.
+        numpy (or any host sequence) in -> numpy out; a CUDA torch tensor in -> tensors on its device out
+        (int32 counts and ids, float64 scores), with no copy through the host."""
+        return _topk_call(lambda *a: self._lib.smatrix_cf_topk_batch(self._handle(), *a), items, k)
 
     # ---- device controls (include/smatrix_b200.h) --------------------------------------------
     def stat(self, name: str) -> int:

@@ -50,7 +50,7 @@ import torch.distributed as dist
 
 import ctypes as C
 
-from .matrix import DevPtr, SparseMatrix
+from .matrix import DevPtr, SparseMatrix, _topk_call
 
 
 class _PeerBuffers:
@@ -722,6 +722,10 @@ class ShardedSparseMatrix:
                                                                   ids.ctypes.data, scores.ctypes.data, max(total, 1)))
         assert got == total
         return offsets, ids[:total], scores[:total]
+
+    def cf_topk_batch(self, items, k: int):
+        """The k best neighbours of THIS rank's items (contract of SparseMatrix.cf_topk_batch); collective."""
+        return _topk_call(lambda *a: self._lib.smatrix_b200_shard_cf_topk_batch(self._handle(), *a), items, k)
 
     def getrow_batch_into(self, d_xs, n: int, d_offsets: int, d_pairs: int, pairs_cap: int) -> int:
         """The raw collective call on device (or host) pointers; returns the total number of pairs."""
