@@ -49,6 +49,23 @@ typedef struct {
   int owned; /* cudaMalloc'ed by us (freed at close); 0 = a block given back to the slab, e.g. a replaced directory */
 } smx_seg_t;
 
+typedef struct { void* p; size_t bytes; } smx_dbuf_t; /* device scratch that grows on demand (dbuf_need) */
+
+/* Pinned host words that small device answers are read back into, and a single op's arguments go up from: one
+ * field per value, so that no two uses share a slot. */
+typedef struct {
+  uint32_t op[3];      /* single ops: x, y, value on their way to d_small[DS_X..DS_V] */
+  uint32_t answer;     /* single ops: the value or row length (d_small[DS_OUT]) */
+  uint64_t row_total;  /* pairs of the rows of a getrow plan / of smatrix_b200_scan_counts (the last offset) */
+  uint32_t n_big_rows; /* rows of a getrow plan that the whole grid compacts */
+  uint32_t n_spill;    /* cells the tile-wise re-placement could not place in their tile */
+  uint32_t probe_max;  /* largest probe step of a directory rehash */
+  uint32_t n_big_sums; /* SMX_STAT_VALUE_SUM: rows with a big bucket, summed by a launch of their own */
+  uint32_t topk_cut;   /* end of the next piece of a cf_topk_batch call */
+  struct { uint32_t n_big, active; uint64_t big_pairs; } topk; /* control words 0..3 of a top-k selection */
+} smx_small_t;
+enum { DS_X, DS_Y, DS_V, DS_OUT, DS_WORDS }; /* the words of d_small: a single op's arguments, a one-word answer */
+
 struct smatrix_s {
   int device;
   int prev_device; /* the caller's current device, restored by leave() */
@@ -91,49 +108,34 @@ struct smatrix_s {
   int wide_slices;        /* SMATRIX_WIDE_SLICES: chunks without ops on column 0 use 256 slices */
 
 
-  uint32_t* d_small; /* 64 words */
-  uint32_t* h_small; /* pinned, 64 words */
+  uint32_t* d_small; /* DS_WORDS words */
+  smx_small_t* h_small; /* pinned */
 
-  uint32_t* d_tmp;   /* general temp (counts / outputs), grows */
-  size_t d_tmp_bytes;
-  uint64_t* d_tmp64;
-  size_t d_tmp64_bytes;
-  uint32_t* d_rowbuf;
-  size_t d_rowbuf_bytes;
-  /* *_batch_out (exact per-op return values): scratch sized for bo_cap ops */
-  uint32_t bo_cap;
-  uint64_t* bo_addr[2];
-  uint32_t* bo_idx[2];
-  uint64_t* bo_seg;
-  uint64_t* bo_tiles;
-  uint32_t* bo_out;
-  void* bo_sort;
-  size_t bo_sort_bytes;
-  uint64_t* d_info;     /* getrow: per-row directory index | caplog << 32 (k_row_counts) */
-  uint32_t* d_big;      /* getrow: indices of big rows in the current query + per-row output cursors */
-  uint32_t* d_cursors;
-  size_t d_big_bytes;
-  uint32_t n_big_rows;
-  /* top-k (smatrix_cf_topk_batch, smatrix_b200_topk_segments): scratch that grows with slack, so that calls of
-   * similar size make no cudaMalloc */
+  /* scratch that grows with slack (dbuf_need), so that calls of similar size make no cudaMalloc; freed at close.
+   * Only smx_dbuf_t members: smatrix_close and SMX_STAT_DEVICE_BYTES walk it as an array. */
+  struct {
+    smx_dbuf_t tmp, tmp64; /* general temp: ids on their way up, counts, partition counters (u32 / u64 words) */
+    smx_dbuf_t plan;       /* getrow plan (rowplan) */
+    smx_dbuf_t rows;       /* pairs of whole rows on their way to host outputs, scores or a snapshot */
+    smx_dbuf_t host_out;   /* cf_neighbors_batch / cf_topk_batch answers on their way to host outputs */
+    smx_dbuf_t spill;      /* cells that did not fit their tile (16 bytes each) */
+    /* *_batch_out (exact per-op return values) */
+    smx_dbuf_t bo_addr[2], bo_idx[2], bo_seg, bo_tiles, bo_out, bo_sort;
+    /* top-k (smatrix_cf_topk_batch, smatrix_b200_topk_segments) */
+    smx_dbuf_t tk_ctl;     /* 16 control words + the list of big segments */
+    smx_dbuf_t tk_off;     /* row offsets of the whole call (piece cuts) */
+    smx_dbuf_t tk_big;     /* select state + histograms of the big segments */
+    smx_dbuf_t tk_cids, tk_cscores; /* compaction regions of the big segments */
+    smx_dbuf_t tk_ids, tk_scores;   /* scores of a piece */
+  } db;
   uint32_t topk_pairs;  /* SMATRIX_TOPK_PAIRS: pairs per piece of a cf_topk_batch call */
-  uint32_t* tk_ctl;     /* 16 control words + the list of big segments */
-  uint64_t* tk_off;     /* row offsets of the whole call (piece cuts) */
-  void* tk_big;         /* select state + histograms of the big segments */
-  uint32_t* tk_cids;    /* compaction regions of the big segments */
-  double* tk_cscores;
-  uint32_t* tk_ids;     /* scores of a piece */
-  double* tk_scores;
-  void* tk_out;         /* a piece's answers on their way to host outputs */
-  size_t tk_bytes[8];
   uint64_t n_topk_big, n_topk_passes;
 
   unsigned long long* free_ptr[SMX_CLASSES]; /* device stacks of vacated buckets, per size class */
   uint32_t free_cap[SMX_CLASSES];
   int debug;                                 /* SMATRIX_DEBUG: growth decisions on stderr */
   int migrate_tiles;                         /* SMATRIX_MIGRATE_TILES (default 1): big rows are re-placed tile by tile in shared memory */
-  unsigned long long* d_spill;               /* cells that did not fit their tile (16 bytes each) */
-  uint32_t spill_cap;
+  uint32_t spill_cap;                        /* cells the spill list (db.spill) is sized for */
   uint64_t n_spilled;
   int recycle;                               /* SMATRIX_RECYCLE (default 1) */
   int presize;                               /* SMATRIX_PRESIZE (default 1): distinct-row estimate before a chunk of new rows */
@@ -190,6 +192,19 @@ static void* dmalloc(smatrix_t* s, size_t bytes) {
   s->alloc_ns += now_ns() - t0; /* SMX_STAT_NS_ALLOC: cudaMalloc stalls for 2 - 150 ms on some hosts */
   s->n_allocs++;
   return p;
+}
+
+/* b, grown to at least `need` bytes.  A replaced block may still be read by work in flight on s->stream: it is
+ * freed after that work; its contents are not kept. */
+static void* dbuf_need(smatrix_t* s, smx_dbuf_t* b, size_t need) {
+  if (need <= b->bytes) return b->p;
+  if (b->p) {
+    CK(cudaStreamSynchronize(s->stream));
+    CK(cudaFree(b->p));
+  }
+  b->bytes = need + need / 4 + 4096;
+  b->p = dmalloc(s, b->bytes);
+  return b->p;
 }
 
 /* host <-> device copies, counted (the end-to-end accounting of bench.py reads the counters) */
@@ -344,19 +359,6 @@ static void ensure_lists(smatrix_t* s, uint32_t n) {
   s->list_cap = cap;
 }
 
-static void ensure_tmp(smatrix_t* s, size_t bytes32, size_t bytes64) {
-  if (bytes32 > s->d_tmp_bytes) {
-    if (s->d_tmp) { CK(cudaStreamSynchronize(s->stream)); cudaFree(s->d_tmp); }
-    s->d_tmp_bytes = bytes32 + bytes32 / 4;
-    s->d_tmp = (uint32_t*)dmalloc(s, s->d_tmp_bytes);
-  }
-  if (bytes64 > s->d_tmp64_bytes) {
-    if (s->d_tmp64) { CK(cudaStreamSynchronize(s->stream)); cudaFree(s->d_tmp64); }
-    s->d_tmp64_bytes = bytes64 + bytes64 / 4;
-    s->d_tmp64 = (uint64_t*)dmalloc(s, s->d_tmp64_bytes);
-  }
-}
-
 static void ensure_stage(smatrix_t* s, uint32_t n) {
   if (n <= s->stage_cap) return;
   uint32_t cap = n < 4096 ? 4096 : n;
@@ -431,22 +433,20 @@ static void grow_rows(smatrix_t* s, uint32_t n_grow) {
   const int tiles = s->migrate_tiles && n_big;
   smx_launch_migrate(s->stream, v, s->lists, n_grow, n_mid, n_big, region, tiles);
   if (tiles) { /* big rows: new buckets built tile by tile in shared memory (k_migrate_tiles) */
+    unsigned long long* spill;
+    uint32_t n_spill;
     for (;;) {
-      if (!s->d_spill) {
-        s->spill_cap = s->spill_cap ? s->spill_cap : (1u << 16);
-        s->d_spill = (unsigned long long*)dmalloc(s, (size_t)s->spill_cap * 16);
-      }
+      spill = dbuf_need(s, &s->db.spill, (size_t)s->spill_cap * 16);
       CK(cudaMemsetAsync(&s->d_ctl->n_spill, 0, 4, s->stream));
-      smx_launch_migrate_tiles(s->stream, v, s->lists, n_big, region, s->d_spill, s->spill_cap);
-      copy_d2h(s, &s->h_small[38], &s->d_ctl->n_spill, 4, s->stream);
+      smx_launch_migrate_tiles(s->stream, v, s->lists, n_big, region, spill, s->spill_cap);
+      copy_d2h(s, &s->h_small->n_spill, &s->d_ctl->n_spill, 4, s->stream);
       CK(cudaStreamSynchronize(s->stream));
-      if (s->h_small[38] <= s->spill_cap) break;
-      CK(cudaFree(s->d_spill)); /* the list was too short: step 1 only reads the old buckets, so it can run again */
-      s->d_spill = NULL;
-      s->spill_cap = s->h_small[38] + s->h_small[38] / 2 + 1024;
+      n_spill = s->h_small->n_spill;
+      if (n_spill <= s->spill_cap) break;
+      s->spill_cap = n_spill + n_spill / 2 + 1024; /* the list was too short: step 1 only reads the old buckets, so it can run again */
     }
-    smx_launch_migrate_tiles_finish(s->stream, v, s->lists, n_big, region, s->d_spill, s->h_small[38]);
-    s->n_spilled += s->h_small[38];
+    smx_launch_migrate_tiles_finish(s->stream, v, s->lists, n_big, region, spill, n_spill);
+    s->n_spilled += n_spill;
   }
   if (s->timing) CK(cudaStreamSynchronize(s->stream)); /* attribute the device time to this phase */
   s->n_launches += (n_grow > n_mid + n_big ? 1 : 0) + (n_mid ? 1 : 0) + (n_big ? 3 : 0);
@@ -482,10 +482,10 @@ static void presize_dir(smatrix_t* s, const smx_ops_t* ops) {
    * 2^27 instead of 2^26 entries for config 2, +2 % per step); the grow loop handles those */
   if (used) return;
   const uint64_t m = 1ull << SMX_SKETCH_BITS_LOG;
-  ensure_tmp(s, (size_t)(m / 8), 0);
-  CK(cudaMemsetAsync(s->d_tmp, 0, (size_t)(m / 8), s->stream));
+  uint32_t* bitmap = dbuf_need(s, &s->db.tmp, (size_t)(m / 8));
+  CK(cudaMemsetAsync(bitmap, 0, (size_t)(m / 8), s->stream));
   CK(cudaMemsetAsync(&s->d_ctl->scratch, 0, 8, s->stream));
-  smx_launch_sketch(s->stream, ops->xs, ops->n, s->d_tmp, SMX_SKETCH_BITS_LOG, s->d_ctl);
+  smx_launch_sketch(s->stream, ops->xs, ops->n, bitmap, SMX_SKETCH_BITS_LOG, s->d_ctl);
   s->n_launches += 2;
   read_ctl(s);
   const double zeros = (double)s->h_ctl->scratch;
@@ -524,12 +524,12 @@ static int resize_dir(smatrix_t* s, uint64_t new_cap, int shrink) {
   smx_view_t to = view_for(s, nd, new_cap);
   smx_launch_dir_rehash(s->stream, from, to);
   s->n_launches++;
-  if (shrink) copy_d2h(s, &s->h_small[39], &s->d_ctl->dir_probe_max, 4, s->stream); /* read in the same wait */
+  if (shrink) copy_d2h(s, &s->h_small->probe_max, &s->d_ctl->dir_probe_max, 4, s->stream); /* read in the same wait */
   CK(cudaStreamSynchronize(s->stream));
-  if (shrink && s->h_small[39] >= SMX_DIR_CREATE_STEPS) {
+  if (shrink && s->h_small->probe_max >= SMX_DIR_CREATE_STEPS) {
     if (s->debug)
       fprintf(stderr, "[smatrix] shrink to %llu entries refused: a row would sit %u probe steps from its home\n",
-              (unsigned long long)new_cap, s->h_small[39]);
+              (unsigned long long)new_cap, s->h_small->probe_max);
     if (in_arena) slab_give_back(s, (char*)nd, (size_t)new_cap * sizeof(smx_row_t));
     else CK(cudaFree(nd));
     /* the rehash counted the rows per slice of the new directory: put back the counts of the current one
@@ -651,8 +651,7 @@ static int partition_chunk(smatrix_t* s, smx_ops_t* ops, int api_op, uint32_t* n
    * use all 256 parts as slices if the twins stay empty — else fold neighbouring bins back. */
   const int fine = s->wide_slices && parts_log == 7 && parts_log + shift > s->slice_log + 7;
   ensure_parts(s, n);
-  ensure_tmp(s, 0, 3 * SMX_MAX_PARTS_H * 8);
-  unsigned long long* d_counts = (unsigned long long*)s->d_tmp64; /* up to 2 * SMX_MAX_PARTS_H bins */
+  unsigned long long* d_counts = dbuf_need(s, &s->db.tmp64, 3 * SMX_MAX_PARTS_H * 8); /* up to 2 * SMX_MAX_PARTS_H bins */
   unsigned long long* d_cursors = d_counts + 2 * SMX_MAX_PARTS_H;
   unsigned long long h[2 * SMX_MAX_PARTS_H], cur[SMX_MAX_PARTS_H];
   double t0 = now_ns();
@@ -767,6 +766,16 @@ static int is_device_ptr(const void* p) {
   return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
+/* The arrays of one batched call must be all host or all device memory: returns 1 for device arrays and dies on a
+ * mix.  Each of arrays[0..n) is checked (NULL counts as host memory), `opt` only when it is not NULL. */
+static int batch_on_device(const void* opt, int n, const void* const* arrays) {
+  const int dev = is_device_ptr(arrays[0]);
+  int mixed = opt && is_device_ptr(opt) != dev;
+  for (int i = 1; i < n; i++) mixed |= is_device_ptr(arrays[i]) != dev;
+  if (mixed) smx_die("batch arrays must be all host or all device pointers");
+  return dev;
+}
+
 /* Every entry point runs on the handle's GPU and puts the caller's current device back afterwards,
  * so a process that holds handles on several GPUs (or mixes the library with other CUDA code) never
  * finds its current device changed by a call. */
@@ -788,10 +797,7 @@ static void write_batch(smatrix_t* s, int api_op, const uint32_t* xs, const uint
                         const uint32_t* vs, size_t n) {
   if (n == 0) return;
   enter(s);
-  const int dev = is_device_ptr(xs);
-  if (is_device_ptr(ys) != dev || (vs && is_device_ptr(vs) != dev))
-    smx_die("batch arrays must be all host or all device pointers");
-  if (dev) {
+  if (batch_on_device(vs, 2, (const void*[]){xs, ys})) {
     /* equal chunks: a batch a little over k * chunk_max must not end in a sliver that pays a whole
      * chunk's launches and round trips (the multi-GPU inbox holds 2^26 +- a few thousand ops) */
     const size_t pieces = (n + s->chunk_max - 1) / s->chunk_max;
@@ -850,35 +856,25 @@ void smatrix_set_batch(smatrix_t* self, const uint32_t* xs, const uint32_t* ys,
 }
 
 /* ---- N1: the same batches, returning every op's value as if applied one by one in input order ---- */
-static void ensure_batch_out(smatrix_t* s, uint32_t n) {
-  if (n <= s->bo_cap) return;
-  if (s->bo_cap) {
-    CK(cudaStreamSynchronize(s->stream));
-    cudaFree(s->bo_addr[0]); cudaFree(s->bo_addr[1]); cudaFree(s->bo_idx[0]); cudaFree(s->bo_idx[1]);
-    cudaFree(s->bo_seg); cudaFree(s->bo_tiles); cudaFree(s->bo_out); cudaFree(s->bo_sort);
-  }
-  uint32_t cap = n < 4096 ? 4096 : n;
-  s->bo_addr[0] = (uint64_t*)dmalloc(s, (size_t)cap * 8);
-  s->bo_addr[1] = (uint64_t*)dmalloc(s, (size_t)cap * 8);
-  s->bo_idx[0] = (uint32_t*)dmalloc(s, (size_t)cap * 4);
-  s->bo_idx[1] = (uint32_t*)dmalloc(s, (size_t)cap * 4);
-  s->bo_seg = (uint64_t*)dmalloc(s, (size_t)cap * 8);
-  s->bo_tiles = (uint64_t*)dmalloc(s, ((size_t)smx_scan_scratch_items(cap) + 1) * 8);
-  s->bo_out = (uint32_t*)dmalloc(s, (size_t)cap * 4);
-  s->bo_sort_bytes = smx_batch_out_sort_bytes(cap);
-  s->bo_sort = dmalloc(s, s->bo_sort_bytes);
-  s->bo_cap = cap;
+/* the *_batch_out launches for the ops of a chunk just applied; their scratch is sized for at least 4096 ops */
+static void batch_out(smatrix_t* s, smx_ops_t ops, int api_op, uint32_t* d_out) {
+  const size_t cap = ops.n < 4096 ? 4096 : ops.n;
+  smx_dbuf_t* sort = &s->db.bo_sort;
+  dbuf_need(s, sort, smx_batch_out_sort_bytes((uint32_t)cap));
+  smx_launch_batch_out(s->stream, view_of(s), ops, api_op == 2 ? SMX_OP_SETZERO : api_op, d_out,
+                       dbuf_need(s, &s->db.bo_addr[0], cap * 8), dbuf_need(s, &s->db.bo_addr[1], cap * 8),
+                       dbuf_need(s, &s->db.bo_idx[0], cap * 4), dbuf_need(s, &s->db.bo_idx[1], cap * 4),
+                       dbuf_need(s, &s->db.bo_seg, cap * 8),
+                       dbuf_need(s, &s->db.bo_tiles, ((size_t)smx_scan_scratch_items((uint32_t)cap) + 1) * 8),
+                       sort->p, sort->bytes);
 }
 
 static void chunk_out(smatrix_t* s, int api_op, const uint32_t* d_xs, const uint32_t* d_ys, const uint32_t* d_vs,
                       uint32_t n, uint32_t* d_out) {
   process_chunk(s, api_op, d_xs, d_ys, d_vs, n);
-  ensure_batch_out(s, n);
   smx_ops_t ops;
   ops.xs = d_xs; ops.ys = d_ys; ops.vs = d_vs; ops.idx = NULL; ops.v_const = 1u; ops.n = n;
-  smx_launch_batch_out(s->stream, view_of(s), ops, api_op == 2 ? SMX_OP_SETZERO : api_op, d_out, s->bo_addr[0],
-                       s->bo_addr[1], s->bo_idx[0], s->bo_idx[1], s->bo_seg, s->bo_tiles, s->bo_sort,
-                       s->bo_sort_bytes);
+  batch_out(s, ops, api_op, d_out);
   s->n_launches += 7;
 }
 
@@ -887,10 +883,7 @@ static void write_batch_out(smatrix_t* s, int api_op, const uint32_t* xs, const 
   if (n == 0) return;
   if (!out) smx_die("batch_out: out must not be NULL");
   enter(s);
-  const int dev = is_device_ptr(xs);
-  if (is_device_ptr(ys) != dev || (vs && is_device_ptr(vs) != dev) || is_device_ptr(out) != dev)
-    smx_die("batch arrays must be all host or all device pointers");
-  if (dev) {
+  if (batch_on_device(vs, 3, (const void*[]){xs, ys, out})) {
     for (size_t off = 0; off < n; off += s->chunk_max) {
       const uint32_t len = (uint32_t)((n - off < s->chunk_max) ? n - off : s->chunk_max);
       chunk_out(s, api_op, xs + off, ys + off, vs ? vs + off : NULL, len, out + off);
@@ -900,14 +893,14 @@ static void write_batch_out(smatrix_t* s, int api_op, const uint32_t* xs, const 
     uint32_t step = s->chunk_max < s->stage_max ? s->chunk_max : s->stage_max;
     if (n < step) step = (uint32_t)n;
     ensure_stage(s, step);
-    ensure_batch_out(s, step);
+    uint32_t* d_out = dbuf_need(s, &s->db.bo_out, (size_t)step * 4);
     const uint32_t* src[3] = {xs, ys, vs};
     for (size_t off = 0; off < n; off += step) {
       const uint32_t len = (uint32_t)((n - off < step) ? n - off : step);
       for (int a = 0; a < 3; a++)
         if (src[a]) copy_h2d(s, s->stage[0][a], src[a] + off, (size_t)len * 4, s->stream);
-      chunk_out(s, api_op, s->stage[0][0], s->stage[0][1], vs ? s->stage[0][2] : NULL, len, s->bo_out);
-      copy_d2h(s, out + off, s->bo_out, (size_t)len * 4, s->stream);
+      chunk_out(s, api_op, s->stage[0][0], s->stage[0][1], vs ? s->stage[0][2] : NULL, len, d_out);
+      copy_d2h(s, out + off, d_out, (size_t)len * 4, s->stream);
       CK(cudaStreamSynchronize(s->stream));
     }
   }
@@ -934,10 +927,7 @@ void smatrix_b200_apply_ordered(smatrix_t* s, int op, const uint32_t* d_xs, cons
   if (op < 0 || op > 2) smx_die("apply_ordered: op must be 0 (incr), 1 (decr) or 2 (set)");
   enter(s);
   if (n > (1u << 30)) smx_die("apply_ordered: at most 2^30 ops per call (one chunk)");
-  const int dev = is_device_ptr(d_xs);
-  if (is_device_ptr(d_ys) != dev || (d_vals && is_device_ptr(d_vals) != dev) || is_device_ptr(d_ords) != dev)
-    smx_die("batch arrays must be all host or all device pointers");
-  if (dev) {
+  if (batch_on_device(d_vals, 3, (const void*[]){d_xs, d_ys, d_ords})) {
     process_chunk_ordered(s, op, d_xs, d_ys, d_vals, d_ords, (uint32_t)n);
     CK(cudaStreamSynchronize(s->stream));
   } else { /* host arrays: one staged copy (this entry point is meant for device-resident batches) */
@@ -965,11 +955,9 @@ void smatrix_b200_apply_ordered_out(smatrix_t* s, int op, const uint32_t* d_xs, 
   if (n > (1u << 30)) smx_die("apply_ordered_out: at most 2^30 ops per call (one chunk)");
   enter(s);
   process_chunk_ordered(s, op, d_xs, d_ys, d_vals, d_ords, (uint32_t)n);
-  ensure_batch_out(s, (uint32_t)n);
   smx_ops_t ops;
   ops.xs = d_xs; ops.ys = d_ys; ops.vs = d_vals; ops.idx = d_ords; ops.v_const = 1u; ops.n = (uint32_t)n;
-  smx_launch_batch_out(s->stream, view_of(s), ops, op == 2 ? SMX_OP_SETZERO : op, d_out, s->bo_addr[0], s->bo_addr[1],
-                       s->bo_idx[0], s->bo_idx[1], s->bo_seg, s->bo_tiles, s->bo_sort, s->bo_sort_bytes);
+  batch_out(s, ops, op, d_out);
   s->n_launches += 9;
   CK(cudaStreamSynchronize(s->stream));
   CK(cudaGetLastError());
@@ -1026,8 +1014,7 @@ static void get_sliced(smatrix_t* s, const uint32_t* d_xs, const uint32_t* d_ys,
   get_geometry(s, &parts_log, &shift);
   const uint32_t slices = 1u << parts_log, mask = (uint32_t)(s->dir_cap - 1);
   ensure_parts(s, n);
-  ensure_tmp(s, 0, 3 * SMX_MAX_PARTS_H * 8);
-  unsigned long long* d_counts = (unsigned long long*)s->d_tmp64;
+  unsigned long long* d_counts = dbuf_need(s, &s->db.tmp64, 3 * SMX_MAX_PARTS_H * 8);
   unsigned long long* d_cursors = d_counts + 2 * SMX_MAX_PARTS_H;
   CK(cudaMemsetAsync(d_counts, 0, slices * 8, s->stream));
   smx_launch_partition_count(s->stream, d_xs, NULL, n, slices, mask, shift, 0, d_counts);
@@ -1046,10 +1033,7 @@ void smatrix_get_batch(smatrix_t* s, const uint32_t* xs, const uint32_t* ys, siz
                        uint32_t* out) {
   if (n == 0) return;
   enter(s);
-  const int dev = is_device_ptr(xs);
-  if (is_device_ptr(ys) != dev || is_device_ptr(out) != dev)
-    smx_die("batch arrays must be all host or all device pointers");
-  if (dev) {
+  if (batch_on_device(NULL, 3, (const void*[]){xs, ys, out})) {
     for (size_t off = 0; off < n; off += READ_STEP) {
       const uint32_t len = (uint32_t)((n - off < READ_STEP) ? n - off : READ_STEP);
       timed_begin(s);
@@ -1100,17 +1084,16 @@ void smatrix_get_batch(smatrix_t* s, const uint32_t* xs, const uint32_t* ys, siz
 void smatrix_rowlen_batch(smatrix_t* s, const uint32_t* xs, size_t n, uint32_t* out) {
   if (n == 0) return;
   enter(s);
-  const int dev = is_device_ptr(xs);
-  if (is_device_ptr(out) != dev) smx_die("batch arrays must be all host or all device pointers");
+  const int dev = batch_on_device(NULL, 2, (const void*[]){xs, out});
   for (size_t off = 0; off < n; off += READ_STEP) {
     const uint32_t len = (uint32_t)((n - off < READ_STEP) ? n - off : READ_STEP);
     if (dev) {
       smx_launch_rowlen(s->stream, view_of(s), xs + off, len, out + off);
     } else {
-      ensure_tmp(s, (size_t)len * 8, 0);
-      copy_h2d(s, s->d_tmp, xs + off, (size_t)len * 4, s->stream);
-      smx_launch_rowlen(s->stream, view_of(s), s->d_tmp, len, s->d_tmp + len);
-      copy_d2h(s, out + off, s->d_tmp + len, (size_t)len * 4, s->stream);
+      uint32_t* tmp = dbuf_need(s, &s->db.tmp, (size_t)len * 8);
+      copy_h2d(s, tmp, xs + off, (size_t)len * 4, s->stream);
+      smx_launch_rowlen(s->stream, view_of(s), tmp, len, tmp + len);
+      copy_d2h(s, out + off, tmp + len, (size_t)len * 4, s->stream);
     }
     s->n_launches++;
     CK(cudaStreamSynchronize(s->stream));
@@ -1119,189 +1102,156 @@ void smatrix_rowlen_batch(smatrix_t* s, const uint32_t* xs, size_t n, uint32_t* 
   leave(s);
 }
 
-/* counts + scan for rows xs[0..n) (device array); leaves offsets in d_tmp64[0..n], the list of
- * big rows in s->d_big[0..s->n_big) and zeroed per-row cursors in s->d_cursors; returns total */
-/* scratch of the getrow plan for n rows: info (u64), list of big rows (u32), output cursors (u32) + counter */
-static uint32_t* ensure_rowplan(smatrix_t* s, uint32_t n) {
-  const size_t need = (size_t)n * 16 + 64;
-  if (need > s->d_big_bytes) {
-    if (s->d_info) { CK(cudaStreamSynchronize(s->stream)); cudaFree(s->d_info); }
-    s->d_big_bytes = need + need / 4 + 4096;
-    s->d_info = (uint64_t*)dmalloc(s, s->d_big_bytes);
-  }
-  s->d_big = (uint32_t*)(s->d_info + n);
-  s->d_cursors = s->d_big + n;
-  CK(cudaMemsetAsync(s->d_cursors, 0, (size_t)n * 4 + 8, s->stream));
-  return s->d_cursors + n; /* one counter word after the cursors */
+/* scratch of the getrow plan for n rows: per-row directory index | caplog << 32 (u64, k_row_counts), row counts,
+ * the list of big rows and the per-row output cursors (u32), and the big-row counter; cursors and counter zeroed */
+typedef struct { uint64_t* info; uint32_t *counts, *big, *cursors, *n_big; } smx_rowplan_t;
+static smx_rowplan_t rowplan(smatrix_t* s, uint32_t n) {
+  smx_rowplan_t p;
+  p.info = dbuf_need(s, &s->db.plan, (size_t)n * 20 + 64);
+  p.counts = (uint32_t*)(p.info + n);
+  p.big = p.counts + n;
+  p.cursors = p.big + n;
+  p.n_big = p.cursors + n;
+  CK(cudaMemsetAsync(p.cursors, 0, (size_t)n * 4 + 8, s->stream));
+  return p;
 }
 
-static uint64_t plan_rows(smatrix_t* s, const uint32_t* d_xs, uint32_t n, uint32_t* d_counts) {
-  uint32_t* d_nbig = ensure_rowplan(s, n);
-  smx_launch_row_counts(s->stream, view_of(s), d_xs, n, d_counts, s->d_info, s->d_big, d_nbig);
-  smx_launch_scan(s->stream, d_counts, n, 0, s->d_tmp64, s->d_tmp64 + (size_t)n + 1);
+typedef struct {
+  uint64_t total;      /* pairs of all the rows */
+  const uint32_t* ids; /* the row ids, on the device */
+  uint64_t* offsets;   /* [n + 1], in db.tmp64 */
+  uint32_t* pairs;     /* where the pairs were filled; NULL if they were not */
+} smx_rows_t;
+
+/* The start of every read that returns whole rows: rows ids[0..n) (host ids go up through db.tmp first) are
+ * counted and scanned, and when 0 < total <= room their pairs are filled into d_pairs, or into db.rows when d_pairs
+ * is NULL (the fill is timed for smatrix_getrow_batch's kernel time). */
+static smx_rows_t gather_rows(smatrix_t* s, const uint32_t* ids, int ids_on_device, uint32_t n, uint64_t room,
+                              uint32_t* d_pairs) {
+  smx_rows_t r;
+  r.ids = ids;
+  if (!ids_on_device) {
+    uint32_t* d_ids = dbuf_need(s, &s->db.tmp, (size_t)n * 4);
+    copy_h2d(s, d_ids, ids, (size_t)n * 4, s->stream);
+    r.ids = d_ids;
+  }
+  r.offsets = dbuf_need(s, &s->db.tmp64, ((size_t)n + 1 + smx_scan_scratch_items(n)) * 8);
+  const smx_rowplan_t p = rowplan(s, n);
+  smx_launch_row_counts(s->stream, view_of(s), r.ids, n, p.counts, p.info, p.big, p.n_big);
+  smx_launch_scan(s->stream, p.counts, n, 0, r.offsets, r.offsets + (size_t)n + 1);
   s->n_launches += 4;
-  uint64_t total = 0;
-  copy_d2h(s, &s->h_small[32], s->d_tmp64 + n, 8, s->stream);
-  copy_d2h(s, &s->h_small[34], d_nbig, 4, s->stream);
+  copy_d2h(s, &s->h_small->row_total, r.offsets + n, 8, s->stream);
+  copy_d2h(s, &s->h_small->n_big_rows, p.n_big, 4, s->stream);
   CK(cudaStreamSynchronize(s->stream));
-  memcpy(&total, &s->h_small[32], 8);
-  s->n_big_rows = s->h_small[34];
-  return total;
+  r.total = s->h_small->row_total;
+  r.pairs = NULL;
+  if (r.total && r.total <= room) {
+    r.pairs = d_pairs ? d_pairs : dbuf_need(s, &s->db.rows, (size_t)r.total * 8);
+    timed_begin(s);
+    smx_launch_getrow_fill(s->stream, view_of(s), p.info, n, r.offsets, 0, r.pairs, p.big, s->h_small->n_big_rows,
+                           p.cursors);
+    timed_end(s);
+    s->n_launches++;
+  }
+  return r;
+}
+
+/* a call for no rows still writes offsets[0] = 0 */
+static uint64_t no_rows(smatrix_t* s, uint64_t* offsets) {
+  if (offsets) {
+    const uint64_t zero = 0;
+    enter(s);
+    CK(cudaMemcpy(offsets, &zero, 8, cudaMemcpyDefault));
+    leave(s);
+  }
+  return 0;
 }
 
 uint64_t smatrix_getrow_batch(smatrix_t* s, const uint32_t* xs, size_t n, uint64_t* offsets,
                               uint32_t* pairs, uint64_t pairs_cap) {
-  if (n == 0) {
-    if (offsets) {
-      uint64_t zero = 0;
-      enter(s);
-      CK(cudaMemcpy(offsets, &zero, 8, cudaMemcpyDefault));
-      leave(s);
-    }
-    return 0;
-  }
+  if (n == 0) return no_rows(s, offsets);
   if (n >= 0xFFFFFFFFull) smx_die("getrow_batch: too many rows in one call");
   enter(s);
   const uint32_t nn = (uint32_t)n;
-  const int dev = is_device_ptr(xs);
-  const uint32_t tiles = smx_scan_scratch_items(nn);
-  ensure_tmp(s, (size_t)nn * 8, ((size_t)nn + 1 + tiles) * 8);
-  const uint32_t* d_xs = xs;
-  uint32_t* d_counts = s->d_tmp + nn;
-  if (!dev) {
-    copy_h2d(s, s->d_tmp, xs, (size_t)nn * 4, s->stream);
-    d_xs = s->d_tmp;
-  }
-  const uint64_t total = plan_rows(s, d_xs, nn, d_counts);
+  const int pairs_dev = is_device_ptr(pairs);
+  const smx_rows_t r = gather_rows(s, xs, is_device_ptr(xs), nn, pairs ? pairs_cap : 0, pairs_dev ? pairs : NULL);
   if (offsets) {
-    CK(cudaMemcpyAsync(offsets, s->d_tmp64, ((size_t)nn + 1) * 8, cudaMemcpyDefault, s->stream));
+    CK(cudaMemcpyAsync(offsets, r.offsets, ((size_t)nn + 1) * 8, cudaMemcpyDefault, s->stream));
     if (!is_device_ptr(offsets)) s->d2h_bytes += ((size_t)nn + 1) * 8;
   }
-  int filled = 0;
-  if (pairs && total <= pairs_cap && total > 0) {
-    filled = 1;
-    if (is_device_ptr(pairs)) {
-      timed_begin(s);
-      smx_launch_getrow_fill(s->stream, view_of(s), s->d_info, nn, s->d_tmp64, 0, pairs, s->d_big, s->n_big_rows, s->d_cursors);
-      timed_end(s);
-      s->n_launches++;
-    } else {
-      if (total * 8 > s->d_rowbuf_bytes) { /* grows with slack: batches of similar size must not re-allocate */
-        if (s->d_rowbuf) cudaFree(s->d_rowbuf);
-        s->d_rowbuf_bytes = (size_t)total * 8 + (size_t)total * 2 + 4096;
-        s->d_rowbuf = (uint32_t*)dmalloc(s, s->d_rowbuf_bytes);
-      }
-      timed_begin(s);
-      smx_launch_getrow_fill(s->stream, view_of(s), s->d_info, nn, s->d_tmp64, 0, s->d_rowbuf, s->d_big, s->n_big_rows, s->d_cursors);
-      timed_end(s);
-      s->n_launches++;
-      copy_d2h(s, pairs, s->d_rowbuf, (size_t)total * 8, s->stream);
-    }
-  }
+  if (r.pairs && !pairs_dev) copy_d2h(s, pairs, r.pairs, (size_t)r.total * 8, s->stream);
   CK(cudaStreamSynchronize(s->stream));
-  if (filled) timed_collect(s);
+  if (r.pairs) timed_collect(s);
   CK(cudaGetLastError());
   leave(s);
-  return total;
+  return r.total;
 }
 
 /* SURVEY.md 8f N4: neighbours + cosine scores for a batch of items (examples/cf_recommender.c:50-86) */
 uint64_t smatrix_cf_neighbors_batch(smatrix_t* s, const uint32_t* items, size_t n, uint64_t* offsets,
                                     uint32_t* ids, double* scores, uint64_t cap) {
-  if (n == 0) {
-    if (offsets) { uint64_t zero = 0; enter(s); CK(cudaMemcpy(offsets, &zero, 8, cudaMemcpyDefault)); leave(s); }
-    return 0;
-  }
+  if (n == 0) return no_rows(s, offsets);
   if (n >= 0xFFFFFFFFull) smx_die("cf_neighbors_batch: too many items in one call");
   enter(s);
   const uint32_t nn = (uint32_t)n;
-  const int dev = is_device_ptr(items);
-  const uint32_t tiles = smx_scan_scratch_items(nn);
-  ensure_tmp(s, (size_t)nn * 8, ((size_t)nn + 1 + tiles) * 8);
-  const uint32_t* d_items = items;
-  if (!dev) {
-    copy_h2d(s, s->d_tmp, items, (size_t)nn * 4, s->stream);
-    d_items = s->d_tmp;
-  }
-  const uint64_t total = plan_rows(s, d_items, nn, s->d_tmp + nn);
-  if (offsets) CK(cudaMemcpyAsync(offsets, s->d_tmp64, ((size_t)nn + 1) * 8, cudaMemcpyDefault, s->stream));
-  if (ids && scores && total <= cap && total > 0) {
-    if (total * 8 > s->d_rowbuf_bytes) {
-      if (s->d_rowbuf) cudaFree(s->d_rowbuf);
-      s->d_rowbuf_bytes = (size_t)total * 8;
-      s->d_rowbuf = (uint32_t*)dmalloc(s, s->d_rowbuf_bytes);
-    }
-    smx_launch_getrow_fill(s->stream, view_of(s), s->d_info, nn, s->d_tmp64, 0, s->d_rowbuf, s->d_big, s->n_big_rows, s->d_cursors);
-    const int out_dev = is_device_ptr(ids);
-    if (is_device_ptr(scores) != out_dev) smx_die("batch arrays must be all host or all device pointers");
+  const smx_rows_t r = gather_rows(s, items, is_device_ptr(items), nn, (ids && scores) ? cap : 0, NULL);
+  if (offsets) CK(cudaMemcpyAsync(offsets, r.offsets, ((size_t)nn + 1) * 8, cudaMemcpyDefault, s->stream));
+  if (r.pairs) {
+    const int out_dev = batch_on_device(NULL, 2, (const void*[]){ids, scores});
     uint32_t* d_ids = ids;
     double* d_scores = scores;
-    void* tmp = NULL;
     if (!out_dev) {
-      tmp = dmalloc(s, (size_t)total * 12 + 64);
-      d_scores = (double*)tmp;
-      d_ids = (uint32_t*)((char*)tmp + (size_t)total * 8);
+      char* o = dbuf_need(s, &s->db.host_out, (size_t)r.total * 12 + 64);
+      d_scores = (double*)o;
+      d_ids = (uint32_t*)(o + (size_t)r.total * 8);
     }
-    smx_launch_cf_scores(s->stream, view_of(s), d_items, nn, s->d_tmp64, s->d_rowbuf, d_ids, d_scores);
-    s->n_launches += 2;
+    smx_launch_cf_scores(s->stream, view_of(s), r.ids, nn, r.offsets, r.pairs, d_ids, d_scores);
+    s->n_launches++;
     if (!out_dev) {
-      copy_d2h(s, ids, d_ids, (size_t)total * 4, s->stream);
-      copy_d2h(s, scores, d_scores, (size_t)total * 8, s->stream);
-      CK(cudaStreamSynchronize(s->stream));
-      CK(cudaFree(tmp));
+      copy_d2h(s, ids, d_ids, (size_t)r.total * 4, s->stream);
+      copy_d2h(s, scores, d_scores, (size_t)r.total * 8, s->stream);
     }
   }
   CK(cudaStreamSynchronize(s->stream));
   CK(cudaGetLastError());
   leave(s);
-  return total;
+  return r.total;
 }
 
 /* ------------------------------------------------------------------------------ top-k */
-/* top-k scratch buffer `b` (an index into tk_bytes) of at least `need` bytes; grows with slack */
-static void* tk_buf(smatrix_t* s, void** p, int b, size_t need) {
-  if (need > s->tk_bytes[b]) {
-    if (*p) { CK(cudaStreamSynchronize(s->stream)); cudaFree(*p); }
-    s->tk_bytes[b] = need + need / 4 + 4096;
-    *p = dmalloc(s, s->tk_bytes[b]);
-  }
-  return *p;
-}
-
 /* the selection of smatrix_b200_topk_segments on device arrays, enqueued on s->stream (synchronises to read
  * the number of big segments and, per digit pass, how many are still selecting) */
 static void topk_run(smatrix_t* s, uint32_t n, const uint64_t* d_off, const uint32_t* d_ids, const double* d_scores,
                      uint32_t k, uint32_t* d_counts, uint32_t* d_oids, double* d_oscores) {
   if (!n) return;
-  uint32_t* ctl = (uint32_t*)tk_buf(s, (void**)&s->tk_ctl, 0, (size_t)n * 4 + 64);
+  uint32_t* ctl = dbuf_need(s, &s->db.tk_ctl, (size_t)n * 4 + 64);
   uint32_t* big_list = ctl + 16;
   CK(cudaMemsetAsync(ctl, 0, 64, s->stream));
   smx_launch_topk_classify(s->stream, n, d_off, big_list, ctl);
-  copy_d2h(s, &s->h_small[40], ctl, 16, s->stream);
+  copy_d2h(s, &s->h_small->topk, ctl, 16, s->stream);
   smx_launch_topk_small(s->stream, n, d_off, d_ids, d_scores, k, d_counts, d_oids, d_oscores);
   s->n_launches += 3;
   CK(cudaStreamSynchronize(s->stream));
-  const uint32_t n_big = s->h_small[40];
+  const uint32_t n_big = s->h_small->topk.n_big;
   if (!n_big) return;
-  uint64_t big_pairs;
-  memcpy(&big_pairs, &s->h_small[42], 8);
-  void* big = tk_buf(s, &s->tk_big, 2, smx_topk_big_bytes(n_big));
-  tk_buf(s, (void**)&s->tk_cids, 3, (size_t)big_pairs * 4);
-  tk_buf(s, (void**)&s->tk_cscores, 4, (size_t)big_pairs * 8);
+  const uint64_t big_pairs = s->h_small->topk.big_pairs;
+  void* big = dbuf_need(s, &s->db.tk_big, smx_topk_big_bytes(n_big));
+  uint32_t* cids = dbuf_need(s, &s->db.tk_cids, (size_t)big_pairs * 4);
+  double* cscores = dbuf_need(s, &s->db.tk_cscores, (size_t)big_pairs * 8);
   CK(cudaMemsetAsync(big, 0, smx_topk_big_bytes(n_big), s->stream));
   smx_launch_topk_init(s->stream, big_list, n_big, d_off, big, ctl);
   s->n_launches++;
   for (uint32_t pass = 1;; pass++) { /* every pass fixes one more digit of the k-th key */
     if (pass > smx_topk_max_passes()) smx_die("topk: the select did not end after %u digit passes", pass - 1);
     CK(cudaMemsetAsync(ctl + 1, 0, 4, s->stream));
-    smx_launch_topk_pass(s->stream, big, n_big, k, d_ids, d_scores, s->tk_cids, s->tk_cscores, ctl);
-    copy_d2h(s, &s->h_small[44], ctl + 1, 4, s->stream);
+    smx_launch_topk_pass(s->stream, big, n_big, k, d_ids, d_scores, cids, cscores, ctl);
+    copy_d2h(s, &s->h_small->topk.active, ctl + 1, 4, s->stream);
     CK(cudaStreamSynchronize(s->stream));
     s->n_launches += 3;
     s->n_topk_passes++;
-    if (!s->h_small[44]) break;
+    if (!s->h_small->topk.active) break;
   }
-  smx_launch_topk_finish(s->stream, big, n_big, s->tk_cids, s->tk_cscores, k, d_counts, d_oids, d_oscores);
+  smx_launch_topk_finish(s->stream, big, n_big, cids, cscores, k, d_counts, d_oids, d_oscores);
   s->n_launches++;
   s->n_topk_big += n_big;
 }
@@ -1327,53 +1277,44 @@ void smatrix_cf_topk_batch(smatrix_t* s, const uint32_t* items, size_t n, uint32
   if (n >= 0xFFFFFFFFull) smx_die("cf_topk_batch: too many items in one call");
   if (!n) return;
   enter(s);
-  const int out_dev = is_device_ptr(counts);
-  if (is_device_ptr(ids) != out_dev || is_device_ptr(scores) != out_dev)
-    smx_die("batch arrays must be all host or all device pointers");
+  const int out_dev = batch_on_device(NULL, 3, (const void*[]){counts, ids, scores});
   const uint32_t nn = (uint32_t)n;
-  const uint32_t tiles = smx_scan_scratch_items(nn);
-  ensure_tmp(s, (size_t)nn * 8, ((size_t)nn + 1 + tiles) * 8);
+  uint32_t* tmp = dbuf_need(s, &s->db.tmp, (size_t)nn * 8);
+  uint64_t* tmp64 = dbuf_need(s, &s->db.tmp64, ((size_t)nn + 1 + smx_scan_scratch_items(nn)) * 8);
   const uint32_t* d_items = items;
   if (!is_device_ptr(items)) {
-    copy_h2d(s, s->d_tmp, items, (size_t)nn * 4, s->stream);
-    d_items = s->d_tmp;
+    copy_h2d(s, tmp, items, (size_t)nn * 4, s->stream);
+    d_items = tmp;
   }
-  uint32_t* d_cnt = s->d_tmp + nn;
+  uint32_t* d_cnt = tmp + nn;
   /* the row lengths of the whole call decide where the pieces end */
-  uint64_t* d_all = (uint64_t*)tk_buf(s, (void**)&s->tk_off, 1, ((size_t)nn + 1) * 8);
+  uint64_t* d_all = dbuf_need(s, &s->db.tk_off, ((size_t)nn + 1) * 8);
   smx_launch_row_counts(s->stream, view_of(s), d_items, nn, d_cnt, NULL, NULL, NULL);
-  smx_launch_scan(s->stream, d_cnt, nn, 0, d_all, s->d_tmp64 + (size_t)nn + 1);
+  smx_launch_scan(s->stream, d_cnt, nn, 0, d_all, tmp64 + (size_t)nn + 1);
   s->n_launches += 4;
   for (uint32_t lo = 0, hi; lo < nn; lo = hi) {
-    smx_launch_topk_cut(s->stream, d_all, nn, lo, s->topk_pairs, s->d_small);
-    copy_d2h(s, &s->h_small[45], s->d_small, 4, s->stream);
+    smx_launch_topk_cut(s->stream, d_all, nn, lo, s->topk_pairs, s->d_small + DS_OUT);
+    copy_d2h(s, &s->h_small->topk_cut, s->d_small + DS_OUT, 4, s->stream);
     CK(cudaStreamSynchronize(s->stream));
-    hi = s->h_small[45];
+    hi = s->h_small->topk_cut;
     const uint32_t np = hi - lo;
-    const uint64_t total = plan_rows(s, d_items + lo, np, d_cnt); /* the piece's offsets: d_tmp64[0..np] */
-    tk_buf(s, (void**)&s->tk_ids, 5, (size_t)total * 4);
-    tk_buf(s, (void**)&s->tk_scores, 6, (size_t)total * 8);
-    if (total) {
-      if (total * 8 > s->d_rowbuf_bytes) {
-        if (s->d_rowbuf) cudaFree(s->d_rowbuf);
-        s->d_rowbuf_bytes = (size_t)total * 8 + (size_t)total * 2 + 4096;
-        s->d_rowbuf = (uint32_t*)dmalloc(s, s->d_rowbuf_bytes);
-      }
-      smx_launch_getrow_fill(s->stream, view_of(s), s->d_info, np, s->d_tmp64, 0, s->d_rowbuf, s->d_big, s->n_big_rows,
-                             s->d_cursors);
-      smx_launch_cf_scores(s->stream, view_of(s), d_items + lo, np, s->d_tmp64, s->d_rowbuf, s->tk_ids, s->tk_scores);
-      s->n_launches += 2;
+    const smx_rows_t r = gather_rows(s, d_items + lo, 1, np, UINT64_MAX, NULL);
+    uint32_t* p_ids = dbuf_need(s, &s->db.tk_ids, (size_t)r.total * 4);
+    double* p_scores = dbuf_need(s, &s->db.tk_scores, (size_t)r.total * 8);
+    if (r.total) {
+      smx_launch_cf_scores(s->stream, view_of(s), r.ids, np, r.offsets, r.pairs, p_ids, p_scores);
+      s->n_launches++;
     }
     uint32_t* oc = counts + lo;
     uint32_t* oi = ids + (size_t)lo * k;
     double* os = scores + (size_t)lo * k;
     if (!out_dev) {
-      char* o = (char*)tk_buf(s, &s->tk_out, 7, (size_t)np * (12ull * k + 4));
+      char* o = dbuf_need(s, &s->db.host_out, (size_t)np * (12ull * k + 4));
       os = (double*)o;
       oi = (uint32_t*)(o + (size_t)np * k * 8);
       oc = oi + (size_t)np * k;
     }
-    topk_run(s, np, s->d_tmp64, s->tk_ids, s->tk_scores, k, oc, oi, os);
+    topk_run(s, np, r.offsets, p_ids, p_scores, k, oc, oi, os);
     if (!out_dev) {
       copy_d2h(s, counts + lo, oc, (size_t)np * 4, s->stream);
       copy_d2h(s, ids + (size_t)lo * k, oi, (size_t)np * k * 4, s->stream);
@@ -1386,16 +1327,22 @@ void smatrix_cf_topk_batch(smatrix_t* s, const uint32_t* items, size_t n, uint32
 }
 
 /* ------------------------------------------------------------------------------ single ops */
+/* the answer of a single op, d_small[DS_OUT] */
+static uint32_t single_answer(smatrix_t* s) {
+  copy_d2h(s, &s->h_small->answer, s->d_small + DS_OUT, 4, s->stream);
+  CK(cudaStreamSynchronize(s->stream));
+  return s->h_small->answer;
+}
+
 static uint32_t single_write(smatrix_t* s, int api_op, uint32_t x, uint32_t y, uint32_t v) {
   enter(s);
-  s->h_small[0] = x; s->h_small[1] = y; s->h_small[2] = v;
-  copy_h2d(s, s->d_small, s->h_small, 12, s->stream);
-  process_chunk(s, api_op, s->d_small, s->d_small + 1, s->d_small + 2, 1);
-  smx_launch_get(s->stream, view_of(s), s->d_small, s->d_small + 1, 1, s->d_small + 3);
+  uint32_t* d = s->d_small;
+  s->h_small->op[0] = x; s->h_small->op[1] = y; s->h_small->op[2] = v;
+  copy_h2d(s, d + DS_X, s->h_small->op, 12, s->stream);
+  process_chunk(s, api_op, d + DS_X, d + DS_Y, d + DS_V, 1);
+  smx_launch_get(s->stream, view_of(s), d + DS_X, d + DS_Y, 1, d + DS_OUT);
   s->n_launches++;
-  copy_d2h(s, &s->h_small[3], s->d_small + 3, 4, s->stream);
-  CK(cudaStreamSynchronize(s->stream));
-  const uint32_t r = s->h_small[3];
+  const uint32_t r = single_answer(s);
   leave(s);
   return r;
 }
@@ -1412,49 +1359,38 @@ uint32_t smatrix_decr(smatrix_t* self, uint32_t x, uint32_t y, uint32_t value) {
 
 uint32_t smatrix_get(smatrix_t* s, uint32_t x, uint32_t y) {
   enter(s);
-  s->h_small[0] = x; s->h_small[1] = y;
-  copy_h2d(s, s->d_small, s->h_small, 8, s->stream);
-  smx_launch_get(s->stream, view_of(s), s->d_small, s->d_small + 1, 1, s->d_small + 3);
+  uint32_t* d = s->d_small;
+  s->h_small->op[0] = x; s->h_small->op[1] = y;
+  copy_h2d(s, d + DS_X, s->h_small->op, 8, s->stream);
+  smx_launch_get(s->stream, view_of(s), d + DS_X, d + DS_Y, 1, d + DS_OUT);
   s->n_launches++;
-  copy_d2h(s, &s->h_small[3], s->d_small + 3, 4, s->stream);
-  CK(cudaStreamSynchronize(s->stream));
-  const uint32_t r = s->h_small[3];
+  const uint32_t r = single_answer(s);
   leave(s);
   return r;
 }
 
 uint32_t smatrix_rowlen(smatrix_t* s, uint32_t x) {
   enter(s);
-  s->h_small[0] = x;
-  copy_h2d(s, s->d_small, s->h_small, 4, s->stream);
-  smx_launch_rowlen(s->stream, view_of(s), s->d_small, 1, s->d_small + 3);
+  uint32_t* d = s->d_small;
+  s->h_small->op[0] = x;
+  copy_h2d(s, d + DS_X, s->h_small->op, 4, s->stream);
+  smx_launch_rowlen(s->stream, view_of(s), d + DS_X, 1, d + DS_OUT);
   s->n_launches++;
-  copy_d2h(s, &s->h_small[3], s->d_small + 3, 4, s->stream);
-  CK(cudaStreamSynchronize(s->stream));
-  const uint32_t r = s->h_small[3];
+  const uint32_t r = single_answer(s);
   leave(s);
   return r;
 }
 
 uint32_t smatrix_getrow(smatrix_t* s, uint32_t x, uint32_t* ret, size_t ret_len) {
   enter(s);
-  s->h_small[0] = x;
-  copy_h2d(s, s->d_small, s->h_small, 4, s->stream);
-  ensure_tmp(s, 64, (2 + smx_scan_scratch_items(1)) * 8);
-  const uint64_t total = plan_rows(s, s->d_small, 1, s->d_small + 4);
+  s->h_small->op[0] = x;
+  const smx_rows_t r = gather_rows(s, s->h_small->op, 0, 1, UINT64_MAX, NULL);
   /* reference loop (src/smatrix.c:196-205): emit, then stop once num*8 >= ret_len */
   uint64_t room = (ret_len + 7) / 8;
   if (room < 1) room = 1;
-  const uint64_t n = total < room ? total : room;
+  const uint64_t n = r.total < room ? r.total : room;
   if (n > 0) {
-    if (total * 8 > s->d_rowbuf_bytes) {
-      if (s->d_rowbuf) cudaFree(s->d_rowbuf);
-      s->d_rowbuf_bytes = (size_t)total * 8;
-      s->d_rowbuf = (uint32_t*)dmalloc(s, s->d_rowbuf_bytes);
-    }
-    smx_launch_getrow_fill(s->stream, view_of(s), s->d_info, 1, s->d_tmp64, 0, s->d_rowbuf, s->d_big, s->n_big_rows, s->d_cursors);
-    s->n_launches++;
-    CK(cudaMemcpyAsync(ret, s->d_rowbuf, (size_t)n * 8, cudaMemcpyDefault, s->stream));
+    CK(cudaMemcpyAsync(ret, r.pairs, (size_t)n * 8, cudaMemcpyDefault, s->stream));
     CK(cudaStreamSynchronize(s->stream));
   }
   leave(s);
@@ -1539,35 +1475,29 @@ static int snapshot_save(smatrix_t* s) {
   for (uint64_t first = 0; first < n_rows && rc == 0; first += SMX_SNAPSHOT_ROWS) {
     const uint32_t len = (uint32_t)((n_rows - first < SMX_SNAPSHOT_ROWS) ? n_rows - first : SMX_SNAPSHOT_ROWS);
     const uint32_t* d_xs = d_keys + first;
-    const uint32_t tiles = smx_scan_scratch_items(len);
-    ensure_tmp(s, (size_t)len * 12, ((size_t)len + 2 + tiles) * 8);
-    uint32_t* d_counts = s->d_tmp;
-    uint32_t* d_slog = s->d_tmp + len;
-    uint32_t* d_units = s->d_tmp + 2 * (size_t)len;
-    uint32_t* d_nbig = ensure_rowplan(s, len);
-    smx_launch_row_counts(s->stream, view_of(s), d_xs, len, d_counts, s->d_info, s->d_big, d_nbig);
+    uint32_t* d_slog = dbuf_need(s, &s->db.tmp, (size_t)len * 8);
+    uint32_t* d_units = d_slog + len;
+    uint64_t* d_off = dbuf_need(s, &s->db.tmp64, ((size_t)len + 2 + smx_scan_scratch_items(len)) * 8);
+    const smx_rowplan_t p = rowplan(s, len);
+    smx_launch_row_counts(s->stream, view_of(s), d_xs, len, p.counts, p.info, p.big, p.n_big);
     smx_launch_row_slog(s->stream, view_of(s), d_xs, len, d_slog);
-    smx_launch_snap_units(s->stream, d_counts, d_slog, len, d_units);
-    smx_launch_scan(s->stream, d_units, len, 0, s->d_tmp64, s->d_tmp64 + (size_t)len + 1);
-    copy_d2h(s, h_off, s->d_tmp64, ((size_t)len + 1) * 8, s->stream);
+    smx_launch_snap_units(s->stream, p.counts, d_slog, len, d_units);
+    smx_launch_scan(s->stream, d_units, len, 0, d_off, d_off + (size_t)len + 1);
+    copy_d2h(s, h_off, d_off, ((size_t)len + 1) * 8, s->stream);
     copy_d2h(s, h_keys, d_xs, (size_t)len * 4, s->stream);
-    copy_d2h(s, &s->h_small[34], d_nbig, 4, s->stream);
+    copy_d2h(s, &s->h_small->n_big_rows, p.n_big, 4, s->stream);
     CK(cudaStreamSynchronize(s->stream));
     const size_t need = (size_t)h_off[len] * 8;
-    if (need > s->d_rowbuf_bytes) {
-      if (s->d_rowbuf) cudaFree(s->d_rowbuf);
-      s->d_rowbuf_bytes = need + need / 8 + 4096;
-      s->d_rowbuf = (uint32_t*)dmalloc(s, s->d_rowbuf_bytes);
-    }
+    uint64_t* rows = dbuf_need(s, &s->db.rows, need);
     if (need > out_cap) {
       if (out) cudaFreeHost(out);
       out_cap = need + need / 8 + 4096;
       CK(cudaHostAlloc((void**)&out, out_cap, cudaHostAllocDefault));
     }
-    CK(cudaMemsetAsync(s->d_rowbuf, 0, need, s->stream));
-    smx_launch_snap_rows(s->stream, view_of(s), s->d_info, len, s->d_tmp64, (uint64_t*)s->d_rowbuf, s->d_big, s->h_small[34]);
+    CK(cudaMemsetAsync(rows, 0, need, s->stream));
+    smx_launch_snap_rows(s->stream, view_of(s), p.info, len, d_off, rows, p.big, s->h_small->n_big_rows);
     s->n_launches += 8;
-    copy_d2h(s, out, s->d_rowbuf, need, s->stream);
+    copy_d2h(s, out, rows, need, s->stream);
     CK(cudaStreamSynchronize(s->stream));
     for (uint32_t i = 0; i < len; i++) {
       unsigned char* de = dir_entries + (first + i) * SMX_F_DIR_SLOT;
@@ -1633,10 +1563,10 @@ static int snapshot_load(smatrix_t* s, int fd) {
   if (!xs || !ys || !vs || !rk || !rs || !block) smx_die("out of host memory");
 #define FLUSH_OPS()  do { if (n) { smatrix_set_batch(s, xs, ys, vs, n); n = 0; } } while (0)
 #define FLUSH_ROWS() do { FLUSH_OPS(); if (nr) {                                                     \
-      enter(s); ensure_tmp(s, nr * 8, 0);                                                             \
-      copy_h2d(s, s->d_tmp, rk, nr * 4, s->stream);                   \
-      copy_h2d(s, s->d_tmp + nr, rs, nr * 4, s->stream);              \
-      smx_launch_load_fixup(s->stream, view_of(s), s->d_tmp, s->d_tmp + nr, (uint32_t)nr);            \
+      enter(s); uint32_t* d_rk = dbuf_need(s, &s->db.tmp, nr * 8);                                    \
+      copy_h2d(s, d_rk, rk, nr * 4, s->stream);                       \
+      copy_h2d(s, d_rk + nr, rs, nr * 4, s->stream);                  \
+      smx_launch_load_fixup(s->stream, view_of(s), d_rk, d_rk + nr, (uint32_t)nr);                    \
       CK(cudaStreamSynchronize(s->stream)); leave(s); nr = 0; } } while (0)
   while (bpos && rc == 0) {
     unsigned char bh[SMX_F_DIR_HEAD];
@@ -1744,6 +1674,7 @@ smatrix_t* smatrix_b200_open_arena(const char* fname, int device, size_t arena_b
   s->debug = (int)env_u32("SMATRIX_DEBUG", 0);
   s->migrate_tiles = (int)env_u32("SMATRIX_MIGRATE_TILES", 1);
   s->spill_cap = env_u32("SMATRIX_SPILL_CAP", 1u << 16);
+  if (s->spill_cap < 1) s->spill_cap = 1u << 16;
   s->presize = (int)env_u32("SMATRIX_PRESIZE", 1);
   s->stage_max = env_u32("SMATRIX_STAGE", SMX_STAGE_MAX);
   if (s->stage_max < 1024) s->stage_max = 1024;
@@ -1769,15 +1700,16 @@ smatrix_t* smatrix_b200_open_arena(const char* fname, int device, size_t arena_b
   CK(cudaMemsetAsync(s->d_ctl, 0, sizeof(smx_ctl_t), s->stream));
   CK(cudaHostAlloc((void**)&s->h_ctl, sizeof(smx_ctl_t), cudaHostAllocDefault));
   memset(s->h_ctl, 0, sizeof(smx_ctl_t));
-  s->d_small = (uint32_t*)dmalloc(s, 64 * 4);
-  CK(cudaHostAlloc((void**)&s->h_small, 64 * 4, cudaHostAllocDefault));
+  s->d_small = (uint32_t*)dmalloc(s, DS_WORDS * 4);
+  CK(cudaHostAlloc((void**)&s->h_small, sizeof(smx_small_t), cudaHostAllocDefault));
   if (s->arena_bytes) {
     /* a table with an arena is a bulk table: take the small cudaMalloc'ed scratch of the write path now (sketch
      * bitmap, partition counters, spill list of the tile-wise re-placement) so that no batch ever waits for
      * cudaMalloc — right after another table's arena went back to the driver a single call was seen to stall
      * for 20 - 150 ms (config 3, first step: profiles/r2_summary.md) */
-    ensure_tmp(s, (size_t)1 << (SMX_SKETCH_BITS_LOG - 3), 3 * SMX_MAX_PARTS_H * 8);
-    s->d_spill = (unsigned long long*)dmalloc(s, (size_t)s->spill_cap * 16);
+    dbuf_need(s, &s->db.tmp, (size_t)1 << (SMX_SKETCH_BITS_LOG - 3));
+    dbuf_need(s, &s->db.tmp64, 3 * SMX_MAX_PARTS_H * 8);
+    dbuf_need(s, &s->db.spill, (size_t)s->spill_cap * 16);
   }
   CK(cudaStreamSynchronize(s->stream));
   if (fname) {
@@ -1828,18 +1760,8 @@ void smatrix_close(smatrix_t* s) {
   if (s->stage_cap)
     for (int b = 0; b < 2; b++)
       for (int a = 0; a < 3; a++) scratch_free(s, s->stage[b][a]);
-  if (s->d_tmp) cudaFree(s->d_tmp);
-  if (s->d_tmp64) cudaFree(s->d_tmp64);
-  if (s->d_rowbuf) cudaFree(s->d_rowbuf);
-  if (s->d_info) cudaFree(s->d_info);
-  if (s->d_spill) cudaFree(s->d_spill);
-  void* tk[] = {s->tk_ctl, s->tk_off, s->tk_big, s->tk_cids, s->tk_cscores, s->tk_ids, s->tk_scores, s->tk_out};
-  for (size_t b = 0; b < sizeof tk / sizeof tk[0]; b++)
-    if (tk[b]) cudaFree(tk[b]);
-  if (s->bo_cap) {
-    cudaFree(s->bo_addr[0]); cudaFree(s->bo_addr[1]); cudaFree(s->bo_idx[0]); cudaFree(s->bo_idx[1]);
-    cudaFree(s->bo_seg); cudaFree(s->bo_tiles); cudaFree(s->bo_out); cudaFree(s->bo_sort);
-  }
+  const smx_dbuf_t* db = (const smx_dbuf_t*)&s->db;
+  for (size_t b = 0; b < sizeof s->db / sizeof *db; b++) cudaFree(db[b].p);
   cudaEventDestroy(s->stage_ready[0]); cudaEventDestroy(s->stage_ready[1]);
   cudaEventDestroy(s->ev0); cudaEventDestroy(s->ev1);
   cudaEventDestroy(s->t_start); cudaEventDestroy(s->t_stop);
@@ -1916,14 +1838,14 @@ uint64_t smatrix_b200_stat(smatrix_t* s, int which) {
     case SMX_STAT_VALUE_SUM: {
       read_ctl(s);
       const size_t rows = (size_t)s->h_ctl->dir_used;
-      ensure_tmp(s, (rows + 2) * 4, 0); /* list of the rows with a big bucket + its counter */
-      uint32_t* d_cnt = s->d_tmp + rows + 1;
+      uint32_t* big = dbuf_need(s, &s->db.tmp, (rows + 2) * 4); /* list of the rows with a big bucket + its counter */
+      uint32_t* d_cnt = big + rows + 1;
       CK(cudaMemsetAsync(&s->d_ctl->scratch, 0, 8, s->stream));
       CK(cudaMemsetAsync(d_cnt, 0, 4, s->stream));
-      smx_launch_sum_values(s->stream, view_of(s), s->d_tmp, d_cnt);
-      copy_d2h(s, &s->h_small[36], d_cnt, 4, s->stream);
+      smx_launch_sum_values(s->stream, view_of(s), big, d_cnt);
+      copy_d2h(s, &s->h_small->n_big_sums, d_cnt, 4, s->stream);
       CK(cudaStreamSynchronize(s->stream));
-      smx_launch_sum_values_big(s->stream, view_of(s), s->d_tmp, s->h_small[36]);
+      smx_launch_sum_values_big(s->stream, view_of(s), big, s->h_small->n_big_sums);
       s->n_launches += 2;
       read_ctl(s);
       r = s->h_ctl->scratch;
@@ -1954,12 +1876,13 @@ uint64_t smatrix_b200_stat(smatrix_t* s, int which) {
     case SMX_STAT_D2H_BYTES: r = s->d2h_bytes; break;
     case SMX_STAT_DIR_CAP: r = s->dir_cap; break;
     case SMX_STAT_SLAB_BYTES: r = s->slab_bytes; break;
-    case SMX_STAT_DEVICE_BYTES:
+    case SMX_STAT_DEVICE_BYTES: {
       r = s->seg_bytes + s->dir_cap * sizeof(smx_row_t) + (uint64_t)s->list_cap * (6 * 4 + sizeof(smx_plan_t)) +
-          (uint64_t)s->stage_cap * 24 + s->d_tmp_bytes + s->d_tmp64_bytes + s->d_rowbuf_bytes +
-          (uint64_t)s->addrs_cap * 8 + (uint64_t)s->part_cap * 16;
-      for (int b = 0; b < 8; b++) r += s->tk_bytes[b];
+          (uint64_t)s->stage_cap * 24 + (uint64_t)s->addrs_cap * 8 + (uint64_t)s->part_cap * 16;
+      const smx_dbuf_t* db = (const smx_dbuf_t*)&s->db;
+      for (size_t b = 0; b < sizeof s->db / sizeof *db; b++) r += db[b].bytes;
       break;
+    }
     case SMX_STAT_LAUNCHES: r = s->n_launches; break;
     case SMX_STAT_ROUNDS: r = s->n_rounds; break;
     case SMX_STAT_ROW_GROWS: r = s->n_row_grows; break;
@@ -2136,8 +2059,7 @@ void smatrix_b200_partition_count(smatrix_t* s, const uint32_t* d_xs, size_t n, 
   if (world == 0 || world > 64) smx_die("partition: world size must be 1..64");
   if (n > 0xFFFFFFFFull) smx_die("partition: batch too large");
   enter(s);
-  ensure_tmp(s, 0, (2 * 64 + 5 * 64) * 8);
-  unsigned long long* d_counts = (unsigned long long*)s->d_tmp64;
+  unsigned long long* d_counts = dbuf_need(s, &s->db.tmp64, (2 * 64 + 5 * 64) * 8);
   unsigned long long h[64];
   CK(cudaMemsetAsync(d_counts, 0, 64 * 8, s->stream));
   smx_launch_partition_count(s->stream, d_xs, NULL, (uint32_t)n, world, 0, SMX_PART_OWNER, 0, d_counts);
@@ -2158,9 +2080,8 @@ void smatrix_b200_route_p2p(smatrix_t* s, const uint32_t* d_xs, const uint32_t* 
   if (n == 0) return;
   if (n > 0xFFFFFFFFull) smx_die("route: batch too large");
   enter(s);
-  ensure_tmp(s, 0, (2 * 64 + 5 * 64) * 8);
-  unsigned long long* d_cursors = (unsigned long long*)s->d_tmp64 + 64;
-  unsigned long long* d_tab = (unsigned long long*)s->d_tmp64 + 128;
+  unsigned long long* d_cursors = (unsigned long long*)dbuf_need(s, &s->db.tmp64, (2 * 64 + 5 * 64) * 8) + 64;
+  unsigned long long* d_tab = d_cursors + 64;
   CK(cudaMemsetAsync(d_cursors, 0, 64 * 8, s->stream));
   copy_h2d(s, d_tab, h_dst, 5 * (size_t)world * 8, s->stream);
   smx_launch_partition_scatter(s->stream, d_xs, d_ys, d_vals, (uint32_t)n, world, 0, SMX_PART_OWNER, 0,
@@ -2200,14 +2121,13 @@ void smatrix_b200_row_counts_batch(smatrix_t* s, const uint32_t* d_xs, size_t n,
 uint64_t smatrix_b200_scan_counts(smatrix_t* s, const uint32_t* d_counts, size_t n, uint64_t* d_offsets) {
   if (n >= 0xFFFFFFFFull) smx_die("scan_counts: batch too large");
   enter(s);
-  ensure_tmp(s, 0, ((size_t)smx_scan_scratch_items((uint32_t)n) + 2) * 8);
-  smx_launch_scan(s->stream, d_counts, (uint32_t)n, 0, d_offsets, s->d_tmp64);
+  smx_launch_scan(s->stream, d_counts, (uint32_t)n, 0, d_offsets,
+                  dbuf_need(s, &s->db.tmp64, ((size_t)smx_scan_scratch_items((uint32_t)n) + 2) * 8));
   s->n_launches += 3;
-  copy_d2h(s, &s->h_small[32], d_offsets + n, 8, s->stream);
+  copy_d2h(s, &s->h_small->row_total, d_offsets + n, 8, s->stream);
   CK(cudaStreamSynchronize(s->stream));
   CK(cudaGetLastError());
-  uint64_t total = 0;
-  memcpy(&total, &s->h_small[32], 8);
+  const uint64_t total = s->h_small->row_total;
   leave(s);
   return total;
 }
@@ -2218,14 +2138,13 @@ void smatrix_b200_getrow_fill_at(smatrix_t* s, const uint32_t* d_xs, size_t n, c
   if (n >= 0xFFFFFFFFull) smx_die("getrow_fill_at: batch too large");
   enter(s);
   const uint32_t nn = (uint32_t)n;
-  ensure_tmp(s, (size_t)nn * 4, 0);
-  uint32_t* d_nbig = ensure_rowplan(s, nn);
+  const smx_rowplan_t p = rowplan(s, nn);
   /* resolve the rows (directory index, bucket size) and find the ones the whole grid compacts */
-  smx_launch_row_counts(s->stream, view_of(s), d_xs, nn, s->d_tmp, s->d_info, s->d_big, d_nbig);
-  copy_d2h(s, &s->h_small[34], d_nbig, 4, s->stream);
+  smx_launch_row_counts(s->stream, view_of(s), d_xs, nn, p.counts, p.info, p.big, p.n_big);
+  copy_d2h(s, &s->h_small->n_big_rows, p.n_big, 4, s->stream);
   CK(cudaStreamSynchronize(s->stream));
   timed_begin(s);
-  smx_launch_getrow_fill(s->stream, view_of(s), s->d_info, nn, d_offsets, 0, d_pairs, s->d_big, s->h_small[34], s->d_cursors);
+  smx_launch_getrow_fill(s->stream, view_of(s), p.info, nn, d_offsets, 0, d_pairs, p.big, s->h_small->n_big_rows, p.cursors);
   timed_end(s);
   s->n_launches += 2;
   CK(cudaStreamSynchronize(s->stream));
@@ -2240,8 +2159,7 @@ void smatrix_b200_route_offsets(smatrix_t* s, const uint64_t* d_offsets, const u
   if (n == 0) return;
   if (n >= 0xFFFFFFFFull) smx_die("route_offsets: batch too large");
   enter(s);
-  ensure_tmp(s, 0, (2 * 64 + 5 * 64) * 8);
-  unsigned long long* d_tab = (unsigned long long*)s->d_tmp64 + 128;
+  unsigned long long* d_tab = (unsigned long long*)dbuf_need(s, &s->db.tmp64, (2 * 64 + 5 * 64) * 8) + 128;
   copy_h2d(s, d_tab, h_tab, 2 * (size_t)world * 8, s->stream);
   smx_launch_route_offsets(s->stream, d_offsets, d_pos, (uint32_t)n, world, d_tab);
   s->n_launches++;
@@ -2322,8 +2240,7 @@ void smatrix_b200_partition2(smatrix_t* s, const uint32_t* d_xs, const uint32_t*
   if (world == 0 || world > 64) smx_die("partition: world size must be 1..64");
   if (n > 0xFFFFFFFFull) smx_die("partition: batch too large");
   enter(s);
-  ensure_tmp(s, 0, 2 * 64 * 8);
-  unsigned long long* d_counts = (unsigned long long*)s->d_tmp64;
+  unsigned long long* d_counts = dbuf_need(s, &s->db.tmp64, 2 * 64 * 8);
   unsigned long long* d_cursors = d_counts + 64;
   unsigned long long h[64], cur[64];
   CK(cudaMemsetAsync(d_counts, 0, 64 * 8, s->stream));
