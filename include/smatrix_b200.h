@@ -130,22 +130,11 @@ void smatrix_b200_gen_c4_ops(smatrix_t* self, uint64_t seed, uint64_t first, siz
 double smatrix_b200_probe_random_read(smatrix_t* self, size_t footprint_bytes, size_t accesses, int width);
 double smatrix_b200_probe_random_atomic(smatrix_t* self, size_t footprint_bytes, size_t accesses);
 
-/* Multi-GPU router, device side (K8): bucket a batch by owner rank = smx_owner(x, world).
- * counts[world] (device or host uint64) receives the ops per owner; the permuted batch is
- * written to out_* grouped by owner in rank order. All arrays are DEVICE pointers. */
+/* Multi-GPU router, device side (K8).  smatrix_b200_owner: the rank that owns row x in a world of
+ * `world` ranks (include/smatrix_shard.h).  smatrix_b200_gather(out, vals, pos, n):
+ * out[i] = vals[pos[i]] puts answers that came back in routed order into input order; all three
+ * arrays are DEVICE pointers. */
 uint32_t smatrix_b200_owner(uint32_t x, uint32_t world);
-void smatrix_b200_partition(smatrix_t* self, const uint32_t* d_xs, const uint32_t* d_ys,
-                            const uint32_t* d_vals, size_t n, uint32_t world, uint64_t* h_counts,
-                            uint32_t* d_out_xs, uint32_t* d_out_ys, uint32_t* d_out_vals,
-                            uint32_t* d_out_src /* nullable: original index of each routed op */);
-
-/* Same, and additionally d_out_pos[i] = position of op i in the routed arrays (the inverse
- * permutation; nullable).  smatrix_b200_gather(out, vals, pos, n): out[i] = vals[pos[i]] puts
- * answers that came back in routed order into input order. */
-void smatrix_b200_partition2(smatrix_t* self, const uint32_t* d_xs, const uint32_t* d_ys,
-                             const uint32_t* d_vals, size_t n, uint32_t world, uint64_t* h_counts,
-                             uint32_t* d_out_xs, uint32_t* d_out_ys, uint32_t* d_out_vals,
-                             uint32_t* d_out_src, uint32_t* d_out_pos);
 void smatrix_b200_gather(smatrix_t* self, uint32_t* d_out, const uint32_t* d_vals,
                          const uint32_t* d_pos, size_t n);
 

@@ -74,9 +74,6 @@ PROTOTYPES = {
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "smatrix_b200_probe_random_read": (C.c_double, [C.c_void_p, C.c_size_t, C.c_size_t, C.c_int]),
     "smatrix_b200_probe_random_atomic": (C.c_double, [C.c_void_p, C.c_size_t, C.c_size_t]),
-    "smatrix_b200_partition2": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-                                       C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                       C.c_void_p, C.c_void_p]),
     "smatrix_b200_partition_count": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p]),
     "smatrix_b200_route_p2p": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32,
                                       C.c_void_p, C.c_uint32, C.c_void_p]),
@@ -102,9 +99,6 @@ PROTOTYPES = {
     "smatrix_b200_apply_ordered_out": (None, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_size_t, C.c_void_p]),
     "smatrix_b200_owner": (C.c_uint32, [C.c_uint32, C.c_uint32]),
-    "smatrix_b200_partition": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
-                                      C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                      C.c_void_p]),
 }
 
 # include/smatrix_shard.h

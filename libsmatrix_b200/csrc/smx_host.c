@@ -1646,14 +1646,7 @@ smatrix_t* smatrix_b200_open_arena(const char* fname, int device, size_t arena_b
   if (!s) return NULL;
   s->device = device;
   pthread_mutex_init(&s->mu, NULL);
-  if (env_u32("SMATRIX_STREAM_HIGH_PRIORITY", 0)) { /* router handles: their kernels must interleave
-                                                       with an update in flight on another handle */
-    int lo = 0, hi = 0;
-    CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-    CK(cudaStreamCreateWithPriority(&s->stream, cudaStreamNonBlocking, hi));
-  } else {
-    CK(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
-  }
+  CK(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&s->read_stream[0], cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&s->read_stream[1], cudaStreamNonBlocking));
@@ -2221,43 +2214,6 @@ void smatrix_b200_memcpy_async(smatrix_t* s, void* dst, const void* src, size_t 
 void smatrix_b200_lane_sync(smatrix_t* s, int lane) {
   enter(s);
   CK(cudaStreamSynchronize(lane_stream(s, lane)));
-  CK(cudaGetLastError());
-  leave(s);
-}
-
-void smatrix_b200_partition(smatrix_t* s, const uint32_t* d_xs, const uint32_t* d_ys,
-                            const uint32_t* d_vals, size_t n, uint32_t world, uint64_t* h_counts,
-                            uint32_t* d_out_xs, uint32_t* d_out_ys, uint32_t* d_out_vals,
-                            uint32_t* d_out_src) {
-  smatrix_b200_partition2(s, d_xs, d_ys, d_vals, n, world, h_counts, d_out_xs, d_out_ys, d_out_vals,
-                          d_out_src, NULL);
-}
-
-void smatrix_b200_partition2(smatrix_t* s, const uint32_t* d_xs, const uint32_t* d_ys,
-                             const uint32_t* d_vals, size_t n, uint32_t world, uint64_t* h_counts,
-                             uint32_t* d_out_xs, uint32_t* d_out_ys, uint32_t* d_out_vals,
-                             uint32_t* d_out_src, uint32_t* d_out_pos) {
-  if (world == 0 || world > 64) smx_die("partition: world size must be 1..64");
-  if (n > 0xFFFFFFFFull) smx_die("partition: batch too large");
-  enter(s);
-  unsigned long long* d_counts = dbuf_need(s, &s->db.tmp64, 2 * 64 * 8);
-  unsigned long long* d_cursors = d_counts + 64;
-  unsigned long long h[64], cur[64];
-  CK(cudaMemsetAsync(d_counts, 0, 64 * 8, s->stream));
-  smx_launch_partition_count(s->stream, d_xs, NULL, (uint32_t)n, world, 0, SMX_PART_OWNER, 0, d_counts);
-  copy_d2h(s, h, d_counts, world * 8, s->stream);
-  CK(cudaStreamSynchronize(s->stream));
-  unsigned long long at = 0;
-  for (uint32_t r = 0; r < world; r++) {
-    cur[r] = at;
-    at += h[r];
-    h_counts[r] = h[r];
-  }
-  copy_h2d(s, d_cursors, cur, world * 8, s->stream);
-  smx_launch_partition_scatter(s->stream, d_xs, d_ys, d_vals, (uint32_t)n, world, 0, SMX_PART_OWNER, 0,
-                               d_cursors, d_out_xs, d_out_ys, d_out_vals, d_out_src, NULL, d_out_pos, NULL, 0);
-  s->n_launches += 2;
-  CK(cudaStreamSynchronize(s->stream));
   CK(cudaGetLastError());
   leave(s);
 }

@@ -33,8 +33,6 @@ cudaError_t cudaMemcpy(void* d, const void* s, size_t n, int kind);
 cudaError_t cudaMemcpyAsync(void* d, const void* s, size_t n, int kind, cudaStream_t st);
 cudaError_t cudaStreamCreateWithFlags(cudaStream_t* s, unsigned flags);
 cudaError_t cudaStreamDestroy(cudaStream_t s);
-cudaError_t cudaDeviceGetStreamPriorityRange(int* lo, int* hi);
-cudaError_t cudaStreamCreateWithPriority(cudaStream_t* s, unsigned flags, int prio);
 cudaError_t cudaStreamSynchronize(cudaStream_t s);
 cudaError_t cudaStreamWaitEvent(cudaStream_t s, cudaEvent_t e, unsigned flags);
 cudaError_t cudaEventCreateWithFlags(cudaEvent_t* e, unsigned flags);

@@ -44,8 +44,6 @@ cudaError_t cudaMemcpy(void* d, const void* s, size_t n, int) { memmove(d, s, n)
 cudaError_t cudaMemcpyAsync(void* d, const void* s, size_t n, int, cudaStream_t) { memmove(d, s, n); return 0; }
 cudaError_t cudaStreamCreateWithFlags(cudaStream_t* s, unsigned) { *s = (void*)1; return 0; }
 cudaError_t cudaStreamDestroy(cudaStream_t) { return 0; }
-cudaError_t cudaDeviceGetStreamPriorityRange(int* lo, int* hi) { *lo = 0; *hi = -1; return 0; }
-cudaError_t cudaStreamCreateWithPriority(cudaStream_t* s, unsigned, int) { *s = (void*)1; return 0; }
 cudaError_t cudaStreamSynchronize(cudaStream_t) { return 0; }
 cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigned) { return 0; }
 cudaError_t cudaEventCreateWithFlags(cudaEvent_t* e, unsigned) { *e = (void*)1; return 0; }

@@ -1,5 +1,5 @@
 """Worker for tests/test_gpu_sharded.py: one rank (= one GPU) of an NCCL group driving the
-row-shard router on the real CUDA library."""
+C router (include/smatrix_shard.h) on the real CUDA library."""
 import os
 import sys
 
@@ -11,7 +11,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
-from libsmatrix_b200.sharded import ShardedSparseMatrix, TorchShardedSparseMatrix  # noqa: E402
+from libsmatrix_b200.sharded import ShardedSparseMatrix  # noqa: E402
 from oracle import cpu  # noqa: E402
 
 U32 = np.uint32
@@ -22,14 +22,9 @@ def main():
     torch.cuda.set_device(rank)
     dev = torch.device("cuda", rank)
     dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
-    kind = os.environ.get("SMX_ROUTER_KIND", "c")     # c = the C router (product); torch-p2p / torch-nccl = fallback
-    sliced = kind == "c-sliced"                       # the C router, shards forced onto their slice-ordered paths
-    kind = "c" if sliced else kind
-    p2p = kind != "torch-nccl"
-    if kind == "c":
-        m = ShardedSparseMatrix(rank, world, rank)
-    else:
-        m = TorchShardedSparseMatrix(rank, world, rank, p2p=p2p)
+    kind = os.environ.get("SMX_SHARD_KIND", "c")
+    sliced = kind == "c-sliced"                       # shards forced onto their slice-ordered paths
+    m = ShardedSparseMatrix(rank, world, rank)
     ref = cpu.CpuMatrix("reference" if cpu.have_reference() else "port")
     rng = np.random.default_rng(321)                  # the same global stream on every rank
     n = 400_000
@@ -48,8 +43,6 @@ def main():
     nz = ys != 0
     ref.apply("incr", xs[nz], ys[nz], np.ones(int(nz.sum()), U32))
     k = int(nz.sum())
-    if kind != "c":
-        m.PIPELINE_MIN, m.PIPELINE_PIECE = 50_000, 40_000                  # force the overlapped pieces
     m.incr_batch(t(xs[nz][sl(k)]), t(ys[nz][sl(k)]), None, ordered=False)  # order-free stream
     allx = np.concatenate([xs, gx]); ally = np.concatenate([ys, gy])
     qx = np.concatenate([allx[rank::7], rng.integers(0, 2**32, 1000, dtype=np.uint64).astype(U32)])
@@ -70,44 +63,40 @@ def main():
     assert (cpu.sort_rows(o1, p1) == cpu.sort_rows(o2, p2)).all(), f"rank {rank}: sharded getrow pairs mismatch"
     o0, p0 = m.getrow_batch(np.zeros(0, U32))
     assert len(o0) == 1 and len(p0) == 0
-    if kind == "c":                                   # per-op return values across ranks (SURVEY.md 8f N1)
-        for op in ("incr", "decr", "set", "incr"):
-            bx = (rng.zipf(1.4, 60000) % 500).astype(U32) * U32(2654435761)
-            by = (rng.zipf(1.3, 60000) % 9).astype(U32)
-            bv = rng.integers(1, 1000, 60000).astype(U32)
-            want = ref.apply(op, bx, by, bv, want_out=True)
-            s6 = sl(60000)
-            got = getattr(m, op + "_batch_out")(bx[s6], by[s6], bv[s6])
-            assert (np.asarray(got) == want[s6]).all(), f"rank {rank}: sharded {op}_batch_out mismatch (host arrays)"
+    for op in ("incr", "decr", "set", "incr"):        # per-op return values across ranks (SURVEY.md 8f N1)
         bx = (rng.zipf(1.4, 60000) % 500).astype(U32) * U32(2654435761)
-        by = (rng.zipf(1.3, 60000) % 9 + 1).astype(U32)
-        want = ref.apply("incr", bx, by, np.ones(60000, U32), want_out=True)
-        got = m.incr_batch_out(t(bx[sl(60000)]), t(by[sl(60000)]), None)          # device arrays, all ones
-        assert (got.cpu().numpy().view(U32) == want[sl(60000)]).all(), f"rank {rank}: sharded incr_batch_out mismatch (device)"
-        allx = np.concatenate([allx, bx]); ally = np.concatenate([ally, by])
-    if kind == "c":                                   # the CF read side across ranks: bit-exact doubles
-        items = np.unique(allx)[rank::11][:200]
-        co, cids, cscores = m.cf_neighbors_batch(items)
-        o3, p3 = ref.getrow_many(items)
-        assert (co == o3).all(), f"rank {rank}: cf offsets mismatch"
-        for i, a in enumerate(items[:40]):
-            lo, hi = int(co[i]), int(co[i + 1])
-            got = dict(zip(cids[lo:hi].tolist(), cscores[lo:hi].tolist()))
-            a_total, want = ref.get(int(a), 0), {}
-            for b, cc in p3[lo:hi]:
-                den = np.sqrt(np.float64(a_total)) * np.sqrt(np.float64(ref.get(int(b), 0) or 1))
-                want[int(b)] = 0.0 if (den == 0.0 or np.float64(cc) > den) else float(np.float64(cc) / den)
-            assert got == want, f"rank {rank}: cf scores of item {a}"
+        by = (rng.zipf(1.3, 60000) % 9).astype(U32)
+        bv = rng.integers(1, 1000, 60000).astype(U32)
+        want = ref.apply(op, bx, by, bv, want_out=True)
+        s6 = sl(60000)
+        got = getattr(m, op + "_batch_out")(bx[s6], by[s6], bv[s6])
+        assert (np.asarray(got) == want[s6]).all(), f"rank {rank}: sharded {op}_batch_out mismatch (host arrays)"
+    bx = (rng.zipf(1.4, 60000) % 500).astype(U32) * U32(2654435761)
+    by = (rng.zipf(1.3, 60000) % 9 + 1).astype(U32)
+    want = ref.apply("incr", bx, by, np.ones(60000, U32), want_out=True)
+    got = m.incr_batch_out(t(bx[sl(60000)]), t(by[sl(60000)]), None)          # device arrays, all ones
+    assert (got.cpu().numpy().view(U32) == want[sl(60000)]).all(), f"rank {rank}: sharded incr_batch_out mismatch (device)"
+    allx = np.concatenate([allx, bx]); ally = np.concatenate([ally, by])
+    items = np.unique(allx)[rank::11][:200]           # the CF read side across ranks: bit-exact doubles
+    co, cids, cscores = m.cf_neighbors_batch(items)
+    o3, p3 = ref.getrow_many(items)
+    assert (co == o3).all(), f"rank {rank}: cf offsets mismatch"
+    for i, a in enumerate(items[:40]):
+        lo, hi = int(co[i]), int(co[i + 1])
+        got = dict(zip(cids[lo:hi].tolist(), cscores[lo:hi].tolist()))
+        a_total, want = ref.get(int(a), 0), {}
+        for b, cc in p3[lo:hi]:
+            den = np.sqrt(np.float64(a_total)) * np.sqrt(np.float64(ref.get(int(b), 0) or 1))
+            want[int(b)] = 0.0 if (den == 0.0 or np.float64(cc) > den) else float(np.float64(cc) / den)
+        assert got == want, f"rank {rank}: cf scores of item {a}"
     tot = torch.tensor([m.stat("rows"), m.stat("nnz")], device=dev)
     dist.all_reduce(tot)
     o, p = ref.getrow_many(np.unique(allx))
     assert int(tot[0]) == len(np.unique(allx)) and int(tot[1]) == len(p)
-    if kind != "c":
-        assert (m._peers is not None) == p2p, "peer-memory route was expected to be active"
     m.close(); ref.close()
     dist.barrier()
     dist.destroy_process_group()
-    print(f"rank {rank} ok (router={kind})")
+    print(f"rank {rank} ok ({kind})")
 
 
 if __name__ == "__main__":

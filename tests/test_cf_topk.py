@@ -132,13 +132,6 @@ def test_device_arrays_sim(sim):
     m.close(); ref.close()
 
 
-def test_torch_sharded_refuses():
-    from libsmatrix_b200.sharded import TorchShardedSparseMatrix
-    m = TorchShardedSparseMatrix.__new__(TorchShardedSparseMatrix)
-    with pytest.raises(AttributeError):
-        m.cf_topk_batch
-
-
 def _rank_main(sim, name, rank, world, errors, device_arrays, rows, want):
     try:
         from libsmatrix_b200.sharded import ShardedSparseMatrix

@@ -100,6 +100,8 @@ def _rank_main(sim, name, rank, world, errors, device_arrays):
         assert (cpu.sort_rows(o1, p1) == cpu.sort_rows(o2, p2)).all(), f"rank {rank}: sharded getrow pairs mismatch"
         o0, p0 = m.getrow_batch(np.zeros(0, U32))                                    # empty request (collective)
         assert len(o0) == 1 and len(p0) == 0
+        owned = sum(1 for x in np.unique(allx) if m._lib.smatrix_b200_owner(int(x), world) == rank)
+        assert m.stat("rows") == owned, f"rank {rank}: the shard holds {m.stat('rows')} rows, it owns {owned}"
         rows_total, nnz_total = m.sum(m.stat("rows")), m.sum(m.stat("nnz"))
         assert rows_total == len(np.unique(allx)), (rows_total, len(np.unique(allx)))
         assert nnz_total == len(ref.getrow_many(np.unique(allx))[1])
