@@ -34,6 +34,40 @@ smatrix_t* smatrix_b200_open_arena(const char* fname, int device, size_t arena_b
  * snapshot — call this at the checkpoints the application can afford. */
 int   smatrix_b200_snapshot(smatrix_t* self);
 
+/* Device-level pieces of the snapshot, used by the multi-GPU router (every rank writes its part of ONE
+ * .smx file, and reads a share of one).  The file is always the reference's format: 512-byte header,
+ * chained directory blocks of 2^22 entries, then the row blocks.
+ *   snap_extent    list this table's rows and lay out their row blocks: returns (rows, row-block bytes).
+ *                  Holds the list until snap_write (or the next extent, or close).
+ *   snap_rows_base where the row blocks start in a file of `total_rows` rows
+ *   snap_layout    header and directory block headers of such a file into `fd`, and its final size
+ *   snap_write     this table's row blocks at byte `byte_base` of fd and its directory entries from entry
+ *                  `first_entry` on (entry e is slot e % 2^22 of block e / 2^22); 0 or -1
+ *   snap_commit    rename(tmp, fname) and fsync of the directory that holds fname; 0 or -1
+ * A table on its own (smatrix_b200_snapshot) is: extent, layout, write at snap_rows_base(rows), fsync,
+ * commit. */
+int      smatrix_b200_snap_extent(smatrix_t* self, uint64_t* rows, uint64_t* bytes);
+uint64_t smatrix_b200_snap_rows_base(uint64_t total_rows);
+int      smatrix_b200_snap_layout(int fd, uint64_t total_rows, uint64_t total_bytes);
+int      smatrix_b200_snap_write(smatrix_t* self, int fd, uint64_t byte_base, uint64_t first_entry);
+int      smatrix_b200_snap_commit(const char* tmp, const char* fname);
+/* The reader of a .smx file: share `share` of `shares` (a contiguous range of directory entries, cut evenly)
+ * is read in file order, window by window ($SMATRIX_LOAD_WINDOW bytes, default 64 MiB; a bigger row grows
+ * it), every row header is checked on the host, and the device expands the raw row blocks into pieces of
+ * at most $SMATRIX_LOAD_CELLS cells (default 2^24; a row never straddles two pieces).
+ *   load_begin   NULL if the header or the directory is unreadable
+ *   load_next    1 = a piece: the op stream (x, y, v; n_ops) as smatrix_set_batch takes it — per row
+ *                (key, 0, 0) first, then its cells with a non-zero value in slot order — and the rows'
+ *                (key, log2 row size) for load_fixup, which goes after the piece's ops.  DEVICE arrays of
+ *                self's scratch, valid until the next call.  0 = the share is done, -1 = corrupt row.
+ *   load_fixup   the rowlen state of loaded rows: S = the file's row size, d = (column 0 != 0) */
+typedef struct smx_loader_s smx_loader_t;
+smx_loader_t* smatrix_b200_load_begin(smatrix_t* self, int fd, int share, int shares);
+int  smatrix_b200_load_next(smx_loader_t* ld, const uint32_t** d_xs, const uint32_t** d_ys, const uint32_t** d_vs,
+                            size_t* n_ops, const uint32_t** d_keys, const uint32_t** d_logs, size_t* n_rows);
+void smatrix_b200_load_end(smx_loader_t* ld);
+void smatrix_b200_load_fixup(smatrix_t* self, const uint32_t* d_keys, const uint32_t* d_logs, size_t n);
+
 int   smatrix_b200_device(smatrix_t* self);   /* CUDA device ordinal                            */
 void* smatrix_b200_stream(smatrix_t* self);   /* the cudaStream_t every kernel is launched on   */
 void  smatrix_b200_sync(smatrix_t* self);     /* cudaStreamSynchronize on that stream            */

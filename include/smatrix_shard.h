@@ -39,7 +39,28 @@ typedef struct smatrix_shard_s smatrix_shard_t;
 smatrix_shard_t* smatrix_b200_shard_open(const char* name, int rank, int world, int device);
 /* the same with this rank's slab arena given explicitly (bytes; 0 = on demand) instead of $SMATRIX_ARENA_GIB */
 smatrix_shard_t* smatrix_b200_shard_open_arena(const char* name, int rank, int world, int device, size_t arena_bytes);
-void smatrix_b200_shard_close(smatrix_shard_t* self);            /* collective */
+/* Collective.  Like smatrix_b200_shard_open_arena, plus file mode as in smatrix_open(fname): the matrix is
+ * loaded from `fname` if the file exists and is non-empty, and written back by smatrix_b200_shard_close.
+ * Every rank passes the same path.  Returns NULL on EVERY rank if any rank fails: the file cannot be
+ * opened or is corrupt, the paths differ, or the usual set-up failures.  A file that could not be read
+ * is never overwritten.
+ * The file is one ordinary .smx file in the reference's format, without sharding metadata: a file written
+ * at one world size loads at any other, on one GPU through smatrix_open, and in the reference; a single-GPU
+ * or reference file loads sharded.  Every rank reads an even share of the file's directory, expands its row
+ * blocks on its GPU and routes the rows to their owners.
+ * Durability is that of a single-GPU handle (smatrix_b200_snapshot): the matrix is persisted only by
+ * smatrix_b200_shard_snapshot and smatrix_b200_shard_close, so a job that dies in between loses the updates
+ * since the last snapshot. */
+smatrix_shard_t* smatrix_b200_shard_open_file(const char* name, int rank, int world, int device,
+                                              size_t arena_bytes, const char* fname);
+/* Collective: write the snapshot now.  The file goes to a temporary name (`fname.tmp`, laid out by rank 0,
+ * then every rank writes its own rows' row blocks and directory entries into it in parallel and fsyncs),
+ * and rank 0 renames it over the old one and syncs the directory.  Returns 0 on every rank, or -1 on every
+ * rank when no rank has a file or any step failed; a failed snapshot leaves the previous file intact. */
+int smatrix_b200_shard_snapshot(smatrix_shard_t* self);
+/* Collective.  With a file (smatrix_b200_shard_open_file) the snapshot is written first; if that fails,
+ * the same message as smatrix_close's goes to stdout and the matrix is closed anyway. */
+void smatrix_b200_shard_close(smatrix_shard_t* self);
 smatrix_t* smatrix_b200_shard_local(smatrix_shard_t* self);      /* this rank's own table (stats, timers) */
 int smatrix_b200_shard_rank(smatrix_shard_t* self);
 int smatrix_b200_shard_world(smatrix_shard_t* self);

@@ -99,12 +99,24 @@ PROTOTYPES = {
     "smatrix_b200_apply_ordered_out": (None, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_size_t, C.c_void_p]),
     "smatrix_b200_owner": (C.c_uint32, [C.c_uint32, C.c_uint32]),
+    "smatrix_b200_snap_extent": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "smatrix_b200_snap_rows_base": (C.c_uint64, [C.c_uint64]),
+    "smatrix_b200_snap_layout": (C.c_int, [C.c_int, C.c_uint64, C.c_uint64]),
+    "smatrix_b200_snap_write": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64, C.c_uint64]),
+    "smatrix_b200_snap_commit": (C.c_int, [C.c_char_p, C.c_char_p]),
+    "smatrix_b200_load_begin": (C.c_void_p, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    "smatrix_b200_load_next": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p]),
+    "smatrix_b200_load_end": (None, [C.c_void_p]),
+    "smatrix_b200_load_fixup": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
 }
 
 # include/smatrix_shard.h
 PROTOTYPES.update({
     "smatrix_b200_shard_open": (C.c_void_p, [C.c_char_p, C.c_int, C.c_int, C.c_int]),
     "smatrix_b200_shard_open_arena": (C.c_void_p, [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_size_t]),
+    "smatrix_b200_shard_open_file": (C.c_void_p, [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_char_p]),
+    "smatrix_b200_shard_snapshot": (C.c_int, [C.c_void_p]),
     "smatrix_b200_shard_close": (None, [C.c_void_p]),
     "smatrix_b200_shard_local": (C.c_void_p, [C.c_void_p]),
     "smatrix_b200_shard_rank": (C.c_int, [C.c_void_p]),

@@ -127,6 +127,9 @@ struct smatrix_s {
     smx_dbuf_t tk_big;     /* select state + histograms of the big segments */
     smx_dbuf_t tk_cids, tk_cscores; /* compaction regions of the big segments */
     smx_dbuf_t tk_ids, tk_scores;   /* scores of a piece */
+    /* loading a snapshot (smatrix_b200_load_next): a window of file bytes, its tiles, their counts and offsets,
+     * the op stream (x, y, v) and the (key, log2 size) fixups of a piece */
+    smx_dbuf_t ld_raw, ld_tiles, ld_cnt, ld_off, ld_ops, ld_fix;
   } db;
   uint32_t topk_pairs;  /* SMATRIX_TOPK_PAIRS: pairs per piece of a cf_topk_batch call */
   uint64_t n_topk_big, n_topk_passes;
@@ -157,6 +160,10 @@ struct smatrix_s {
   double kernel_ns;
   int preagg;
   char* fname;
+  uint32_t* snap_keys; /* the rows smatrix_b200_snap_extent listed, until smatrix_b200_snap_write */
+  uint64_t snap_rows;
+  uint64_t* snap_hoff; /* a table of one chunk of rows: its layout (offsets, keys, big rows) as snap_extent */
+  uint32_t* snap_hkeys; /* read it back, so that snap_write neither lays it out nor reads it again */
 };
 
 /* ------------------------------------------------------------------------------ errors */
@@ -1436,6 +1443,189 @@ static void sync_parent_dir(const char* fname) { /* make the rename itself durab
   free(dir);
 }
 
+#define SMX_F_BLOCK_BYTES (SMX_F_DIR_HEAD + SMX_F_DIR_ENTRIES * SMX_F_DIR_SLOT)
+#define SMX_LOAD_WINDOW_DEFAULT (64u << 20) /* bytes of file per pread */
+#define SMX_LOAD_CELLS_DEFAULT (1u << 24)   /* cells per piece: bounds the loader's device scratch */
+
+/* ---- save, in two device-level pieces (include/smatrix_b200.h): a table's extent in the file, then its
+ * row blocks and directory entries at a given place.  One table writes a whole file (snapshot_save); the
+ * ranks of a sharded matrix write their parts of one file side by side (smx_router.c). */
+static void snap_free_keys(smatrix_t* s) {
+  if (s->snap_keys) cudaFree(s->snap_keys);
+  free(s->snap_hoff); free(s->snap_hkeys);
+  s->snap_keys = s->snap_hkeys = NULL;
+  s->snap_hoff = NULL;
+  s->snap_rows = 0;
+}
+
+/* rows [first, first + len) of the listed keys: row sizes -> 8-byte units -> offsets (d_off[0..len]) */
+typedef struct { smx_rowplan_t p; uint64_t* d_off; uint32_t* d_slog; } smx_snapchunk_t;
+static smx_snapchunk_t snap_chunk_bufs(smatrix_t* s, uint32_t len) { /* the same buffers for the same len */
+  smx_snapchunk_t c;
+  c.d_slog = dbuf_need(s, &s->db.tmp, (size_t)len * 8);
+  c.d_off = dbuf_need(s, &s->db.tmp64, ((size_t)len + 2 + smx_scan_scratch_items(len)) * 8);
+  c.p = rowplan(s, len);
+  return c;
+}
+static smx_snapchunk_t snap_chunk(smatrix_t* s, uint64_t first, uint32_t len) {
+  const uint32_t* d_xs = s->snap_keys + first;
+  smx_snapchunk_t c = snap_chunk_bufs(s, len);
+  uint32_t* d_slog = c.d_slog;
+  uint32_t* d_units = d_slog + len;
+  smx_launch_row_counts(s->stream, view_of(s), d_xs, len, c.p.counts, c.p.info, c.p.big, c.p.n_big);
+  smx_launch_row_slog(s->stream, view_of(s), d_xs, len, d_slog);
+  smx_launch_snap_units(s->stream, c.p.counts, d_slog, len, d_units);
+  smx_launch_scan(s->stream, d_units, len, 0, c.d_off, c.d_off + (size_t)len + 1);
+  s->n_launches += 6;
+  return c;
+}
+
+/* caller holds the handle lock, the stream is idle */
+static void snap_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes) {
+  snap_free_keys(s);
+  read_ctl(s);
+  const uint64_t n_rows = s->h_ctl->dir_used;
+  if (n_rows) {
+    s->snap_keys = (uint32_t*)dmalloc(s, n_rows * 4);
+    CK(cudaMemsetAsync(&s->d_ctl->scratch, 0, 8, s->stream));
+    smx_launch_list_rows(s->stream, view_of(s), s->snap_keys, (uint32_t*)&s->d_ctl->scratch);
+  }
+  s->snap_rows = n_rows;
+  uint64_t total = 0;
+  for (uint64_t first = 0; first < n_rows; first += SMX_SNAPSHOT_ROWS) {
+    const uint32_t len = (uint32_t)((n_rows - first < SMX_SNAPSHOT_ROWS) ? n_rows - first : SMX_SNAPSHOT_ROWS);
+    const smx_snapchunk_t c = snap_chunk(s, first, len);
+    if (n_rows <= SMX_SNAPSHOT_ROWS) {
+      s->snap_hoff = (uint64_t*)malloc(((size_t)len + 1) * 8);
+      s->snap_hkeys = (uint32_t*)malloc((size_t)len * 4);
+      if (!s->snap_hoff || !s->snap_hkeys) smx_die("out of host memory");
+      copy_d2h(s, s->snap_hoff, c.d_off, ((size_t)len + 1) * 8, s->stream);
+      copy_d2h(s, s->snap_hkeys, s->snap_keys, (size_t)len * 4, s->stream);
+      copy_d2h(s, &s->h_small->n_big_rows, c.p.n_big, 4, s->stream);
+      CK(cudaStreamSynchronize(s->stream));
+      total = s->snap_hoff[len] * 8;
+    } else {
+      copy_d2h(s, &s->h_small->row_total, c.d_off + len, 8, s->stream);
+      CK(cudaStreamSynchronize(s->stream));
+      total += s->h_small->row_total * 8;
+    }
+  }
+  CK(cudaGetLastError());
+  *rows = n_rows;
+  *bytes = total;
+}
+
+/* directory entries e0 .. e0 + n - 1 (12 bytes each in `ents`): entry e is slot e % 2^22 of block e / 2^22 */
+static int snap_write_entries(int fd, const unsigned char* ents, uint64_t e0, uint64_t n) {
+  while (n) {
+    const uint64_t b = e0 / SMX_F_DIR_ENTRIES, slot = e0 % SMX_F_DIR_ENTRIES;
+    const uint64_t run = (n < SMX_F_DIR_ENTRIES - slot) ? n : SMX_F_DIR_ENTRIES - slot;
+    if (write_all(fd, ents, run * SMX_F_DIR_SLOT, SMX_F_META + b * SMX_F_BLOCK_BYTES + SMX_F_DIR_HEAD + slot * SMX_F_DIR_SLOT))
+      return -1;
+    ents += run * SMX_F_DIR_SLOT; e0 += run; n -= run;
+  }
+  return 0;
+}
+
+/* caller holds the handle lock; the rows snap_extent listed */
+static int snap_write(smatrix_t* s, int fd, uint64_t fpos, uint64_t first_entry) {
+  const uint64_t n_rows = s->snap_rows;
+  unsigned char* ents = (unsigned char*)malloc((size_t)SMX_SNAPSHOT_ROWS * SMX_F_DIR_SLOT);
+  uint32_t* h_keys = (uint32_t*)malloc(SMX_SNAPSHOT_ROWS * 4);
+  uint64_t* h_off = (uint64_t*)malloc(((size_t)SMX_SNAPSHOT_ROWS + 1) * 8);
+  unsigned char* out = NULL; /* pinned: the row blocks come down at PCIe speed */
+  size_t out_cap = 0;
+  int rc = 0;
+  if (!ents || !h_keys || !h_off) smx_die("out of host memory");
+  /* K9: every chunk of rows is laid out ON THE DEVICE in the reference's row-block format (sizes ->
+   * scan -> k_snap_rows / k_snap_big place every cell by column % size); the host only moves bytes */
+  for (uint64_t first = 0; first < n_rows && rc == 0; first += SMX_SNAPSHOT_ROWS) {
+    const uint32_t len = (uint32_t)((n_rows - first < SMX_SNAPSHOT_ROWS) ? n_rows - first : SMX_SNAPSHOT_ROWS);
+    smx_snapchunk_t c;
+    if (s->snap_hoff) { /* one chunk, laid out by snap_extent: its buffers still hold it */
+      c = snap_chunk_bufs(s, len);
+      memcpy(h_off, s->snap_hoff, ((size_t)len + 1) * 8);
+      memcpy(h_keys, s->snap_hkeys, (size_t)len * 4);
+    } else {
+      c = snap_chunk(s, first, len);
+      copy_d2h(s, h_off, c.d_off, ((size_t)len + 1) * 8, s->stream);
+      copy_d2h(s, h_keys, s->snap_keys + first, (size_t)len * 4, s->stream);
+      copy_d2h(s, &s->h_small->n_big_rows, c.p.n_big, 4, s->stream);
+      CK(cudaStreamSynchronize(s->stream));
+    }
+    const size_t need = (size_t)h_off[len] * 8;
+    uint64_t* rows = dbuf_need(s, &s->db.rows, need);
+    if (need > out_cap) {
+      if (out) cudaFreeHost(out);
+      out_cap = need + need / 8 + 4096;
+      CK(cudaHostAlloc((void**)&out, out_cap, cudaHostAllocDefault));
+    }
+    CK(cudaMemsetAsync(rows, 0, need, s->stream));
+    smx_launch_snap_rows(s->stream, view_of(s), c.p.info, len, c.d_off, rows, c.p.big, s->h_small->n_big_rows);
+    s->n_launches += 2;
+    copy_d2h(s, out, rows, need, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    for (uint32_t i = 0; i < len; i++) {
+      unsigned char* de = ents + (size_t)i * SMX_F_DIR_SLOT;
+      const uint64_t row_fpos = fpos + h_off[i] * 8;
+      memcpy(de, &h_keys[i], 4);
+      memcpy(de + 4, &row_fpos, 8);
+    }
+    if (write_all(fd, out, need, fpos) || snap_write_entries(fd, ents, first_entry + first, len)) rc = -1;
+    fpos += need;
+  }
+  CK(cudaGetLastError());
+  if (out) cudaFreeHost(out);
+  free(ents); free(h_keys); free(h_off);
+  snap_free_keys(s);
+  return rc;
+}
+
+uint64_t smatrix_b200_snap_rows_base(uint64_t total_rows) {
+  const uint64_t n_blocks = total_rows ? (total_rows + SMX_F_DIR_ENTRIES - 1) / SMX_F_DIR_ENTRIES : 1;
+  return SMX_F_META + n_blocks * SMX_F_BLOCK_BYTES;
+}
+
+int smatrix_b200_snap_layout(int fd, uint64_t total_rows, uint64_t total_bytes) {
+  const uint64_t n_blocks = total_rows ? (total_rows + SMX_F_DIR_ENTRIES - 1) / SMX_F_DIR_ENTRIES : 1;
+  unsigned char head[SMX_F_META];
+  memset(head, 0, sizeof head);
+  memset(head, 0x17, 8);
+  { uint64_t first = SMX_F_META; memcpy(head + 8, &first, 8); }
+  if (write_all(fd, head, sizeof head, 0)) return -1;
+  for (uint64_t b = 0; b < n_blocks; b++) {
+    const uint64_t bpos = SMX_F_META + b * SMX_F_BLOCK_BYTES;
+    unsigned char bh[SMX_F_DIR_HEAD];
+    const uint64_t entries = SMX_F_DIR_ENTRIES, next = (b + 1 < n_blocks) ? bpos + SMX_F_BLOCK_BYTES : 0;
+    memcpy(bh, &entries, 8);
+    memcpy(bh + 8, &next, 8);
+    if (write_all(fd, bh, sizeof bh, bpos)) return -1;
+  }
+  /* unused directory entries read back as zeros */
+  return ftruncate(fd, (off_t)(smatrix_b200_snap_rows_base(total_rows) + total_bytes)) == -1 ? -1 : 0;
+}
+
+int smatrix_b200_snap_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes) {
+  enter(s);
+  CK(cudaStreamSynchronize(s->stream));
+  snap_extent(s, rows, bytes);
+  leave(s);
+  return 0;
+}
+
+int smatrix_b200_snap_write(smatrix_t* s, int fd, uint64_t byte_base, uint64_t first_entry) {
+  enter(s);
+  const int rc = snap_write(s, fd, byte_base, first_entry);
+  leave(s);
+  return rc;
+}
+
+int smatrix_b200_snap_commit(const char* tmp, const char* fname) {
+  if (rename(tmp, fname) == -1) return -1;
+  sync_parent_dir(fname);
+  return 0;
+}
+
 /* caller holds the handle lock */
 static int snapshot_save(smatrix_t* s) {
   size_t fl = strlen(s->fname);
@@ -1445,92 +1635,18 @@ static int snapshot_save(smatrix_t* s) {
   memcpy(tmp + fl, ".tmp", 5);
   int fd = open(tmp, O_RDWR | O_CREAT | O_TRUNC, 00600);
   if (fd == -1) { perror("cannot open file"); free(tmp); return -1; }
-  read_ctl(s);
-  const uint64_t n_rows = s->h_ctl->dir_used;
-  const uint64_t n_blocks = n_rows ? (n_rows + SMX_F_DIR_ENTRIES - 1) / SMX_F_DIR_ENTRIES : 1;
-  const uint64_t block_bytes = SMX_F_DIR_HEAD + SMX_F_DIR_ENTRIES * SMX_F_DIR_SLOT;
-  uint64_t fpos = SMX_F_META + n_blocks * block_bytes; /* row blocks start after the directory */
-  int rc = 0;
-  unsigned char head[SMX_F_META];
-  memset(head, 0, sizeof head);
-  memset(head, 0x17, 8);
-  { uint64_t first = SMX_F_META; memcpy(head + 8, &first, 8); }
-  if (write_all(fd, head, sizeof head, 0)) rc = -1;
-
-  uint32_t* d_keys = NULL;
-  unsigned char* dir_entries = (unsigned char*)calloc(n_rows ? n_rows : 1, SMX_F_DIR_SLOT);
-  uint32_t* h_keys = (uint32_t*)malloc(SMX_SNAPSHOT_ROWS * 4);
-  uint64_t* h_off = (uint64_t*)malloc(((size_t)SMX_SNAPSHOT_ROWS + 1) * 8);
-  unsigned char* out = NULL; /* pinned: the row blocks come down at PCIe speed */
-  size_t out_cap = 0;
-  if (!dir_entries || !h_keys || !h_off) smx_die("out of host memory");
-  if (n_rows) {
-    d_keys = (uint32_t*)dmalloc(s, n_rows * 4);
-    CK(cudaMemsetAsync(&s->d_ctl->scratch, 0, 8, s->stream));
-    smx_launch_list_rows(s->stream, view_of(s), d_keys, (uint32_t*)&s->d_ctl->scratch);
-    CK(cudaStreamSynchronize(s->stream));
-  }
-  /* K9: every chunk of rows is laid out ON THE DEVICE in the reference's row-block format (sizes ->
-   * scan -> k_snap_rows / k_snap_big place every cell by column % size); the host only moves bytes */
-  for (uint64_t first = 0; first < n_rows && rc == 0; first += SMX_SNAPSHOT_ROWS) {
-    const uint32_t len = (uint32_t)((n_rows - first < SMX_SNAPSHOT_ROWS) ? n_rows - first : SMX_SNAPSHOT_ROWS);
-    const uint32_t* d_xs = d_keys + first;
-    uint32_t* d_slog = dbuf_need(s, &s->db.tmp, (size_t)len * 8);
-    uint32_t* d_units = d_slog + len;
-    uint64_t* d_off = dbuf_need(s, &s->db.tmp64, ((size_t)len + 2 + smx_scan_scratch_items(len)) * 8);
-    const smx_rowplan_t p = rowplan(s, len);
-    smx_launch_row_counts(s->stream, view_of(s), d_xs, len, p.counts, p.info, p.big, p.n_big);
-    smx_launch_row_slog(s->stream, view_of(s), d_xs, len, d_slog);
-    smx_launch_snap_units(s->stream, p.counts, d_slog, len, d_units);
-    smx_launch_scan(s->stream, d_units, len, 0, d_off, d_off + (size_t)len + 1);
-    copy_d2h(s, h_off, d_off, ((size_t)len + 1) * 8, s->stream);
-    copy_d2h(s, h_keys, d_xs, (size_t)len * 4, s->stream);
-    copy_d2h(s, &s->h_small->n_big_rows, p.n_big, 4, s->stream);
-    CK(cudaStreamSynchronize(s->stream));
-    const size_t need = (size_t)h_off[len] * 8;
-    uint64_t* rows = dbuf_need(s, &s->db.rows, need);
-    if (need > out_cap) {
-      if (out) cudaFreeHost(out);
-      out_cap = need + need / 8 + 4096;
-      CK(cudaHostAlloc((void**)&out, out_cap, cudaHostAllocDefault));
-    }
-    CK(cudaMemsetAsync(rows, 0, need, s->stream));
-    smx_launch_snap_rows(s->stream, view_of(s), p.info, len, d_off, rows, p.big, s->h_small->n_big_rows);
-    s->n_launches += 8;
-    copy_d2h(s, out, rows, need, s->stream);
-    CK(cudaStreamSynchronize(s->stream));
-    for (uint32_t i = 0; i < len; i++) {
-      unsigned char* de = dir_entries + (first + i) * SMX_F_DIR_SLOT;
-      const uint64_t row_fpos = fpos + h_off[i] * 8;
-      memcpy(de, &h_keys[i], 4);
-      memcpy(de + 4, &row_fpos, 8);
-    }
-    if (write_all(fd, out, need, fpos)) rc = -1;
-    fpos += need;
-  }
-  for (uint64_t b = 0; b < n_blocks && rc == 0; b++) {
-    const uint64_t bpos = SMX_F_META + b * block_bytes;
-    unsigned char bh[SMX_F_DIR_HEAD];
-    const uint64_t entries = SMX_F_DIR_ENTRIES, next = (b + 1 < n_blocks) ? bpos + block_bytes : 0;
-    memcpy(bh, &entries, 8);
-    memcpy(bh + 8, &next, 8);
-    if (write_all(fd, bh, sizeof bh, bpos)) rc = -1;
-    const uint64_t lo = b * SMX_F_DIR_ENTRIES;
-    const uint64_t cnt = (n_rows > lo) ? ((n_rows - lo < SMX_F_DIR_ENTRIES) ? n_rows - lo : SMX_F_DIR_ENTRIES) : 0;
-    if (cnt && write_all(fd, dir_entries + lo * SMX_F_DIR_SLOT, cnt * SMX_F_DIR_SLOT, bpos + SMX_F_DIR_HEAD)) rc = -1;
-  }
-  if (rc == 0 && ftruncate(fd, (off_t)fpos) == -1) rc = -1; /* unused directory entries read back as zeros */
+  uint64_t rows = 0, bytes = 0;
+  snap_extent(s, &rows, &bytes);
+  int rc = smatrix_b200_snap_layout(fd, rows, bytes);
+  if (snap_write(s, fd, smatrix_b200_snap_rows_base(rows), 0)) rc = -1;
   if (rc == 0 && fsync(fd) == -1) rc = -1; /* the data is on disk before the old file is replaced */
   if (close(fd) == -1) rc = -1;
-  if (rc == 0 && rename(tmp, s->fname) == -1) rc = -1;
-  if (rc == 0) sync_parent_dir(s->fname);
+  if (rc == 0) rc = smatrix_b200_snap_commit(tmp, s->fname);
   if (rc) {
     perror("libsmatrix: writing the snapshot failed");
     unlink(tmp); /* the previous snapshot, if any, is still intact */
   }
-  if (d_keys) cudaFree(d_keys);
-  if (out) cudaFreeHost(out);
-  free(dir_entries); free(h_keys); free(h_off); free(tmp);
+  free(tmp);
   return rc;
 }
 
@@ -1544,77 +1660,236 @@ static int read_all(int fd, void* buf, size_t bytes, uint64_t at) {
   return 0;
 }
 
-/* handle is complete and not yet published: public entry points may be used */
-static int snapshot_load(smatrix_t* s, int fd) {
+/* ---- load: one reader of row blocks for a share of the directory (include/smatrix_b200.h) ----
+ * The share's rows are read in file order, window by window, into pinned memory; every row header is
+ * checked here; the raw bytes go up with a tile table and k_load_count / k_load_emit expand them into
+ * the op stream on the device. */
+typedef struct { uint64_t rpos; uint32_t key; } smx_ldrow_t;
+struct smx_loader_s {
+  smatrix_t* s;
+  int fd;
+  uint64_t fsize;
+  smx_ldrow_t* rows; /* this share, by file offset */
+  uint64_t n, next;
+  size_t window;     /* SMATRIX_LOAD_WINDOW: bytes per pread (grown for a bigger row) */
+  uint64_t cells;    /* SMATRIX_LOAD_CELLS: cells per piece (a bigger row is a piece of its own) */
+  unsigned char* win; size_t win_cap;   /* pinned */
+  smx_load_tile_t* tiles; size_t tiles_cap;
+  uint32_t* fix; size_t fix_cap;        /* keys, then log2 sizes */
+};
+
+static int ldrow_cmp(const void* a, const void* b) {
+  const uint64_t x = ((const smx_ldrow_t*)a)->rpos, y = ((const smx_ldrow_t*)b)->rpos;
+  return x < y ? -1 : x > y;
+}
+
+void smatrix_b200_load_end(smx_loader_t* ld) {
+  if (!ld) return;
+  if (ld->win) cudaFreeHost(ld->win);
+  free(ld->rows); free(ld->tiles); free(ld->fix);
+  free(ld);
+}
+
+smx_loader_t* smatrix_b200_load_begin(smatrix_t* s, int fd, int share, int shares) {
   unsigned char head[SMX_F_META];
+  struct stat st;
+  if (shares < 1 || share < 0 || share >= shares || fstat(fd, &st) != 0) return NULL;
   if (read_all(fd, head, sizeof head, 0) || head[0] != 0x17 || head[1] != 0x17) {
     fprintf(stderr, "libsmatrix: invalid file header\n");
-    return -1;
+    return NULL;
   }
-  uint64_t bpos;
-  memcpy(&bpos, head + 8, 8);
-  size_t cap = 1u << 22; /* triples per flush (grows for rows larger than that) */
-  uint32_t* xs = (uint32_t*)malloc(cap * 4), * ys = (uint32_t*)malloc(cap * 4), * vs = (uint32_t*)malloc(cap * 4);
-  uint32_t* rk = (uint32_t*)malloc(cap * 4), * rs = (uint32_t*)malloc(cap * 4);
+  smx_loader_t* ld = (smx_loader_t*)calloc(1, sizeof *ld);
   unsigned char* block = (unsigned char*)malloc(SMX_F_DIR_ENTRIES * SMX_F_DIR_SLOT);
-  uint32_t* cells = NULL;
-  size_t cells_cap = 0, n = 0, nr = 0;
+  if (!ld || !block) smx_die("out of host memory");
+  ld->s = s;
+  ld->fd = fd;
+  ld->fsize = (uint64_t)st.st_size;
+  ld->window = env_u32("SMATRIX_LOAD_WINDOW", SMX_LOAD_WINDOW_DEFAULT);
+  if (ld->window < 64) ld->window = 64;
+  ld->cells = env_u32("SMATRIX_LOAD_CELLS", SMX_LOAD_CELLS_DEFAULT);
+  if (ld->cells < 1) ld->cells = 1;
+  /* the chain of directory blocks (a slot with rpos = 0 ends its block, src/smatrix.c:814-815): count the
+   * entries, then read this share's contiguous range of them */
+  uint64_t bpos, total = 0, nblk = 0, blk_cap = 0;
+  uint64_t* blk = NULL; /* per block: position, entries in use */
+  memcpy(&bpos, head + 8, 8);
   int rc = 0;
-  if (!xs || !ys || !vs || !rk || !rs || !block) smx_die("out of host memory");
-#define FLUSH_OPS()  do { if (n) { smatrix_set_batch(s, xs, ys, vs, n); n = 0; } } while (0)
-#define FLUSH_ROWS() do { FLUSH_OPS(); if (nr) {                                                     \
-      enter(s); uint32_t* d_rk = dbuf_need(s, &s->db.tmp, nr * 8);                                    \
-      copy_h2d(s, d_rk, rk, nr * 4, s->stream);                       \
-      copy_h2d(s, d_rk + nr, rs, nr * 4, s->stream);                  \
-      smx_launch_load_fixup(s->stream, view_of(s), d_rk, d_rk + nr, (uint32_t)nr);                    \
-      CK(cudaStreamSynchronize(s->stream)); leave(s); nr = 0; } } while (0)
   while (bpos && rc == 0) {
     unsigned char bh[SMX_F_DIR_HEAD];
-    if (read_all(fd, bh, sizeof bh, bpos)) { rc = -1; break; }
-    uint64_t entries, next;
+    uint64_t entries, next, used = 0;
+    if (nblk > ld->fsize / SMX_F_DIR_HEAD || read_all(fd, bh, sizeof bh, bpos)) { rc = -1; break; } /* or a loop */
     memcpy(&entries, bh, 8);
     memcpy(&next, bh + 8, 8);
-    if (entries > SMX_F_DIR_ENTRIES) { rc = -1; break; }
-    if (read_all(fd, block, entries * SMX_F_DIR_SLOT, bpos + SMX_F_DIR_HEAD)) { rc = -1; break; }
-    for (uint64_t i = 0; i < entries; i++) {
-      uint32_t key;
+    if (entries > SMX_F_DIR_ENTRIES || read_all(fd, block, entries * SMX_F_DIR_SLOT, bpos + SMX_F_DIR_HEAD)) { rc = -1; break; }
+    for (; used < entries; used++) {
       uint64_t rpos;
-      memcpy(&key, block + i * SMX_F_DIR_SLOT, 4);
-      memcpy(&rpos, block + i * SMX_F_DIR_SLOT + 4, 8);
-      if (!rpos) break; /* src/smatrix.c:814-815 */
-      unsigned char rh[SMX_F_ROW_HEAD];
-      uint64_t size;
-      if (read_all(fd, rh, sizeof rh, rpos) || rh[0] != 0x23 || rh[7] != 0x23) { rc = -1; break; }
-      memcpy(&size, rh + 8, 8);
-      if (size == 0 || (size & (size - 1)) || size > (1ull << 32)) { rc = -1; break; }
-      if (size * 2 > cells_cap) {
-        free(cells);
-        cells_cap = size * 2;
-        cells = (uint32_t*)malloc(cells_cap * 4);
-        if (!cells) smx_die("out of host memory");
-      }
-      if (read_all(fd, cells, size * 8, rpos + SMX_F_ROW_HEAD)) { rc = -1; break; }
-      if (n + size + 1 > cap) FLUSH_OPS();
-      if (size + 1 > cap) { /* a single row larger than the staging buffers: grow them */
-        cap = size + 1;
-        xs = (uint32_t*)realloc(xs, cap * 4); ys = (uint32_t*)realloc(ys, cap * 4); vs = (uint32_t*)realloc(vs, cap * 4);
-        if (!xs || !ys || !vs) smx_die("out of host memory");
-      }
-      xs[n] = key; ys[n] = 0; vs[n] = 0; n++; /* the row exists even when it is empty */
-      for (uint64_t c = 0; c < size; c++)
-        if (cells[2 * c + 1] != 0) { xs[n] = key; ys[n] = cells[2 * c]; vs[n] = cells[2 * c + 1]; n++; }
-      uint32_t lg = 0;
-      while ((1ull << lg) < size) lg++;
-      rk[nr] = key; rs[nr] = lg; nr++;
-      if (nr == (1u << 22)) FLUSH_ROWS();
+      memcpy(&rpos, block + used * SMX_F_DIR_SLOT + 4, 8);
+      if (!rpos) break;
     }
+    if (nblk == blk_cap) {
+      blk_cap = blk_cap * 2 + 16;
+      blk = (uint64_t*)realloc(blk, blk_cap * 16);
+      if (!blk) smx_die("out of host memory");
+    }
+    blk[2 * nblk] = bpos; blk[2 * nblk + 1] = used; nblk++;
+    total += used;
     bpos = next;
   }
-  if (rc == 0) FLUSH_ROWS();
-#undef FLUSH_OPS
-#undef FLUSH_ROWS
+  const uint64_t lo = total * (uint64_t)share / (uint64_t)shares, hi = total * ((uint64_t)share + 1) / (uint64_t)shares;
+  ld->n = hi - lo;
+  ld->rows = (smx_ldrow_t*)malloc((ld->n ? ld->n : 1) * sizeof(smx_ldrow_t));
+  if (!ld->rows) smx_die("out of host memory");
+  for (uint64_t b = 0, e = 0; b < nblk && rc == 0; e += blk[2 * b + 1], b++) {
+    const uint64_t a = lo > e ? lo : e, z = hi < e + blk[2 * b + 1] ? hi : e + blk[2 * b + 1];
+    if (a >= z) continue;
+    if (read_all(fd, block, (z - a) * SMX_F_DIR_SLOT, blk[2 * b] + SMX_F_DIR_HEAD + (a - e) * SMX_F_DIR_SLOT)) { rc = -1; break; }
+    for (uint64_t k = a; k < z; k++) {
+      smx_ldrow_t* r = &ld->rows[k - lo];
+      memcpy(&r->key, block + (k - a) * SMX_F_DIR_SLOT, 4);
+      memcpy(&r->rpos, block + (k - a) * SMX_F_DIR_SLOT + 4, 8);
+    }
+  }
+  free(blk);
+  free(block);
+  if (rc) {
+    fprintf(stderr, "libsmatrix: file is corrupt\n");
+    smatrix_b200_load_end(ld);
+    return NULL;
+  }
+  /* reads go forward through the file even where a foreign file's rows are not in directory order */
+  for (uint64_t i = 1; i < ld->n; i++)
+    if (ld->rows[i].rpos < ld->rows[i - 1].rpos) { qsort(ld->rows, ld->n, sizeof(smx_ldrow_t), ldrow_cmp); break; }
+  return ld;
+}
+
+/* the window holds file bytes [at, at + len) */
+static int load_window(smx_loader_t* ld, uint64_t at, size_t len) {
+  if (len > ld->win_cap) {
+    if (ld->win) cudaFreeHost(ld->win);
+    ld->win_cap = len;
+    CK(cudaHostAlloc((void**)&ld->win, ld->win_cap, cudaHostAllocDefault));
+  }
+  return read_all(ld->fd, ld->win, len, at);
+}
+
+int smatrix_b200_load_next(smx_loader_t* ld, const uint32_t** d_xs, const uint32_t** d_ys, const uint32_t** d_vs,
+                           size_t* n_ops, const uint32_t** d_keys, const uint32_t** d_logs, size_t* n_rows) {
+  smatrix_t* s = ld->s;
+  *n_ops = *n_rows = 0;
+  if (ld->next == ld->n) return 0;
+  const uint64_t wstart = ld->rows[ld->next].rpos & ~7ull; /* our files keep every cell 8-byte aligned */
+  size_t len = ld->window;
+  uint64_t i = ld->next, cells = 0, nt = 0, nf = 0, end = 0;
+  if (ld->rows[i].rpos + SMX_F_ROW_HEAD > ld->fsize) return -1;
+  for (;;) { /* read; grow the window if its first row does not fit */
+    if (len > ld->fsize - wstart) len = (size_t)(ld->fsize - wstart);
+    if (load_window(ld, wstart, len)) return -1;
+    const uint64_t rpos = ld->rows[i].rpos;
+    if (rpos + SMX_F_ROW_HEAD <= wstart + len) {
+      uint64_t size;
+      memcpy(&size, ld->win + (rpos - wstart) + 8, 8);
+      if (size == 0 || (size & (size - 1)) || size > (1ull << 32) || rpos + SMX_F_ROW_HEAD + size * 8 > ld->fsize) return -1;
+      if (rpos + SMX_F_ROW_HEAD + size * 8 <= wstart + len) break;
+      len = (size_t)(rpos + SMX_F_ROW_HEAD + size * 8 - wstart);
+    } else {
+      len = (size_t)(rpos + SMX_F_ROW_HEAD - wstart);
+    }
+  }
+  for (; i < ld->n; i++) {
+    const uint64_t rpos = ld->rows[i].rpos;
+    if (rpos + SMX_F_ROW_HEAD > wstart + len) break;
+    const unsigned char* rh = ld->win + (rpos - wstart);
+    uint64_t size;
+    memcpy(&size, rh + 8, 8);
+    if (rh[0] != 0x23 || rh[7] != 0x23 || size == 0 || (size & (size - 1)) || size > (1ull << 32) ||
+        rpos + SMX_F_ROW_HEAD + size * 8 > ld->fsize)
+      return -1;
+    if (rpos + SMX_F_ROW_HEAD + size * 8 > wstart + len) break;
+    if (i > ld->next && cells + size > ld->cells) break;
+    const uint64_t tile = 1ull << SMX_LOAD_TILE_LOG, ntiles = (size + tile - 1) / tile;
+    if (nt + ntiles > ld->tiles_cap) {
+      ld->tiles_cap = (nt + ntiles) * 2 + 1024;
+      ld->tiles = (smx_load_tile_t*)realloc(ld->tiles, ld->tiles_cap * sizeof(smx_load_tile_t));
+      if (!ld->tiles) smx_die("out of host memory");
+    }
+    for (uint64_t k = 0; k < ntiles; k++) {
+      smx_load_tile_t* t = &ld->tiles[nt++];
+      t->off = rpos - wstart + SMX_F_ROW_HEAD + k * tile * 8;
+      t->key = ld->rows[i].key;
+      t->cells = (uint32_t)(size < tile ? size : tile) | (k == 0 ? SMX_LOAD_FIRST : 0u);
+    }
+    if (nf + 1 > ld->fix_cap) {
+      ld->fix_cap = nf * 2 + 1024;
+      ld->fix = (uint32_t*)realloc(ld->fix, ld->fix_cap * 2 * 4);
+      if (!ld->fix) smx_die("out of host memory");
+    }
+    ld->fix[nf++] = ld->rows[i].key;
+    cells += size;
+    end = rpos + SMX_F_ROW_HEAD + size * 8 - wstart;
+  }
+  for (uint64_t r = 0; r < nf; r++) { /* keys, then the log2 row sizes */
+    uint64_t size;
+    memcpy(&size, ld->win + (ld->rows[ld->next + r].rpos - wstart) + 8, 8);
+    ld->fix[nf + r] = log2_u64(size);
+  }
+  ld->next = i;
+  if (nt >= 0xFFFFFFFFull) smx_die("load: too many rows in one window");
+  enter(s);
+  /* the window up to the end of its last row goes to the device */
+  void* raw = dbuf_need(s, &s->db.ld_raw, end);
+  smx_load_tile_t* tiles = dbuf_need(s, &s->db.ld_tiles, nt * sizeof(smx_load_tile_t));
+  uint32_t* cnt = dbuf_need(s, &s->db.ld_cnt, nt * 4);
+  uint64_t* off = dbuf_need(s, &s->db.ld_off, (nt + 2 + smx_scan_scratch_items((uint32_t)nt)) * 8);
+  uint32_t* fix = dbuf_need(s, &s->db.ld_fix, nf * 8);
+  copy_h2d(s, raw, ld->win, end, s->stream);
+  copy_h2d(s, tiles, ld->tiles, nt * sizeof(smx_load_tile_t), s->stream);
+  copy_h2d(s, fix, ld->fix, nf * 8, s->stream);
+  smx_launch_load_count(s->stream, raw, tiles, (uint32_t)nt, cnt);
+  smx_launch_scan(s->stream, cnt, (uint32_t)nt, 0, off, off + nt + 1);
+  copy_d2h(s, &s->h_small->row_total, off + nt, 8, s->stream);
+  CK(cudaStreamSynchronize(s->stream));
+  const uint64_t ops = s->h_small->row_total;
+  uint32_t* xs = dbuf_need(s, &s->db.ld_ops, ops * 12);
+  smx_launch_load_emit(s->stream, raw, tiles, (uint32_t)nt, off, xs, xs + ops, xs + 2 * ops);
+  s->n_launches += 5;
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+  *d_xs = xs; *d_ys = xs + ops; *d_vs = xs + 2 * ops;
+  *n_ops = (size_t)ops;
+  *d_keys = fix; *d_logs = fix + nf;
+  *n_rows = (size_t)nf;
+  return 1;
+}
+
+void smatrix_b200_load_fixup(smatrix_t* s, const uint32_t* d_keys, const uint32_t* d_logs, size_t n) {
+  if (!n) return;
+  if (n >= 0xFFFFFFFFull) smx_die("load_fixup: batch too large");
+  enter(s);
+  smx_launch_load_fixup(s->stream, view_of(s), d_keys, d_logs, (uint32_t)n);
+  s->n_launches++;
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+}
+
+/* handle is complete and not yet published: public entry points may be used.  One GPU reads the whole
+ * directory as its share; every piece is applied as a device-array set batch, then its rows take the
+ * file's row sizes (k_load_fixup) — the rowlen automaton continues from there. */
+static int snapshot_load(smatrix_t* s, int fd) {
+  smx_loader_t* ld = smatrix_b200_load_begin(s, fd, 0, 1);
+  if (!ld) return -1;
+  int rc;
+  for (;;) {
+    const uint32_t *xs, *ys, *vs, *keys, *logs;
+    size_t n, nr;
+    rc = smatrix_b200_load_next(ld, &xs, &ys, &vs, &n, &keys, &logs, &nr);
+    if (rc <= 0) break;
+    smatrix_set_batch(s, xs, ys, vs, n);
+    smatrix_b200_load_fixup(s, keys, logs, nr);
+  }
   if (rc) fprintf(stderr, "libsmatrix: file is corrupt\n");
-  free(xs); free(ys); free(vs); free(rk); free(rs); free(block); free(cells);
+  smatrix_b200_load_end(ld);
   return rc;
 }
 
@@ -1738,6 +2013,7 @@ void smatrix_close(smatrix_t* s) {
     if (s->segs[i].owned) cudaFree(s->segs[i].base);
   free(s->segs);
   if (!s->dir_in_arena) cudaFree(s->dir);
+  snap_free_keys(s);
   cudaFree(s->d_ctl);
   cudaFreeHost(s->h_ctl);
   cudaFree(s->d_small);

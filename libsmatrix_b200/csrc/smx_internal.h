@@ -213,6 +213,21 @@ void smx_launch_snap_rows(smx_stream_t stream, smx_view_t v, const uint64_t* inf
                           const uint32_t* big_list, uint32_t n_big);
 void smx_launch_load_fixup(smx_stream_t stream, smx_view_t v, const uint32_t* xs, const uint32_t* slogs,
                            uint32_t n);
+/* a snapshot's row blocks on the device: `raw` is a window of file bytes, a tile is a row or a
+ * 2^SMX_LOAD_TILE_LOG-cell part of one; count -> smx_launch_scan -> emit writes every row's
+ * (key, 0, 0) op and then its cells with a non-zero value, in slot order */
+#define SMX_LOAD_TILE_LOG 12u
+#define SMX_LOAD_FIRST 0x80000000u /* smx_load_tile_t.cells: the row's first tile */
+typedef struct {
+  uint64_t off;   /* byte offset of the tile's first cell in the window */
+  uint32_t key;   /* row id */
+  uint32_t cells; /* cells in the tile | SMX_LOAD_FIRST */
+} smx_load_tile_t;
+void smx_launch_load_count(smx_stream_t stream, const void* raw, const smx_load_tile_t* tiles, uint32_t n,
+                           uint32_t* counts);
+void smx_launch_load_emit(smx_stream_t stream, const void* raw, const smx_load_tile_t* tiles, uint32_t n,
+                          const uint64_t* offsets /* n + 1, from smx_launch_scan */, uint32_t* xs, uint32_t* ys,
+                          uint32_t* vs);
 void smx_launch_gen_c2_ops(smx_stream_t stream, uint64_t seed, uint64_t first, uint64_t count,
                            uint32_t rows, uint32_t ycols, uint32_t* xs, uint32_t* ys);
 void smx_launch_gen_c2_queries(smx_stream_t stream, uint64_t seed_get, uint64_t seed_build,

@@ -19,6 +19,7 @@
  *   k_set_max/mark/commit  last-writer-wins resolution for smatrix_set batches (:225-234 applied
  *                       sequentially)
  *   k_snap_units / _rows / _big   the row blocks of the .smx file (:454-482) in the loader's layout (:499-545)
+ *   k_load_count / _emit          the loader's parse of raw row blocks into (x, y, v) ops (:499-545)
  *   k_partition_count / _scatter  no counterpart: chunk ordering by directory slice (writes and large read
  *                       calls), and the multi-GPU route (every owner's run stored straight into that
  *                       owner's inbox over NVLink)
@@ -1726,6 +1727,68 @@ k_load_fixup(smx_view_t V, const uint32_t* xs, const uint32_t* slogs, uint32_t n
   }
 }
 
+/* ---- loading a snapshot: raw row blocks -> the op stream of the loader ------------------------
+ * The host uploads a window of file bytes and a tile table (smx_load_tile_t): a row of up to
+ * 2^SMX_LOAD_TILE_LOG cells is one tile, a bigger row is cut into tiles of that many cells.  One warp
+ * per tile, two passes: k_load_count counts every tile's ops, smx_launch_scan turns the counts into
+ * offsets, and k_load_emit writes them in order — the first tile of a row leads with (key, 0, 0) so
+ * that the row exists even when it holds no live cell, then every cell with a non-zero value follows
+ * in slot order (a ballot per 32 cells, each lane's place = the popcount of the lanes below it).
+ * Header checks are the host's: the device only sees validated sizes. */
+__device__ __forceinline__ ull ld_file_cell(const unsigned char* p) { /* {u32 column, u32 value} */
+  if (((uintptr_t)p & 7u) == 0u) return *(const ull*)p;
+  ull c;
+  memcpy(&c, p, 8); /* a row block at an odd offset of a foreign file */
+  return c;
+}
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_load_count(const unsigned char* raw, const smx_load_tile_t* tiles, uint32_t n, uint32_t* counts) {
+  const uint32_t lane = lane_id();
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) / SMX_WARP;
+  const uint32_t nwarps = gridDim.x * blockDim.x / SMX_WARP;
+  for (uint32_t t = warp; t < n; t += nwarps) {
+    const smx_load_tile_t T = tiles[t];
+    const uint32_t cells = T.cells & ~SMX_LOAD_FIRST;
+    const unsigned char* p = raw + T.off;
+    uint32_t live = 0;
+    for (uint32_t base = 0; base < cells; base += SMX_WARP) {
+      const uint32_t c = base + lane;
+      const bool nz = c < cells && (uint32_t)(ld_file_cell(p + 8ull * c) >> 32) != 0u;
+      live += (uint32_t)__popc(__ballot_sync(SMX_FULL, nz));
+    }
+    if (lane == 0) counts[t] = live + ((T.cells & SMX_LOAD_FIRST) ? 1u : 0u);
+  }
+}
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_load_emit(const unsigned char* raw, const smx_load_tile_t* tiles, uint32_t n, const ull* offsets,
+            uint32_t* xs, uint32_t* ys, uint32_t* vs) {
+  const uint32_t lane = lane_id();
+  const uint32_t below = (1u << lane) - 1u;
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) / SMX_WARP;
+  const uint32_t nwarps = gridDim.x * blockDim.x / SMX_WARP;
+  for (uint32_t t = warp; t < n; t += nwarps) {
+    const smx_load_tile_t T = tiles[t];
+    const uint32_t cells = T.cells & ~SMX_LOAD_FIRST;
+    const unsigned char* p = raw + T.off;
+    ull at = offsets[t];
+    if (T.cells & SMX_LOAD_FIRST) {
+      if (lane == 0) { xs[at] = T.key; ys[at] = 0u; vs[at] = 0u; }
+      at++;
+    }
+    for (uint32_t base = 0; base < cells; base += SMX_WARP) {
+      const uint32_t c = base + lane;
+      const ull cell = c < cells ? ld_file_cell(p + 8ull * c) : 0ull;
+      const uint32_t v = (uint32_t)(cell >> 32);
+      const uint32_t m = __ballot_sync(SMX_FULL, v != 0u);
+      if (v != 0u) {
+        const ull j = at + (ull)__popc(m & below);
+        xs[j] = T.key; ys[j] = (uint32_t)cell; vs[j] = v;
+      }
+      at += (ull)__popc(m);
+    }
+  }
+}
+
 /* sum of every stored value (all cells + column 0) mod 2^64 -> ctl->scratch: one warp per
  * directory entry walks that row's bucket.  For an incr-only build this must equal the sum of all
  * increments — the size-independent invariant bench.py checks at full scale. */
@@ -2482,6 +2545,17 @@ extern "C" void smx_launch_load_fixup(smx_stream_t st, smx_view_t v, const uint3
                                       const uint32_t* slogs, uint32_t n) {
   if (!n) return;
   SMX_LAUNCH(k_load_fixup, grid_for(n), SMX_BLOCK, st, v, xs, slogs, n);
+}
+extern "C" void smx_launch_load_count(smx_stream_t st, const void* raw, const smx_load_tile_t* tiles, uint32_t n,
+                                      uint32_t* counts) {
+  if (!n) return;
+  SMX_LAUNCH(k_load_count, grid_for((ull)n * SMX_WARP), SMX_BLOCK, st, (const unsigned char*)raw, tiles, n, counts);
+}
+extern "C" void smx_launch_load_emit(smx_stream_t st, const void* raw, const smx_load_tile_t* tiles, uint32_t n,
+                                     const uint64_t* offsets, uint32_t* xs, uint32_t* ys, uint32_t* vs) {
+  if (!n) return;
+  SMX_LAUNCH(k_load_emit, grid_for((ull)n * SMX_WARP), SMX_BLOCK, st, (const unsigned char*)raw, tiles, n,
+             (const ull*)offsets, xs, ys, vs);
 }
 extern "C" void smx_launch_cf_scores(smx_stream_t st, smx_view_t v, const uint32_t* items, uint32_t n,
                                      const uint64_t* offsets, const uint32_t* pairs, uint32_t* ids,

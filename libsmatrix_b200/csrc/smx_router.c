@@ -85,6 +85,7 @@ struct smatrix_shard_s {
   uint32_t piece;
   uint32_t taper_min; /* 0 = off; else the last staged piece is cut into 1/2, 1/4, 1/4 if a quarter has this many ops */
   uint64_t stat[8]; /* SMX_SHARD_STAT_* */
+  char* fname;        /* file mode: the .smx file every rank loaded from and writes back to */
 };
 
 /* inbox layout for capacity `cap` ops (cap is a multiple of 256): shared arrays first, then the
@@ -329,8 +330,14 @@ smatrix_shard_t* smatrix_b200_shard_open_arena(const char* name, int rank, int w
   return sh;
 }
 
+static int rt_snapshot(smatrix_shard_t* sh);
 void smatrix_b200_shard_close(smatrix_shard_t* sh) {
   if (!sh) return;
+  if (sh->fname && rt_snapshot(sh) != 0 && sh->rank == 0) { /* close() is void: be loud instead */
+    printf("libsmatrix error: could not write %s; the previous snapshot (if any) was kept\n", sh->fname);
+    fflush(stdout);
+  }
+  free(sh->fname);
   rt_barrier(sh);
   rt_unmap(sh, sh->peer_inbox);
   rt_unmap(sh, sh->peer_rowbuf);
@@ -912,4 +919,131 @@ void smatrix_b200_shard_cf_topk_batch(smatrix_shard_t* sh, const uint32_t* items
     if (!c.scratch) smatrix_b200_dev_free(sh->local, extra);
   }
   if (c.scratch) smatrix_b200_dev_free(sh->local, c.scratch);
+}
+
+/* ------------------------------------------------------------------------------ file mode */
+/* Collective: the .smx snapshot of the whole sharded matrix, one ordinary file in the reference's format.
+ * Every rank lays out its own rows (snap_extent); exclusive prefixes of the (rows, bytes) pairs give each rank
+ * its first directory entry and the byte where its row blocks go.  Rank 0 creates `fname.tmp` with the header
+ * and directory block headers at its final size, then every rank writes its part and fsyncs, and rank 0
+ * renames the file over the old one.  The outcome is agreed on: 0 or -1 on every rank. */
+static int rt_all_ok(smatrix_shard_t* sh, int ok) {
+  uint64_t mine[4] = {(uint64_t)(ok != 0), 0, 0, 0}, all[RT_MAXW][4];
+  rt_allgather(sh, mine, all);
+  for (int r = 0; r < sh->world; r++) ok = ok && all[r][0];
+  return ok;
+}
+
+static int rt_snapshot(smatrix_shard_t* sh) {
+  const int W = sh->world, me = sh->rank;
+  uint64_t rows = 0, bytes = 0;
+  if (sh->fname) smatrix_b200_snap_extent(sh->local, &rows, &bytes);
+  uint64_t mine[4] = {sh->fname != NULL, rows, bytes, 0}, all[RT_MAXW][4];
+  rt_allgather(sh, mine, all);
+  uint64_t total_rows = 0, total_bytes = 0, first = 0, base = 0;
+  int have = 1;
+  for (int r = 0; r < W; r++) {
+    have = have && all[r][0];
+    if (r == me) { first = total_rows; base = total_bytes; }
+    total_rows += all[r][1];
+    total_bytes += all[r][2];
+  }
+  if (!have) return -1;
+  base += smatrix_b200_snap_rows_base(total_rows);
+  const size_t fl = strlen(sh->fname);
+  char* tmp = (char*)malloc(fl + 8);
+  if (!tmp) rt_die(sh, "out of host memory");
+  memcpy(tmp, sh->fname, fl);
+  memcpy(tmp + fl, ".tmp", 5);
+  int fd = -1, ok = 1;
+  if (me == 0) {
+    fd = open(tmp, O_RDWR | O_CREAT | O_TRUNC, 00600);
+    ok = fd != -1 && smatrix_b200_snap_layout(fd, total_rows, total_bytes) == 0;
+  }
+  if (rt_all_ok(sh, ok)) { /* the file exists at its final size: the others open it without O_TRUNC */
+    if (me != 0) fd = open(tmp, O_RDWR);
+    ok = fd != -1 && smatrix_b200_snap_write(sh->local, fd, base, first) == 0 && fsync(fd) == 0;
+  } else {
+    ok = 0;
+  }
+  if (fd != -1 && close(fd) == -1) ok = 0;
+  ok = rt_all_ok(sh, ok);
+  if (me == 0) {
+    if (ok && smatrix_b200_snap_commit(tmp, sh->fname) != 0) ok = 0;
+    if (!ok) {
+      perror("libsmatrix: writing the snapshot failed");
+      unlink(tmp); /* the previous snapshot, if any, is still intact */
+    }
+  }
+  free(tmp);
+  return rt_all_ok(sh, ok) ? 0 : -1;
+}
+
+int smatrix_b200_shard_snapshot(smatrix_shard_t* sh) { return rt_snapshot(sh); }
+
+static uint64_t rt_fnv(const char* p) {
+  uint64_t h = 0xcbf29ce484222325ull;
+  for (; *p; p++) h = (h ^ (unsigned char)*p) * 0x100000001b3ull;
+  return h;
+}
+
+/* Collective: every rank reads its share of the file's directory (smatrix_b200_load_next) and routes each
+ * piece to the rows' owners as an ordered set batch, then the pieces' (key, log2 size) fixups, which every
+ * owner applies after the ops.  Ranks whose share has run out join with n = 0 until no rank has more. */
+static int rt_load(smatrix_shard_t* sh, int fd) {
+  smx_loader_t* ld = smatrix_b200_load_begin(sh->local, fd, sh->rank, sh->world);
+  int bad = ld == NULL;
+  for (;;) {
+    const uint32_t *xs = NULL, *ys = NULL, *vs = NULL, *keys = NULL, *logs = NULL;
+    size_t n = 0, nr = 0;
+    const int r = bad ? 0 : smatrix_b200_load_next(ld, &xs, &ys, &vs, &n, &keys, &logs, &nr);
+    if (r < 0) bad = 1;
+    if (r <= 0) n = nr = 0;
+    uint64_t mine[4] = {(uint64_t)bad, (uint64_t)(r > 0), 0, 0}, all[RT_MAXW][4];
+    rt_allgather(sh, mine, all);
+    int any_bad = 0, any_more = 0;
+    for (int k = 0; k < sh->world; k++) { any_bad |= (int)all[k][0]; any_more |= (int)all[k][1]; }
+    if (any_bad) { bad = 1; break; }
+    if (!any_more) break;
+    rt_write(sh, 2, xs, ys, vs, n, 1);
+    rt_route_t R;
+    rt_route(sh, keys, logs, NULL, nr, 0, 0, &R);
+    if (R.n_recv)
+      smatrix_b200_load_fixup(sh->local, (const uint32_t*)(sh->inbox + OFF_X(sh->cap)),
+                              (const uint32_t*)(sh->inbox + OFF_Y(sh->cap)), (size_t)R.n_recv);
+  }
+  smatrix_b200_load_end(ld);
+  if (bad && sh->rank == 0) fprintf(stderr, "libsmatrix: file is corrupt\n");
+  return bad ? -1 : 0;
+}
+
+smatrix_shard_t* smatrix_b200_shard_open_file(const char* name, int rank, int world, int device, size_t arena_bytes,
+                                              const char* fname) {
+  smatrix_shard_t* sh = smatrix_b200_shard_open_arena(name, rank, world, device, arena_bytes);
+  if (!sh || !fname) return sh;
+  /* like smatrix_open(fname): the file must be creatable / readable, on every rank, under one path */
+  const int fd = open(fname, O_RDWR | O_CREAT, 00600);
+  if (fd == -1) perror("cannot open file");
+  struct stat st;
+  const int has_data = fd != -1 && fstat(fd, &st) == 0 && st.st_size > 0;
+  uint64_t mine[4] = {(uint64_t)(fd != -1), rt_fnv(fname), (uint64_t)has_data, 0}, all[RT_MAXW][4];
+  rt_allgather(sh, mine, all);
+  int ok = 1, same = 1;
+  for (int r = 0; r < world; r++) {
+    ok = ok && all[r][0];
+    same = same && all[r][1] == all[0][1] && all[r][2] == all[0][2];
+  }
+  if (ok && !same) {
+    if (rank == 0) fprintf(stderr, "libsmatrix: shard_open_file: the ranks were given different files\n");
+    ok = 0;
+  }
+  if (ok && all[0][2] && rt_load(sh, fd) != 0) ok = 0;
+  if (fd != -1) close(fd);
+  if (!ok) { /* every rank takes this branch together; a file we could not read is not overwritten */
+    smatrix_b200_shard_close(sh);
+    return NULL;
+  }
+  sh->fname = strdup(fname);
+  if (!sh->fname) rt_die(sh, "out of host memory");
+  return sh;
 }

@@ -50,18 +50,28 @@ class ShardedSparseMatrix:
     """ctypes wrapper of smatrix_b200_shard_* — no computation and no routing logic here."""
 
     def __init__(self, rank: int, world: int, device: int = 0, name: str | None = None,
-                 _lib_path: str | None = None, arena_gib: float | None = None):
+                 _lib_path: str | None = None, arena_gib: float | None = None, fname: str | None = None):
+        """fname: file mode (include/smatrix_shard.h, smatrix_b200_shard_open_file) — the matrix is loaded from
+        that .smx file if it exists and is non-empty and written back by snapshot() and close(); every rank
+        passes the same path."""
         from . import binding
         self._lib = binding.load(_lib_path)
         self.rank, self.world = rank, world
         self._name = name or default_name()
-        if arena_gib is not None:
+        self.filename = fname
+        if fname is not None:
+            arena = (int(arena_gib * (1 << 30)) if arena_gib is not None
+                     else int(os.environ.get("SMATRIX_ARENA_GIB") or "0", 0) << 30)
+            self._h = self._lib.smatrix_b200_shard_open_file(self._name.encode(), rank, world, int(device), arena,
+                                                             fname.encode())
+        elif arena_gib is not None:
             self._h = self._lib.smatrix_b200_shard_open_arena(self._name.encode(), rank, world, int(device),
                                                               int(arena_gib * (1 << 30)))
         else:
             self._h = self._lib.smatrix_b200_shard_open(self._name.encode(), rank, world, int(device))
         if not self._h:
-            raise RuntimeError("smatrix_b200_shard_open failed (no CUDA device or no peer access)")
+            raise RuntimeError("smatrix_b200_shard_open failed (no CUDA device or no peer access"
+                               + (", or the file cannot be opened or is corrupt)" if fname is not None else ")"))
         self.local = SparseMatrix._borrow(self._lib, self._lib.smatrix_b200_shard_local(self._h))
         self._cuda = _lib_path is None
 
@@ -193,6 +203,10 @@ class ShardedSparseMatrix:
             self._lib.smatrix_b200_shard_stat_reset(self._handle())
         return d
 
+    def snapshot(self) -> int:
+        """Collective: write the .smx file now (smatrix_b200_shard_snapshot); 0, or -1 on every rank."""
+        return int(self._lib.smatrix_b200_shard_snapshot(self._handle()))
+
     def barrier(self):
         self._lib.smatrix_b200_shard_barrier(self._handle())
 
@@ -228,7 +242,8 @@ class ShardedSparseMatrix:
 
 
 def open_sharded(rank: int, world: int, device: int = 0, name: str | None = None,
-                 arena_gib: float | None = None) -> ShardedSparseMatrix:
-    """Collective: open this rank's part of a sharded matrix.  Raises RuntimeError on every rank alike
-    (shard_open agrees on the outcome before anyone returns) when the router cannot be set up."""
-    return ShardedSparseMatrix(rank, world, device, name=name, arena_gib=arena_gib)
+                 arena_gib: float | None = None, fname: str | None = None) -> ShardedSparseMatrix:
+    """Collective: open this rank's part of a sharded matrix, file-backed when `fname` is given.  Raises
+    RuntimeError on every rank alike (shard_open agrees on the outcome before anyone returns) when the router
+    cannot be set up or the file cannot be opened or read."""
+    return ShardedSparseMatrix(rank, world, device, name=name, arena_gib=arena_gib, fname=fname)
