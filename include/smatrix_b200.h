@@ -21,7 +21,9 @@ extern "C" {
  * (see smatrix_b200_set_get_slices), SMATRIX_WIDE_SLICES (default 1: a write chunk without ops on column 0
  * is ordered over 256 directory slices instead of 128 + their column-0 twins), SMATRIX_TOPK_PAIRS (default
  * 2^28: smatrix_cf_topk_batch scores and ranks the items of a call in pieces whose rows hold at most that
- * many pairs, 32 bytes of device scratch per pair; a row longer than that is a piece of its own). */
+ * many pairs, 32 bytes of device scratch per pair; a row longer than that is a piece of its own.
+ * smatrix_cf_recommend_batch cuts its baskets the same way, at basket boundaries, with up to about 100 bytes of
+ * device scratch per pair; a basket whose rows hold more is a piece of its own). */
 smatrix_t* smatrix_b200_open(const char* fname, int device);
 /* the same with the slab arena given explicitly (bytes; 0 = segments on demand) instead of through
  * $SMATRIX_ARENA_GIB — for hosts that open several handles with different needs from several threads */
@@ -104,7 +106,8 @@ enum {
   SMX_STAT_NS_ALLOC = 26,   /* host time inside cudaMalloc on behalf of this handle so far, ns */
   SMX_STAT_ALLOCS = 27,     /* number of those cudaMalloc calls */
   SMX_STAT_TOPK_BIG = 28,   /* top-k segments (items) longer than 4096 pairs: ranked by the multi-block radix select */
-  SMX_STAT_TOPK_PASSES = 29 /* digit passes that select ran so far */
+  SMX_STAT_TOPK_PASSES = 29,/* digit passes that select ran so far */
+  SMX_STAT_REC_BIG = 30     /* baskets longer than 4096 pairs: aggregated by the global sort of smatrix_cf_recommend_batch */
 };
 uint64_t smatrix_b200_stat(smatrix_t* self, int which);
 
@@ -216,6 +219,14 @@ void smatrix_b200_cf_scores_totals(smatrix_t* self, size_t n, const uint64_t* d_
 void smatrix_b200_topk_segments(smatrix_t* self, size_t n, const uint64_t* d_offsets, const uint32_t* d_ids,
                                 const double* d_scores, uint32_t k, uint32_t* d_counts, uint32_t* d_out_ids,
                                 double* d_out_scores);
+/* The aggregation and ranking of smatrix_cf_recommend_batch over neighbour lists that are already on the device:
+ * basket i is positions d_basket_off[i] .. d_basket_off[i+1] (n + 1 entries, d_basket_off[0] = 0) of d_items,
+ * and position j's list is d_ids / d_scores[d_offsets[j] .. d_offsets[j+1]), the layout smatrix_cf_neighbors_batch
+ * produces.  Candidates, summation order, exclusions and the fixed-width outputs are those of
+ * smatrix_cf_recommend_batch.  1 <= k <= 1024.  All arrays DEVICE. */
+void smatrix_b200_basket_topk(smatrix_t* self, size_t n_baskets, const uint64_t* d_basket_off, const uint32_t* d_items,
+                              const uint64_t* d_offsets, const uint32_t* d_ids, const double* d_scores, uint32_t k,
+                              uint32_t* d_counts, uint32_t* d_out_ids, double* d_out_scores);
 int  smatrix_b200_is_device_ptr(smatrix_t* self, const void* p);   /* device (or managed) memory? */
 /* peers in the SAME process (one thread per GPU) need no IPC: enable direct access to `peer_device` */
 int  smatrix_b200_enable_peer(smatrix_t* self, int peer_device);

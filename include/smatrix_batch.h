@@ -81,6 +81,22 @@ uint64_t smatrix_cf_neighbors_batch(smatrix_t* self, const uint32_t* items, size
 void smatrix_cf_topk_batch(smatrix_t* self, const uint32_t* items, size_t n, uint32_t k,
                            uint32_t* counts, uint32_t* ids, double* scores);
 
+/* Item-based recommendations for baskets (a user's items): basket i is items[basket_off[i] .. basket_off[i+1]);
+ * basket_off has n + 1 entries, starts at 0, never decreases and ends at most at 2^32 - 2.  For every position j,
+ * L_j is exactly the list smatrix_cf_neighbors_batch returns for items[j] (empty for an absent item).  The
+ * candidates of basket i are the ids of its lists, minus its own items and minus id 0 (the column-0 pair holds the
+ * item's total, not a co-occurrence).  A candidate's score is (((0.0 + s_j1) + s_j2) + ...) over the positions
+ * j1 < j2 < ... of the basket whose list holds it, in IEEE double with one rounding per addition, in that order:
+ * the answer is bit-exact and reproducible; an item repeated in a basket counts once per position.  Output as
+ * smatrix_cf_topk_batch: counts[n] = min(k, candidates), ids[n*k] / scores[n*k] by score descending, then id
+ * ascending, slots past the count hold id 0xFFFFFFFF and score -1.0; an empty basket, or one of absent items only,
+ * has count 0.  1 <= k <= 1024.  basket_off and items are both host or both device arrays, the three outputs all
+ * host or all device (host outputs: n * (12k + 4) bytes come down; the neighbour lists never leave the device).
+ * Baskets are processed in pieces whose rows hold at most $SMATRIX_TOPK_PAIRS pairs (a basket over that is a piece
+ * of its own, see smatrix_b200.h). */
+void smatrix_cf_recommend_batch(smatrix_t* self, const uint64_t* basket_off, const uint32_t* items,
+                                size_t n_baskets, uint32_t k, uint32_t* counts, uint32_t* ids, double* scores);
+
 #ifdef __cplusplus
 }
 #endif

@@ -120,6 +120,15 @@ uint64_t smatrix_b200_shard_cf_neighbors_batch(smatrix_shard_t* self, const uint
 void smatrix_b200_shard_cf_topk_batch(smatrix_shard_t* self, const uint32_t* items, size_t n, uint32_t k,
                                       uint32_t* counts, uint32_t* ids, double* scores);
 
+/* Basket recommendations for this rank's baskets across ranks: same contract as smatrix_cf_recommend_batch
+ * (basket_off[n_baskets + 1], items, counts[n], ids / scores[n*k], 1 <= k <= 1024; a rank may pass no baskets).
+ * The lists of the flattened items come as in smatrix_b200_shard_cf_neighbors_batch and are aggregated and ranked
+ * by smatrix_b200_basket_topk on this rank's GPU, so the answers equal the single-GPU ones bit for bit at every
+ * world size.  One piece per call, as smatrix_b200_shard_cf_topk_batch. */
+void smatrix_b200_shard_cf_recommend_batch(smatrix_shard_t* self, const uint64_t* basket_off, const uint32_t* items,
+                                           size_t n_baskets, uint32_t k, uint32_t* counts, uint32_t* ids,
+                                           double* scores);
+
 /* Host wall-clock accounting of this rank since the last reset (not collective): time spent routing
  * (count, count exchange, scatter over NVLink, arrival barrier), time spent applying the inbox,
  * number of routes, bytes this rank stored into OTHER ranks' inboxes. */

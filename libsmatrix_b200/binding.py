@@ -42,6 +42,8 @@ PROTOTYPES = {
                                                C.c_void_p, C.c_uint64]),
     "smatrix_cf_topk_batch": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p, C.c_void_p,
                                      C.c_void_p]),
+    "smatrix_cf_recommend_batch": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p,
+                                          C.c_void_p, C.c_void_p]),
     # include/smatrix_b200.h
     "smatrix_b200_open": (C.c_void_p, [C.c_char_p, C.c_int]),
     "smatrix_b200_open_arena": (C.c_void_p, [C.c_char_p, C.c_int, C.c_size_t]),
@@ -90,6 +92,8 @@ PROTOTYPES = {
                                              C.c_void_p, C.c_void_p]),
     "smatrix_b200_topk_segments": (None, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                           C.c_void_p, C.c_void_p, C.c_void_p]),
+    "smatrix_b200_basket_topk": (None, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "smatrix_b200_enable_peer": (C.c_int, [C.c_void_p, C.c_int]),
     "smatrix_b200_is_device_ptr": (C.c_int, [C.c_void_p, C.c_void_p]),
     "smatrix_b200_memcpy_async": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int]),
@@ -134,6 +138,8 @@ PROTOTYPES.update({
                                                           C.c_void_p, C.c_uint64]),
     "smatrix_b200_shard_cf_topk_batch": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p,
                                                 C.c_void_p, C.c_void_p]),
+    "smatrix_b200_shard_cf_recommend_batch": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32,
+                                                     C.c_void_p, C.c_void_p, C.c_void_p]),
     "smatrix_b200_shard_getrow_batch": (C.c_uint64, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                                     C.c_uint64]),
     "smatrix_b200_shard_stat": (C.c_uint64, [C.c_void_p, C.c_int]),
@@ -148,7 +154,7 @@ STAT = {"rows": 0, "nnz": 1, "dir_cap": 2, "slab_bytes": 3, "device_bytes": 4, "
         "ns_grow_plan": 12, "ns_slab": 13, "ns_migrate": 14, "ns_dir": 15, "value_sum": 16,
         "live_bucket_bytes": 17, "free_bytes": 18, "recycled": 19, "h2d_bytes": 20, "d2h_bytes": 21, "bucket_bytes": 22, "spilled": 23,
         "sliced_gets": 24, "wide_chunks": 25, "ns_alloc": 26, "allocs": 27,
-        "topk_big": 28, "topk_passes": 29}
+        "topk_big": 28, "topk_passes": 29, "rec_big": 30}
 
 _cache: dict[str, C.CDLL] = {}
 

@@ -63,6 +63,9 @@ typedef struct {
   uint32_t n_big_sums; /* SMX_STAT_VALUE_SUM: rows with a big bucket, summed by a launch of their own */
   uint32_t topk_cut;   /* end of the next piece of a cf_topk_batch call */
   struct { uint32_t n_big, active; uint64_t big_pairs; } topk; /* control words 0..3 of a top-k selection */
+  uint32_t rec_cut[3]; /* end of the next piece of a cf_recommend_batch call, its first and end position */
+  struct { uint32_t bad, pad; uint64_t n_pos; } rec_check; /* device basket offsets: malformed?, positions */
+  struct { uint32_t n_big, pad; uint64_t big_pairs; } rec;  /* big baskets of a piece and their pairs */
 } smx_small_t;
 enum { DS_X, DS_Y, DS_V, DS_OUT, DS_WORDS }; /* the words of d_small: a single op's arguments, a one-word answer */
 
@@ -127,12 +130,19 @@ struct smatrix_s {
     smx_dbuf_t tk_big;     /* select state + histograms of the big segments */
     smx_dbuf_t tk_cids, tk_cscores; /* compaction regions of the big segments */
     smx_dbuf_t tk_ids, tk_scores;   /* scores of a piece */
+    /* basket recommendations (smatrix_cf_recommend_batch, smatrix_b200_basket_topk): the call's offsets and items
+     * on their way up, its positions' row counts and pair offsets, control words + big list + survivor counts,
+     * sorted item keys, the radix sorts' storage, staged survivors, reduced offsets and the reduced CSR, and the
+     * big baskets' lengths / offsets, sort keys, values, marks and their scan */
+    smx_dbuf_t rc_in, rc_pos, rc_ctl, rc_items, rc_sort, rc_tids, rc_tscores, rc_red, rc_rids, rc_rscores;
+    smx_dbuf_t rc_big, rc_keys, rc_vals, rc_flags;
     /* loading a snapshot (smatrix_b200_load_next): a window of file bytes, its tiles, their counts and offsets,
      * the op stream (x, y, v) and the (key, log2 size) fixups of a piece */
     smx_dbuf_t ld_raw, ld_tiles, ld_cnt, ld_off, ld_ops, ld_fix;
   } db;
   uint32_t topk_pairs;  /* SMATRIX_TOPK_PAIRS: pairs per piece of a cf_topk_batch call */
   uint64_t n_topk_big, n_topk_passes;
+  uint64_t n_rec_big; /* SMX_STAT_REC_BIG */
 
   unsigned long long* free_ptr[SMX_CLASSES]; /* device stacks of vacated buckets, per size class */
   uint32_t free_cap[SMX_CLASSES];
@@ -1333,6 +1343,178 @@ void smatrix_cf_topk_batch(smatrix_t* s, const uint32_t* items, size_t n, uint32
   leave(s);
 }
 
+/* ------------------------------------------------------------------------------ basket recommendations */
+#define REC_ITEM_BUDGET (1u << 30) /* positions per piece (the radix sorts count items in an int) */
+
+/* Aggregation and ranking of one piece of baskets, enqueued on s->stream (synchronises to read the number of big
+ * baskets and their pairs, and inside topk_run).  d_boff[0..nb] are absolute positions, base = d_boff[0], n_pos
+ * positions; d_items is indexed by absolute position; d_off[0..n_pos] is the per-position CSR of d_ids / d_scores
+ * (`pairs` pairs).  db.rc_ctl must already hold 64 + 8 * nb bytes. */
+static void rec_run(smatrix_t* s, uint32_t nb, const uint64_t* d_boff, uint64_t base, uint64_t n_pos,
+                    const uint32_t* d_items, const uint64_t* d_off, uint64_t pairs, const uint32_t* d_ids,
+                    const double* d_scores, uint32_t k, uint32_t* d_counts, uint32_t* d_oids, double* d_oscores) {
+  if (n_pos >= (1ull << 31)) smx_die("cf_recommend_batch: a piece of %llu items is more than 2^31 - 1",
+                                     (unsigned long long)n_pos);
+  uint32_t* ctl = s->db.rc_ctl.p;
+  uint32_t* big_list = ctl + 16;
+  uint32_t* cnt = big_list + nb;
+  uint64_t* keys = dbuf_need(s, &s->db.rc_items, (size_t)n_pos * 16 + 16);
+  uint64_t* sitems = keys + n_pos;
+  uint32_t* t_ids = dbuf_need(s, &s->db.rc_tids, (size_t)pairs * 4);
+  double* t_scores = dbuf_need(s, &s->db.rc_tscores, (size_t)pairs * 8);
+  uint64_t* red_off = dbuf_need(s, &s->db.rc_red, ((size_t)nb + 1 + smx_scan_scratch_items(nb)) * 8);
+  uint32_t* r_ids = dbuf_need(s, &s->db.rc_rids, (size_t)pairs * 4);
+  double* r_scores = dbuf_need(s, &s->db.rc_rscores, (size_t)pairs * 8);
+  size_t sort_bytes = smx_rec_sort_bytes((uint32_t)n_pos);
+  void* sort_tmp = dbuf_need(s, &s->db.rc_sort, sort_bytes);
+  CK(cudaMemsetAsync(ctl, 0, 64, s->stream));
+  smx_launch_rec_items(s->stream, nb, d_boff, base, d_items, (uint32_t)n_pos, keys, sitems, sort_tmp, sort_bytes);
+  smx_launch_rec_small(s->stream, nb, d_boff, base, d_off, d_ids, d_scores, sitems, big_list, ctl, t_ids, t_scores,
+                       cnt);
+  copy_d2h(s, &s->h_small->rec, ctl, 16, s->stream);
+  s->n_launches += 5;
+  CK(cudaStreamSynchronize(s->stream));
+  const uint32_t n_big = s->h_small->rec.n_big;
+  const uint64_t big_pairs = s->h_small->rec.big_pairs;
+  uint64_t *big_off = NULL, *bkeys = NULL, *fpos = NULL;
+  uint32_t* bvals = NULL;
+  if (n_big) {
+    if (big_pairs >= (1ull << 31))
+      smx_die("cf_recommend_batch: the big baskets of a piece hold %llu pairs, more than 2^31 - 1",
+              (unsigned long long)big_pairs);
+    const uint32_t P = (uint32_t)big_pairs;
+    const size_t scan_items = smx_scan_scratch_items(P > n_big ? P : n_big);
+    uint32_t* lens = dbuf_need(s, &s->db.rc_big, (size_t)n_big * 4 + ((size_t)n_big + 1 + scan_items) * 8 + 16);
+    big_off = (uint64_t*)(((uintptr_t)(lens + n_big) + 7) & ~(uintptr_t)7);
+    uint64_t* scan_tmp = big_off + n_big + 1;
+    uint64_t* keys_a = dbuf_need(s, &s->db.rc_keys, (size_t)P * 16);
+    bkeys = keys_a + P;
+    uint32_t* vals_a = dbuf_need(s, &s->db.rc_vals, (size_t)P * 8);
+    bvals = vals_a + P;
+    uint32_t* flags = dbuf_need(s, &s->db.rc_flags, (size_t)P * 4 + ((size_t)P + 1) * 8 + 16);
+    fpos = (uint64_t*)(((uintptr_t)(flags + P) + 7) & ~(uintptr_t)7);
+    sort_bytes = smx_rec_sort_bytes(P);
+    sort_tmp = dbuf_need(s, &s->db.rc_sort, sort_bytes);
+    smx_launch_rec_big(s->stream, big_list, n_big, P, d_boff, base, d_off, d_ids, sitems, lens, big_off, keys_a, bkeys,
+                       vals_a, bvals, flags, fpos, scan_tmp, sort_tmp, sort_bytes, cnt);
+    s->n_launches += 12;
+    s->n_rec_big += n_big;
+  }
+  smx_launch_scan(s->stream, cnt, nb, 0, red_off, red_off + (size_t)nb + 1);
+  smx_launch_rec_emit(s->stream, nb, d_boff, base, d_off, d_scores, cnt, red_off, t_ids, t_scores, big_list, n_big,
+                      (uint32_t)big_pairs, big_off, bkeys, bvals, fpos, r_ids, r_scores);
+  s->n_launches += n_big ? 5 : 4;
+  topk_run(s, nb, red_off, r_ids, r_scores, k, d_counts, d_oids, d_oscores);
+}
+
+void smatrix_b200_basket_topk(smatrix_t* s, size_t n, const uint64_t* d_basket_off, const uint32_t* d_items,
+                              const uint64_t* d_offsets, const uint32_t* d_ids, const double* d_scores, uint32_t k,
+                              uint32_t* d_counts, uint32_t* d_out_ids, double* d_out_scores) {
+  if (k < 1 || k > SMX_TOPK_MAX_K) smx_die("basket_topk: k = %u is outside 1..%u", k, SMX_TOPK_MAX_K);
+  if (n >= 0xFFFFFFFFull) smx_die("basket_topk: too many baskets in one call");
+  if (!n) return;
+  enter(s);
+  const uint32_t nb = (uint32_t)n;
+  dbuf_need(s, &s->db.rc_ctl, 64 + (size_t)nb * 8);
+  copy_d2h(s, &s->h_small->rec_check.n_pos, d_basket_off + nb, 8, s->stream);
+  CK(cudaStreamSynchronize(s->stream));
+  const uint64_t n_pos = s->h_small->rec_check.n_pos;
+  copy_d2h(s, &s->h_small->row_total, d_offsets + n_pos, 8, s->stream);
+  CK(cudaStreamSynchronize(s->stream));
+  rec_run(s, nb, d_basket_off, 0, n_pos, d_items, d_offsets, s->h_small->row_total, d_ids, d_scores, k, d_counts,
+          d_out_ids, d_out_scores);
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+}
+
+/* per basket, the k best items by the summed scores of the basket's neighbour lists: the lists as
+ * smatrix_cf_neighbors_batch computes them, for pieces of baskets whose rows fit SMATRIX_TOPK_PAIRS, each piece
+ * aggregated and ranked by rec_run */
+void smatrix_cf_recommend_batch(smatrix_t* s, const uint64_t* basket_off, const uint32_t* items, size_t n,
+                                uint32_t k, uint32_t* counts, uint32_t* ids, double* scores) {
+  if (k < 1 || k > SMX_TOPK_MAX_K) smx_die("cf_recommend_batch: k = %u is outside 1..%u", k, SMX_TOPK_MAX_K);
+  if (n >= 0xFFFFFFFFull) smx_die("cf_recommend_batch: too many baskets in one call");
+  if (!n) return;
+  if (!basket_off) smx_die("cf_recommend_batch: basket_off is NULL");
+  enter(s);
+  const int out_dev = is_device_ptr(counts);
+  if (is_device_ptr(ids) != out_dev || is_device_ptr(scores) != out_dev)
+    smx_die("cf_recommend_batch: counts, ids and scores must be all host or all device arrays");
+  const uint32_t nb = (uint32_t)n;
+  const int in_dev = is_device_ptr(basket_off);
+  uint32_t* ctl = dbuf_need(s, &s->db.rc_ctl, 64 + (size_t)nb * 8);
+  uint64_t n_pos;
+  if (in_dev) {
+    CK(cudaMemsetAsync(ctl, 0, 16, s->stream));
+    smx_launch_rec_check(s->stream, basket_off, nb, ctl);
+    copy_d2h(s, &s->h_small->rec_check, ctl, 16, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    s->n_launches++;
+    n_pos = s->h_small->rec_check.n_pos;
+    if (s->h_small->rec_check.bad) n_pos = ~0ull;
+  } else {
+    n_pos = basket_off[0] == 0 ? basket_off[n] : ~0ull;
+    for (size_t i = 0; i < n && n_pos != ~0ull; i++)
+      if (basket_off[i + 1] < basket_off[i]) n_pos = ~0ull;
+  }
+  if (n_pos > 0xFFFFFFFEull)
+    smx_die("cf_recommend_batch: malformed basket offsets (they must start at 0, never decrease and end at most at "
+            "2^32 - 2)");
+  if (n_pos && is_device_ptr(items) != in_dev)
+    smx_die("cf_recommend_batch: basket_off and items must both be host or both be device arrays");
+  const uint32_t npos = (uint32_t)n_pos;
+  const uint64_t* d_boff = basket_off;
+  const uint32_t* d_items = items;
+  if (!in_dev) {
+    char* in = dbuf_need(s, &s->db.rc_in, ((size_t)nb + 1) * 8 + (size_t)npos * 4);
+    copy_h2d(s, in, basket_off, ((size_t)nb + 1) * 8, s->stream);
+    d_boff = (const uint64_t*)in;
+    if (npos) copy_h2d(s, in + ((size_t)nb + 1) * 8, items, (size_t)npos * 4, s->stream);
+    d_items = (const uint32_t*)(in + ((size_t)nb + 1) * 8);
+  }
+  /* the row lengths of the whole call decide where the pieces end */
+  const size_t scan_items = smx_scan_scratch_items(npos);
+  uint64_t* d_pos = dbuf_need(s, &s->db.rc_pos, ((size_t)npos + 1 + scan_items) * 8 + (size_t)npos * 4);
+  uint32_t* d_cnt = (uint32_t*)(d_pos + npos + 1 + scan_items);
+  smx_launch_row_counts(s->stream, view_of(s), d_items, npos, d_cnt, NULL, NULL, NULL);
+  smx_launch_scan(s->stream, d_cnt, npos, 0, d_pos, d_pos + (size_t)npos + 1);
+  s->n_launches += 4;
+  for (uint32_t lo = 0, hi; lo < nb; lo = hi) {
+    smx_launch_rec_cut(s->stream, d_pos, d_boff, nb, lo, s->topk_pairs, REC_ITEM_BUDGET, ctl + 4);
+    copy_d2h(s, s->h_small->rec_cut, ctl + 4, 12, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    s->n_launches++;
+    hi = s->h_small->rec_cut[0];
+    const uint32_t p_lo = s->h_small->rec_cut[1], p_n = s->h_small->rec_cut[2] - p_lo, np = hi - lo;
+    const smx_rows_t r = gather_rows(s, d_items + p_lo, 1, p_n, UINT64_MAX, NULL);
+    uint32_t* p_ids = dbuf_need(s, &s->db.tk_ids, (size_t)r.total * 4);
+    double* p_scores = dbuf_need(s, &s->db.tk_scores, (size_t)r.total * 8);
+    if (r.total) {
+      smx_launch_cf_scores(s->stream, view_of(s), r.ids, p_n, r.offsets, r.pairs, p_ids, p_scores);
+      s->n_launches++;
+    }
+    uint32_t* oc = counts + lo;
+    uint32_t* oi = ids + (size_t)lo * k;
+    double* os = scores + (size_t)lo * k;
+    if (!out_dev) {
+      char* o = dbuf_need(s, &s->db.host_out, (size_t)np * (12ull * k + 4));
+      os = (double*)o;
+      oi = (uint32_t*)(o + (size_t)np * k * 8);
+      oc = oi + (size_t)np * k;
+    }
+    rec_run(s, np, d_boff + lo, p_lo, p_n, d_items, r.offsets, r.total, p_ids, p_scores, k, oc, oi, os);
+    if (!out_dev) {
+      copy_d2h(s, counts + lo, oc, (size_t)np * 4, s->stream);
+      copy_d2h(s, ids + (size_t)lo * k, oi, (size_t)np * k * 4, s->stream);
+      copy_d2h(s, scores + (size_t)lo * k, os, (size_t)np * k * 8, s->stream);
+    }
+  }
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+}
+
 /* ------------------------------------------------------------------------------ single ops */
 /* the answer of a single op, d_small[DS_OUT] */
 static uint32_t single_answer(smatrix_t* s) {
@@ -2141,6 +2323,7 @@ uint64_t smatrix_b200_stat(smatrix_t* s, int which) {
     case SMX_STAT_ALLOCS: r = s->n_allocs; break;
     case SMX_STAT_TOPK_BIG: r = s->n_topk_big; break;
     case SMX_STAT_TOPK_PASSES: r = s->n_topk_passes; break;
+    case SMX_STAT_REC_BIG: r = s->n_rec_big; break;
     case SMX_STAT_H2D_BYTES: r = s->h2d_bytes; break;
     case SMX_STAT_D2H_BYTES: r = s->d2h_bytes; break;
     case SMX_STAT_DIR_CAP: r = s->dir_cap; break;

@@ -204,6 +204,36 @@ void smx_launch_topk_finish(smx_stream_t stream, const void* big_scratch, uint32
                             const double* c_scores, uint32_t k, uint32_t* counts, uint32_t* out_ids, double* out_scores);
 void smx_launch_topk_cut(smx_stream_t stream, const uint64_t* offsets, uint32_t n, uint32_t lo, uint64_t budget,
                          uint32_t* out);
+/* basket recommendations (kernel comment in smx_kernels.cu).  A piece of nb baskets: boff[0..nb] absolute
+ * positions, base = boff[0]; items indexed by position; off[0 .. boff[nb] - base] the per-position CSR of ids /
+ * scores.  Order: rec_items (sorted item keys) -> rec_small (classify into ctl as top-k's: ctl[0] big count,
+ * ctl[2..3] big pairs; small baskets into the staging arrays t_*, cnt[b] survivors) -> (host reads ctl) ->
+ * rec_big (cnt of the big baskets) -> smx_launch_scan(cnt) = red_off -> rec_emit (the reduced CSR r_*).
+ * sort_tmp: smx_rec_sort_bytes(max(n_pos, n_pairs)); scan_tmp: smx_scan_scratch_items(max(n_big, n_pairs)). */
+size_t smx_rec_sort_bytes(uint32_t n);
+void smx_launch_rec_items(smx_stream_t stream, uint32_t nb, const uint64_t* boff, uint64_t base, const uint32_t* items,
+                          uint32_t n_pos, uint64_t* keys, uint64_t* sitems, void* sort_tmp, size_t sort_bytes);
+void smx_launch_rec_small(smx_stream_t stream, uint32_t nb, const uint64_t* boff, uint64_t base, const uint64_t* off,
+                          const uint32_t* ids, const double* scores, const uint64_t* sitems, uint32_t* big_list,
+                          uint32_t* ctl, uint32_t* t_ids, double* t_scores, uint32_t* cnt);
+void smx_launch_rec_big(smx_stream_t stream, const uint32_t* big_list, uint32_t n_big, uint32_t n_pairs,
+                        const uint64_t* boff, uint64_t base, const uint64_t* off, const uint32_t* ids,
+                        const uint64_t* sitems, uint32_t* lens, uint64_t* big_off /* n_big + 1 */, uint64_t* keys_a,
+                        uint64_t* keys_b, uint32_t* vals_a, uint32_t* vals_b, uint32_t* flags,
+                        uint64_t* fpos /* n_pairs + 1 */, uint64_t* scan_tmp, void* sort_tmp, size_t sort_bytes,
+                        uint32_t* cnt);
+void smx_launch_rec_emit(smx_stream_t stream, uint32_t nb, const uint64_t* boff, uint64_t base, const uint64_t* off,
+                         const double* scores, const uint32_t* cnt, const uint64_t* red_off, const uint32_t* t_ids,
+                         const double* t_scores, const uint32_t* big_list, uint32_t n_big, uint32_t n_pairs,
+                         const uint64_t* big_off, const uint64_t* keys /* rec_big's keys_b */,
+                         const uint32_t* vals /* vals_b */, const uint64_t* fpos, uint32_t* r_ids, double* r_scores);
+/* one thread: out[0] = end of the piece of baskets from lo whose rows hold <= budget pairs (pos_off: positions'
+ * pair offsets of the whole call) and <= item_budget items, at least one basket; out[1..2] = its positions */
+void smx_launch_rec_cut(smx_stream_t stream, const uint64_t* pos_off, const uint64_t* boff, uint32_t nb, uint32_t lo,
+                        uint64_t budget, uint64_t item_budget, uint32_t* out);
+/* out[0] |= 1 if boff[0..nb] is not a valid basket CSR (starts at 0, never decreases, ends <= 2^32 - 2);
+ * out[2..3] = boff[nb] as u64.  out[0] zeroed. */
+void smx_launch_rec_check(smx_stream_t stream, const uint64_t* boff, uint32_t nb, uint32_t* out);
 void smx_launch_list_rows(smx_stream_t stream, smx_view_t v, uint32_t* keys, uint32_t* counter /* zeroed */);
 void smx_launch_row_slog(smx_stream_t stream, smx_view_t v, const uint32_t* xs, uint32_t n, uint32_t* out);
 void smx_launch_snap_units(smx_stream_t stream, const uint32_t* counts, const uint32_t* slogs, uint32_t n,

@@ -1601,6 +1601,244 @@ __global__ void k_topk_cut(const ull* offsets, uint32_t n, uint32_t lo, ull budg
   out[0] = a;
 }
 
+/* ---- basket recommendations (smatrix_cf_recommend_batch, smatrix_b200_basket_topk) ---------------------------
+ * A piece of nb baskets: boff[0..nb] are absolute positions (base = boff[0]), items[p] is the item at position p,
+ * and off[p - base] .. off[p - base + 1] is that position's neighbour list in ids / scores.  Basket b's pairs are
+ * [off[boff[b] - base], off[boff[b + 1] - base]), position-major, so ordering them stably by id puts every id's
+ * contributions in position order, and one thread adds each run up left to right (IEEE double, one rounding per
+ * addition).  A run survives unless its id is 0 or an item of the basket (binary search in the basket's items,
+ * sorted once by k_rec_item_keys + a radix sort of (basket << 32 | item) keys).  The survivors, in id order, are
+ * a reduced CSR that the top-k selection ranks.  Size classes as top-k's:
+ *   k_rec_warp / k_rec_block  baskets of <= TOPK_WARP_MAX / TOPK_BLOCK_MAX pairs: bitonic sort of (id << 32 |
+ *                             local index) keys in shared memory; survivors go to the basket's own slots of the
+ *                             staging arrays, their number to cnt[b]
+ *   big baskets               all of a piece's at once: (slot << 32 | id) keys of their pairs with the local index
+ *                             as value, one stable radix sort, k_rec_big_flag marks the surviving run heads, a scan
+ *                             of the marks ranks them and k_rec_big_emit sums each run straight into the reduced CSR
+ * k_rec_compact moves the small baskets' survivors from the staging arrays to the reduced CSR. */
+__device__ __forceinline__ double rec_add(double a, double b) {
+#ifdef SMX_HOSTSIM
+  return a + b;
+#else
+  return __dadd_rn(a, b); /* never contracted or reordered */
+#endif
+}
+/* is `id` excluded from basket b, whose sorted (b << 32 | item) keys are sitems[lo..hi)? */
+__device__ __forceinline__ bool rec_excluded(uint32_t id, uint32_t b, const ull* sitems, ull lo, ull hi) {
+  if (id == 0u) return true;
+  const ull want = ((ull)b << 32) | id;
+  while (lo < hi) {
+    const ull m = lo + (hi - lo) / 2u;
+    const ull v = sitems[m];
+    if (v == want) return true;
+    if (v < want) lo = m + 1u; else hi = m;
+  }
+  return false;
+}
+/* bitonic sort of N (power of two) keys, ascending */
+template <bool BLOCK>
+__device__ void rec_sort(ull* key, uint32_t N, uint32_t t, uint32_t T) {
+  for (uint32_t run = 2; run <= N; run <<= 1)
+    for (uint32_t j = run >> 1; j > 0; j >>= 1) {
+      for (uint32_t i = t; i < N; i += T) {
+        const uint32_t l = i ^ j;
+        if (l <= i) continue;
+        const ull a = key[i], c = key[l];
+        if ((i & run) == 0 ? a > c : a < c) {
+          key[i] = c;
+          key[l] = a;
+        }
+      }
+      topk_sync<BLOCK>();
+    }
+}
+/* one small basket by a warp or a block: sort, run sums, survivors in id order to t_ids / t_scores[lo..) */
+template <bool BLOCK>
+__device__ void rec_segment(uint32_t b, ull p0, ull p1, ull lo, uint32_t len, const uint32_t* ids,
+                            const double* scores, const ull* sitems, ull* key, uint32_t t, uint32_t T,
+                            uint32_t* t_ids, double* t_scores, uint32_t* cnt) {
+  uint32_t N = 1u;
+  while (N < len) N <<= 1;
+  for (uint32_t i = t; i < N; i += T) key[i] = i < len ? ((ull)ids[lo + i] << 32) | i : ~0ull;
+  topk_sync<BLOCK>();
+  rec_sort<BLOCK>(key, N, t, T);
+  uint32_t kept = 0u;
+  for (uint32_t c0 = 0; c0 < len; c0 += T) { /* every thread takes the same number of turns */
+    const uint32_t j = c0 + t;
+    bool keep = false;
+    uint32_t id = 0u;
+    double sum = 0.0;
+    if (j < len) {
+      id = (uint32_t)(key[j] >> 32);
+      keep = (j == 0u || (uint32_t)(key[j - 1] >> 32) != id) && !rec_excluded(id, b, sitems, p0, p1);
+      if (keep)
+        for (uint32_t q = j; q < len && (uint32_t)(key[q] >> 32) == id; ++q)
+          sum = rec_add(sum, scores[lo + (uint32_t)key[q]]);
+    }
+    uint32_t w, tot;
+    if (BLOCK) {
+      ull all;
+      w = (uint32_t)block_exclusive_scan(keep ? 1ull : 0ull, &all);
+      tot = (uint32_t)all;
+    } else {
+      const unsigned m = __ballot_sync(SMX_FULL, keep);
+      w = (uint32_t)__popc(m & ((1u << t) - 1u));
+      tot = (uint32_t)__popc(m);
+    }
+    if (keep) {
+      t_ids[lo + kept + w] = id;
+      t_scores[lo + kept + w] = sum;
+    }
+    kept += tot;
+  }
+  if (t == 0u) cnt[b] = kept;
+  topk_sync<BLOCK>(); /* before the buffer takes the next basket */
+}
+
+/* keys of the piece's items: (basket << 32 | item) at position p - base; one warp per basket */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_item_keys(uint32_t nb, const ull* boff, ull base, const uint32_t* items, ull* keys) {
+  const uint32_t lane = lane_id();
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) / SMX_WARP;
+  const uint32_t nwarps = gridDim.x * blockDim.x / SMX_WARP;
+  for (uint32_t b = warp; b < nb; b += nwarps)
+    for (ull p = boff[b] + lane; p < boff[b + 1]; p += SMX_WARP) keys[p - base] = ((ull)b << 32) | items[p];
+}
+
+/* big baskets -> list; ctl[0] = their number, ctl[2..3] = their pairs (u64) */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_classify(uint32_t nb, const ull* boff, ull base, const ull* off, uint32_t* big_list, uint32_t* ctl) {
+  for (uint32_t b = blockIdx.x * blockDim.x + threadIdx.x; b < nb; b += gridDim.x * blockDim.x) {
+    const ull len = off[boff[b + 1] - base] - off[boff[b] - base];
+    if (len <= TOPK_BLOCK_MAX) continue;
+    big_list[agg_inc(&ctl[0])] = b;
+    atomicAdd((ull*)(ctl + 2), len);
+  }
+}
+
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_warp(uint32_t nb, const ull* boff, ull base, const ull* off, const uint32_t* ids, const double* scores,
+           const ull* sitems, uint32_t* t_ids, double* t_scores, uint32_t* cnt) {
+  __shared__ ull s_key[SMX_BLOCK / SMX_WARP][TOPK_WARP_MAX];
+  const uint32_t lane = lane_id(), wib = threadIdx.x / SMX_WARP;
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) / SMX_WARP;
+  const uint32_t nwarps = gridDim.x * blockDim.x / SMX_WARP;
+  for (uint32_t b = warp; b < nb; b += nwarps) {
+    const ull p0 = boff[b] - base, p1 = boff[b + 1] - base, lo = off[p0], len = off[p1] - lo;
+    if (len > TOPK_WARP_MAX) continue;
+    rec_segment<false>(b, p0, p1, lo, (uint32_t)len, ids, scores, sitems, s_key[wib], lane, SMX_WARP, t_ids, t_scores,
+                       cnt);
+  }
+}
+
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_block(uint32_t nb, const ull* boff, ull base, const ull* off, const uint32_t* ids, const double* scores,
+            const ull* sitems, uint32_t* t_ids, double* t_scores, uint32_t* cnt) {
+  __shared__ ull s_key[TOPK_BLOCK_MAX];
+  for (uint32_t b = blockIdx.x; b < nb; b += gridDim.x) {
+    const ull p0 = boff[b] - base, p1 = boff[b + 1] - base, lo = off[p0], len = off[p1] - lo;
+    if (len <= TOPK_WARP_MAX || len > TOPK_BLOCK_MAX) continue;
+    rec_segment<true>(b, p0, p1, lo, (uint32_t)len, ids, scores, sitems, s_key, threadIdx.x, blockDim.x, t_ids,
+                      t_scores, cnt);
+  }
+}
+
+/* pairs of big basket j (= big_list[j]) */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_big_lens(const uint32_t* big_list, uint32_t n_big, const ull* boff, ull base, const ull* off, uint32_t* lens) {
+  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n_big; j += gridDim.x * blockDim.x) {
+    const uint32_t b = big_list[j];
+    lens[j] = (uint32_t)(off[boff[b + 1] - base] - off[boff[b] - base]);
+  }
+}
+/* (slot << 32 | id) keys and local indices of the big baskets' pairs, slot j at big_off[j] */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_big_keys(const uint32_t* big_list, uint32_t first, const ull* boff, ull base, const ull* off,
+               const uint32_t* ids, const ull* big_off, ull* keys, uint32_t* vals) {
+  const uint32_t j = first + blockIdx.y, b = big_list[j];
+  const ull lo = off[boff[b] - base], len = off[boff[b + 1] - base] - lo, at = big_off[j];
+  for (ull q = (ull)blockIdx.x * blockDim.x + threadIdx.x; q < len; q += (ull)gridDim.x * blockDim.x) {
+    keys[at + q] = ((ull)j << 32) | ids[lo + q];
+    vals[at + q] = (uint32_t)q;
+  }
+}
+/* flags[p] = 1 where a run of equal keys starts and its id survives */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_big_flag(const ull* keys, uint32_t P, const uint32_t* big_list, const ull* boff, ull base, const ull* sitems,
+               uint32_t* flags) {
+  for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
+    const ull key = keys[p];
+    bool keep = p == 0u || keys[p - 1] != key;
+    if (keep) {
+      const uint32_t b = big_list[(uint32_t)(key >> 32)];
+      keep = !rec_excluded((uint32_t)key, b, sitems, boff[b] - base, boff[b + 1] - base);
+    }
+    flags[p] = keep ? 1u : 0u;
+  }
+}
+/* survivors per big basket from the scan of the flags */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_big_count(const uint32_t* big_list, uint32_t n_big, const ull* big_off, const ull* fpos, uint32_t* cnt) {
+  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n_big; j += gridDim.x * blockDim.x)
+    cnt[big_list[j]] = (uint32_t)(fpos[big_off[j + 1]] - fpos[big_off[j]]);
+}
+/* every surviving run of the big baskets: its sum, at its rank inside the basket's reduced segment */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_big_emit(const ull* keys, const uint32_t* vals, uint32_t P, const uint32_t* big_list, const ull* big_off,
+               const ull* boff, ull base, const ull* off, const double* scores, const ull* fpos, const ull* red_off,
+               uint32_t* r_ids, double* r_scores) {
+  for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
+    if (fpos[p + 1] == fpos[p]) continue;
+    const ull key = keys[p];
+    const uint32_t j = (uint32_t)(key >> 32), b = big_list[j];
+    const ull lo = off[boff[b] - base];
+    double sum = 0.0;
+    for (uint32_t q = p; q < P && keys[q] == key; ++q) sum = rec_add(sum, scores[lo + vals[q]]);
+    const ull at = red_off[b] + (fpos[p] - fpos[big_off[j]]);
+    r_ids[at] = (uint32_t)key;
+    r_scores[at] = sum;
+  }
+}
+/* the small baskets' survivors from their staging slots into the reduced CSR; one warp per basket */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_rec_compact(uint32_t nb, const ull* boff, ull base, const ull* off, const uint32_t* cnt, const ull* red_off,
+              const uint32_t* t_ids, const double* t_scores, uint32_t* r_ids, double* r_scores) {
+  const uint32_t lane = lane_id();
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) / SMX_WARP;
+  const uint32_t nwarps = gridDim.x * blockDim.x / SMX_WARP;
+  for (uint32_t b = warp; b < nb; b += nwarps) {
+    const ull lo = off[boff[b] - base];
+    if (off[boff[b + 1] - base] - lo > TOPK_BLOCK_MAX) continue;
+    const ull to = red_off[b];
+    for (uint32_t q = lane; q < cnt[b]; q += SMX_WARP) {
+      r_ids[to + q] = t_ids[lo + q];
+      r_scores[to + q] = t_scores[lo + q];
+    }
+  }
+}
+/* one thread: the end of the piece of baskets that starts at basket lo = the last basket whose rows still fit the
+ * pair budget and whose items fit the item budget (at least one basket) -> out[0]; its positions -> out[1..2] */
+__global__ void k_rec_cut(const ull* pos_off, const ull* boff, uint32_t nb, uint32_t lo, ull budget, ull item_budget,
+                          uint32_t* out) {
+  uint32_t a = lo + 1u, b = nb; /* answer in [a, b] */
+  while (a < b) {
+    const uint32_t m = a + (b - a + 1u) / 2u;
+    if (pos_off[boff[m]] - pos_off[boff[lo]] <= budget && boff[m] - boff[lo] <= item_budget) a = m; else b = m - 1u;
+  }
+  out[0] = a;
+  out[1] = (uint32_t)boff[lo];
+  out[2] = (uint32_t)boff[a];
+}
+/* basket offsets that do not start at 0, decrease or end past 2^32 - 2 set out[0]; out[2..3] = boff[nb] (u64) */
+__global__ void __launch_bounds__(SMX_BLOCK) k_rec_check(const ull* boff, uint32_t nb, uint32_t* out) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < nb; i += gridDim.x * blockDim.x)
+    if (boff[i + 1] < boff[i] || (i == 0u && boff[0] != 0ull)) atomicOr(&out[0], 1u);
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    if (boff[nb] > 0xFFFFFFFEull) atomicOr(&out[0], 1u);
+    *(ull*)(out + 2) = boff[nb];
+  }
+}
+
 /* ---- snapshot support (file mode, reference src/smatrix.c:30-72) --------------------------- */
 /* all row ids of the directory, in no particular order */
 __global__ void __launch_bounds__(SMX_BLOCK) k_list_rows(smx_view_t V, uint32_t* keys, uint32_t* counter) {
@@ -2628,6 +2866,107 @@ extern "C" void smx_launch_topk_finish(smx_stream_t st, const void* big_scratch,
 extern "C" void smx_launch_topk_cut(smx_stream_t st, const uint64_t* offsets, uint32_t n, uint32_t lo, uint64_t budget,
                                     uint32_t* out) {
   SMX_LAUNCH(k_topk_cut, 1, 1, st, (const ull*)offsets, n, lo, (ull)budget, out);
+}
+
+static inline int rec_key_bits(uint32_t n) { /* 32 id bits + enough for slots 0 .. n-1 */
+  int b = 32;
+  while (b < 64 && (1ull << (b - 32)) < (ull)n) b++;
+  return b;
+}
+extern "C" size_t smx_rec_sort_bytes(uint32_t n) {
+#ifdef SMX_HOSTSIM
+  (void)n;
+  return 64;
+#else
+  size_t bytes = 0, bytes_keys = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, bytes, (const ull*)nullptr, (ull*)nullptr, (const uint32_t*)nullptr,
+                                  (uint32_t*)nullptr, (int)n, 0, 64);
+  cub::DeviceRadixSort::SortKeys(nullptr, bytes_keys, (const ull*)nullptr, (ull*)nullptr, (int)n, 0, 64);
+  return (bytes > bytes_keys ? bytes : bytes_keys) + 256;
+#endif
+}
+extern "C" void smx_launch_rec_items(smx_stream_t st, uint32_t nb, const uint64_t* boff, uint64_t base,
+                                     const uint32_t* items, uint32_t n_pos, uint64_t* keys, uint64_t* sitems,
+                                     void* sort_tmp, size_t sort_bytes) {
+  if (!n_pos) return;
+  SMX_LAUNCH(k_rec_item_keys, grid_for((ull)nb * SMX_WARP), SMX_BLOCK, st, nb, (const ull*)boff, (ull)base, items,
+             (ull*)keys);
+#ifdef SMX_HOSTSIM
+  (void)sort_tmp; (void)sort_bytes;
+  memcpy(sitems, keys, (size_t)n_pos * 8);
+  std::sort(sitems, sitems + n_pos);
+#else
+  cub::DeviceRadixSort::SortKeys(sort_tmp, sort_bytes, (const ull*)keys, (ull*)sitems, (int)n_pos, 0, rec_key_bits(nb),
+                                 (cudaStream_t)st);
+#endif
+}
+extern "C" void smx_launch_rec_small(smx_stream_t st, uint32_t nb, const uint64_t* boff, uint64_t base,
+                                     const uint64_t* off, const uint32_t* ids, const double* scores,
+                                     const uint64_t* sitems, uint32_t* big_list, uint32_t* ctl, uint32_t* t_ids,
+                                     double* t_scores, uint32_t* cnt) {
+  if (!nb) return;
+  SMX_LAUNCH(k_rec_classify, grid_for(nb), SMX_BLOCK, st, nb, (const ull*)boff, (ull)base, (const ull*)off, big_list,
+             ctl);
+  SMX_LAUNCH(k_rec_warp, grid_for((ull)nb * SMX_WARP), SMX_BLOCK, st, nb, (const ull*)boff, (ull)base, (const ull*)off,
+             ids, scores, (const ull*)sitems, t_ids, t_scores, cnt);
+  const uint32_t cap = (uint32_t)smx_grid_blocks();
+  SMX_LAUNCH(k_rec_block, nb < cap ? nb : cap, SMX_BLOCK, st, nb, (const ull*)boff, (ull)base, (const ull*)off, ids,
+             scores, (const ull*)sitems, t_ids, t_scores, cnt);
+}
+extern "C" void smx_launch_rec_big(smx_stream_t st, const uint32_t* big_list, uint32_t n_big, uint32_t n_pairs,
+                                   const uint64_t* boff, uint64_t base, const uint64_t* off, const uint32_t* ids,
+                                   const uint64_t* sitems, uint32_t* lens, uint64_t* big_off, uint64_t* keys_a,
+                                   uint64_t* keys_b, uint32_t* vals_a, uint32_t* vals_b, uint32_t* flags,
+                                   uint64_t* fpos, uint64_t* scan_tmp, void* sort_tmp, size_t sort_bytes,
+                                   uint32_t* cnt) {
+  if (!n_big) return;
+  SMX_LAUNCH(k_rec_big_lens, grid_for(n_big), SMX_BLOCK, st, big_list, n_big, (const ull*)boff, (ull)base,
+             (const ull*)off, lens);
+  smx_launch_scan(st, lens, n_big, 0, big_off, scan_tmp);
+  for (uint32_t first = 0; first < n_big; first += 32768u) {
+    const uint32_t c = (n_big - first < 32768u) ? n_big - first : 32768u;
+    SMX_LAUNCH(k_rec_big_keys, dim3(TOPK_BIG_BLOCKS, c, 1u), SMX_BLOCK, st, big_list, first, (const ull*)boff,
+               (ull)base, (const ull*)off, ids, (const ull*)big_off, (ull*)keys_a, vals_a);
+  }
+#ifdef SMX_HOSTSIM
+  (void)sort_tmp; (void)sort_bytes;
+  {
+    std::vector<uint32_t> order(n_pairs);
+    for (uint32_t p = 0; p < n_pairs; p++) order[p] = p;
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return keys_a[a] < keys_a[b]; });
+    for (uint32_t p = 0; p < n_pairs; p++) { keys_b[p] = keys_a[order[p]]; vals_b[p] = vals_a[order[p]]; }
+  }
+#else
+  /* LSD radix sort: stable, so the pairs of one (basket, id) stay in position order */
+  cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, (const ull*)keys_a, (ull*)keys_b, (const uint32_t*)vals_a,
+                                  vals_b, (int)n_pairs, 0, rec_key_bits(n_big), (cudaStream_t)st);
+#endif
+  SMX_LAUNCH(k_rec_big_flag, grid_for(n_pairs), SMX_BLOCK, st, (const ull*)keys_b, n_pairs, big_list, (const ull*)boff,
+             (ull)base, (const ull*)sitems, flags);
+  smx_launch_scan(st, flags, n_pairs, 0, fpos, scan_tmp);
+  SMX_LAUNCH(k_rec_big_count, grid_for(n_big), SMX_BLOCK, st, big_list, n_big, (const ull*)big_off, (const ull*)fpos,
+             cnt);
+}
+extern "C" void smx_launch_rec_emit(smx_stream_t st, uint32_t nb, const uint64_t* boff, uint64_t base,
+                                    const uint64_t* off, const double* scores, const uint32_t* cnt,
+                                    const uint64_t* red_off, const uint32_t* t_ids, const double* t_scores,
+                                    const uint32_t* big_list, uint32_t n_big, uint32_t n_pairs, const uint64_t* big_off,
+                                    const uint64_t* keys, const uint32_t* vals, const uint64_t* fpos, uint32_t* r_ids,
+                                    double* r_scores) {
+  if (!nb) return;
+  SMX_LAUNCH(k_rec_compact, grid_for((ull)nb * SMX_WARP), SMX_BLOCK, st, nb, (const ull*)boff, (ull)base,
+             (const ull*)off, cnt, (const ull*)red_off, t_ids, t_scores, r_ids, r_scores);
+  if (n_big)
+    SMX_LAUNCH(k_rec_big_emit, grid_for(n_pairs), SMX_BLOCK, st, (const ull*)keys, vals, n_pairs, big_list,
+               (const ull*)big_off, (const ull*)boff, (ull)base, (const ull*)off, scores, (const ull*)fpos,
+               (const ull*)red_off, r_ids, r_scores);
+}
+extern "C" void smx_launch_rec_cut(smx_stream_t st, const uint64_t* pos_off, const uint64_t* boff, uint32_t nb,
+                                   uint32_t lo, uint64_t budget, uint64_t item_budget, uint32_t* out) {
+  SMX_LAUNCH(k_rec_cut, 1, 1, st, (const ull*)pos_off, (const ull*)boff, nb, lo, (ull)budget, (ull)item_budget, out);
+}
+extern "C" void smx_launch_rec_check(smx_stream_t st, const uint64_t* boff, uint32_t nb, uint32_t* out) {
+  SMX_LAUNCH(k_rec_check, grid_for(nb), SMX_BLOCK, st, (const ull*)boff, nb, out);
 }
 extern "C" void smx_launch_sum_values(smx_stream_t st, smx_view_t v, uint32_t* big_list, uint32_t* big_counter) {
   SMX_LAUNCH(k_sum_values, grid_for(v.dir_cap * SMX_WARP), SMX_BLOCK, st, v, big_list, big_counter);

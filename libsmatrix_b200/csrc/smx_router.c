@@ -921,6 +921,75 @@ void smatrix_b200_shard_cf_topk_batch(smatrix_shard_t* sh, const uint32_t* items
   if (c.scratch) smatrix_b200_dev_free(sh->local, c.scratch);
 }
 
+/* Basket recommendations across ranks: the flattened items' lists come as in shard_cf_neighbors_batch, and
+ * smatrix_b200_basket_topk aggregates and ranks them on this rank's GPU, the same code as the single-GPU call. */
+void smatrix_b200_shard_cf_recommend_batch(smatrix_shard_t* sh, const uint64_t* basket_off, const uint32_t* items,
+                                           size_t n, uint32_t k, uint32_t* counts, uint32_t* ids, double* scores) {
+  if (k < 1 || k > 1024u) rt_die(sh, "cf_recommend_batch: k = %u is outside 1..1024", k);
+  if (n >= 0xFFFFFFFEull) rt_die(sh, "cf_recommend_batch: too many baskets in one call");
+  const int out_dev = rt_is_dev(sh, counts);
+  if (n && (rt_is_dev(sh, ids) != out_dev || rt_is_dev(sh, scores) != out_dev))
+    rt_die(sh, "cf_recommend_batch: counts, ids and scores must be all host or all device arrays");
+  /* the offsets on the host, to check them and to know the number of items */
+  const int in_dev = n && rt_is_dev(sh, basket_off);
+  uint64_t* hb = NULL;
+  uint64_t n_pos = 0;
+  if (n) {
+    if (!basket_off) rt_die(sh, "cf_recommend_batch: basket_off is NULL");
+    hb = (uint64_t*)malloc((n + 1) * 8);
+    if (!hb) rt_die(sh, "out of host memory");
+    smatrix_b200_memcpy(sh->local, hb, basket_off, (n + 1) * 8);
+    int bad = hb[0] != 0 || hb[n] > 0xFFFFFFFEull;
+    for (size_t i = 0; i < n && !bad; i++) bad = hb[i + 1] < hb[i];
+    if (bad)
+      rt_die(sh, "cf_recommend_batch: malformed basket offsets (they must start at 0, never decrease and end at "
+                 "most at 2^32 - 2)");
+    n_pos = hb[n];
+    if (n_pos && rt_is_dev(sh, items) != in_dev)
+      rt_die(sh, "cf_recommend_batch: basket_off and items must both be host or both be device arrays");
+  }
+  /* room for: the answers when they go to host arrays, all-zero offsets when this rank's rows are empty, the
+   * offsets and items when they are host arrays */
+  const size_t out_bytes = out_dev ? 0 : n * (12ull * k + 4);
+  const size_t in_bytes = in_dev ? 0 : (n + 1) * 8 + n_pos * 4;
+  const size_t extra = out_bytes + (n_pos + 1) * 8 + in_bytes + 64;
+  rt_cf_t c;
+  rt_cf_scores(sh, items, n_pos, 1, ~0ull, NULL, extra, &c);
+  if (n) {
+    char* ex = c.scratch ? (char*)(((uintptr_t)c.extra + 7) & ~(uintptr_t)7)
+                         : (char*)smatrix_b200_dev_alloc(sh->local, extra);
+    const uint64_t* d_off = c.off;
+    char* at = ex;
+    if (!c.filled) {
+      smatrix_b200_memset0(sh->local, at, (n_pos + 1) * 8);
+      d_off = (const uint64_t*)at;
+    }
+    at += (n_pos + 1) * 8;
+    const uint64_t* d_boff = basket_off;
+    const uint32_t* d_items = items;
+    if (!in_dev) {
+      smatrix_b200_memcpy(sh->local, at, hb, (n + 1) * 8);
+      d_boff = (const uint64_t*)at;
+      at += (n + 1) * 8;
+      if (n_pos) smatrix_b200_memcpy(sh->local, at, items, n_pos * 4);
+      d_items = (const uint32_t*)at;
+      at += (n_pos * 4 + 7) & ~(size_t)7;
+    }
+    double* os = out_dev ? scores : (double*)at;
+    uint32_t* oi = out_dev ? ids : (uint32_t*)(os + n * k);
+    uint32_t* oc = out_dev ? counts : oi + n * k;
+    smatrix_b200_basket_topk(sh->local, n, d_boff, d_items, d_off, c.ids, c.scores, k, oc, oi, os);
+    if (!out_dev) {
+      smatrix_b200_memcpy(sh->local, counts, oc, n * 4);
+      smatrix_b200_memcpy(sh->local, ids, oi, n * k * 4);
+      smatrix_b200_memcpy(sh->local, scores, os, n * k * 8);
+    }
+    if (!c.scratch) smatrix_b200_dev_free(sh->local, ex);
+  }
+  free(hb);
+  if (c.scratch) smatrix_b200_dev_free(sh->local, c.scratch);
+}
+
 /* ------------------------------------------------------------------------------ file mode */
 /* Collective: the .smx snapshot of the whole sharded matrix, one ordinary file in the reference's format.
  * Every rank lays out its own rows (snap_extent); exclusive prefixes of the (rows, bytes) pairs give each rank

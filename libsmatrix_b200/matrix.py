@@ -53,6 +53,53 @@ def _topk_call(fn, items, k):
     return counts, ids, scores
 
 
+def _rec_call(fn, basket_offsets, items, k):
+    """fn(off_ptr, items_ptr, n_baskets, k, counts_ptr, ids_ptr, scores_ptr) on outputs allocated where the baskets
+    live; the offsets, the items and k are checked here, before any call into the library."""
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= int(k) <= TOPK_MAX_K:
+        raise ValueError(f"k must be an integer in 1..{TOPK_MAX_K}, got {k!r}")
+    k = int(k)
+    on_cuda = [_is_torch(a) and a.is_cuda for a in (basket_offsets, items)]
+    if on_cuda[0] != on_cuda[1]:
+        raise ValueError("basket offsets and items must both be CUDA tensors or both be host arrays")
+    if on_cuda[0]:
+        import torch
+        if basket_offsets.device != items.device:
+            raise ValueError("basket offsets and items must be on the same device")
+        if basket_offsets.dtype != torch.int64 or items.dtype not in (torch.int32, torch.uint32):
+            raise TypeError("torch baskets: int64 offsets and int32/uint32 items")
+        off, items = basket_offsets.contiguous(), items.contiguous()
+        if off.dim() != 1 or off.numel() < 1:
+            raise ValueError("basket offsets need n_baskets + 1 entries")
+        n = off.numel() - 1
+        ok = torch.stack([off[0] == 0, off[-1] == items.numel(), (off[1:] >= off[:-1]).all()]).all()
+        if not bool(ok):
+            raise ValueError("basket offsets must start at 0, never decrease and end at len(items)")
+        counts = torch.empty(n, dtype=torch.int32, device=items.device)
+        ids = torch.empty((n, k), dtype=torch.int32, device=items.device)
+        scores = torch.empty((n, k), dtype=torch.float64, device=items.device)
+        torch.cuda.current_stream(items.device).synchronize()      # the inputs may still be in flight on torch's stream
+        fn(off.data_ptr(), items.data_ptr(), n, k, counts.data_ptr(), ids.data_ptr(), scores.data_ptr())
+        return counts, ids, scores
+    if _is_torch(basket_offsets):
+        basket_offsets = basket_offsets.numpy()
+    if _is_torch(items):
+        items = items.numpy()
+    raw = np.asarray(basket_offsets)
+    if raw.ndim != 1 or len(raw) < 1 or (len(raw) and raw.dtype.kind not in "iu"):
+        raise ValueError("basket offsets need n_baskets + 1 integer entries")
+    items = np.ascontiguousarray(items, dtype=np.uint32)
+    if raw[0] != 0 or raw[-1] != len(items) or (np.diff(raw.astype(np.int64)) < 0).any():
+        raise ValueError("basket offsets must start at 0, never decrease and end at len(items)")
+    off = np.ascontiguousarray(raw, dtype=np.uint64)
+    n = len(off) - 1
+    counts = np.empty(n, dtype=np.uint32)
+    ids = np.empty((n, k), dtype=np.uint32)
+    scores = np.empty((n, k), dtype=np.float64)
+    fn(off.ctypes.data, items.ctypes.data, n, k, counts.ctypes.data, ids.ctypes.data, scores.ctypes.data)
+    return counts, ids, scores
+
+
 class DevPtr:
     """A raw device array of `n` uint32 (library- or peer-allocated memory that is not a tensor)."""
     __slots__ = ("ptr", "n")
@@ -317,6 +364,14 @@ class SparseMatrix:
         numpy (or any host sequence) in -> numpy out; a CUDA torch tensor in -> tensors on its device out
         (int32 counts and ids, float64 scores), with no copy through the host."""
         return _topk_call(lambda *a: self._lib.smatrix_cf_topk_batch(self._handle(), *a), items, k)
+
+    def cf_recommend_batch(self, basket_offsets, items, k: int):
+        """Per basket (items[basket_offsets[i]:basket_offsets[i+1]], e.g. one user's items), the k best other items
+        by their summed neighbour scores, summed in basket order, ranked on the device (score descending, then id
+        ascending) -> (counts[n], ids[n, k], scores[n, k]); slots past counts[i] hold id 0xFFFFFFFF and score -1.0.
+        The basket's own items and id 0 are never recommended.  numpy in -> numpy out; CUDA torch tensors in (int64
+        offsets, int32 items) -> tensors on their device out, with no copy through the host."""
+        return _rec_call(lambda *a: self._lib.smatrix_cf_recommend_batch(self._handle(), *a), basket_offsets, items, k)
 
     # ---- device controls (include/smatrix_b200.h) --------------------------------------------
     def stat(self, name: str) -> int:

@@ -27,7 +27,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from .matrix import DevPtr, SparseMatrix, _topk_call
+from .matrix import DevPtr, SparseMatrix, _rec_call, _topk_call
 
 _seq = [0]
 
@@ -187,6 +187,12 @@ class ShardedSparseMatrix:
     def cf_topk_batch(self, items, k: int):
         """The k best neighbours of THIS rank's items (contract of SparseMatrix.cf_topk_batch); collective."""
         return _topk_call(lambda *a: self._lib.smatrix_b200_shard_cf_topk_batch(self._handle(), *a), items, k)
+
+    def cf_recommend_batch(self, basket_offsets, items, k: int):
+        """Recommendations for THIS rank's baskets (contract of SparseMatrix.cf_recommend_batch); collective, and a
+        rank may pass no baskets (offsets [0])."""
+        return _rec_call(lambda *a: self._lib.smatrix_b200_shard_cf_recommend_batch(self._handle(), *a),
+                         basket_offsets, items, k)
 
     def getrow_batch_into(self, d_xs, n: int, d_offsets: int, d_pairs: int, pairs_cap: int) -> int:
         """The raw collective call on device (or host) pointers; returns the total number of pairs."""
