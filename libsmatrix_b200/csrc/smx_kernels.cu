@@ -1868,12 +1868,21 @@ k_row_slog(smx_view_t V, const uint32_t* xs, uint32_t n, uint32_t* out) {
  * Three phases keep every probe chain intact when the loader later drops zero-valued cells
  * (src/smatrix.c:533-540): (1) cells with a non-zero value, in any order (unique keys: any insertion
  * order gives a valid table), (2) column 0 into the first cell whose column is 0, (3) zero-valued
- * cells last.  units[i] = 2 + size_i (in 8-byte units) is scanned into the block offsets. */
+ * cells last.  units[i] = 2 + size_i (in 8-byte units) is scanned into the block offsets.
+ * size_i is the reference's row size S, exactly: the reference grows a row only before placing a new
+ * column when used > S/2, so a row can hold S/2 + 1 columns, plus column 0 set after the last growth.
+ * The cells always fit: live + (c0 != 0) <= S/2 + 2 <= S for S >= 16. */
 __global__ void __launch_bounds__(SMX_BLOCK)
 k_snap_units(const uint32_t* counts, const uint32_t* slogs, uint32_t n, uint32_t* units) {
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    ull size = 1ull << (slogs[i] < 4u ? 4u : slogs[i]);
-    while ((ull)counts[i] > size / 2) size *= 2; /* never fuller than the reference lets a row get */
+    const ull size = 1ull << (slogs[i] < 4u ? 4u : slogs[i]);
+    if ((ull)counts[i] > size) { /* a broken rowlen state: snap_place would never return */
+#ifdef SMX_HOSTSIM
+      abort();
+#else
+      __trap();
+#endif
+    }
     units[i] = (uint32_t)(size + 2ull);
   }
 }
@@ -1973,10 +1982,18 @@ k_load_fixup(smx_view_t V, const uint32_t* xs, const uint32_t* slogs, uint32_t n
  * that the row exists even when it holds no live cell, then every cell with a non-zero value follows
  * in slot order (a ballot per 32 cells, each lane's place = the popcount of the lanes below it).
  * Header checks are the host's: the device only sees validated sizes. */
-__device__ __forceinline__ ull ld_file_cell(const unsigned char* p) { /* {u32 column, u32 value} */
-  if (((uintptr_t)p & 7u) == 0u) return *(const ull*)p;
-  ull c;
-  memcpy(&c, p, 8); /* a row block at an odd offset of a foreign file */
+/* {u32 column, u32 value}.  A foreign file can put a row block at any offset (the reference's files at 4 mod
+ * 8).  Those cells are read in 4-byte words or bytes, spelled out: a memcpy here was compiled into the same
+ * 8-byte load as the aligned branch, which faults with "misaligned address" on the device. */
+__device__ __forceinline__ ull ld_file_cell(const unsigned char* p) {
+  const uintptr_t a = (uintptr_t)p;
+  if ((a & 7u) == 0u) return *(const ull*)p;
+  if ((a & 3u) == 0u) {
+    const uint32_t* w = (const uint32_t*)p;
+    return (ull)__ldcg(w) | ((ull)__ldcg(w + 1) << 32);
+  }
+  ull c = 0;
+  for (int k = 7; k >= 0; --k) c = (c << 8) | (ull)__ldcg(p + k);
   return c;
 }
 __global__ void __launch_bounds__(SMX_BLOCK)

@@ -115,7 +115,7 @@ class CpuMatrix:
         self._f["getrow"].argtypes = [C.c_void_p, C.c_uint32, _u32p, C.c_size_t]
         self.h = C.c_void_p(self._f["open"](fname.encode() if fname else None))
         if not self.h:
-            raise MemoryError("open failed")
+            raise ValueError(f"cannot load {fname}") if fname else MemoryError("open failed")
 
     def fnptr(self, name: str) -> C.c_void_p:
         return C.cast(self._f[name], C.c_void_p)
@@ -135,6 +135,26 @@ class CpuMatrix:
 
     def rowlen(self, x):
         return self._f["rowlen"](self.h, x)
+
+    # the restatement only: its row sizes and its file writer --------------------------------
+    def rowsize(self, x) -> int:
+        """Slot capacity S of row x (0 if the row does not exist)."""
+        f = self.lib.smx_oracle_rowsize
+        f.restype, f.argtypes = C.c_uint32, [C.c_void_p, C.c_uint32]
+        return f(self.h, x)
+
+    def save(self, fname: str, shuffled: bool = False, dead: bool = False, unaligned: bool = False,
+             small_dir: bool = False) -> None:
+        """Write the matrix as a .smx file (the rows' cell arrays as they are in memory).  The layout
+        switches make the file look like one the reference's append-only writer leaves behind
+        (oracle/smatrix_oracle.h: SMX_ORACLE_SAVE_*); the rows and cells are the same either way."""
+        if self.kind != "port":
+            raise NotImplementedError("the reference writes its file at close")
+        flags = 1 * shuffled | 2 * dead | 4 * unaligned | 8 * small_dir
+        f = self.lib.smx_oracle_save
+        f.restype, f.argtypes = C.c_int, [C.c_void_p, C.c_char_p, C.c_int]
+        if f(self.h, fname.encode(), flags) != 0:
+            raise OSError(f"cannot write {fname}")
 
     def getrow_raw(self, x, ret_len_bytes: int, slack_pairs: int = 2) -> np.ndarray:
         """The literal C call with a caller buffer of `ret_len_bytes` (plus slack for the

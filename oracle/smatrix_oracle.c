@@ -3,9 +3,9 @@
  * open-addressing hash maps (row directory "cmap" -> per-row column map "rmap").
  *
  * TEST INFRASTRUCTURE ONLY (see smatrix_oracle.h).  Written from the reference's behaviour,
- * not from its text: no locks, no file mode, index-based instead of pointer-based.  Every
- * function names the reference lines whose behaviour it restates (paths relative to the
- * reference checkout).
+ * not from its text: no locks, no IO thread (the file is read at open and written whole at
+ * save / close), index-based instead of pointer-based.  Every function names the reference
+ * lines whose behaviour it restates (paths relative to the reference checkout).
  *
  * What has to be reproduced for bit-exact results (SURVEY.md 8a):
  *   - column map: identity hash `y % size`, linear probing, EMPTY <=> key==0 && value==0
@@ -18,6 +18,9 @@
  *   - directory: `x % size`, linear probing over {used flag, key}, grow x2 when
  *     used*4 >= size*3 (:673-741), initial 65536 entries (src/smatrix.h:24), rows start with
  *     16 cells (src/smatrix.h:21)
+ *   - file mode (.smx, :30-72): a row block is the row's own cell array (:454-482); loading is
+ *     positional — a row keeps its file size and its cells' slots, slots with value == 0 are
+ *     cleared in place and `used` is the count of the non-empty slots left (:499-545)
  */
 #include "smatrix_oracle.h"
 
@@ -49,6 +52,7 @@ struct smx_oracle_s {
   uint64_t dsize;
   uint64_t dused;
   dirent_t* dir;
+  char* fname; /* file mode: written back at close */
 };
 
 static void* zalloc(size_t bytes) {
@@ -121,6 +125,7 @@ static void dir_double(smx_oracle_t* m) {
   bigger.dsize = m->dsize * 2;
   bigger.dused = 0;
   bigger.dir = zalloc(sizeof(dirent_t) * bigger.dsize);
+  bigger.fname = m->fname;
   for (uint64_t i = 0; i < m->dsize; i++) {
     if (!m->dir[i].taken) continue;
     uint64_t at = dir_place(&bigger, m->dir[i].x);
@@ -170,23 +175,172 @@ static cell_t* resolve(smx_oracle_t* m, uint32_t x, uint32_t y, int write, row_t
   return &r->cell[at];
 }
 
+/* ---- file mode (.smx, src/smatrix.c:30-72) -------------------------------------------------
+ *   header     512 bytes: 8 x 0x17, u64 offset of the first directory block (:564-596)
+ *   directory  blocks of {u64 entries, u64 next} + entries x {u32 row, u64 row offset}, chained;
+ *              an entry with offset 0 ends its block (:744-830)
+ *   row block  8 x 0x23, u64 size, then the row's cell array as it is in memory (:454-482) */
+#define F_HEAD 512ull
+#define F_DIR_ENTRIES 4194304ull
+#define F_DIR_HEAD 16ull
+#define F_DIR_SLOT 12ull
+#define F_ROW_HEAD 16ull
+#define F_SMALL_DIR_ENTRIES 5ull /* SMX_ORACLE_SAVE_SMALL_DIR */
+#define F_DEAD_CELLS 16ull       /* SMX_ORACLE_SAVE_DEAD: a row's stale first block */
+
+static void put64(unsigned char* p, uint64_t v) { memcpy(p, &v, 8); }
+static uint64_t get64(const unsigned char* p) { uint64_t v; memcpy(&v, p, 8); return v; }
+
+/* src/smatrix.c:499-545 — one row block, positionally: the row keeps the file's size and every
+ * cell's slot; a slot whose value is 0 is cleared, and `used` is the count of what is left
+ * (column-0 slot included).  Returns 0, or -1 when the block does not fit the file. */
+static int load_row(smx_oracle_t* m, uint32_t x, const unsigned char* d, uint64_t n, uint64_t rpos) {
+  if (rpos > n || n - rpos < F_ROW_HEAD) return -1;
+  for (int k = 0; k < 8; k++)
+    if (d[rpos + k] != 0x23) return -1;
+  const uint64_t size = get64(d + rpos + 8);
+  if (size == 0 || (size & (size - 1)) || size > (1ull << 32) || (n - rpos - F_ROW_HEAD) / 8 < size) return -1;
+  uint64_t at = dir_probe(m, x);
+  if (m->dir[at].taken && m->dir[at].x == x) return -1; /* a row listed twice */
+  row_t* r = zalloc(sizeof(row_t));
+  r->size = (uint32_t)size;
+  r->cell = zalloc(sizeof(cell_t) * size);
+  memcpy(r->cell, d + rpos + F_ROW_HEAD, sizeof(cell_t) * size);
+  r->used = 0;
+  for (uint64_t i = 0; i < size; i++) {
+    if (r->cell[i].val == 0) r->cell[i].key = 0;
+    if (!cell_is_empty(&r->cell[i])) r->used++;
+  }
+  at = dir_place(m, x);
+  m->dir[at].row = r;
+  return 0;
+}
+
+/* src/smatrix.c:744-830 — the header, then the chain of directory blocks, every entry's row */
+static int load_file(smx_oracle_t* m, const unsigned char* d, uint64_t n) {
+  if (n < F_HEAD) return -1;
+  for (int k = 0; k < 8; k++)
+    if (d[k] != 0x17) return -1;
+  uint64_t bpos = get64(d + 8), blocks = 0;
+  while (bpos) {
+    if (++blocks > n / F_DIR_HEAD || bpos > n || n - bpos < F_DIR_HEAD) return -1; /* a loop, or past the end */
+    const uint64_t entries = get64(d + bpos), next = get64(d + bpos + 8);
+    if (entries > F_DIR_ENTRIES || (n - bpos - F_DIR_HEAD) / F_DIR_SLOT < entries) return -1;
+    for (uint64_t e = 0; e < entries; e++) {
+      const unsigned char* ent = d + bpos + F_DIR_HEAD + e * F_DIR_SLOT;
+      uint32_t x;
+      memcpy(&x, ent, 4);
+      const uint64_t rpos = get64(ent + 4);
+      if (!rpos) break;
+      if (load_row(m, x, d, n, rpos)) return -1;
+    }
+    bpos = next;
+  }
+  return 0;
+}
+
+int smx_oracle_save(smx_oracle_t* m, const char* fname, int flags) {
+  uint64_t n = 0;
+  for (uint64_t i = 0; i < m->dsize; i++) n += m->dir[i].taken;
+  row_t** rows = malloc(sizeof(row_t*) * (n ? n : 1));
+  uint32_t* keys = malloc(sizeof(uint32_t) * (n ? n : 1));
+  uint64_t* rpos = malloc(sizeof(uint64_t) * (n ? n : 1));
+  uint64_t* dead = malloc(sizeof(uint64_t) * (n ? n : 1));
+  if (!rows || !keys || !rpos || !dead) abort();
+  for (uint64_t i = 0, k = 0; i < m->dsize; i++) /* directory order = table order */
+    if (m->dir[i].taken) { rows[k] = m->dir[i].row; keys[k] = m->dir[i].x; k++; }
+  const uint64_t per = (flags & SMX_ORACLE_SAVE_SMALL_DIR) ? F_SMALL_DIR_ENTRIES : F_DIR_ENTRIES;
+  const uint64_t nblk = n ? (n + per - 1) / per : 1, blk_bytes = F_DIR_HEAD + per * F_DIR_SLOT;
+  /* layout: header, first directory block, row blocks, then the later directory blocks at the end
+   * of the file, where an append-only writer puts the next block once the previous one is full */
+  uint64_t pos = F_HEAD + blk_bytes;
+  for (uint64_t k = 0; k < n; k++) {
+    const uint64_t i = (flags & SMX_ORACLE_SAVE_SHUFFLED) ? n - 1 - k : k;
+    /* two row blocks off alignment: one at 4 mod 8, one at 1 mod 8, the blocks behind them aligned */
+    const uint64_t odd = !(flags & SMX_ORACLE_SAVE_UNALIGNED) ? 0 : k == n / 2 ? 4 : k == n / 2 + 1 ? 1 : 0;
+    dead[i] = 0;
+    if ((flags & SMX_ORACLE_SAVE_DEAD) && k % 2 == 0) { /* a row's earlier, smaller block */
+      dead[i] = pos;
+      pos += F_ROW_HEAD + 8 * F_DEAD_CELLS;
+    }
+    pos += odd;
+    rpos[i] = pos;
+    pos += F_ROW_HEAD + 8ull * rows[i]->size + (odd ? 8 - odd : 0);
+  }
+  const uint64_t later_dirs = pos;
+  pos += (nblk - 1) * blk_bytes;
+  unsigned char* d = calloc(1, pos);
+  if (!d) abort();
+  memset(d, 0x17, 8);
+  put64(d + 8, F_HEAD);
+  for (uint64_t b = 0; b < nblk; b++) {
+    const uint64_t at = b ? later_dirs + (b - 1) * blk_bytes : F_HEAD;
+    put64(d + at, per);
+    put64(d + at + 8, b + 1 < nblk ? later_dirs + b * blk_bytes : 0);
+    for (uint64_t e = 0; e < per && b * per + e < n; e++) {
+      unsigned char* ent = d + at + F_DIR_HEAD + e * F_DIR_SLOT;
+      memcpy(ent, &keys[b * per + e], 4);
+      put64(ent + 4, rpos[b * per + e]);
+    }
+  }
+  for (uint64_t i = 0; i < n; i++) {
+    memset(d + rpos[i], 0x23, 8);
+    put64(d + rpos[i] + 8, rows[i]->size);
+    memcpy(d + rpos[i] + F_ROW_HEAD, rows[i]->cell, 8ull * rows[i]->size);
+    if (dead[i]) { /* stale: every value off by one, unreferenced */
+      memset(d + dead[i], 0x23, 8);
+      put64(d + dead[i] + 8, F_DEAD_CELLS);
+      for (uint64_t c = 0; c < F_DEAD_CELLS && c < rows[i]->size; c++) {
+        cell_t stale = rows[i]->cell[c];
+        stale.val += 1;
+        memcpy(d + dead[i] + F_ROW_HEAD + 8 * c, &stale, 8);
+      }
+    }
+  }
+  FILE* f = fopen(fname, "wb");
+  int rc = f && fwrite(d, 1, pos, f) == pos ? 0 : -1;
+  if (f && fclose(f) != 0) rc = -1;
+  free(d); free(rows); free(keys); free(rpos); free(dead);
+  return rc;
+}
+
 smx_oracle_t* smx_oracle_open(const char* fname) {
-  if (fname) return NULL; /* memory mode only */
   smx_oracle_t* m = zalloc(sizeof(*m));
   m->dsize = DIR_ENTRIES0; /* src/smatrix.c:598-612 */
   m->dused = 0;
   m->dir = zalloc(sizeof(dirent_t) * m->dsize);
+  if (!fname) return m;
+  m->fname = strdup(fname);
+  FILE* f = fopen(fname, "rb"); /* a missing or empty file is a new matrix (:90-111) */
+  if (!f) return m;
+  fseek(f, 0, SEEK_END);
+  const long n = ftell(f);
+  fseek(f, 0, SEEK_SET);
+  unsigned char* d = n > 0 ? malloc((size_t)n) : NULL;
+  int rc = 0;
+  if (n > 0) rc = (!d || fread(d, 1, (size_t)n, f) != (size_t)n) ? -1 : load_file(m, d, (uint64_t)n);
+  fclose(f);
+  free(d);
+  if (rc) {
+    fprintf(stderr, "smx_oracle: %s is not a valid .smx file\n", fname);
+    free(m->fname);
+    m->fname = NULL; /* never overwrite it */
+    smx_oracle_close(m);
+    return NULL;
+  }
   return m;
 }
 
 void smx_oracle_close(smx_oracle_t* m) { /* src/smatrix.c:113-133 */
   if (!m) return;
+  if (m->fname && smx_oracle_save(m, m->fname, 0)) fprintf(stderr, "smx_oracle: cannot write %s\n", m->fname);
   for (uint64_t i = 0; i < m->dsize; i++) {
     if (m->dir[i].taken && m->dir[i].row) {
       free(m->dir[i].row->cell);
       free(m->dir[i].row);
     }
   }
+  free(m->fname);
   free(m->dir);
   free(m);
 }

@@ -18,7 +18,9 @@
 
 typedef struct smx_oracle_s smx_oracle_t;
 
-smx_oracle_t* smx_oracle_open(const char* fname); /* fname must be NULL (memory mode)        */
+/* fname == NULL: memory mode.  Otherwise the file (if it exists and is not empty) is loaded the
+ * reference's way, and the matrix is written back to it at close; NULL for a corrupt file. */
+smx_oracle_t* smx_oracle_open(const char* fname);
 void     smx_oracle_close(smx_oracle_t* m);
 uint32_t smx_oracle_get(smx_oracle_t* m, uint32_t x, uint32_t y);
 uint32_t smx_oracle_set(smx_oracle_t* m, uint32_t x, uint32_t y, uint32_t v);
@@ -31,5 +33,14 @@ uint32_t smx_oracle_getrow(smx_oracle_t* m, uint32_t x, uint32_t* ret, size_t re
 uint64_t smx_oracle_nrows(smx_oracle_t* m);       /* directory entries in use               */
 uint64_t smx_oracle_dirsize(smx_oracle_t* m);     /* directory capacity                     */
 uint32_t smx_oracle_rowsize(smx_oracle_t* m, uint32_t x); /* slot capacity of row x, 0 if absent */
+
+/* Write the matrix as a .smx file now; 0 or -1.  With flags 0 the file is laid out like a fresh
+ * snapshot (rows in directory order, one directory block).  The flags make it look like a file the
+ * reference's append-only writer leaves behind, with the same rows and cells: */
+#define SMX_ORACLE_SAVE_SHUFFLED  1 /* row blocks in reverse directory order                        */
+#define SMX_ORACLE_SAVE_DEAD      2 /* an unreferenced stale block before every other row block      */
+#define SMX_ORACLE_SAVE_UNALIGNED 4 /* the middle row block at 4 mod 8, the one after it at 1 mod 8  */
+#define SMX_ORACLE_SAVE_SMALL_DIR 8 /* directory blocks of 5 entries, chained, the last partly used  */
+int smx_oracle_save(smx_oracle_t* m, const char* fname, int flags);
 
 #endif

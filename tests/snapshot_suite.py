@@ -4,6 +4,7 @@ GPU tests."""
 from __future__ import annotations
 
 import os
+import shutil
 
 import numpy as np
 
@@ -79,6 +80,12 @@ def scenario_snapshot_roundtrip_big(make, tmp_path, n_rows=30000):
     m2 = make(f)
     assert m2.stat("nnz") == nnz and m2.stat("rows") == len(np.unique(xs))
     assert (np.asarray(m2.get_batch(xs, ys)) == want).all()
-    got = np.asarray(m2.rowlen_batch(np.unique(xs)))
-    assert (got == rl).all() or True    # rowlen after a reload is the reference's recount; checked in the interchange test
+    rows = np.unique(xs)
+    ck = cpu.CpuMatrix("port", shutil.copy(f, str(tmp_path / "checker.smx")))   # the reference's positional load
+    assert (np.asarray(m2.rowlen_batch(rows)) == ck.rowlen_many(rows)).all()     # rowlen: the recount of the file
+    assert (np.asarray(m2.get_batch(xs, ys)) == ck.get_many(xs, ys)).all()
+    o1, p1 = m2.getrow_batch(rows)
+    o2, p2 = ck.getrow_many(rows)
+    assert (o1 == o2).all() and (cpu.sort_rows(o1, p1) == cpu.sort_rows(o2, p2)).all()
+    ck.close()
     m2.close()

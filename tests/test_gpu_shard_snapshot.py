@@ -93,6 +93,17 @@ def test_save_at_w_reload_at_any_world(world, tmp_path):
         shutil.copy(f, g)
         shutil.copy(f + ".npz", g + ".npz")
         _run("load", g, w, f"load{world}_{w}")
+    import smx_file                                     # the file is the checker's format, row by row,
+    import snapshot_oracle_suite as so                  # and its positional load reads the same table
+    xs = np.unique(np.asarray(__import__("shard_snapshot_gpu_worker").stream()[0]))
+    for x, (size, cells) in smx_file.read(f).items():
+        smx_file.check_row(x, size, cells)
+    want = np.load(f + ".npz")
+    ck = cpu.CpuMatrix("port", shutil.copy(f, str(tmp_path / "ck.smx")))
+    assert not so.hidden(smx_file.read(f))
+    o, p = ck.getrow_many(xs)
+    assert (o == want["offsets"]).all() and (cpu.sort_rows(o, p) == want["pairs"]).all()
+    ck.close()
     if cpu.have_reference():                            # the reference reads the sharded file
         want = np.load(f + ".npz")
         r = cpu.CpuMatrix("reference", shutil.copy(f, str(tmp_path / "ref.smx")))

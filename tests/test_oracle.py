@@ -248,3 +248,33 @@ def test_lazy_rowlen_automaton_equals_stepwise():
                 z = True
             s2, d2 = catch_up(slog, d, c, z)
             assert c + d2 == want[c], (n_total, flip, c)
+
+
+# ------------------------------------------------------------------ file mode
+@need_ref
+def test_file_mode_matches_reference(tmp_path):
+    """The restatement's .smx writer and positional loader against the reference's file mode: each loads the
+    other's file (and its own), and all four give the same answers, getrow in table order included."""
+    import shutil
+    rng = np.random.default_rng(77)
+    rf = str(tmp_path / "ref.smx")
+    ref, port = cpu.CpuMatrix("reference", rf), cpu.CpuMatrix("port")
+    for op in ("incr", "set", "incr"):
+        xs, ys, vs = safe_stream(rng, 20000, 120, 90, op, col0_rate=0.05, max_val=3)   # zero-valued cells too
+        ref.apply(op, xs, ys, vs); port.apply(op, xs, ys, vs)
+    rows = np.unique(xs)
+    pf = str(tmp_path / "port.smx")
+    port.save(pf, shuffled=True, dead=True, unaligned=True, small_dir=True)
+    ref.close(); port.close()
+    loaded = [cpu.CpuMatrix(kind, shutil.copy(src, str(tmp_path / f"{kind}_{k}.smx")))
+              for k, src in enumerate((rf, pf)) for kind in ("reference", "port")]
+    qx, qy = np.repeat(rows, 92), np.tile(np.arange(92, dtype=np.uint32), len(rows))
+    want = loaded[0]
+    for m in loaded[1:]:
+        assert (m.get_many(qx, qy) == want.get_many(qx, qy)).all()
+        assert (m.rowlen_many(rows) == want.rowlen_many(rows)).all()
+        oa, pa = m.getrow_many(rows)
+        ob, pb = want.getrow_many(rows)
+        assert (oa == ob).all() and (pa == pb).all()
+    for m in loaded:
+        m.close()
