@@ -107,7 +107,8 @@ enum {
   SMX_STAT_ALLOCS = 27,     /* number of those cudaMalloc calls */
   SMX_STAT_TOPK_BIG = 28,   /* top-k segments (items) longer than 4096 pairs: ranked by the multi-block radix select */
   SMX_STAT_TOPK_PASSES = 29,/* digit passes that select ran so far */
-  SMX_STAT_REC_BIG = 30     /* baskets longer than 4096 pairs: aggregated by the global sort of smatrix_cf_recommend_batch */
+  SMX_STAT_REC_BIG = 30,    /* baskets longer than 4096 pairs: aggregated by the global sort of smatrix_cf_recommend_batch */
+  SMX_STAT_SORT_BIG = 31    /* segments longer than 4096 pairs: sorted by the global radix sort of smatrix_b200_sort_rows */
 };
 uint64_t smatrix_b200_stat(smatrix_t* self, int which);
 
@@ -227,6 +228,15 @@ void smatrix_b200_topk_segments(smatrix_t* self, size_t n, const uint64_t* d_off
 void smatrix_b200_basket_topk(smatrix_t* self, size_t n_baskets, const uint64_t* d_basket_off, const uint32_t* d_items,
                               const uint64_t* d_offsets, const uint32_t* d_ids, const double* d_scores, uint32_t k,
                               uint32_t* d_counts, uint32_t* d_out_ids, double* d_out_scores);
+/* The sort of smatrix_getrow_sorted_batch over any CSR of (column, value) pairs on the device: segment i is
+ * d_pairs[2 d_offsets[i] .. 2 d_offsets[i+1]), sorted in place by column (unsigned).  Columns must be unique inside a
+ * segment.  Segments of up to 4096 pairs are sorted in shared memory; longer ones together, in groups of at most
+ * $SMATRIX_TOPK_PAIRS pairs (a longer segment is a group of its own), by a radix sort with up to about 40
+ * bytes of device scratch per pair (SMX_STAT_SORT_BIG counts them).  All arrays DEVICE. */
+void smatrix_b200_sort_rows(smatrix_t* self, size_t n, const uint64_t* d_offsets, uint32_t* d_pairs);
+/* The sort of smatrix_list_rows, used by the multi-GPU router: the n keys d_keys[0..n) (DEVICE, left as they are)
+ * in ascending order, the first min(cap, n) of them to out (host or device). */
+void smatrix_b200_sort_keys(smatrix_t* self, const uint32_t* d_keys, size_t n, uint32_t* out, uint64_t cap);
 int  smatrix_b200_is_device_ptr(smatrix_t* self, const void* p);   /* device (or managed) memory? */
 /* peers in the SAME process (one thread per GPU) need no IPC: enable direct access to `peer_device` */
 int  smatrix_b200_enable_peer(smatrix_t* self, int peer_device);

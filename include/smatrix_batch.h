@@ -97,6 +97,19 @@ void smatrix_cf_topk_batch(smatrix_t* self, const uint32_t* items, size_t n, uin
 void smatrix_cf_recommend_batch(smatrix_t* self, const uint64_t* basket_off, const uint32_t* items,
                                 size_t n_baskets, uint32_t k, uint32_t* counts, uint32_t* ids, double* scores);
 
+/* The rows of the matrix in ascending key order, starting at the first key >= from: keys[0 .. min(cap, m)) where
+ * m is the number of rows with key >= from; returns m.  Size query with keys == NULL.  The rows are exactly those a
+ * snapshot of the matrix would list (the reference's row map: a row exists from the first incr / decr / set on any
+ * of its columns, set 0 included, and is never removed); a row may have no pairs.  keys may be host or device.
+ * Page through the matrix with from = last key + 1 (stop after key 0xFFFFFFFF).  Cost: one pass over the
+ * directory per call, whatever cap is. */
+uint64_t smatrix_list_rows(smatrix_t* self, uint32_t from, uint32_t* keys, uint64_t cap);
+
+/* smatrix_getrow_batch with every row's pairs in ascending column order (so (0, c0) first when column 0 is
+ * non-zero).  Same CSR contract, size query and host / device rules as smatrix_getrow_batch. */
+uint64_t smatrix_getrow_sorted_batch(smatrix_t* self, const uint32_t* xs, size_t n, uint64_t* offsets,
+                                     uint32_t* pairs, uint64_t pairs_cap);
+
 #ifdef __cplusplus
 }
 #endif

@@ -129,6 +129,17 @@ void smatrix_b200_shard_cf_recommend_batch(smatrix_shard_t* self, const uint64_t
                                            size_t n_baskets, uint32_t k, uint32_t* counts, uint32_t* ids,
                                            double* scores);
 
+/* Collective: smatrix_list_rows of the sharded matrix.  Every rank passes the same `from` and `cap` and gets the
+ * same answer, equal to one GPU's (keys host or device, NULL for a size query).  Every rank lists its own keys
+ * >= from, at most cap of them; the counts go round, every rank writes its list into every rank's row buffer at its
+ * rank's place, and every rank sorts those at most world * cap keys and keeps the first cap. */
+uint64_t smatrix_b200_shard_list_rows(smatrix_shard_t* self, uint32_t from, uint32_t* keys, uint64_t cap);
+
+/* Collective: smatrix_getrow_sorted_batch for this rank's rows, with the contract of smatrix_b200_shard_getrow_batch;
+ * the pairs that land in this rank's row buffer are sorted there by smatrix_b200_sort_rows. */
+uint64_t smatrix_b200_shard_getrow_sorted_batch(smatrix_shard_t* self, const uint32_t* xs, size_t n,
+                                                uint64_t* offsets, uint32_t* pairs, uint64_t pairs_cap);
+
 /* Host wall-clock accounting of this rank since the last reset (not collective): time spent routing
  * (count, count exchange, scatter over NVLink, arrival barrier), time spent applying the inbox,
  * number of routes, bytes this rank stored into OTHER ranks' inboxes. */

@@ -66,6 +66,9 @@ typedef struct {
   uint32_t rec_cut[3]; /* end of the next piece of a cf_recommend_batch call, its first and end position */
   struct { uint32_t bad, pad; uint64_t n_pos; } rec_check; /* device basket offsets: malformed?, positions */
   struct { uint32_t n_big, pad; uint64_t big_pairs; } rec;  /* big baskets of a piece and their pairs */
+  struct { uint32_t n_big, pad; uint64_t big_pairs; } sort; /* big segments of a sort_rows call and their pairs */
+  struct { uint32_t end, pad; uint64_t pairs; } sort_cut;   /* end of the next group of big segments, its pairs */
+  uint32_t listed;     /* rows smatrix_list_rows found */
 } smx_small_t;
 enum { DS_X, DS_Y, DS_V, DS_OUT, DS_WORDS }; /* the words of d_small: a single op's arguments, a one-word answer */
 
@@ -125,7 +128,7 @@ struct smatrix_s {
     /* *_batch_out (exact per-op return values) */
     smx_dbuf_t bo_addr[2], bo_idx[2], bo_seg, bo_tiles, bo_out, bo_sort;
     /* top-k (smatrix_cf_topk_batch, smatrix_b200_topk_segments) */
-    smx_dbuf_t tk_ctl;     /* 16 control words + the list of big segments */
+    smx_dbuf_t tk_ctl;     /* 16 control words + the list of big segments (also of smatrix_b200_sort_rows) */
     smx_dbuf_t tk_off;     /* row offsets of the whole call (piece cuts) */
     smx_dbuf_t tk_big;     /* select state + histograms of the big segments */
     smx_dbuf_t tk_cids, tk_cscores; /* compaction regions of the big segments */
@@ -136,6 +139,10 @@ struct smatrix_s {
      * big baskets' lengths / offsets, sort keys, values, marks and their scan */
     smx_dbuf_t rc_in, rc_pos, rc_ctl, rc_items, rc_sort, rc_tids, rc_tscores, rc_red, rc_rids, rc_rscores;
     smx_dbuf_t rc_big, rc_keys, rc_vals, rc_flags;
+    /* rows sorted by column (smatrix_b200_sort_rows): the big segments' lengths, offsets and scan, the sort keys and
+     * values of a group of them, the radix sort's storage; the listing (smatrix_list_rows): the keys as found and
+     * sorted, its radix sort's storage */
+    smx_dbuf_t sr_big, sr_keys, sr_vals, sr_sort, ls_keys, ls_sort;
     /* loading a snapshot (smatrix_b200_load_next): a window of file bytes, its tiles, their counts and offsets,
      * the op stream (x, y, v) and the (key, log2 size) fixups of a piece */
     smx_dbuf_t ld_raw, ld_tiles, ld_cnt, ld_off, ld_ops, ld_fix;
@@ -143,6 +150,7 @@ struct smatrix_s {
   uint32_t topk_pairs;  /* SMATRIX_TOPK_PAIRS: pairs per piece of a cf_topk_batch call */
   uint64_t n_topk_big, n_topk_passes;
   uint64_t n_rec_big; /* SMX_STAT_REC_BIG */
+  uint64_t n_sort_big; /* SMX_STAT_SORT_BIG */
 
   unsigned long long* free_ptr[SMX_CLASSES]; /* device stacks of vacated buckets, per size class */
   uint32_t free_cap[SMX_CLASSES];
@@ -1184,14 +1192,19 @@ static uint64_t no_rows(smatrix_t* s, uint64_t* offsets) {
   return 0;
 }
 
-uint64_t smatrix_getrow_batch(smatrix_t* s, const uint32_t* xs, size_t n, uint64_t* offsets,
-                              uint32_t* pairs, uint64_t pairs_cap) {
+static void sort_run(smatrix_t* s, uint32_t n, const uint64_t* d_off, uint32_t* d_pairs);
+
+/* smatrix_getrow_batch, and with sorted != 0 smatrix_getrow_sorted_batch: the filled rows are sorted by column on the
+ * device before they go anywhere */
+static uint64_t getrow_rows(smatrix_t* s, const char* what, int sorted, const uint32_t* xs, size_t n,
+                            uint64_t* offsets, uint32_t* pairs, uint64_t pairs_cap) {
   if (n == 0) return no_rows(s, offsets);
-  if (n >= 0xFFFFFFFFull) smx_die("getrow_batch: too many rows in one call");
+  if (n >= 0xFFFFFFFFull) smx_die("%s: too many rows in one call", what);
   enter(s);
   const uint32_t nn = (uint32_t)n;
   const int pairs_dev = is_device_ptr(pairs);
   const smx_rows_t r = gather_rows(s, xs, is_device_ptr(xs), nn, pairs ? pairs_cap : 0, pairs_dev ? pairs : NULL);
+  if (sorted && r.pairs) sort_run(s, nn, r.offsets, r.pairs);
   if (offsets) {
     CK(cudaMemcpyAsync(offsets, r.offsets, ((size_t)nn + 1) * 8, cudaMemcpyDefault, s->stream));
     if (!is_device_ptr(offsets)) s->d2h_bytes += ((size_t)nn + 1) * 8;
@@ -1202,6 +1215,15 @@ uint64_t smatrix_getrow_batch(smatrix_t* s, const uint32_t* xs, size_t n, uint64
   CK(cudaGetLastError());
   leave(s);
   return r.total;
+}
+
+uint64_t smatrix_getrow_batch(smatrix_t* s, const uint32_t* xs, size_t n, uint64_t* offsets,
+                              uint32_t* pairs, uint64_t pairs_cap) {
+  return getrow_rows(s, "getrow_batch", 0, xs, n, offsets, pairs, pairs_cap);
+}
+uint64_t smatrix_getrow_sorted_batch(smatrix_t* s, const uint32_t* xs, size_t n, uint64_t* offsets,
+                                     uint32_t* pairs, uint64_t pairs_cap) {
+  return getrow_rows(s, "getrow_sorted_batch", 1, xs, n, offsets, pairs, pairs_cap);
 }
 
 /* SURVEY.md 8f N4: neighbours + cosine scores for a batch of items (examples/cf_recommender.c:50-86) */
@@ -1515,6 +1537,102 @@ void smatrix_cf_recommend_batch(smatrix_t* s, const uint64_t* basket_off, const 
   leave(s);
 }
 
+/* ------------------------------------------------------------------------------ enumeration */
+/* Segments d_off[0..n] of d_pairs sorted by column in place, enqueued on s->stream (synchronises to read the number
+ * of big segments and, per group of them, its end): the small ones by sort_small, the big ones a group of at most
+ * SMATRIX_TOPK_PAIRS pairs at a time (a longer segment is a group of its own) by one radix sort each. */
+static void sort_run(smatrix_t* s, uint32_t n, const uint64_t* d_off, uint32_t* d_pairs) {
+  if (!n) return;
+  uint32_t* ctl = dbuf_need(s, &s->db.tk_ctl, (size_t)n * 4 + 64);
+  uint32_t* big_list = ctl + 16;
+  CK(cudaMemsetAsync(ctl, 0, 64, s->stream));
+  smx_launch_topk_classify(s->stream, n, d_off, big_list, ctl);
+  copy_d2h(s, &s->h_small->sort, ctl, 16, s->stream);
+  smx_launch_sort_small(s->stream, n, d_off, d_pairs);
+  s->n_launches += 3;
+  CK(cudaStreamSynchronize(s->stream));
+  const uint32_t n_big = s->h_small->sort.n_big;
+  if (!n_big) return;
+  const size_t scan_items = smx_scan_scratch_items(n_big);
+  uint32_t* lens = dbuf_need(s, &s->db.sr_big, (size_t)n_big * 4 + ((size_t)n_big + 1 + scan_items) * 8 + 16);
+  uint64_t* big_off = (uint64_t*)(((uintptr_t)(lens + n_big) + 7) & ~(uintptr_t)7);
+  smx_launch_sort_big_lens(s->stream, big_list, n_big, d_off, lens);
+  smx_launch_scan(s->stream, lens, n_big, 0, big_off, big_off + n_big + 1);
+  s->n_launches += 4;
+  for (uint32_t lo = 0, hi; lo < n_big; lo = hi) {
+    smx_launch_sort_cut(s->stream, big_off, n_big, lo, s->topk_pairs, ctl + 4);
+    copy_d2h(s, &s->h_small->sort_cut, ctl + 4, 16, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    s->n_launches++;
+    hi = s->h_small->sort_cut.end;
+    const uint64_t P = s->h_small->sort_cut.pairs;
+    if (P >= (1ull << 31)) smx_die("sort_rows: a row of %llu pairs is more than 2^31 - 1", (unsigned long long)P);
+    uint64_t* keys = dbuf_need(s, &s->db.sr_keys, (size_t)P * 16);
+    uint32_t* vals = dbuf_need(s, &s->db.sr_vals, (size_t)P * 8);
+    const size_t sort_bytes = smx_rec_sort_bytes((uint32_t)P);
+    void* sort_tmp = dbuf_need(s, &s->db.sr_sort, sort_bytes);
+    smx_launch_sort_big(s->stream, big_list, lo, hi - lo, (uint32_t)P, big_off, d_off, d_pairs, keys, keys + P, vals,
+                        vals + P, sort_tmp, sort_bytes);
+    s->n_launches += 3;
+  }
+  s->n_sort_big += n_big;
+}
+
+void smatrix_b200_sort_rows(smatrix_t* s, size_t n, const uint64_t* d_offsets, uint32_t* d_pairs) {
+  if (n >= 0xFFFFFFFFull) smx_die("sort_rows: too many segments in one call");
+  if (!n) return;
+  enter(s);
+  sort_run(s, (uint32_t)n, d_offsets, d_pairs);
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+}
+
+/* the n keys d_in (device) in ascending order into d_tmp (device, n keys), the first min(cap, n) of them to out */
+static void sort_keys_to(smatrix_t* s, const uint32_t* d_in, uint32_t* d_tmp, uint32_t n, uint32_t* out, uint64_t cap) {
+  const size_t sort_bytes = smx_sort_keys_bytes(n);
+  void* sort_tmp = dbuf_need(s, &s->db.ls_sort, sort_bytes);
+  smx_launch_sort_keys(s->stream, d_in, d_tmp, n, sort_tmp, sort_bytes);
+  s->n_launches++;
+  const size_t bytes = (size_t)(cap < n ? cap : n) * 4;
+  CK(cudaMemcpyAsync(out, d_tmp, bytes, cudaMemcpyDefault, s->stream));
+  if (!is_device_ptr(out)) s->d2h_bytes += bytes;
+}
+
+/* one pass over the directory for the keys >= from, then a radix sort of them (not in a size query) */
+uint64_t smatrix_list_rows(smatrix_t* s, uint32_t from, uint32_t* keys, uint64_t cap) {
+  enter(s);
+  read_ctl(s);
+  const uint64_t rows = s->h_ctl->dir_used;
+  if (rows >= (1ull << 31)) smx_die("list_rows: %llu rows are more than 2^31 - 1", (unsigned long long)rows);
+  uint64_t m = 0;
+  if (rows) {
+    uint32_t* d_keys = dbuf_need(s, &s->db.ls_keys, (size_t)rows * 8 + 4); /* as found, sorted, the counter */
+    uint32_t* d_cnt = d_keys + 2 * rows;
+    CK(cudaMemsetAsync(d_cnt, 0, 4, s->stream));
+    smx_launch_list_rows(s->stream, view_of(s), from, d_keys, d_cnt);
+    copy_d2h(s, &s->h_small->listed, d_cnt, 4, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    s->n_launches++;
+    m = s->h_small->listed;
+    if (keys && cap && m) sort_keys_to(s, d_keys, d_keys + rows, (uint32_t)m, keys, cap);
+  }
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+  return m;
+}
+
+void smatrix_b200_sort_keys(smatrix_t* s, const uint32_t* d_keys, size_t n, uint32_t* out, uint64_t cap) {
+  if (n >= (1ull << 31)) smx_die("sort_keys: %zu keys are more than 2^31 - 1", n);
+  if (!n || !cap) return;
+  enter(s);
+  sort_keys_to(s, d_keys, dbuf_need(s, &s->db.ls_keys, n * 4), (uint32_t)n, out, cap);
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  leave(s);
+}
+
 /* ------------------------------------------------------------------------------ single ops */
 /* the answer of a single op, d_small[DS_OUT] */
 static uint32_t single_answer(smatrix_t* s) {
@@ -1670,7 +1788,7 @@ static void snap_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes) {
   if (n_rows) {
     s->snap_keys = (uint32_t*)dmalloc(s, n_rows * 4);
     CK(cudaMemsetAsync(&s->d_ctl->scratch, 0, 8, s->stream));
-    smx_launch_list_rows(s->stream, view_of(s), s->snap_keys, (uint32_t*)&s->d_ctl->scratch);
+    smx_launch_list_rows(s->stream, view_of(s), 0, s->snap_keys, (uint32_t*)&s->d_ctl->scratch);
   }
   s->snap_rows = n_rows;
   uint64_t total = 0;
@@ -2324,6 +2442,7 @@ uint64_t smatrix_b200_stat(smatrix_t* s, int which) {
     case SMX_STAT_TOPK_BIG: r = s->n_topk_big; break;
     case SMX_STAT_TOPK_PASSES: r = s->n_topk_passes; break;
     case SMX_STAT_REC_BIG: r = s->n_rec_big; break;
+    case SMX_STAT_SORT_BIG: r = s->n_sort_big; break;
     case SMX_STAT_H2D_BYTES: r = s->h2d_bytes; break;
     case SMX_STAT_D2H_BYTES: r = s->d2h_bytes; break;
     case SMX_STAT_DIR_CAP: r = s->dir_cap; break;

@@ -234,7 +234,24 @@ void smx_launch_rec_cut(smx_stream_t stream, const uint64_t* pos_off, const uint
 /* out[0] |= 1 if boff[0..nb] is not a valid basket CSR (starts at 0, never decreases, ends <= 2^32 - 2);
  * out[2..3] = boff[nb] as u64.  out[0] zeroed. */
 void smx_launch_rec_check(smx_stream_t stream, const uint64_t* boff, uint32_t nb, uint32_t* out);
-void smx_launch_list_rows(smx_stream_t stream, smx_view_t v, uint32_t* keys, uint32_t* counter /* zeroed */);
+/* rows sorted by column (kernel comment in smx_kernels.cu): sort_small sorts the segments of <= TOPK_BLOCK_MAX
+ * pairs in place; the big ones, listed by smx_launch_topk_classify: sort_big_lens -> smx_launch_scan = big_off
+ * (n_big + 1) -> per group: sort_cut (out[0] = end of the group from lo, out[2..3] = its pairs as u64) -> sort_big
+ * (keys / vals: P each; sort_tmp: smx_rec_sort_bytes(P)) */
+void smx_launch_sort_small(smx_stream_t stream, uint32_t n, const uint64_t* offsets, uint32_t* pairs);
+void smx_launch_sort_big_lens(smx_stream_t stream, const uint32_t* big_list, uint32_t n_big, const uint64_t* offsets,
+                              uint32_t* lens);
+void smx_launch_sort_cut(smx_stream_t stream, const uint64_t* big_off, uint32_t n_big, uint32_t lo, uint64_t budget,
+                         uint32_t* out);
+void smx_launch_sort_big(smx_stream_t stream, const uint32_t* big_list, uint32_t lo, uint32_t n_grp, uint32_t P,
+                         const uint64_t* big_off, const uint64_t* offsets, uint32_t* pairs, uint64_t* keys_a,
+                         uint64_t* keys_b, uint32_t* vals_a, uint32_t* vals_b, void* sort_tmp, size_t sort_bytes);
+/* the row ids >= from (a snapshot: from = 0), in directory order; then an ascending radix sort of n u32 keys */
+void smx_launch_list_rows(smx_stream_t stream, smx_view_t v, uint32_t from, uint32_t* keys,
+                          uint32_t* counter /* zeroed */);
+size_t smx_sort_keys_bytes(uint32_t n);
+void smx_launch_sort_keys(smx_stream_t stream, const uint32_t* in, uint32_t* out, uint32_t n, void* sort_tmp,
+                          size_t sort_bytes);
 void smx_launch_row_slog(smx_stream_t stream, smx_view_t v, const uint32_t* xs, uint32_t n, uint32_t* out);
 void smx_launch_snap_units(smx_stream_t stream, const uint32_t* counts, const uint32_t* slogs, uint32_t n,
                            uint32_t* units /* 2 + reference row size, in 8-byte units */);

@@ -1839,13 +1839,101 @@ __global__ void __launch_bounds__(SMX_BLOCK) k_rec_check(const ull* boff, uint32
   }
 }
 
+/* ---- rows sorted by column (smatrix_getrow_sorted_batch, smatrix_b200_sort_rows) -----------------------------
+ * Segment i is pairs[2 offsets[i] .. 2 offsets[i+1]) of (column, value) pairs.  Columns are unique in a segment, so
+ * ordering the u64 keys (column << 32 | value) ascending orders it by column, unsigned.  Size classes as top-k's:
+ *   k_sort_warp / k_sort_block  segments of <= TOPK_WARP_MAX / TOPK_BLOCK_MAX pairs: the keys in shared memory,
+ *                               padded with ~0 to a power of two, rec_sort, written back in place
+ *   big segments                a group of them at a time (k_topk_classify lists them, k_sort_cut cuts the list into
+ *                               groups of at most $SMATRIX_TOPK_PAIRS pairs): (slot << 32 | column) keys with the
+ *                               value as payload, one radix sort, k_sort_big_scatter writes slot j's run back to its
+ *                               segment */
+__device__ __forceinline__ ull sort_key(const uint32_t* p) { return ((ull)p[0] << 32) | p[1]; }
+template <bool BLOCK>
+__device__ void sort_segment(uint32_t* pairs, uint32_t len, ull* key, uint32_t t, uint32_t T) {
+  uint32_t N = 1u;
+  while (N < len) N <<= 1;
+  for (uint32_t i = t; i < N; i += T) key[i] = i < len ? sort_key(pairs + 2ull * i) : ~0ull;
+  topk_sync<BLOCK>();
+  rec_sort<BLOCK>(key, N, t, T);
+  for (uint32_t i = t; i < len; i += T) {
+    pairs[2ull * i] = (uint32_t)(key[i] >> 32);
+    pairs[2ull * i + 1] = (uint32_t)key[i];
+  }
+  topk_sync<BLOCK>(); /* before the buffer takes the next segment */
+}
+
+__global__ void __launch_bounds__(SMX_BLOCK) k_sort_warp(uint32_t n, const ull* offsets, uint32_t* pairs) {
+  __shared__ ull s_key[SMX_BLOCK / SMX_WARP][TOPK_WARP_MAX];
+  const uint32_t lane = lane_id(), wib = threadIdx.x / SMX_WARP;
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) / SMX_WARP;
+  const uint32_t nwarps = gridDim.x * blockDim.x / SMX_WARP;
+  for (uint32_t i = warp; i < n; i += nwarps) {
+    const ull lo = offsets[i], len = offsets[i + 1] - lo;
+    if (len < 2u || len > TOPK_WARP_MAX) continue;
+    sort_segment<false>(pairs + 2ull * lo, (uint32_t)len, s_key[wib], lane, SMX_WARP);
+  }
+}
+
+__global__ void __launch_bounds__(SMX_BLOCK) k_sort_block(uint32_t n, const ull* offsets, uint32_t* pairs) {
+  __shared__ ull s_key[TOPK_BLOCK_MAX]; /* 32 KB */
+  for (uint32_t i = blockIdx.x; i < n; i += gridDim.x) {
+    const ull lo = offsets[i], len = offsets[i + 1] - lo;
+    if (len <= TOPK_WARP_MAX || len > TOPK_BLOCK_MAX) continue;
+    sort_segment<true>(pairs + 2ull * lo, (uint32_t)len, s_key, threadIdx.x, blockDim.x);
+  }
+}
+
+/* pairs of big segment j (= big_list[j]) */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_sort_big_lens(const uint32_t* big_list, uint32_t n_big, const ull* offsets, uint32_t* lens) {
+  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < n_big; j += gridDim.x * blockDim.x)
+    lens[j] = (uint32_t)(offsets[big_list[j] + 1] - offsets[big_list[j]]);
+}
+/* one thread: the end of the group of big segments that starts at lo (big_off: their exclusive prefix) = the last
+ * segment whose pairs still fit the budget, at least one -> out[0]; the group's pairs -> out[2..3] (u64) */
+__global__ void k_sort_cut(const ull* big_off, uint32_t n_big, uint32_t lo, ull budget, uint32_t* out) {
+  uint32_t a = lo + 1u, b = n_big; /* answer in [a, b] */
+  while (a < b) {
+    const uint32_t m = a + (b - a + 1u) / 2u;
+    if (big_off[m] - big_off[lo] <= budget) a = m; else b = m - 1u;
+  }
+  out[0] = a;
+  *(ull*)(out + 2) = big_off[a] - big_off[lo];
+}
+/* (slot << 32 | column) keys and values of the group's pairs, slot s = segment big_list[lo + s] at big_off[lo + s] */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_sort_big_keys(const uint32_t* big_list, uint32_t lo, uint32_t first, const ull* big_off, const ull* offsets,
+                const uint32_t* pairs, ull* keys, uint32_t* vals) {
+  const uint32_t s = first + blockIdx.y, j = lo + s;
+  const ull at = big_off[j] - big_off[lo], len = big_off[j + 1] - big_off[j];
+  const uint32_t* p = pairs + 2ull * offsets[big_list[j]];
+  for (ull q = (ull)blockIdx.x * blockDim.x + threadIdx.x; q < len; q += (ull)gridDim.x * blockDim.x) {
+    keys[at + q] = ((ull)s << 32) | p[2ull * q];
+    vals[at + q] = p[2ull * q + 1];
+  }
+}
+/* the sorted group back into its segments: slot s's run starts at big_off[lo + s] - big_off[lo] */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_sort_big_scatter(const ull* keys, const uint32_t* vals, uint32_t P, const uint32_t* big_list, uint32_t lo,
+                   const ull* big_off, const ull* offsets, uint32_t* pairs) {
+  for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
+    const ull key = keys[p];
+    const uint32_t j = lo + (uint32_t)(key >> 32);
+    const ull at = offsets[big_list[j]] + (p - (big_off[j] - big_off[lo]));
+    pairs[2ull * at] = (uint32_t)key;
+    pairs[2ull * at + 1] = vals[p];
+  }
+}
+
 /* ---- snapshot support (file mode, reference src/smatrix.c:30-72) --------------------------- */
-/* all row ids of the directory, in no particular order */
-__global__ void __launch_bounds__(SMX_BLOCK) k_list_rows(smx_view_t V, uint32_t* keys, uint32_t* counter) {
+/* the row ids >= from of the directory, in no particular order (a snapshot lists them all: from = 0) */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_list_rows(smx_view_t V, uint32_t from, uint32_t* keys, uint32_t* counter) {
   for (ull pos = blockIdx.x * blockDim.x + threadIdx.x; pos < V.dir_cap;
        pos += (ull)gridDim.x * blockDim.x) {
     Hdr h = ld_hdr(V.dir + pos);
-    if (h.meta & SMX_META_USED) keys[agg_inc(counter)] = h.key;
+    if ((h.meta & SMX_META_USED) && h.key >= from) keys[agg_inc(counter)] = h.key;
   }
 }
 /* log2 of the reference's row size as of now (the caught-up automaton state), per row */
@@ -2770,8 +2858,9 @@ extern "C" void smx_launch_getrow_fill(smx_stream_t st, smx_view_t v, const uint
   }
 }
 
-extern "C" void smx_launch_list_rows(smx_stream_t st, smx_view_t v, uint32_t* keys, uint32_t* counter) {
-  SMX_LAUNCH(k_list_rows, grid_for(v.dir_cap), SMX_BLOCK, st, v, keys, counter);
+extern "C" void smx_launch_list_rows(smx_stream_t st, smx_view_t v, uint32_t from, uint32_t* keys,
+                                     uint32_t* counter) {
+  SMX_LAUNCH(k_list_rows, grid_for(v.dir_cap), SMX_BLOCK, st, v, from, keys, counter);
 }
 extern "C" void smx_launch_row_slog(smx_stream_t st, smx_view_t v, const uint32_t* xs, uint32_t n,
                                     uint32_t* out) {
@@ -2984,6 +3073,67 @@ extern "C" void smx_launch_rec_cut(smx_stream_t st, const uint64_t* pos_off, con
 }
 extern "C" void smx_launch_rec_check(smx_stream_t st, const uint64_t* boff, uint32_t nb, uint32_t* out) {
   SMX_LAUNCH(k_rec_check, grid_for(nb), SMX_BLOCK, st, (const ull*)boff, nb, out);
+}
+extern "C" size_t smx_sort_keys_bytes(uint32_t n) {
+#ifdef SMX_HOSTSIM
+  (void)n;
+  return 64;
+#else
+  size_t bytes = 0;
+  cub::DeviceRadixSort::SortKeys(nullptr, bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n, 0, 32);
+  return bytes + 256;
+#endif
+}
+extern "C" void smx_launch_sort_keys(smx_stream_t st, const uint32_t* in, uint32_t* out, uint32_t n, void* sort_tmp,
+                                     size_t sort_bytes) {
+  if (!n) return;
+#ifdef SMX_HOSTSIM
+  (void)st; (void)sort_tmp; (void)sort_bytes;
+  memcpy(out, in, (size_t)n * 4);
+  std::sort(out, out + n);
+#else
+  cub::DeviceRadixSort::SortKeys(sort_tmp, sort_bytes, in, out, (int)n, 0, 32, (cudaStream_t)st);
+#endif
+}
+extern "C" void smx_launch_sort_small(smx_stream_t st, uint32_t n, const uint64_t* offsets, uint32_t* pairs) {
+  if (!n) return;
+  SMX_LAUNCH(k_sort_warp, grid_for((ull)n * SMX_WARP), SMX_BLOCK, st, n, (const ull*)offsets, pairs);
+  const uint32_t cap = (uint32_t)smx_grid_blocks();
+  SMX_LAUNCH(k_sort_block, n < cap ? n : cap, SMX_BLOCK, st, n, (const ull*)offsets, pairs);
+}
+extern "C" void smx_launch_sort_big_lens(smx_stream_t st, const uint32_t* big_list, uint32_t n_big,
+                                         const uint64_t* offsets, uint32_t* lens) {
+  if (!n_big) return;
+  SMX_LAUNCH(k_sort_big_lens, grid_for(n_big), SMX_BLOCK, st, big_list, n_big, (const ull*)offsets, lens);
+}
+extern "C" void smx_launch_sort_cut(smx_stream_t st, const uint64_t* big_off, uint32_t n_big, uint32_t lo,
+                                    uint64_t budget, uint32_t* out) {
+  SMX_LAUNCH(k_sort_cut, 1, 1, st, (const ull*)big_off, n_big, lo, (ull)budget, out);
+}
+extern "C" void smx_launch_sort_big(smx_stream_t st, const uint32_t* big_list, uint32_t lo, uint32_t n_grp, uint32_t P,
+                                    const uint64_t* big_off, const uint64_t* offsets, uint32_t* pairs, uint64_t* keys_a,
+                                    uint64_t* keys_b, uint32_t* vals_a, uint32_t* vals_b, void* sort_tmp,
+                                    size_t sort_bytes) {
+  if (!n_grp) return;
+  for (uint32_t first = 0; first < n_grp; first += 32768u) {
+    const uint32_t c = (n_grp - first < 32768u) ? n_grp - first : 32768u;
+    SMX_LAUNCH(k_sort_big_keys, dim3(TOPK_BIG_BLOCKS, c, 1u), SMX_BLOCK, st, big_list, lo, first, (const ull*)big_off,
+               (const ull*)offsets, (const uint32_t*)pairs, (ull*)keys_a, vals_a);
+  }
+#ifdef SMX_HOSTSIM
+  (void)sort_tmp; (void)sort_bytes;
+  {
+    std::vector<uint32_t> order(P);
+    for (uint32_t p = 0; p < P; p++) order[p] = p;
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return keys_a[a] < keys_a[b]; });
+    for (uint32_t p = 0; p < P; p++) { keys_b[p] = keys_a[order[p]]; vals_b[p] = vals_a[order[p]]; }
+  }
+#else
+  cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, (const ull*)keys_a, (ull*)keys_b, (const uint32_t*)vals_a,
+                                  vals_b, (int)P, 0, rec_key_bits(n_grp), (cudaStream_t)st);
+#endif
+  SMX_LAUNCH(k_sort_big_scatter, grid_for(P), SMX_BLOCK, st, (const ull*)keys_b, (const uint32_t*)vals_b, P, big_list,
+             lo, (const ull*)big_off, (const ull*)offsets, pairs);
 }
 extern "C" void smx_launch_sum_values(smx_stream_t st, smx_view_t v, uint32_t* big_list, uint32_t* big_counter) {
   SMX_LAUNCH(k_sum_values, grid_for(v.dir_cap * SMX_WARP), SMX_BLOCK, st, v, big_list, big_counter);

@@ -794,11 +794,15 @@ static const uint32_t* rt_ids_on_device(smatrix_shard_t* sh, const uint32_t* xs,
   return sh->stage[0][0];
 }
 
-uint64_t smatrix_b200_shard_getrow_batch(smatrix_shard_t* sh, const uint32_t* xs, size_t n, uint64_t* offsets,
-                                         uint32_t* pairs, uint64_t pairs_cap) {
-  if (n >= 0xFFFFFFFEull) rt_die(sh, "getrow_batch: too many rows in one call");
+/* smatrix_b200_shard_getrow_batch, and with sorted != 0 shard_getrow_sorted_batch: the pairs are sorted by column in
+ * this rank's row buffer before they are copied out */
+static uint64_t rt_getrow(smatrix_shard_t* sh, const char* what, int sorted, const uint32_t* xs, size_t n,
+                          uint64_t* offsets, uint32_t* pairs, uint64_t pairs_cap) {
+  if (n >= 0xFFFFFFFEull) rt_die(sh, "%s: too many rows in one call", what);
   int filled = 0, any = 0;
   const uint64_t total = rt_getrow_core(sh, rt_ids_on_device(sh, xs, n), n, pairs != NULL, pairs_cap, &filled, &any);
+  if (filled && sorted)
+    smatrix_b200_sort_rows(sh->local, n, (const uint64_t*)(sh->inbox + OFF_OFS(sh->cap)), (uint32_t*)sh->rowbuf);
   if (offsets) {
     if (n) {
       smatrix_b200_memcpy(sh->local, offsets, sh->inbox + OFF_OFS(sh->cap), (n + 1) * 8);
@@ -809,6 +813,45 @@ uint64_t smatrix_b200_shard_getrow_batch(smatrix_shard_t* sh, const uint32_t* xs
   }
   if (filled) smatrix_b200_memcpy(sh->local, pairs, sh->rowbuf, (size_t)total * 8);
   return total;
+}
+
+uint64_t smatrix_b200_shard_getrow_batch(smatrix_shard_t* sh, const uint32_t* xs, size_t n, uint64_t* offsets,
+                                         uint32_t* pairs, uint64_t pairs_cap) {
+  return rt_getrow(sh, "getrow_batch", 0, xs, n, offsets, pairs, pairs_cap);
+}
+uint64_t smatrix_b200_shard_getrow_sorted_batch(smatrix_shard_t* sh, const uint32_t* xs, size_t n, uint64_t* offsets,
+                                                uint32_t* pairs, uint64_t pairs_cap) {
+  return rt_getrow(sh, "getrow_sorted_batch", 1, xs, n, offsets, pairs, pairs_cap);
+}
+
+/* The first cap keys >= from of the whole matrix are among the first cap of every rank's own.  Those lists (their
+ * lengths all-gathered) go into every rank's row buffer side by side, in rank order, and every rank sorts the lot. */
+uint64_t smatrix_b200_shard_list_rows(smatrix_shard_t* sh, uint32_t from, uint32_t* keys, uint64_t cap) {
+  const int W = sh->world, me = sh->rank;
+  const uint64_t mine_m = smatrix_list_rows(sh->local, from, NULL, 0);
+  const uint64_t take = mine_m < cap ? mine_m : cap;
+  uint64_t mine[4] = {mine_m, take, (uint64_t)(keys != NULL && cap > 0), 0}, all[RT_MAXW][4];
+  rt_allgather(sh, mine, all);
+  uint64_t m = 0, T = 0, at = 0;
+  int want = 0;
+  for (int r = 0; r < W; r++) {
+    m += all[r][0];
+    if (r < me) at += all[r][1];
+    T += all[r][1];
+    want |= (int)all[r][2];
+  }
+  if (!want || !T) return m;
+  rt_need_rowbuf(sh, (T + 1) / 2); /* T keys of 4 bytes in a buffer of 8-byte pairs; the same T on every rank */
+  uint32_t* d_keys = (uint32_t*)sh->rowbuf;
+  if (take) {
+    smatrix_list_rows(sh->local, from, d_keys + at, cap);
+    for (int r = 0; r < W; r++)
+      if (r != me) smatrix_b200_memcpy(sh->local, (uint32_t*)sh->peer_rowbuf[r] + at, d_keys + at, (size_t)take * 4);
+  }
+  rt_barrier(sh);
+  if (keys) smatrix_b200_sort_keys(sh->local, d_keys, (size_t)T, keys, cap);
+  rt_barrier(sh); /* nobody writes into a row buffer that its rank still sorts from */
+  return m;
 }
 
 /* The collective core of both CF calls: rows through the getrow route, totals through two sharded gets, scores

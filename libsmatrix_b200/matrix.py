@@ -100,6 +100,71 @@ def _rec_call(fn, basket_offsets, items, k):
     return counts, ids, scores
 
 
+def _check_key(name, v) -> int:
+    if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not 0 <= int(v) <= 0xFFFFFFFF:
+        raise ValueError(f"{name} must be an integer row key in 0..2^32 - 1, got {v!r}")
+    return int(v)
+
+
+def _check_count(name, v) -> int:
+    if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or int(v) < 1:
+        raise ValueError(f"{name} must be an integer >= 1, got {v!r}")
+    return int(v)
+
+
+def _list_rows(fn, start, limit, bound, device, dev):
+    """fn(from, keys_ptr, cap) -> m, into an array of min(limit, bound) keys (bound >= m) on the host or on CUDA
+    device `dev`; -> the first min(limit, m) keys."""
+    n = bound if limit is None else min(limit, bound)
+    if device:
+        import torch
+        keys = torch.empty(n, dtype=torch.int32, device=torch.device("cuda", dev))
+        ptr = keys.data_ptr()
+    else:
+        keys = np.empty(n, dtype=np.uint32)
+        ptr = keys.ctypes.data
+    got = min(int(fn(start, ptr if n else None, n)), n)
+    if got == n:
+        return keys
+    return keys[:got].clone() if device else keys[:got].copy()
+
+
+def _getrow_sorted(fn, xs):
+    """fn(xs_ptr, n, offsets_ptr, pairs_ptr, cap) -> total: a CUDA tensor in -> (int64 offsets, int32 pairs) on its
+    device; anything else -> numpy (uint64 offsets, uint32 pairs)."""
+    if _is_torch(xs) and xs.is_cuda:
+        import torch
+        if xs.dtype not in (torch.int32, torch.uint32):
+            raise TypeError("torch batch arrays must be int32/uint32")
+        xs = xs.contiguous()
+        n = xs.numel()
+        offsets = torch.empty(n + 1, dtype=torch.int64, device=xs.device)
+        torch.cuda.current_stream(xs.device).synchronize()      # the rows may still be in flight on torch's stream
+        total = int(fn(xs.data_ptr(), n, None, None, 0))
+        pairs = torch.empty((total, 2), dtype=torch.int32, device=xs.device)
+        assert int(fn(xs.data_ptr(), n, offsets.data_ptr(), pairs.data_ptr() if total else None, total)) == total
+        return offsets, pairs
+    xs = np.ascontiguousarray(xs.numpy() if _is_torch(xs) else xs, dtype=np.uint32)
+    n = len(xs)
+    offsets = np.zeros(n + 1, dtype=np.uint64)
+    total = int(fn(xs.ctypes.data, n, None, None, 0))          # the size query; the offsets come down once
+    pairs = np.zeros((total, 2), dtype=np.uint32)
+    assert int(fn(xs.ctypes.data, n, offsets.ctypes.data, pairs.ctypes.data if total else None, total)) == total
+    return offsets, pairs
+
+
+def _pages(m, start, rows_per_page, device):
+    while True:
+        keys = m.rows(start, rows_per_page, device)
+        if len(keys) == 0:
+            return
+        yield (keys,) + tuple(m.getrow_sorted_batch(keys))
+        last = int(keys[-1]) & 0xFFFFFFFF
+        if len(keys) < rows_per_page or last == 0xFFFFFFFF:
+            return
+        start = last + 1
+
+
 class DevPtr:
     """A raw device array of `n` uint32 (library- or peer-allocated memory that is not a tensor)."""
     __slots__ = ("ptr", "n")
@@ -372,6 +437,29 @@ class SparseMatrix:
         The basket's own items and id 0 are never recommended.  numpy in -> numpy out; CUDA torch tensors in (int64
         offsets, int32 items) -> tensors on their device out, with no copy through the host."""
         return _rec_call(lambda *a: self._lib.smatrix_cf_recommend_batch(self._handle(), *a), basket_offsets, items, k)
+
+    # ---- enumeration -------------------------------------------------------------------------
+    def rows(self, start: int = 0, limit: int | None = None, device: bool = False):
+        """The row keys >= start in ascending order, at most `limit` of them (all by default): the rows a snapshot
+        lists, including rows without pairs.  A uint32 numpy array, or with device=True an int32 CUDA tensor on the
+        matrix's GPU that is filled without a copy through the host.  One pass over the directory per call."""
+        start = _check_key("start", start)
+        limit = None if limit is None else _check_count("limit", limit)
+        return _list_rows(lambda *a: self._lib.smatrix_list_rows(self._handle(), *a), start, limit,
+                          self.stat("rows"), device, self.device)
+
+    def getrow_sorted_batch(self, xs):
+        """getrow_batch with every row's pairs in ascending column order -> (offsets[n+1], pairs[total, 2]): numpy
+        (uint64, uint32) for host rows, or int64 / int32 tensors on the device of a CUDA tensor of rows, with no copy
+        through the host."""
+        return _getrow_sorted(lambda *a: self._lib.smatrix_getrow_sorted_batch(self._handle(), *a), xs)
+
+    def iter_rows(self, start: int = 0, rows_per_page: int = 1 << 20, device: bool = False):
+        """Every row with key >= start exactly once, in key order, a page of at most rows_per_page rows at a time:
+        yields (keys, offsets, pairs) = (rows(...), *getrow_sorted_batch(keys)), numpy or (device=True) CUDA tensors."""
+        start = _check_key("start", start)
+        rows_per_page = _check_count("rows_per_page", rows_per_page)
+        return _pages(self, start, rows_per_page, device)
 
     # ---- device controls (include/smatrix_b200.h) --------------------------------------------
     def stat(self, name: str) -> int:

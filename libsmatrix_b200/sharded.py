@@ -27,7 +27,8 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from .matrix import DevPtr, SparseMatrix, _rec_call, _topk_call
+from .matrix import (DevPtr, SparseMatrix, _check_count, _check_key, _getrow_sorted, _list_rows, _rec_call,
+                     _topk_call)
 
 _seq = [0]
 
@@ -193,6 +194,18 @@ class ShardedSparseMatrix:
         rank may pass no baskets (offsets [0])."""
         return _rec_call(lambda *a: self._lib.smatrix_b200_shard_cf_recommend_batch(self._handle(), *a),
                          basket_offsets, items, k)
+
+    def rows(self, start: int = 0, limit: int | None = None, device: bool = False):
+        """Collective: SparseMatrix.rows of the whole sharded matrix.  Every rank passes the same start and limit
+        and gets the same keys (device=True: on this rank's GPU)."""
+        start = _check_key("start", start)
+        limit = None if limit is None else _check_count("limit", limit)
+        fn = lambda *a: self._lib.smatrix_b200_shard_list_rows(self._handle(), *a)
+        return _list_rows(fn, start, limit, int(fn(start, None, 0)), device, self.local.device)
+
+    def getrow_sorted_batch(self, xs):
+        """Collective: SparseMatrix.getrow_sorted_batch for THIS rank's rows (a rank may pass none)."""
+        return _getrow_sorted(lambda *a: self._lib.smatrix_b200_shard_getrow_sorted_batch(self._handle(), *a), xs)
 
     def getrow_batch_into(self, d_xs, n: int, d_offsets: int, d_pairs: int, pairs_cap: int) -> int:
         """The raw collective call on device (or host) pointers; returns the total number of pairs."""
