@@ -41,8 +41,10 @@ typedef struct smatrix_s smatrix_t;
  * DURABILITY differs from the reference: the reference's IO thread streams dirty rows to the
  * file all the time (src/smatrix.c:418-596); here the file changes only in smatrix_close and in
  * smatrix_b200_snapshot (smatrix_b200.h) — written to a temporary file, fsync'ed, then renamed
- * over the old one, so the file on disk is always a complete snapshot.  Updates made after the
- * last snapshot are lost if the process dies (every "libsmatrix error" path abort()s). */
+ * over the old one — and in smatrix_b200_checkpoint, which appends the rows written since the
+ * last save and then switches the header's directory pointer, so the file on disk always loads
+ * to a complete persisted state.  Updates made after the last snapshot or checkpoint are lost if
+ * the process dies (every "libsmatrix error" path abort()s). */
 smatrix_t* smatrix_open(const char* fname);
 
 /* replaces src/smatrix.c:113-133.  Writes the snapshot (file mode) and frees all device memory. */

@@ -31,10 +31,26 @@ smatrix_t* smatrix_b200_open_arena(const char* fname, int device, size_t arena_b
 
 /* File-backed handles: write the snapshot NOW (temporary file, fsync, atomic rename) and return 0
  * on success, -1 on failure (or when the handle has no file).  The reference streams dirty rows to
- * its file continuously from an IO thread (src/smatrix.c:418-596); this build persists only here
- * and in smatrix_close, so a process that abort()s in between loses the updates since the last
- * snapshot — call this at the checkpoints the application can afford. */
+ * its file continuously from an IO thread (src/smatrix.c:418-596); this build persists only here,
+ * in smatrix_b200_checkpoint and in smatrix_close, so a process that abort()s in between loses the
+ * updates since the last snapshot or checkpoint — call one of them at the moments the application
+ * can afford.  A snapshot rewrites the whole file; a checkpoint costs about what the rows written
+ * since the last save take in the file. */
 int   smatrix_b200_snapshot(smatrix_t* self);
+/* File-backed handles: persist the matrix by appending to the file only the row blocks of rows written since the
+ * file last matched the table, then a new directory, then switching the header to it.  0 or -1 (-1 also when the
+ * handle has no file).  Afterwards the file loads — here at any world size, in the C checker, in the reference — to
+ * exactly what a full snapshot taken at the same moment would load to.
+ * Crash safety: the blocks go to E = the file size rounded up to 8, the directory chain behind them, fsync, then
+ * the header's 8-byte pointer at offset 8, fsync; nothing else before E is written, so the file on disk loads to
+ * the previous state or to the new one at every moment.  A checkpoint that fails keeps the rows dirty.
+ * It takes a full snapshot instead (temporary file, rename) when the file was missing or empty at open or is now,
+ * when its directory does not list the table's rows (a listed row is missing from the table, or the counts do not
+ * add up), or when the file would grow past twice the size of a full snapshot.  Only the row SET is checked: a
+ * file replaced behind the handle's back by one with the same rows and other cells is not detected.  With no row
+ * written since the last save it returns 0 and does not open the file for writing.  smatrix_close and
+ * smatrix_b200_snapshot keep writing full snapshots. */
+int   smatrix_b200_checkpoint(smatrix_t* self);
 
 /* Device-level pieces of the snapshot, used by the multi-GPU router (every rank writes its part of ONE
  * .smx file, and reads a share of one).  The file is always the reference's format: 512-byte header,
@@ -53,6 +69,31 @@ uint64_t smatrix_b200_snap_rows_base(uint64_t total_rows);
 int      smatrix_b200_snap_layout(int fd, uint64_t total_rows, uint64_t total_bytes);
 int      smatrix_b200_snap_write(smatrix_t* self, int fd, uint64_t byte_base, uint64_t first_entry);
 int      smatrix_b200_snap_commit(const char* tmp, const char* fname);
+/* Device-level pieces of smatrix_b200_checkpoint, for the router in the same way (every rank appends its part):
+ *   ckpt_extent     snap_extent over the rows written since the marks were last cleared (held until
+ *                   snap_write_at, or ckpt_reset)
+ *   snap_write_at   snap_write with the directory chain at byte dir_base instead of 512
+ *   load_entries    the directory entries of a loader's share in DIRECTORY order, before any load_next: returns
+ *                   their number; entries [first, first + n) go to DEVICE arrays (key, row offset low / high word)
+ *                   when d_keys is not NULL
+ *   ckpt_keep       the keep filter over n old entries (DEVICE arrays as load_entries fills them): returns how many
+ *                   of them name a row that is not in the table; the entries of clean rows are appended, in their
+ *                   order, to the handle's kept list, *kept = its length
+ *   ckpt_write_kept the kept list as entries first_entry.. of the chain at dir_base, then empties it
+ *   ckpt_reset      empties the kept list and drops the held extent (a checkpoint that falls back)
+ *   ckpt_layout     the directory block headers of a chain of `entries` entries at dir_base, the file extended to
+ *                   its end (sparse)
+ *   ckpt_switch     fsync, the header's pointer := dir_base, fsync
+ *   clear_dirty     the file matches the table: clear the marks */
+int      smatrix_b200_ckpt_extent(smatrix_t* self, uint64_t* rows, uint64_t* bytes);
+int      smatrix_b200_snap_write_at(smatrix_t* self, int fd, uint64_t byte_base, uint64_t dir_base, uint64_t first_entry);
+uint64_t smatrix_b200_ckpt_keep(smatrix_t* self, const uint32_t* d_keys, const uint32_t* d_lo, const uint32_t* d_hi,
+                                size_t n, uint64_t* kept);
+int      smatrix_b200_ckpt_write_kept(smatrix_t* self, int fd, uint64_t dir_base, uint64_t first_entry);
+void     smatrix_b200_ckpt_reset(smatrix_t* self);
+int      smatrix_b200_ckpt_layout(int fd, uint64_t dir_base, uint64_t entries);
+int      smatrix_b200_ckpt_switch(int fd, uint64_t dir_base);
+void     smatrix_b200_clear_dirty(smatrix_t* self);
 /* The reader of a .smx file: share `share` of `shares` (a contiguous range of directory entries, cut evenly)
  * is read in file order, window by window ($SMATRIX_LOAD_WINDOW bytes, default 64 MiB; a bigger row grows
  * it), every row header is checked on the host, and the device expands the raw row blocks into pieces of
@@ -68,6 +109,8 @@ smx_loader_t* smatrix_b200_load_begin(smatrix_t* self, int fd, int share, int sh
 int  smatrix_b200_load_next(smx_loader_t* ld, const uint32_t** d_xs, const uint32_t** d_ys, const uint32_t** d_vs,
                             size_t* n_ops, const uint32_t** d_keys, const uint32_t** d_logs, size_t* n_rows);
 void smatrix_b200_load_end(smx_loader_t* ld);
+uint64_t smatrix_b200_load_entries(smx_loader_t* ld, uint64_t first, uint64_t n, uint32_t* d_keys, uint32_t* d_lo,
+                                   uint32_t* d_hi);
 void smatrix_b200_load_fixup(smatrix_t* self, const uint32_t* d_keys, const uint32_t* d_logs, size_t n);
 
 int   smatrix_b200_device(smatrix_t* self);   /* CUDA device ordinal                            */
@@ -84,7 +127,8 @@ enum {
   SMX_STAT_DIR_CAP = 2,     /* directory capacity in entries                              */
   SMX_STAT_SLAB_BYTES = 3,  /* bytes handed out by the slab allocator                     */
   SMX_STAT_DEVICE_BYTES = 4,/* bytes of device memory held (directory + slab segments + scratch) */
-  SMX_STAT_LAUNCHES = 5,    /* kernels launched by this handle so far                     */
+  SMX_STAT_LAUNCHES = 5,    /* kernels launched by this handle so far (not counted: the row listing of a snapshot
+                               and the pass that clears the checkpoint marks after a load or a save) */
   SMX_STAT_ROUNDS = 6,      /* upsert rounds (1 per pass + 1 per growth retry) so far     */
   SMX_STAT_ROW_GROWS = 7,   /* row growth (rehash) events so far                          */
   SMX_STAT_DIR_GROWS = 8,   /* directory rehash events so far                             */
@@ -108,7 +152,8 @@ enum {
   SMX_STAT_TOPK_BIG = 28,   /* top-k segments (items) longer than 4096 pairs: ranked by the multi-block radix select */
   SMX_STAT_TOPK_PASSES = 29,/* digit passes that select ran so far */
   SMX_STAT_REC_BIG = 30,    /* baskets longer than 4096 pairs: aggregated by the global sort of smatrix_cf_recommend_batch */
-  SMX_STAT_SORT_BIG = 31    /* segments longer than 4096 pairs: sorted by the global radix sort of smatrix_b200_sort_rows */
+  SMX_STAT_SORT_BIG = 31,   /* segments longer than 4096 pairs: sorted by the global radix sort of smatrix_b200_sort_rows */
+  SMX_STAT_DIRTY_ROWS = 32  /* rows written since the file last matched the table (since open without a file); scans the directory */
 };
 uint64_t smatrix_b200_stat(smatrix_t* self, int which);
 

@@ -48,9 +48,9 @@ smatrix_shard_t* smatrix_b200_shard_open_arena(const char* name, int rank, int w
  * at one world size loads at any other, on one GPU through smatrix_open, and in the reference; a single-GPU
  * or reference file loads sharded.  Every rank reads an even share of the file's directory, expands its row
  * blocks on its GPU and routes the rows to their owners.
- * Durability is that of a single-GPU handle (smatrix_b200_snapshot): the matrix is persisted only by
- * smatrix_b200_shard_snapshot and smatrix_b200_shard_close, so a job that dies in between loses the updates
- * since the last snapshot. */
+ * Durability is that of a single-GPU handle (smatrix_b200_snapshot, smatrix_b200_checkpoint): the matrix is
+ * persisted only by smatrix_b200_shard_snapshot, smatrix_b200_shard_checkpoint and smatrix_b200_shard_close, so a
+ * job that dies in between loses the updates since the last of them. */
 smatrix_shard_t* smatrix_b200_shard_open_file(const char* name, int rank, int world, int device,
                                               size_t arena_bytes, const char* fname);
 /* Collective: write the snapshot now.  The file goes to a temporary name (`fname.tmp`, laid out by rank 0,
@@ -58,6 +58,14 @@ smatrix_shard_t* smatrix_b200_shard_open_file(const char* name, int rank, int wo
  * and rank 0 renames it over the old one and syncs the directory.  Returns 0 on every rank, or -1 on every
  * rank when no rank has a file or any step failed; a failed snapshot leaves the previous file intact. */
 int smatrix_b200_shard_snapshot(smatrix_shard_t* self);
+/* Collective: smatrix_b200_checkpoint for the sharded matrix — append the row blocks of the rows written since
+ * the file last matched the table, a new directory behind them, then switch the header.  Every rank reads an even
+ * share of the old directory and routes its entries to the rows' owners, which keep the entries of their clean
+ * rows; every rank appends its dirty rows' blocks and its entries side by side, rank 0 switches the header.  The
+ * fall-backs to the full snapshot (no base, a directory that does not list the table's rows, a file past twice a
+ * full snapshot) are decided collectively.  Returns the same value on every rank: 0, or -1 when no rank has a file
+ * or any step failed (the file then still loads to the previous state and the rows stay dirty). */
+int smatrix_b200_shard_checkpoint(smatrix_shard_t* self);
 /* Collective.  With a file (smatrix_b200_shard_open_file) the snapshot is written first; if that fails,
  * the same message as smatrix_close's goes to stdout and the matrix is closed anyway. */
 void smatrix_b200_shard_close(smatrix_shard_t* self);

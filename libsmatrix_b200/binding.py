@@ -51,6 +51,7 @@ PROTOTYPES = {
     "smatrix_b200_open": (C.c_void_p, [C.c_char_p, C.c_int]),
     "smatrix_b200_open_arena": (C.c_void_p, [C.c_char_p, C.c_int, C.c_size_t]),
     "smatrix_b200_snapshot": (C.c_int, [C.c_void_p]),
+    "smatrix_b200_checkpoint": (C.c_int, [C.c_void_p]),
     "smatrix_b200_device": (C.c_int, [C.c_void_p]),
     "smatrix_b200_stream": (C.c_void_p, [C.c_void_p]),
     "smatrix_b200_sync": (None, [C.c_void_p]),
@@ -118,6 +119,16 @@ PROTOTYPES = {
                                          C.c_void_p, C.c_void_p]),
     "smatrix_b200_load_end": (None, [C.c_void_p]),
     "smatrix_b200_load_fixup": (None, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
+    "smatrix_b200_load_entries": (C.c_uint64, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
+                                               C.c_void_p]),
+    "smatrix_b200_ckpt_extent": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "smatrix_b200_snap_write_at": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64, C.c_uint64, C.c_uint64]),
+    "smatrix_b200_ckpt_keep": (C.c_uint64, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "smatrix_b200_ckpt_write_kept": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64, C.c_uint64]),
+    "smatrix_b200_ckpt_reset": (None, [C.c_void_p]),
+    "smatrix_b200_ckpt_layout": (C.c_int, [C.c_int, C.c_uint64, C.c_uint64]),
+    "smatrix_b200_ckpt_switch": (C.c_int, [C.c_int, C.c_uint64]),
+    "smatrix_b200_clear_dirty": (None, [C.c_void_p]),
 }
 
 # include/smatrix_shard.h
@@ -126,6 +137,7 @@ PROTOTYPES.update({
     "smatrix_b200_shard_open_arena": (C.c_void_p, [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_size_t]),
     "smatrix_b200_shard_open_file": (C.c_void_p, [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_char_p]),
     "smatrix_b200_shard_snapshot": (C.c_int, [C.c_void_p]),
+    "smatrix_b200_shard_checkpoint": (C.c_int, [C.c_void_p]),
     "smatrix_b200_shard_close": (None, [C.c_void_p]),
     "smatrix_b200_shard_local": (C.c_void_p, [C.c_void_p]),
     "smatrix_b200_shard_rank": (C.c_int, [C.c_void_p]),
@@ -162,7 +174,7 @@ STAT = {"rows": 0, "nnz": 1, "dir_cap": 2, "slab_bytes": 3, "device_bytes": 4, "
         "ns_grow_plan": 12, "ns_slab": 13, "ns_migrate": 14, "ns_dir": 15, "value_sum": 16,
         "live_bucket_bytes": 17, "free_bytes": 18, "recycled": 19, "h2d_bytes": 20, "d2h_bytes": 21, "bucket_bytes": 22, "spilled": 23,
         "sliced_gets": 24, "wide_chunks": 25, "ns_alloc": 26, "allocs": 27,
-        "topk_big": 28, "topk_passes": 29, "rec_big": 30, "sort_big": 31}
+        "topk_big": 28, "topk_passes": 29, "rec_big": 30, "sort_big": 31, "dirty_rows": 32}
 
 _cache: dict[str, C.CDLL] = {}
 

@@ -69,6 +69,8 @@ typedef struct {
   struct { uint32_t n_big, pad; uint64_t big_pairs; } sort; /* big segments of a sort_rows call and their pairs */
   struct { uint32_t end, pad; uint64_t pairs; } sort_cut;   /* end of the next group of big segments, its pairs */
   uint32_t listed;     /* rows smatrix_list_rows found */
+  uint32_t ck_missing; /* old directory entries of a checkpoint whose row is not in the table */
+  uint64_t ck_kept;    /* ... and the number of them the keep filter kept (its last offset) */
 } smx_small_t;
 enum { DS_X, DS_Y, DS_V, DS_OUT, DS_WORDS }; /* the words of d_small: a single op's arguments, a one-word answer */
 
@@ -146,6 +148,9 @@ struct smatrix_s {
     /* loading a snapshot (smatrix_b200_load_next): a window of file bytes, its tiles, their counts and offsets,
      * the op stream (x, y, v) and the (key, log2 size) fixups of a piece */
     smx_dbuf_t ld_raw, ld_tiles, ld_cnt, ld_off, ld_ops, ld_fix;
+    /* checkpoints (smatrix_b200_ckpt_keep): old directory entries on their way up (key, row offset lo / hi), their
+     * keep flags, its scan and the kept entries packed as in the file */
+    smx_dbuf_t ck_in, ck_flags, ck_off, ck_out;
   } db;
   uint32_t topk_pairs;  /* SMATRIX_TOPK_PAIRS: pairs per piece of a cf_topk_batch call */
   uint64_t n_topk_big, n_topk_passes;
@@ -182,6 +187,9 @@ struct smatrix_s {
   uint64_t snap_rows;
   uint64_t* snap_hoff; /* a table of one chunk of rows: its layout (offsets, keys, big rows) as snap_extent */
   uint32_t* snap_hkeys; /* read it back, so that snap_write neither lays it out nor reads it again */
+  int ck_base;          /* the file matched the table at some point (a load, a snapshot or a checkpoint) */
+  unsigned char* ck_kept; /* kept directory entries of the checkpoint in progress (12 bytes each, file order) */
+  uint64_t ck_kept_n, ck_kept_cap;
 };
 
 /* ------------------------------------------------------------------------------ errors */
@@ -1610,7 +1618,7 @@ uint64_t smatrix_list_rows(smatrix_t* s, uint32_t from, uint32_t* keys, uint64_t
     uint32_t* d_keys = dbuf_need(s, &s->db.ls_keys, (size_t)rows * 8 + 4); /* as found, sorted, the counter */
     uint32_t* d_cnt = d_keys + 2 * rows;
     CK(cudaMemsetAsync(d_cnt, 0, 4, s->stream));
-    smx_launch_list_rows(s->stream, view_of(s), from, d_keys, d_cnt);
+    smx_launch_list_rows(s->stream, view_of(s), from, SMX_META_USED, d_keys, d_cnt);
     copy_d2h(s, &s->h_small->listed, d_cnt, 4, s->stream);
     CK(cudaStreamSynchronize(s->stream));
     s->n_launches++;
@@ -1758,6 +1766,15 @@ static void snap_free_keys(smatrix_t* s) {
   s->snap_rows = 0;
 }
 
+/* caller holds the handle lock: the file matches the table again (after a load, a snapshot or a checkpoint).  Like
+ * the snapshot's listing, the pass is not counted in SMX_STAT_LAUNCHES, so that a snapshot or a load counts the
+ * launches it always did */
+static void clear_dirty(smatrix_t* s) {
+  smx_launch_clear_dirty(s->stream, view_of(s));
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+}
+
 /* rows [first, first + len) of the listed keys: row sizes -> 8-byte units -> offsets (d_off[0..len]) */
 typedef struct { smx_rowplan_t p; uint64_t* d_off; uint32_t* d_slog; } smx_snapchunk_t;
 static smx_snapchunk_t snap_chunk_bufs(smatrix_t* s, uint32_t len) { /* the same buffers for the same len */
@@ -1780,15 +1797,21 @@ static smx_snapchunk_t snap_chunk(smatrix_t* s, uint64_t first, uint32_t len) {
   return c;
 }
 
-/* caller holds the handle lock, the stream is idle */
-static void snap_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes) {
+/* caller holds the handle lock, the stream is idle.  need = SMX_META_USED: every row (a snapshot);
+ * | SMX_META_DIRTY: the rows written since the file last matched the table (a checkpoint) */
+static void snap_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes, uint32_t need) {
   snap_free_keys(s);
   read_ctl(s);
-  const uint64_t n_rows = s->h_ctl->dir_used;
+  uint64_t n_rows = s->h_ctl->dir_used;
   if (n_rows) {
     s->snap_keys = (uint32_t*)dmalloc(s, n_rows * 4);
     CK(cudaMemsetAsync(&s->d_ctl->scratch, 0, 8, s->stream));
-    smx_launch_list_rows(s->stream, view_of(s), 0, s->snap_keys, (uint32_t*)&s->d_ctl->scratch);
+    smx_launch_list_rows(s->stream, view_of(s), 0, need, s->snap_keys, (uint32_t*)&s->d_ctl->scratch);
+    if (need != SMX_META_USED) {
+      copy_d2h(s, &s->h_small->listed, &s->d_ctl->scratch, 4, s->stream);
+      CK(cudaStreamSynchronize(s->stream));
+      n_rows = s->h_small->listed;
+    }
   }
   s->snap_rows = n_rows;
   uint64_t total = 0;
@@ -1815,20 +1838,22 @@ static void snap_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes) {
   *bytes = total;
 }
 
-/* directory entries e0 .. e0 + n - 1 (12 bytes each in `ents`): entry e is slot e % 2^22 of block e / 2^22 */
-static int snap_write_entries(int fd, const unsigned char* ents, uint64_t e0, uint64_t n) {
+/* directory entries e0 .. e0 + n - 1 (12 bytes each in `ents`) of the chain at dir_base: entry e is slot e % 2^22
+ * of block e / 2^22 */
+static int snap_write_entries(int fd, const unsigned char* ents, uint64_t dir_base, uint64_t e0, uint64_t n) {
   while (n) {
     const uint64_t b = e0 / SMX_F_DIR_ENTRIES, slot = e0 % SMX_F_DIR_ENTRIES;
     const uint64_t run = (n < SMX_F_DIR_ENTRIES - slot) ? n : SMX_F_DIR_ENTRIES - slot;
-    if (write_all(fd, ents, run * SMX_F_DIR_SLOT, SMX_F_META + b * SMX_F_BLOCK_BYTES + SMX_F_DIR_HEAD + slot * SMX_F_DIR_SLOT))
+    if (write_all(fd, ents, run * SMX_F_DIR_SLOT, dir_base + b * SMX_F_BLOCK_BYTES + SMX_F_DIR_HEAD + slot * SMX_F_DIR_SLOT))
       return -1;
     ents += run * SMX_F_DIR_SLOT; e0 += run; n -= run;
   }
   return 0;
 }
 
-/* caller holds the handle lock; the rows snap_extent listed */
-static int snap_write(smatrix_t* s, int fd, uint64_t fpos, uint64_t first_entry) {
+/* caller holds the handle lock; the rows snap_extent listed, their blocks from byte fpos on, their entries from
+ * first_entry on in the directory chain at dir_base */
+static int snap_write(smatrix_t* s, int fd, uint64_t fpos, uint64_t dir_base, uint64_t first_entry) {
   const uint64_t n_rows = s->snap_rows;
   unsigned char* ents = (unsigned char*)malloc((size_t)SMX_SNAPSHOT_ROWS * SMX_F_DIR_SLOT);
   uint32_t* h_keys = (uint32_t*)malloc(SMX_SNAPSHOT_ROWS * 4);
@@ -1871,7 +1896,7 @@ static int snap_write(smatrix_t* s, int fd, uint64_t fpos, uint64_t first_entry)
       memcpy(de, &h_keys[i], 4);
       memcpy(de + 4, &row_fpos, 8);
     }
-    if (write_all(fd, out, need, fpos) || snap_write_entries(fd, ents, first_entry + first, len)) rc = -1;
+    if (write_all(fd, out, need, fpos) || snap_write_entries(fd, ents, dir_base, first_entry + first, len)) rc = -1;
     fpos += need;
   }
   CK(cudaGetLastError());
@@ -1908,14 +1933,18 @@ int smatrix_b200_snap_layout(int fd, uint64_t total_rows, uint64_t total_bytes) 
 int smatrix_b200_snap_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes) {
   enter(s);
   CK(cudaStreamSynchronize(s->stream));
-  snap_extent(s, rows, bytes);
+  snap_extent(s, rows, bytes, SMX_META_USED);
   leave(s);
   return 0;
 }
 
 int smatrix_b200_snap_write(smatrix_t* s, int fd, uint64_t byte_base, uint64_t first_entry) {
+  return smatrix_b200_snap_write_at(s, fd, byte_base, SMX_F_META, first_entry);
+}
+
+int smatrix_b200_snap_write_at(smatrix_t* s, int fd, uint64_t byte_base, uint64_t dir_base, uint64_t first_entry) {
   enter(s);
-  const int rc = snap_write(s, fd, byte_base, first_entry);
+  const int rc = snap_write(s, fd, byte_base, dir_base, first_entry);
   leave(s);
   return rc;
 }
@@ -1936,15 +1965,18 @@ static int snapshot_save(smatrix_t* s) {
   int fd = open(tmp, O_RDWR | O_CREAT | O_TRUNC, 00600);
   if (fd == -1) { perror("cannot open file"); free(tmp); return -1; }
   uint64_t rows = 0, bytes = 0;
-  snap_extent(s, &rows, &bytes);
+  snap_extent(s, &rows, &bytes, SMX_META_USED);
   int rc = smatrix_b200_snap_layout(fd, rows, bytes);
-  if (snap_write(s, fd, smatrix_b200_snap_rows_base(rows), 0)) rc = -1;
+  if (snap_write(s, fd, smatrix_b200_snap_rows_base(rows), SMX_F_META, 0)) rc = -1;
   if (rc == 0 && fsync(fd) == -1) rc = -1; /* the data is on disk before the old file is replaced */
   if (close(fd) == -1) rc = -1;
   if (rc == 0) rc = smatrix_b200_snap_commit(tmp, s->fname);
   if (rc) {
     perror("libsmatrix: writing the snapshot failed");
     unlink(tmp); /* the previous snapshot, if any, is still intact */
+  } else {
+    clear_dirty(s); /* the file matches the table */
+    s->ck_base = 1;
   }
   free(tmp);
   return rc;
@@ -1973,6 +2005,7 @@ struct smx_loader_s {
   uint64_t n, next;
   size_t window;     /* SMATRIX_LOAD_WINDOW: bytes per pread (grown for a bigger row) */
   uint64_t cells;    /* SMATRIX_LOAD_CELLS: cells per piece (a bigger row is a piece of its own) */
+  int sorted;        /* rows are in file order (load_next); until then in directory order (load_entries) */
   unsigned char* win; size_t win_cap;   /* pinned */
   smx_load_tile_t* tiles; size_t tiles_cap;
   uint32_t* fix; size_t fix_cap;        /* keys, then log2 sizes */
@@ -2056,10 +2089,31 @@ smx_loader_t* smatrix_b200_load_begin(smatrix_t* s, int fd, int share, int share
     smatrix_b200_load_end(ld);
     return NULL;
   }
-  /* reads go forward through the file even where a foreign file's rows are not in directory order */
-  for (uint64_t i = 1; i < ld->n; i++)
-    if (ld->rows[i].rpos < ld->rows[i - 1].rpos) { qsort(ld->rows, ld->n, sizeof(smx_ldrow_t), ldrow_cmp); break; }
   return ld;
+}
+
+uint64_t smatrix_b200_load_entries(smx_loader_t* ld, uint64_t first, uint64_t n, uint32_t* d_keys, uint32_t* d_lo,
+                                   uint32_t* d_hi) {
+  if (ld->sorted) smx_die("load_entries: the loader has started reading rows");
+  if (!d_keys || first >= ld->n) return ld->n;
+  if (n > ld->n - first) n = ld->n - first;
+  smatrix_t* s = ld->s;
+  uint32_t* h = (uint32_t*)malloc((size_t)n * 12 + 4);
+  if (!h) smx_die("out of host memory");
+  for (uint64_t i = 0; i < n; i++) {
+    const smx_ldrow_t* r = &ld->rows[first + i];
+    h[i] = r->key;
+    h[n + i] = (uint32_t)r->rpos;
+    h[2 * n + i] = (uint32_t)(r->rpos >> 32);
+  }
+  enter(s);
+  copy_h2d(s, d_keys, h, (size_t)n * 4, s->stream);
+  copy_h2d(s, d_lo, h + n, (size_t)n * 4, s->stream);
+  copy_h2d(s, d_hi, h + 2 * n, (size_t)n * 4, s->stream);
+  CK(cudaStreamSynchronize(s->stream));
+  leave(s);
+  free(h);
+  return ld->n;
 }
 
 /* the window holds file bytes [at, at + len) */
@@ -2076,6 +2130,11 @@ int smatrix_b200_load_next(smx_loader_t* ld, const uint32_t** d_xs, const uint32
                            size_t* n_ops, const uint32_t** d_keys, const uint32_t** d_logs, size_t* n_rows) {
   smatrix_t* s = ld->s;
   *n_ops = *n_rows = 0;
+  if (!ld->sorted) { /* reads go forward through the file even where a foreign file's rows are not in directory order */
+    ld->sorted = 1;
+    for (uint64_t i = 1; i < ld->n; i++)
+      if (ld->rows[i].rpos < ld->rows[i - 1].rpos) { qsort(ld->rows, ld->n, sizeof(smx_ldrow_t), ldrow_cmp); break; }
+  }
   if (ld->next == ld->n) return 0;
   const uint64_t wstart = ld->rows[ld->next].rpos & ~7ull; /* our files keep every cell 8-byte aligned */
   size_t len = ld->window;
@@ -2190,6 +2249,196 @@ static int snapshot_load(smatrix_t* s, int fd) {
   }
   if (rc) fprintf(stderr, "libsmatrix: file is corrupt\n");
   smatrix_b200_load_end(ld);
+  if (rc == 0) { /* the loaded rows are what the file holds */
+    enter(s);
+    clear_dirty(s);
+    s->ck_base = 1;
+    leave(s);
+  }
+  return rc;
+}
+
+/* ------------------------------------------------------------------------------ checkpoint (.smx)
+ * An incremental save: only the row blocks of the rows written since the file last matched the table (the
+ * SMX_META_DIRTY marks k_upsert leaves) are appended, behind them a new directory chain that lists the clean rows'
+ * old entries (their blocks in the file are still right) and the dirty rows' new ones, and then the header is
+ * switched to that chain.  The reference's own writer leaves dead blocks behind and chains directory blocks at the
+ * end of its file in the same way, so every reader of the format follows the header's pointer.  Order of the
+ * steps, so that the file loads to the old or the new state at every moment: blocks at E = round_up(size, 8),
+ * directory at D behind them (full 2^22-entry blocks, the unused entries left to ftruncate: sparse), fsync, the 8
+ * header bytes at offset 8 := D, fsync.  Nothing before E but those 8 bytes is written. */
+void smatrix_b200_clear_dirty(smatrix_t* s) {
+  enter(s);
+  CK(cudaStreamSynchronize(s->stream));
+  clear_dirty(s);
+  leave(s);
+}
+
+int smatrix_b200_ckpt_extent(smatrix_t* s, uint64_t* rows, uint64_t* bytes) {
+  enter(s);
+  CK(cudaStreamSynchronize(s->stream));
+  snap_extent(s, rows, bytes, SMX_META_USED | SMX_META_DIRTY);
+  leave(s);
+  return 0;
+}
+
+static uint64_t count_dirty(smatrix_t* s) { /* caller holds the handle lock */
+  read_ctl(s);
+  if (!s->h_ctl->dir_used) return 0;
+  CK(cudaMemsetAsync(&s->d_ctl->scratch, 0, 8, s->stream));
+  smx_launch_list_rows(s->stream, view_of(s), 0, SMX_META_USED | SMX_META_DIRTY, NULL, (uint32_t*)&s->d_ctl->scratch);
+  s->n_launches++;
+  copy_d2h(s, &s->h_small->listed, &s->d_ctl->scratch, 4, s->stream);
+  CK(cudaStreamSynchronize(s->stream));
+  CK(cudaGetLastError());
+  return s->h_small->listed;
+}
+
+uint64_t smatrix_b200_ckpt_keep(smatrix_t* s, const uint32_t* d_keys, const uint32_t* d_lo, const uint32_t* d_hi,
+                                size_t n, uint64_t* kept) {
+  uint64_t missing = 0;
+  enter(s);
+  for (size_t first = 0; first < n;) {
+    const uint32_t len = (uint32_t)(n - first < SMX_SNAPSHOT_ROWS ? n - first : SMX_SNAPSHOT_ROWS);
+    uint32_t* flags = dbuf_need(s, &s->db.ck_flags, (size_t)len * 4 + 8);
+    uint64_t* off = dbuf_need(s, &s->db.ck_off, ((size_t)len + 2 + smx_scan_scratch_items(len)) * 8);
+    uint32_t* out = dbuf_need(s, &s->db.ck_out, (size_t)len * SMX_F_DIR_SLOT);
+    uint32_t* d_missing = flags + len;
+    CK(cudaMemsetAsync(d_missing, 0, 4, s->stream));
+    smx_launch_keep(s->stream, view_of(s), d_keys + first, d_lo + first, d_hi + first, len, flags, off,
+                    off + (size_t)len + 1, d_missing, out);
+    s->n_launches += 5;
+    copy_d2h(s, &s->h_small->ck_missing, d_missing, 4, s->stream);
+    copy_d2h(s, &s->h_small->ck_kept, off + len, 8, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    const uint64_t k = s->h_small->ck_kept;
+    missing += s->h_small->ck_missing;
+    if (s->ck_kept_n + k > s->ck_kept_cap) {
+      s->ck_kept_cap = (s->ck_kept_n + k) * 2 + 1024;
+      s->ck_kept = (unsigned char*)realloc(s->ck_kept, (size_t)s->ck_kept_cap * SMX_F_DIR_SLOT);
+      if (!s->ck_kept) smx_die("out of host memory");
+    }
+    copy_d2h(s, s->ck_kept + s->ck_kept_n * SMX_F_DIR_SLOT, out, (size_t)k * SMX_F_DIR_SLOT, s->stream);
+    CK(cudaStreamSynchronize(s->stream));
+    s->ck_kept_n += k;
+    first += len;
+  }
+  CK(cudaGetLastError());
+  *kept = s->ck_kept_n;
+  leave(s);
+  return missing;
+}
+
+int smatrix_b200_ckpt_write_kept(smatrix_t* s, int fd, uint64_t dir_base, uint64_t first_entry) {
+  enter(s);
+  const int rc = snap_write_entries(fd, s->ck_kept, dir_base, first_entry, s->ck_kept_n);
+  s->ck_kept_n = 0;
+  leave(s);
+  return rc;
+}
+
+void smatrix_b200_ckpt_reset(smatrix_t* s) {
+  enter(s);
+  s->ck_kept_n = 0;
+  snap_free_keys(s);
+  leave(s);
+}
+
+int smatrix_b200_ckpt_layout(int fd, uint64_t dir_base, uint64_t entries) {
+  const uint64_t n_blocks = entries ? (entries + SMX_F_DIR_ENTRIES - 1) / SMX_F_DIR_ENTRIES : 1;
+  /* the file first reaches its final size: the unused entries read back as zeros */
+  if (ftruncate(fd, (off_t)(dir_base + n_blocks * SMX_F_BLOCK_BYTES)) == -1) return -1;
+  for (uint64_t b = 0; b < n_blocks; b++) {
+    const uint64_t bpos = dir_base + b * SMX_F_BLOCK_BYTES;
+    unsigned char bh[SMX_F_DIR_HEAD];
+    const uint64_t cnt = SMX_F_DIR_ENTRIES, next = (b + 1 < n_blocks) ? bpos + SMX_F_BLOCK_BYTES : 0;
+    memcpy(bh, &cnt, 8);
+    memcpy(bh + 8, &next, 8);
+    if (write_all(fd, bh, sizeof bh, bpos)) return -1;
+  }
+  return 0;
+}
+
+int smatrix_b200_ckpt_switch(int fd, uint64_t dir_base) {
+  if (fsync(fd) == -1) return -1; /* blocks and directory are on disk before the header points at them */
+  if (write_all(fd, &dir_base, 8, 8)) return -1;
+  return fsync(fd) == -1 ? -1 : 0;
+}
+
+/* caller holds the handle lock, the stream is idle */
+static int checkpoint(smatrix_t* s) {
+  const uint64_t dirty = count_dirty(s);
+  if (!dirty) return 0;
+  if (!s->ck_base) return snapshot_save(s); /* the file never matched the table */
+  const int fd = open(s->fname, O_RDWR);
+  if (fd == -1) {
+    if (errno == ENOENT) return snapshot_save(s);
+    perror("libsmatrix: cannot open the file for a checkpoint");
+    return -1;
+  }
+  struct stat st;
+  if (fstat(fd, &st) != 0) { perror("libsmatrix: checkpoint"); close(fd); return -1; }
+  if (st.st_size == 0) { close(fd); return snapshot_save(s); }
+  const uint64_t fsize = (uint64_t)st.st_size;
+  uint64_t rows = 0, all_bytes = 0, drows = 0, dbytes = 0, kept = 0, missing = 0;
+  snap_extent(s, &rows, &all_bytes, SMX_META_USED); /* the size of a full snapshot */
+  snap_free_keys(s);
+  leave(s); /* the pieces below take the lock themselves */
+  s->ck_kept_n = 0;
+  smx_loader_t* ld = smatrix_b200_load_begin(s, fd, 0, 1);
+  int match = ld != NULL;
+  if (ld) {
+    const uint64_t n = smatrix_b200_load_entries(ld, 0, 0, NULL, NULL, NULL);
+    enter(s);
+    uint32_t* d_in = dbuf_need(s, &s->db.ck_in, (size_t)(n < SMX_SNAPSHOT_ROWS ? n : SMX_SNAPSHOT_ROWS) * 12 + 16);
+    leave(s);
+    const uint64_t piece = SMX_SNAPSHOT_ROWS;
+    for (uint64_t first = 0; first < n; first += piece) {
+      const uint64_t len = n - first < piece ? n - first : piece;
+      smatrix_b200_load_entries(ld, first, len, d_in, d_in + len, d_in + 2 * len);
+      missing += smatrix_b200_ckpt_keep(s, d_in, d_in + len, d_in + 2 * len, (size_t)len, &kept);
+    }
+    smatrix_b200_load_end(ld);
+  }
+  enter(s);
+  snap_extent(s, &drows, &dbytes, SMX_META_USED | SMX_META_DIRTY); /* held until snap_write */
+  /* the old directory lists exactly the table's rows: every listed row is in the table, and the clean ones and the
+   * dirty ones add up to all of them (a dirty row may be new, so it need not be listed) */
+  match = match && missing == 0 && kept + drows == rows;
+  const uint64_t E = (fsize + 7) & ~7ull, D = E + dbytes;
+  const uint64_t end = D + smatrix_b200_snap_rows_base(kept + drows) - SMX_F_META;
+  if (!match || end > 2 * (smatrix_b200_snap_rows_base(rows) + all_bytes)) {
+    /* a file that does not describe this table, or one that has grown to twice a full snapshot: rewrite it */
+    close(fd);
+    s->ck_kept_n = 0;
+    snap_free_keys(s);
+    return snapshot_save(s);
+  }
+  int rc = smatrix_b200_ckpt_layout(fd, D, kept + drows);
+  if (rc == 0 && snap_write(s, fd, E, D, kept)) rc = -1;
+  snap_free_keys(s);
+  if (rc == 0 && snap_write_entries(fd, s->ck_kept, D, 0, kept)) rc = -1;
+  s->ck_kept_n = 0;
+  if (rc) {
+    (void)!ftruncate(fd, (off_t)fsize); /* the header was not switched: the old file as it was */
+  } else if (smatrix_b200_ckpt_switch(fd, D)) {
+    rc = -1;
+  }
+  if (close(fd) == -1) rc = -1;
+  if (rc) {
+    perror("libsmatrix: writing the checkpoint failed");
+    return -1;
+  }
+  clear_dirty(s);
+  return 0;
+}
+
+int smatrix_b200_checkpoint(smatrix_t* s) {
+  if (!s->fname) return -1;
+  enter(s);
+  CK(cudaStreamSynchronize(s->stream));
+  const int rc = checkpoint(s);
+  leave(s);
   return rc;
 }
 
@@ -2284,7 +2533,7 @@ smatrix_t* smatrix_b200_open_arena(const char* fname, int device, size_t arena_b
     s->fname = strdup(fname);
     struct stat st;
     int bad = 0;
-    if (fstat(fd, &st) == 0 && st.st_size > 0) bad = snapshot_load(s, fd);
+    if (fstat(fd, &st) == 0 && st.st_size > 0) bad = snapshot_load(s, fd); /* a file that loads is the base of checkpoints */
     close(fd);
     if (bad) {
       free(s->fname);
@@ -2314,6 +2563,7 @@ void smatrix_close(smatrix_t* s) {
   free(s->segs);
   if (!s->dir_in_arena) cudaFree(s->dir);
   snap_free_keys(s);
+  free(s->ck_kept);
   cudaFree(s->d_ctl);
   cudaFreeHost(s->h_ctl);
   cudaFree(s->d_small);
@@ -2443,6 +2693,7 @@ uint64_t smatrix_b200_stat(smatrix_t* s, int which) {
     case SMX_STAT_TOPK_PASSES: r = s->n_topk_passes; break;
     case SMX_STAT_REC_BIG: r = s->n_rec_big; break;
     case SMX_STAT_SORT_BIG: r = s->n_sort_big; break;
+    case SMX_STAT_DIRTY_ROWS: r = count_dirty(s); break;
     case SMX_STAT_H2D_BYTES: r = s->h2d_bytes; break;
     case SMX_STAT_D2H_BYTES: r = s->d2h_bytes; break;
     case SMX_STAT_DIR_CAP: r = s->dir_cap; break;

@@ -36,6 +36,7 @@ extern "C" {
 #define SMX_META_SLOG   (0x1Fu << SMX_META_SLOG_SHIFT)
 #define SMX_META_T0P    0x800u  /* column 0 turns non-zero inside the current batch at t0     */
 #define SMX_META_GROW   0x1000u /* row is queued for growth in the current round              */
+#define SMX_META_DIRTY  0x2000u /* row was written since the file last matched the table (checkpoints) */
 #define SMX_INLINE_LOG  2u
 #define SMX_MIN_SLAB_LOG 4u     /* first slab bucket: 16 cells = 128 B (src/smatrix.h:21)     */
 #define SMX_MAX_CAPLOG  31u
@@ -246,9 +247,18 @@ void smx_launch_sort_cut(smx_stream_t stream, const uint64_t* big_off, uint32_t 
 void smx_launch_sort_big(smx_stream_t stream, const uint32_t* big_list, uint32_t lo, uint32_t n_grp, uint32_t P,
                          const uint64_t* big_off, const uint64_t* offsets, uint32_t* pairs, uint64_t* keys_a,
                          uint64_t* keys_b, uint32_t* vals_a, uint32_t* vals_b, void* sort_tmp, size_t sort_bytes);
-/* the row ids >= from (a snapshot: from = 0), in directory order; then an ascending radix sort of n u32 keys */
-void smx_launch_list_rows(smx_stream_t stream, smx_view_t v, uint32_t from, uint32_t* keys,
+/* the row ids >= from whose meta has every flag of `need` (SMX_META_USED: every row; | SMX_META_DIRTY: the rows
+ * written since the last checkpoint), in directory order (keys = NULL: count only); then an ascending radix sort of
+ * n u32 keys */
+void smx_launch_list_rows(smx_stream_t stream, smx_view_t v, uint32_t from, uint32_t need, uint32_t* keys,
                           uint32_t* counter /* zeroed */);
+void smx_launch_clear_dirty(smx_stream_t stream, smx_view_t v);
+/* the keep filter of a checkpoint over n old directory entries (keys, row offsets as lo / hi words): *missing +=
+ * entries whose row is not in the table; the entries of clean rows go to out as packed 12-byte entries in their
+ * order, offsets[n] = their number.  flags: n words; offsets: n + 1; tile_sums: smx_scan_scratch_items(n) */
+void smx_launch_keep(smx_stream_t stream, smx_view_t v, const uint32_t* keys, const uint32_t* lo, const uint32_t* hi,
+                     uint32_t n, uint32_t* flags, uint64_t* offsets, uint64_t* tile_sums, uint32_t* missing,
+                     uint32_t* out);
 size_t smx_sort_keys_bytes(uint32_t n);
 void smx_launch_sort_keys(smx_stream_t stream, const uint32_t* in, uint32_t* out, uint32_t n, void* sort_tmp,
                           size_t sort_bytes);

@@ -342,6 +342,8 @@ __device__ __forceinline__ int upsert_one(const smx_view_t& V, const smx_lists_t
   Hdr h;
   int r = dir_find(V, x, true, &e, &h);
   if (r == DIR_FULL) return ST_DIRFULL; /* counted per block by the caller */
+  /* the row is written: the next checkpoint appends it (one atomic per row per checkpoint interval) */
+  if (!(h.meta & SMX_META_DIRTY)) atomicOr(&e->meta, SMX_META_DIRTY);
   if (pass == SMX_PASS_COL0) {
     apply_value<OP>(&e->c0, v);
     /* column 0 of this row turns non-zero inside this batch: remember the first such op
@@ -1927,13 +1929,53 @@ k_sort_big_scatter(const ull* keys, const uint32_t* vals, uint32_t P, const uint
 }
 
 /* ---- snapshot support (file mode, reference src/smatrix.c:30-72) --------------------------- */
-/* the row ids >= from of the directory, in no particular order (a snapshot lists them all: from = 0) */
+/* the row ids >= from of the directory whose flags include all of `need`, in no particular order (a snapshot
+ * lists every row: from = 0, need = USED; a checkpoint the written ones: need = USED | DIRTY).  keys = NULL:
+ * only count them */
 __global__ void __launch_bounds__(SMX_BLOCK)
-k_list_rows(smx_view_t V, uint32_t from, uint32_t* keys, uint32_t* counter) {
+k_list_rows(smx_view_t V, uint32_t from, uint32_t need, uint32_t* keys, uint32_t* counter) {
   for (ull pos = blockIdx.x * blockDim.x + threadIdx.x; pos < V.dir_cap;
        pos += (ull)gridDim.x * blockDim.x) {
     Hdr h = ld_hdr(V.dir + pos);
-    if ((h.meta & SMX_META_USED) && h.key >= from) keys[agg_inc(counter)] = h.key;
+    if ((h.meta & need) == need && h.key >= from) {
+      const uint32_t at = agg_inc(counter);
+      if (keys) keys[at] = h.key;
+    }
+  }
+}
+/* the file matches the table again: no row is written since */
+__global__ void __launch_bounds__(SMX_BLOCK) k_clear_dirty(smx_view_t V) {
+  for (ull pos = blockIdx.x * blockDim.x + threadIdx.x; pos < V.dir_cap;
+       pos += (ull)gridDim.x * blockDim.x) {
+    smx_row_t* e = V.dir + pos;
+    if (__ldcg(&e->meta) & SMX_META_DIRTY) atomicAnd(&e->meta, ~SMX_META_DIRTY);
+  }
+}
+/* ---- the keep filter of a checkpoint: the old directory's entries (key, row offset as lo / hi words) against
+ * the table.  k_keep_flags: flags[i] = 1 for an entry whose row is in the table and clean (its block in the file
+ * is still right); an entry whose row is not in the table at all is counted in *missing (the file does not
+ * describe this table).  smx_launch_scan turns the flags into positions; k_keep_emit writes the kept entries as
+ * packed 12-byte .smx directory entries, in their old order. */
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_keep_flags(smx_view_t V, const uint32_t* keys, uint32_t n, uint32_t* flags, uint32_t* missing) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    smx_row_t* e;
+    Hdr h;
+    uint32_t keep = 0u;
+    if (dir_find(V, keys[i], false, &e, &h) != DIR_FOUND) atomicAdd(missing, 1u);
+    else keep = (h.meta & SMX_META_DIRTY) ? 0u : 1u;
+    flags[i] = keep;
+  }
+}
+__global__ void __launch_bounds__(SMX_BLOCK)
+k_keep_emit(const uint32_t* keys, const uint32_t* lo, const uint32_t* hi, uint32_t n, const uint32_t* flags,
+            const ull* offsets, uint32_t* out) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    if (!flags[i]) continue;
+    uint32_t* de = out + 3ull * offsets[i]; /* {u32 row, u64 row offset}, 4-byte aligned */
+    de[0] = keys[i];
+    de[1] = lo[i];
+    de[2] = hi[i];
   }
 }
 /* log2 of the reference's row size as of now (the caught-up automaton state), per row */
@@ -2858,9 +2900,20 @@ extern "C" void smx_launch_getrow_fill(smx_stream_t st, smx_view_t v, const uint
   }
 }
 
-extern "C" void smx_launch_list_rows(smx_stream_t st, smx_view_t v, uint32_t from, uint32_t* keys,
+extern "C" void smx_launch_list_rows(smx_stream_t st, smx_view_t v, uint32_t from, uint32_t need, uint32_t* keys,
                                      uint32_t* counter) {
-  SMX_LAUNCH(k_list_rows, grid_for(v.dir_cap), SMX_BLOCK, st, v, from, keys, counter);
+  SMX_LAUNCH(k_list_rows, grid_for(v.dir_cap), SMX_BLOCK, st, v, from, need, keys, counter);
+}
+extern "C" void smx_launch_clear_dirty(smx_stream_t st, smx_view_t v) {
+  SMX_LAUNCH(k_clear_dirty, grid_for(v.dir_cap), SMX_BLOCK, st, v);
+}
+extern "C" void smx_launch_keep(smx_stream_t st, smx_view_t v, const uint32_t* keys, const uint32_t* lo,
+                                const uint32_t* hi, uint32_t n, uint32_t* flags, uint64_t* offsets, uint64_t* tile_sums,
+                                uint32_t* missing, uint32_t* out) {
+  if (!n) return;
+  SMX_LAUNCH(k_keep_flags, grid_for(n), SMX_BLOCK, st, v, keys, n, flags, missing);
+  smx_launch_scan(st, flags, n, 0, offsets, tile_sums);
+  SMX_LAUNCH(k_keep_emit, grid_for(n), SMX_BLOCK, st, keys, lo, hi, n, flags, (const ull*)offsets, out);
 }
 extern "C" void smx_launch_row_slog(smx_stream_t st, smx_view_t v, const uint32_t* xs, uint32_t n,
                                     uint32_t* out) {

@@ -86,6 +86,7 @@ struct smatrix_shard_s {
   uint32_t taper_min; /* 0 = off; else the last staged piece is cut into 1/2, 1/4, 1/4 if a quarter has this many ops */
   uint64_t stat[8]; /* SMX_SHARD_STAT_* */
   char* fname;        /* file mode: the .smx file every rank loaded from and writes back to */
+  int ck_base;        /* the file matched the table at some point (a load, a snapshot or a checkpoint) */
 };
 
 /* inbox layout for capacity `cap` ops (cap is a multiple of 256): shared arrays first, then the
@@ -1088,10 +1089,118 @@ static int rt_snapshot(smatrix_shard_t* sh) {
     }
   }
   free(tmp);
-  return rt_all_ok(sh, ok) ? 0 : -1;
+  if (!rt_all_ok(sh, ok)) return -1;
+  smatrix_b200_clear_dirty(sh->local); /* the file matches the table */
+  sh->ck_base = 1;
+  return 0;
 }
 
 int smatrix_b200_shard_snapshot(smatrix_shard_t* sh) { return rt_snapshot(sh); }
+
+/* Collective: the checkpoint of smatrix_b200_checkpoint for the whole sharded matrix.  Every decision is taken from
+ * all-gathered values, so every rank takes the same branch: no file -> -1; nothing written -> 0; no base (the file
+ * was or is missing or empty) -> the full snapshot.  Then every rank reads an even share of the old directory and
+ * routes its (key, row offset lo, hi) entries to the rows' owners in pieces, and each owner runs the keep filter on
+ * its inbox.  A listed row missing anywhere, Σ (kept + dirty) != Σ rows, or an appended file past twice a full
+ * snapshot -> the full snapshot.  Otherwise exclusive prefixes give every rank the byte where its dirty rows' blocks
+ * go behind E and its first entry in the new chain at D (its kept entries, then its dirty rows'); rank 0 extends the
+ * file and writes the block headers, every rank writes its part and fsyncs, rank 0 switches the header and fsyncs,
+ * and every rank clears its marks.  Each step's outcome is agreed on: 0 or -1 on every rank. */
+static int rt_checkpoint(smatrix_shard_t* sh) {
+  const int W = sh->world, me = sh->rank;
+  uint64_t dirty = sh->fname ? smatrix_b200_stat(sh->local, SMX_STAT_DIRTY_ROWS) : 0;
+  uint64_t fstate = 0; /* rank 0: 0 = the file is missing, 1 = it cannot be read, else its size + 2 */
+  if (me == 0 && sh->fname) {
+    struct stat st;
+    if (stat(sh->fname, &st) == 0) fstate = S_ISREG(st.st_mode) ? (uint64_t)st.st_size + 2 : 1;
+    else fstate = errno == ENOENT ? 0 : 1;
+  }
+  uint64_t mine[4] = {sh->fname != NULL, dirty, fstate, 0}, all[RT_MAXW][4];
+  rt_allgather(sh, mine, all);
+  uint64_t total_dirty = 0;
+  int have = 1;
+  for (int r = 0; r < W; r++) { have = have && all[r][0]; total_dirty += all[r][1]; }
+  if (!have) return -1;
+  if (!total_dirty) return 0;
+  fstate = all[0][2];
+  if (fstate == 1) {
+    if (me == 0) fprintf(stderr, "libsmatrix: cannot open %s for a checkpoint\n", sh->fname);
+    return -1;
+  }
+  if (!sh->ck_base || fstate <= 2) return rt_snapshot(sh); /* the file never matched the table, or is gone */
+  const uint64_t fsize = fstate - 2;
+  uint64_t rows = 0, bytes = 0, drows = 0, dbytes = 0;
+  smatrix_b200_snap_extent(sh->local, &rows, &bytes);
+  const int fd = open(sh->fname, O_RDWR);
+  smx_loader_t* ld = fd == -1 ? NULL : smatrix_b200_load_begin(sh->local, fd, me, W);
+  const uint64_t n = ld ? smatrix_b200_load_entries(ld, 0, 0, NULL, NULL, NULL) : 0;
+  const uint64_t piece = sh->piece, pieces = (n + piece - 1) / piece;
+  uint64_t m1[4] = {ld != NULL, pieces, 0, 0};
+  rt_allgather(sh, m1, all);
+  int ok = 1;
+  uint64_t max_pieces = 0;
+  for (int r = 0; r < W; r++) { ok = ok && all[r][0]; if (all[r][1] > max_pieces) max_pieces = all[r][1]; }
+  uint64_t missing = 0, kept = 0;
+  if (ok) {
+    rt_need_stage(sh, (size_t)(n < piece ? n : piece) + 1);
+    for (uint64_t k = 0; k < max_pieces; k++) { /* the same number of routes on every rank */
+      const uint64_t lo = k * piece < n ? k * piece : n, len = (n - lo < piece) ? n - lo : piece;
+      if (len) smatrix_b200_load_entries(ld, lo, len, sh->stage[0][0], sh->stage[0][1], sh->stage[0][2]);
+      rt_route_t R;
+      rt_route(sh, sh->stage[0][0], sh->stage[0][1], sh->stage[0][2], (size_t)len, 0, 0, &R);
+      const uint64_t cap = sh->cap;
+      missing += smatrix_b200_ckpt_keep(sh->local, (const uint32_t*)(sh->inbox + OFF_X(cap)),
+                                        (const uint32_t*)(sh->inbox + OFF_Y(cap)),
+                                        (const uint32_t*)(sh->inbox + OFF_V(cap)), (size_t)R.n_recv, &kept);
+      rt_barrier(sh); /* the inboxes are read before the next route fills them */
+    }
+  }
+  smatrix_b200_load_end(ld);
+  /* held until snap_write_at; laid out only now, because the routes above reuse the scratch that holds it */
+  smatrix_b200_ckpt_extent(sh->local, &drows, &dbytes);
+  uint64_t m2[4] = {(uint64_t)ok, missing, kept, 0}, m3[4] = {rows, bytes, drows, dbytes}, all3[RT_MAXW][4];
+  rt_allgather(sh, m2, all);
+  rt_allgather(sh, m3, all3);
+  uint64_t t_rows = 0, t_bytes = 0, t_drows = 0, t_dbytes = 0, t_missing = 0, t_kept = 0, byte_off = 0, first = 0;
+  for (int r = 0; r < W; r++) {
+    ok = ok && all[r][0];
+    if (r == me) { byte_off = t_dbytes; first = t_kept + t_drows; }
+    t_missing += all[r][1]; t_kept += all[r][2];
+    t_rows += all3[r][0]; t_bytes += all3[r][1]; t_drows += all3[r][2]; t_dbytes += all3[r][3];
+  }
+  const uint64_t E = (fsize + 7) & ~7ull, D = E + t_dbytes;
+  const uint64_t end = D + smatrix_b200_snap_rows_base(t_kept + t_drows) - 512; /* the chain without the header */
+  const int match = ok && t_missing == 0 && t_kept + t_drows == t_rows;
+  if (!match || end > 2 * (smatrix_b200_snap_rows_base(t_rows) + t_bytes)) {
+    /* a file that does not describe this table, or one that has grown to twice a full snapshot: rewrite it */
+    if (fd != -1) close(fd);
+    smatrix_b200_ckpt_reset(sh->local);
+    return rt_snapshot(sh);
+  }
+  ok = me != 0 || smatrix_b200_ckpt_layout(fd, D, t_kept + t_drows) == 0;
+  if (rt_all_ok(sh, ok)) { /* the file has its final size */
+    ok = smatrix_b200_snap_write_at(sh->local, fd, E + byte_off, D, first + kept) == 0;
+    ok = smatrix_b200_ckpt_write_kept(sh->local, fd, D, first) == 0 && ok;
+    ok = ok && fsync(fd) == 0;
+  } else {
+    ok = 0;
+  }
+  smatrix_b200_ckpt_reset(sh->local);
+  ok = rt_all_ok(sh, ok);
+  if (me == 0) {
+    if (!ok) (void)!ftruncate(fd, (off_t)fsize); /* the header was not switched: the old file as it was */
+    else if (smatrix_b200_ckpt_switch(fd, D) != 0) ok = 0;
+  }
+  if (close(fd) == -1) ok = 0;
+  if (!rt_all_ok(sh, ok)) {
+    if (me == 0) perror("libsmatrix: writing the checkpoint failed");
+    return -1;
+  }
+  smatrix_b200_clear_dirty(sh->local);
+  return 0;
+}
+
+int smatrix_b200_shard_checkpoint(smatrix_shard_t* sh) { return rt_checkpoint(sh); }
 
 static uint64_t rt_fnv(const char* p) {
   uint64_t h = 0xcbf29ce484222325ull;
@@ -1151,6 +1260,10 @@ smatrix_shard_t* smatrix_b200_shard_open_file(const char* name, int rank, int wo
   }
   if (ok && all[0][2] && rt_load(sh, fd) != 0) ok = 0;
   if (fd != -1) close(fd);
+  if (ok) { /* the loaded rows are what the file holds */
+    smatrix_b200_clear_dirty(sh->local);
+    sh->ck_base = all[0][2] != 0;
+  }
   if (!ok) { /* every rank takes this branch together; a file we could not read is not overwritten */
     smatrix_b200_shard_close(sh);
     return NULL;

@@ -226,6 +226,18 @@ class SparseMatrix:
     def getFilename(self):
         return self.filename
 
+    # ---- file mode ---------------------------------------------------------------------------
+    def snapshot(self) -> int:
+        """Write the whole .smx file now (temporary file, fsync, rename): 0, or -1 on failure or without a file."""
+        return int(self._lib.smatrix_b200_snapshot(self._handle()))
+
+    def checkpoint(self) -> int:
+        """Persist only what changed: append the blocks of the rows written since the file last matched the table,
+        a new directory, then switch the header to it (smatrix_b200_checkpoint).  The file loads to what a snapshot
+        taken now would load to.  0, or -1 on failure or without a file; stat("dirty_rows") counts the rows the
+        next checkpoint writes."""
+        return int(self._lib.smatrix_b200_checkpoint(self._handle()))
+
     # ---- the reference API -----------------------------------------------------------------
     def get(self, x: int, y: int) -> int:
         return self._lib.smatrix_get(self._handle(), x & 0xFFFFFFFF, y & 0xFFFFFFFF)

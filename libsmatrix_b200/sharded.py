@@ -226,6 +226,11 @@ class ShardedSparseMatrix:
         """Collective: write the .smx file now (smatrix_b200_shard_snapshot); 0, or -1 on every rank."""
         return int(self._lib.smatrix_b200_shard_snapshot(self._handle()))
 
+    def checkpoint(self) -> int:
+        """Collective: append the rows written since the file last matched the table and switch its header to a
+        new directory (smatrix_b200_shard_checkpoint); 0, or -1 on every rank."""
+        return int(self._lib.smatrix_b200_shard_checkpoint(self._handle()))
+
     def barrier(self):
         self._lib.smatrix_b200_shard_barrier(self._handle())
 
